@@ -48,6 +48,38 @@ def load_golden(name: str):
     return c, scene, inp, z
 
 
+class ReferenceGolden:
+    """tests/golden/reference/oracle_vs_reference.npz (tests/golden/make_reference_golden.py): what the tests that compare
+    with the unmodified reference compare against where it is not installed."""
+
+    def __init__(self, path: str) -> None:
+        self.z = np.load(path, allow_pickle=False)
+
+    def check(self, key: str, got, rtol: float = 0.0, atol: float = 0.0) -> None:
+        """Row count, the stored sample of rows and the column sums of ``got`` against the record ``key``; floats within
+        rtol / atol per element (LAPACK / BLAS may differ in the last bits between CPUs), everything else exactly."""
+        from tests.golden.make_reference_golden import column_stats, sample_rows
+        got = np.asarray(got)
+        stats = self.z[f"{key}.stats"]
+        n = int(stats[0])
+        assert got.shape[0] == n, (key, got.shape, n)
+        rows, want = got[sample_rows(n)], self.z[f"{key}.rows"]
+        assert rows.dtype == want.dtype and rows.shape == want.shape, (key, rows.dtype, rows.shape, want.dtype, want.shape)
+        if want.dtype.kind != "f":
+            assert np.array_equal(rows, want), key
+            return
+        np.testing.assert_allclose(rows, want, rtol=rtol, atol=atol, equal_nan=True, err_msg=key)
+        mine = column_stats(got)
+        c = (len(stats) - 1) // 2
+        s, w = mine[1:1 + c], stats[1:1 + c]
+        tol = n * atol + rtol * stats[1 + c:]
+        assert np.array_equal(np.isnan(s), np.isnan(w)) and np.all(np.nan_to_num(np.abs(s - w)) <= tol), (key, s, w)
+
+
+def load_reference_golden() -> ReferenceGolden:
+    return ReferenceGolden(os.path.join(GOLDEN_DIR, "reference", "oracle_vs_reference.npz"))
+
+
 def oracle_cam(c) -> O.OracleCamera:
     return O.OracleCamera(c.uid, c.width, c.height, c.K, c.R, c.t, c.P, c.C)
 

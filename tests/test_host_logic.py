@@ -1,5 +1,7 @@
 """CPU: host-side mirrors of the reference's configuration and seeds (no device work)."""
 import dataclasses
+import json
+import types
 
 import numpy as np
 import pytest
@@ -8,18 +10,28 @@ from lichtfeld_densification_plugin_b200.core.config import DensePipelineConfig,
 from oracle import ref_import
 
 
+def reference_config_fields():
+    """(name, default or None) of the reference's DensePipelineConfig: live where the reference is installed, otherwise
+    the stored record (tests/golden/make_reference_golden.py)."""
+    if ref_import.reference_available():
+        ref = ref_import.import_reference(full_pipeline=False)
+        return [(f.name, None if f.default is dataclasses.MISSING else f.default)
+                for f in dataclasses.fields(ref.config.DensePipelineConfig)]
+    from tests.helpers import load_reference_golden
+    return [tuple(f) for f in json.loads(str(load_reference_golden().z["config/fields"]))]
+
+
 def test_config_is_a_field_for_field_superset_of_the_reference():
-    if not ref_import.reference_available():
-        pytest.skip("reference tree not present (GPU box)")
-    ref = ref_import.import_reference(full_pipeline=False)
-    ref_fields = dataclasses.fields(ref.config.DensePipelineConfig)
+    ref_fields = reference_config_fields()
     ours = {f.name: f for f in dataclasses.fields(DensePipelineConfig)}
     names = [f.name for f in dataclasses.fields(DensePipelineConfig)]
-    assert names[:len(ref_fields)] == [f.name for f in ref_fields]                 # same names, same order
-    for f in ref_fields:
-        if f.default is not dataclasses.MISSING:
-            assert ours[f.name].default == f.default, f.name                       # same defaults
-    cfg = DensePipelineConfig.from_reference(ref.config.DensePipelineConfig(output_path="/tmp/a.ply", matches_per_ref=123, no_filter=True))
+    assert names[:len(ref_fields)] == [name for name, _ in ref_fields]             # same names, same order
+    for name, default in ref_fields:
+        if default is not None:
+            assert ours[name].default == default, name                             # same defaults
+    ref_cfg = types.SimpleNamespace(**{name: default for name, default in ref_fields})
+    ref_cfg.output_path, ref_cfg.matches_per_ref, ref_cfg.no_filter = "a.ply", 123, True
+    cfg = DensePipelineConfig.from_reference(ref_cfg)
     assert cfg.matches_per_ref == 123 and cfg.no_filter and cfg.rng_mode == "philox"
     with pytest.raises(ValueError):
         DensePipelineConfig(output_path="x", rng_mode="nope").validate()
@@ -46,16 +58,18 @@ def test_preview_seed_formula():
 
 
 def test_estimate_total_pairs_matches_reference():
-    if not ref_import.reference_available():
-        pytest.skip("reference tree not present (GPU box)")
-    ref = ref_import.import_reference(full_pipeline=True)
     from lichtfeld_densification_plugin_b200.core.selection import _estimate_total_pairs
     rs = np.random.RandomState(1)
     nn = rs.randint(0, 20, size=(20, 5))
     ids = [int(v) for v in rs.randint(0, 12, size=20)]                                # duplicate image ids: self-pairs are skipped
     refs = [0, 3, 7, 19]
-    for k in (1, 3, 5):
-        assert _estimate_total_pairs(refs, nn, ids, k) == ref.pipeline._estimate_total_pairs(refs, nn, ids, k)
+    if ref_import.reference_available():
+        ref = ref_import.import_reference(full_pipeline=True)
+        want = [ref.pipeline._estimate_total_pairs(refs, nn, ids, k) for k in (1, 3, 5)]
+    else:
+        from tests.helpers import load_reference_golden
+        want = [int(v) for v in load_reference_golden().z["pairs/estimate"]]
+    assert [_estimate_total_pairs(refs, nn, ids, k) for k in (1, 3, 5)] == want
 
 
 def test_packed_cloud_layout_is_one_allocation():

@@ -58,11 +58,8 @@ def test_explicit_index_arithmetic_equals_aten(shape):
         assert np.array_equal(e, t, equal_nan=True)
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="/root/reference not present")
-def test_prologue_vs_live_collect_reference_matches():
-    """Build container only: fresh inputs through the unmodified ``_collect_reference_matches`` with a stub matcher."""
-    ref = ref_import.import_reference(full_pipeline=True)
-    P = ref.pipeline
+def collect_case():
+    """Raw certainty, warp and masks of three neighbours (80^2 maps, 50^2 masks, the second neighbour without a mask)."""
     rs = np.random.RandomState(77)
     H = W = 80
     hm = wm = 50
@@ -71,6 +68,22 @@ def test_prologue_vs_live_collect_reference_matches():
     warp = rs.rand(nn, H, W, 4).astype(np.float32) * 2.2 - 1.1
     mA = (rs.rand(hm, wm) > 0.2).astype(np.uint8)
     mBs = [(rs.rand(hm, wm) > 0.4).astype(np.uint8), None, (rs.rand(hm, wm) > 0.1).astype(np.uint8)]
+    return raw, warp, mA, mBs
+
+
+def test_prologue_vs_live_collect_reference_matches():
+    """Fresh inputs through the unmodified ``_collect_reference_matches`` with a stub matcher where the reference is
+    installed; elsewhere against its stored output (tests/golden/make_reference_golden.py)."""
+    raw, warp, mA, mBs = collect_case()
+    nn, (hm, wm) = raw.shape[0], mA.shape
+    if not ref_import.reference_available():
+        from tests.helpers import load_reference_golden
+        stored = load_reference_golden()
+        for k in range(nn):
+            stored.check(f"collect/cert/{k}", O.certainty_prologue(raw[k], warp[k], mA, mBs[k], 0.35).ravel())
+        return
+    ref = ref_import.import_reference(full_pipeline=True)
+    P = ref.pipeline
 
     class Stub:
         def match_grids_batch(self, imA, nn_images):
