@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define LDP_ABI_VERSION 12
+#define LDP_ABI_VERSION 13
 #define LDP_MAX_NN 16          /* neighbours per reference view (the panel clamps to 10) */
 #define LDP_MAX_BINS 4096      /* coverage tiles per map: ceil(W/tile)*ceil(H/tile), tile = max(1, W/24) */
 
@@ -88,8 +88,33 @@ typedef struct ldp_params {
     int32_t sm_reserve;        /* SMs the one-CTA-per-SM first draw kernel leaves to kernels of OTHER launches in flight on other
                                   streams (engine.DensifyRing passes 16) or to a collective; 0 = take every SM; -1 = the
                                   process-wide default of ldp_set_sm_reserve.  Per call: no shared state between engines */
-    int32_t reserved3;
+    int32_t lens;              /* 1: some camera of the launch has a lens model (ldp_ref_desc.lens_a / lens_b[k] not PINHOLE): the geometry
+                                  kernels' lens instantiation runs.  0: the caller guarantees that every camera is pinhole; the lens
+                                  fields of the descriptors are not read */
 } ldp_params;
+
+/* Lens model of a camera (COLMAP's models map onto two families; see CameraRecord.from_colmap).  Pixel coordinates are
+ * normalised with the record's f32 intrinsics, x = (u - cx) / fx, y = (v - cy) / fy, in f64; with r^2 = x^2 + y^2:
+ *   LDP_LENS_OPENCV   k = {k1, k2, p1, p2, k3, k4, k5, k6} (cv2.projectPoints order):
+ *                       radial = (1 + k1 r^2 + k2 r^4 + k3 r^6) / (1 + k4 r^2 + k5 r^4 + k6 r^6)
+ *                       x_d = x radial + 2 p1 x y + p2 (r^2 + 2 x^2),  y_d = y radial + p1 (r^2 + 2 y^2) + 2 p2 x y
+ *   LDP_LENS_FISHEYE  k = {k1, k2, k3, k4, 0...} (cv2.fisheye): theta = atan(r),
+ *                       theta_d = theta (1 + k1 theta^2 + k2 theta^4 + k3 theta^6 + k4 theta^8), (x_d, y_d) = theta_d / r (x, y)
+ * The observed (distorted) pixels are undistorted by Newton's method in f64 (ldp_undistort_points); a point with no valid
+ * inverse (no convergence, non-positive Jacobian determinant: past the fold of the polynomial; fisheye theta outside
+ * [0, pi/2)) becomes NaN and its sample is dropped. */
+typedef enum ldp_lens_model {
+    LDP_LENS_PINHOLE = 0,
+    LDP_LENS_OPENCV = 1,
+    LDP_LENS_FISHEYE = 2
+} ldp_lens_model;
+
+typedef struct ldp_lens {
+    int32_t model;             /* ldp_lens_model */
+    float fx, fy, cx, cy;      /* the record's f32 K[0,0], K[1,1], K[0,2], K[1,2] (the K that built P and F) */
+    int32_t pad;
+    double k[8];               /* coefficients, unused ones zero */
+} ldp_lens;
 
 /* Per reference view: where its matcher outputs live and its camera constants.  Array of n_refs in
  * DEVICE memory.  Camera constants are computed on the host exactly like the reference does
@@ -119,6 +144,9 @@ typedef struct ldp_ref_desc {
     int32_t mask_w, mask_h;
     float mask_sx, mask_sy;          /* f32(mask_w) / f32(W), f32(mask_h) / f32(H): F.interpolate(mode="nearest") source
                                         index = min(floor(dst * scale), size - 1) (core/pipeline.py:373-378) */
+    /* read only when ldp_params.lens is set */
+    ldp_lens lens_a;                 /* reference camera */
+    ldp_lens lens_b[LDP_MAX_NN];     /* neighbour cameras */
 } ldp_ref_desc;
 
 /* Caller-allocated DEVICE outputs.  Optional pointers may be NULL. */
@@ -172,6 +200,11 @@ int ldp_sample_refs(const ldp_params* params, const ldp_ref_desc* refs, const do
                     const ldp_outputs* out, void* workspace, size_t workspace_bytes, void* stream);
 int ldp_triangulate_samples(const ldp_params* params, const ldp_ref_desc* refs,
                             const ldp_outputs* out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* The lens inversion the geometry kernels apply to the observed pixels, alone: uv_out[i] = the ideal pinhole pixel of the
+ * distorted pixel uv_in[i] (f32 [n,2] DEVICE arrays; may alias), NaN where the lens has no valid inverse (see ldp_lens).
+ * `lens` is a HOST pointer.  A PINHOLE lens copies the input.  For tests of the lens arithmetic and for integrators. */
+int ldp_undistort_points(const ldp_lens* lens, int64_t n, const float* uv_in, float* uv_out, void* stream);
 
 /* The certainty post-processing alone (core/pipeline.py:405-430), for callers that want the reference's
  * cert_list tensors and for stage-level parity tests: for every view r and neighbour k < nn,

@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-LDP_ABI_VERSION = 12
+LDP_ABI_VERSION = 13
 LDP_MAX_NN = 16
 LDP_MAX_BINS = 4096
 
@@ -31,6 +31,10 @@ LDP_REF_CODE_MASK = 0xFF
 
 LDP_RNG_PHILOX = 0
 LDP_RNG_EXPLICIT = 1
+
+LDP_LENS_PINHOLE = 0
+LDP_LENS_OPENCV = 1
+LDP_LENS_FISHEYE = 2
 
 REF_STATUS_MESSAGES = {
     LDP_REF_EMPTY: "all sampling weights are zero",
@@ -58,7 +62,14 @@ class LdpParams(C.Structure):
         ("nn_max", C.c_int32), ("prologue", C.c_int32),
         ("certainty_floor", C.c_float), ("no_warped_masks", C.c_int32),
         ("seed", C.c_uint64), ("uniforms_per_ref", C.c_int64),
-        ("sm_reserve", C.c_int32), ("reserved3", C.c_int32),
+        ("sm_reserve", C.c_int32), ("lens", C.c_int32),
+    ]
+
+
+class LdpLens(C.Structure):
+    _fields_ = [
+        ("model", C.c_int32), ("fx", C.c_float), ("fy", C.c_float), ("cx", C.c_float), ("cy", C.c_float),
+        ("pad", C.c_int32), ("k", C.c_double * 8),
     ]
 
 
@@ -77,6 +88,7 @@ class LdpRefDesc(C.Structure):
         ("group", C.c_int32 * LDP_MAX_NN),
         ("mask_a", C.c_uint64), ("mask_b", C.c_uint64 * LDP_MAX_NN),
         ("mask_w", C.c_int32), ("mask_h", C.c_int32), ("mask_sx", C.c_float), ("mask_sy", C.c_float),
+        ("lens_a", LdpLens), ("lens_b", LdpLens * LDP_MAX_NN),
     ]
 
 
@@ -99,6 +111,7 @@ EXPORTS = [
     "ldp_struct_size", "ldp_profile_enable", "ldp_profile_read", "ldp_profile_name", "ldp_debug_set_cluster", "ldp_debug_last_cluster", "ldp_debug_set_subbatches", "ldp_debug_read_clocks", "ldp_debug_launch_stream",
     "ldp_pack_ply_records", "ldp_pack_points3d_records", "ldp_rgb_to_uint8", "ldp_gather_points", "ldp_gather_rows", "ldp_concat_points", "ldp_scatter_points",
     "ldp_select_kcenters", "ldp_nearest_neighbors", "ldp_voxel_workspace_bytes", "ldp_voxel_downsample", "ldp_set_sm_reserve",
+    "ldp_undistort_points",
 ]
 
 _lock = threading.Lock()
@@ -190,9 +203,11 @@ def load(build_if_missing: bool = False):
                                              C.c_void_p, C.c_size_t, C.c_void_p]
         lib.ldp_set_sm_reserve.restype = C.c_int
         lib.ldp_set_sm_reserve.argtypes = [C.c_int]
+        lib.ldp_undistort_points.restype = C.c_int
+        lib.ldp_undistort_points.argtypes = [C.POINTER(LdpLens), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
         if lib.ldp_abi_version() != LDP_ABI_VERSION:
             raise NativeLibraryError(f"ABI version mismatch: library {lib.ldp_abi_version()}, binding {LDP_ABI_VERSION}")
-        for which, struct in enumerate((LdpParams, LdpRefDesc, LdpOutputs)):
+        for which, struct in enumerate((LdpParams, LdpRefDesc, LdpOutputs, LdpLens)):
             if lib.ldp_struct_size(which) != C.sizeof(struct):
                 raise NativeLibraryError(f"struct layout mismatch for {struct.__name__}: "
                                          f"library {lib.ldp_struct_size(which)}, binding {C.sizeof(struct)}")

@@ -159,7 +159,8 @@ def _record_for(cameras, uid: int, size: Optional[Tuple[int, int]] = None) -> Ca
         sized = table.get(key)
         if sized is None:
             sized = CameraRecord(uid=rec.uid, image_path=rec.image_path, width=int(size[0]), height=int(size[1]),
-                                 K=rec.K, R=rec.R, t=rec.t, P=rec.P, C=rec.C)
+                                 K=rec.K, R=rec.R, t=rec.t, P=rec.P, C=rec.C,
+                                 lens_model=getattr(rec, "lens_model", None), lens_coeffs=getattr(rec, "lens_coeffs", None))
             table[key] = sized
         rec = sized
     return rec

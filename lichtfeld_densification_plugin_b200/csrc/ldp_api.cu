@@ -603,11 +603,13 @@ int launch_geometry(const ldp_params* p, const ldp_ref_desc* refs, const ldp_out
         if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_gather_kernel");
     }
     { KernelTimer kt(st, "ldp_geometry_kernel");
-      (void)launch_k(ldp::ldp_geometry_kernel, dim3(grid), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
+      if (p->lens) (void)launch_k(ldp::ldp_geometry_kernel<true>, dim3(grid), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga);
+      else (void)launch_k(ldp::ldp_geometry_kernel<false>, dim3(grid), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
     ++g_launches;
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_geometry_kernel");
     { KernelTimer kt(st, "ldp_fix_kernel");
-      (void)launch_k(ldp::ldp_fix_kernel, dim3(nsubrefs), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
+      if (p->lens) (void)launch_k(ldp::ldp_fix_kernel<true>, dim3(nsubrefs), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga);
+      else (void)launch_k(ldp::ldp_fix_kernel<false>, dim3(nsubrefs), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
     ++g_launches;
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_fix_kernel");
     return LDP_OK;
@@ -766,6 +768,23 @@ int ldp_pack_ply_records(const float* xyz, const float* rgb, int64_t n, const in
 int ldp_pack_points3d_records(const float* xyz, const float* rgb, const float* err, int64_t n, const int64_t* n_dev,
                               uint64_t first_id, uint8_t* records_out, void* stream) {
     return pack_records(1, xyz, rgb, err, n, n_dev, first_id, records_out, stream);
+}
+
+int ldp_undistort_points(const ldp_lens* lens, int64_t n, const float* uv_in, float* uv_out, void* stream) {
+    if (!lens || n < 0) return fail(LDP_ERR_INVALID, "bad arguments");
+    if (lens->model < LDP_LENS_PINHOLE || lens->model > LDP_LENS_FISHEYE) return fail(LDP_ERR_INVALID, "unknown lens model");
+    g_launches = 0;
+    if (n == 0) return LDP_OK;
+    if (!uv_in || !uv_out) return fail(LDP_ERR_INVALID, "null pointer");
+    if ((reinterpret_cast<size_t>(uv_in) | reinterpret_cast<size_t>(uv_out)) & 7) return fail(LDP_ERR_INVALID, "uv arrays must be 8-byte aligned");
+    const long long blocks = (n + ldp::KU_THREADS - 1) / ldp::KU_THREADS;
+    const unsigned grid = (unsigned)std::min<long long>(blocks, (long long)sm_count() * 16);
+    (void)launch_k(ldp::ldp_undistort_kernel, dim3(grid), dim3(ldp::KU_THREADS), 0, reinterpret_cast<cudaStream_t>(stream), *lens,
+                   (long long)n, reinterpret_cast<const float2*>(uv_in), reinterpret_cast<float2*>(uv_out));
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "ldp_undistort_kernel");
+    return LDP_OK;
 }
 
 int ldp_rgb_to_uint8(const float* rgb, int64_t n_values, uint8_t* out, void* stream) {
@@ -993,6 +1012,7 @@ int64_t ldp_struct_size(int which) {
         case 0: return (int64_t)sizeof(ldp_params);
         case 1: return (int64_t)sizeof(ldp_ref_desc);
         case 2: return (int64_t)sizeof(ldp_outputs);
+        case 3: return (int64_t)sizeof(ldp_lens);
         default: return -1;
     }
 }

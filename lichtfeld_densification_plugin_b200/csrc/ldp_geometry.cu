@@ -327,6 +327,103 @@ __device__ __forceinline__ void fetch_texel_pair(const uint8_t* __restrict__ im,
     }
 }
 
+// ---- lens models (include/ldp_b200.h: ldp_lens).  Not in the reference, which triangulates every camera as a pinhole.
+// The inversion is Newton's method in f64 from the distorted point; it stops when the step is below LENS_STEP_TOL normalised
+// units, and fails (NaN) after LENS_MAX_ITERS steps, or when the Jacobian determinant (fisheye: d theta_d / d theta) is not
+// positive at an iterate -- past the fold of the polynomial, where the inverse is not unique -- or when the fisheye angle
+// it converges to lies outside [0, pi/2).  tests/lens_oracle.py restates the same rule.
+constexpr int LENS_MAX_ITERS = 20;
+constexpr double LENS_STEP_TOL = 1e-12;
+constexpr double LENS_HALF_PI = 1.5707963267948966;
+constexpr double LENS_FISHEYE_THETA0_MAX = 1.5707963267948966 - 1e-6;   // fisheye: the first iterate lies inside [0, pi/2)
+
+__device__ __forceinline__ void lens_distort(const ldp_lens& L, double x, double y, double& xd, double& yd) {
+    const double* k = L.k;
+    const double r2 = x * x + y * y;
+    if (L.model == LDP_LENS_FISHEYE) {
+        const double r = sqrt(r2);
+        const double th = atan(r), t2 = th * th;
+        const double thd = th * (1.0 + t2 * (k[0] + t2 * (k[1] + t2 * (k[2] + t2 * k[3]))));
+        const double s = (r > 0.0) ? thd / r : 1.0;
+        xd = x * s; yd = y * s;
+    } else {
+        const double radial = (1.0 + r2 * (k[0] + r2 * (k[1] + r2 * k[4]))) / (1.0 + r2 * (k[5] + r2 * (k[6] + r2 * k[7])));
+        xd = x * radial + 2.0 * k[2] * x * y + k[3] * (r2 + 2.0 * x * x);
+        yd = y * radial + k[2] * (r2 + 2.0 * y * y) + 2.0 * k[3] * x * y;
+    }
+}
+
+// normalised distorted (xd, yd) -> normalised ideal (x, y); false (and NaN) where there is no valid inverse
+__device__ __forceinline__ bool lens_undistort(const ldp_lens& L, double xd, double yd, double& x, double& y) {
+    const double* k = L.k;
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    if (L.model == LDP_LENS_FISHEYE) {
+        const double rd = sqrt(xd * xd + yd * yd);
+        if (rd == 0.0) { x = xd; y = yd; return true; }
+        // start at r_d, clamped into the valid range like cv2.fisheye: when theta_d(pi/2) > pi/2 (positive coefficients) the
+        // distorted radii in [pi/2, theta_d(pi/2)) have a solution inside it; only the solution's range is checked
+        double th = fmin(rd, LENS_FISHEYE_THETA0_MAX);
+        bool ok = false;
+        for (int it = 0; it < LENS_MAX_ITERS; ++it) {
+            const double t2 = th * th;
+            const double f = th * (1.0 + t2 * (k[0] + t2 * (k[1] + t2 * (k[2] + t2 * k[3])))) - rd;
+            const double d = 1.0 + t2 * (3.0 * k[0] + t2 * (5.0 * k[1] + t2 * (7.0 * k[2] + t2 * 9.0 * k[3])));
+            if (!(d > 0.0)) break;
+            const double step = f / d;
+            th -= step;
+            if (fabs(step) < LENS_STEP_TOL) { ok = th >= 0.0 && th < LENS_HALF_PI; break; }
+        }
+        if (!ok) { x = y = nan; return false; }
+        const double s = tan(th) / rd;
+        x = xd * s; y = yd * s;
+        return true;
+    }
+    double u = xd, v = yd;
+    for (int it = 0; it < LENS_MAX_ITERS; ++it) {
+        const double r2 = u * u + v * v;
+        const double a = 1.0 + r2 * (k[0] + r2 * (k[1] + r2 * k[4]));
+        const double b = 1.0 + r2 * (k[5] + r2 * (k[6] + r2 * k[7]));
+        const double da = k[0] + r2 * (2.0 * k[1] + r2 * 3.0 * k[4]);      // d a / d r2
+        const double db = k[5] + r2 * (2.0 * k[6] + r2 * 3.0 * k[7]);
+        const double radial = a / b;
+        const double drad = (da * b - a * db) / (b * b);                     // d radial / d r2
+        const double fx = u * radial + 2.0 * k[2] * u * v + k[3] * (r2 + 2.0 * u * u) - xd;
+        const double fy = v * radial + k[2] * (r2 + 2.0 * v * v) + 2.0 * k[3] * u * v - yd;
+        const double j00 = radial + 2.0 * u * u * drad + 2.0 * k[2] * v + 6.0 * k[3] * u;
+        const double j01 = 2.0 * u * v * drad + 2.0 * k[2] * u + 2.0 * k[3] * v;
+        const double j10 = 2.0 * u * v * drad + 2.0 * k[2] * u + 2.0 * k[3] * v;
+        const double j11 = radial + 2.0 * v * v * drad + 6.0 * k[2] * v + 2.0 * k[3] * u;
+        const double det = j00 * j11 - j01 * j10;
+        if (!(det > 0.0)) break;
+        const double du = (j11 * fx - j01 * fy) / det, dv = (j00 * fy - j10 * fx) / det;
+        u -= du; v -= dv;
+        if (du * du + dv * dv < LENS_STEP_TOL * LENS_STEP_TOL) { x = u; y = v; return true; }
+    }
+    x = y = nan;
+    return false;
+}
+
+// f32 observed pixel -> f32 ideal pinhole pixel of the same camera (NaN where the lens has no valid inverse)
+__device__ __forceinline__ void lens_undistort_px(const ldp_lens& L, float u, float v, float& ui, float& vi) {
+    const double fx = L.fx, fy = L.fy, cx = L.cx, cy = L.cy;
+    double x, y;
+    lens_undistort(L, ((double)u - cx) / fx, ((double)v - cy) / fy, x, y);
+    ui = (float)(fx * x + cx); vi = (float)(fy * y + cy);
+}
+
+// reprojection error in the distorted image: the f32 projection q (as reproj_err forms it) through the forward lens, in f64
+__device__ __forceinline__ float lens_reproj_err(const ldp_lens& L, const float* P, float X0, float X1, float X2, float X3,
+                                                 float u, float v, float* zout) {
+    const float q0 = proj_row(P, X0, X1, X2, X3), q1 = proj_row(P + 4, X0, X1, X2, X3), q2 = proj_row(P + 8, X0, X1, X2, X3);
+    *zout = q2;
+    const double z = (double)fmaxf(q2, 1e-12f);
+    const double fx = L.fx, fy = L.fy, cx = L.cx, cy = L.cy;
+    double xd, yd;
+    lens_distort(L, ((double)q0 / z - cx) / fx, ((double)q1 / z - cy) / fy, xd, yd);
+    const double du = fx * xd + cx - (double)u, dv = fy * yd + cy - (double)v;
+    return (float)sqrt(du * du + dv * dv);
+}
+
 struct SampleResult {
     float X0, X1, X2, err;
     float cr, cg, cb, dcert;
@@ -409,9 +506,12 @@ __device__ __forceinline__ void gather_sample(const ldp_params& P, const RefCons
 }
 
 // ---- compute: everything else the reference computes for one sampled pixel (core/pipeline.py:653-769)
-template <bool ROBUST>
+// LENS: the launch has lens cameras (ldp_params.lens); lt = the view's staged lens table, [0] reference camera, [1 + k]
+// neighbour k.  A lens camera's observed pixels are undistorted before the Sampson gate and the DLT, and its reprojection
+// error is measured in the distorted image; a pinhole camera's arithmetic is the same as without LENS.
+template <bool ROBUST, bool LENS>
 __device__ __forceinline__ void eval_sample(const ldp_params& P, const RefConst& rc, const PairTable& pc, const GeomArgs& ga,
-                                            const SampleRec& rec, float craw, SampleResult& o GCLK_ARGS) {
+                                            const ldp_lens* lt, const SampleRec& rec, float craw, SampleResult& o GCLK_ARGS) {
     const int k = (int)(rec.k_cert & 0xffu);
     const PairView pk = pair_view(pc, k);
     o.grp = pk.group;
@@ -437,8 +537,14 @@ __device__ __forceinline__ void eval_sample(const ldp_params& P, const RefConst&
     t11[0] = (float)((rec.tex[2] >> 8) & 0xffu);  t11[1] = (float)((rec.tex[2] >> 16) & 0xffu); t11[2] = (float)(rec.tex[2] >> 24);
 
     // ---- full-resolution pixel coordinates: core/pipeline.py:681-683, 697-703
-    const float uA = __fmul_rn(xA, rc.sxA), vA = __fmul_rn(yA, rc.syA);
-    const float uB = __fmul_rn(xB, pk.sxB), vB = __fmul_rn(yB, pk.syB);
+    const float uA_obs = __fmul_rn(xA, rc.sxA), vA_obs = __fmul_rn(yA, rc.syA);
+    const float uB_obs = __fmul_rn(xB, pk.sxB), vB_obs = __fmul_rn(yB, pk.syB);
+    // the ideal pinhole pixels that P, F and the DLT assume
+    float uA = uA_obs, vA = vA_obs, uB = uB_obs, vB = vB_obs;
+    if constexpr (LENS) {
+        if (lt[0].model != LDP_LENS_PINHOLE) lens_undistort_px(lt[0], uA_obs, vA_obs, uA, vA);
+        if (lt[1 + k].model != LDP_LENS_PINHOLE) lens_undistort_px(lt[1 + k], uB_obs, vB_obs, uB, vB);
+    }
 
     // ---- Sampson gate in f64: core/geometry.py:133-141, core/pipeline.py:708-727.  se < thr is decided on
     //      num^2 vs thr*den outside a 2^-50 band, by the reference's quotient inside it.
@@ -512,8 +618,16 @@ __device__ __forceinline__ void eval_sample(const ldp_params& P, const RefConst&
         }
         // ---- reprojection errors + cheirality: core/geometry.py:91-110, core/pipeline.py:735-737
         float z1, z2;
-        const float e1 = reproj_err(rc.P1, X0, X1, X2, X3, uA, vA, &z1);
-        const float e2 = reproj_err(pk.P2, X0, X1, X2, X3, uB, vB, &z2);
+        float e1, e2;
+        if constexpr (LENS) {       // a lens camera's error is measured against its observed (distorted) pixel
+            e1 = (lt[0].model != LDP_LENS_PINHOLE) ? lens_reproj_err(lt[0], rc.P1, X0, X1, X2, X3, uA_obs, vA_obs, &z1)
+                                                   : reproj_err(rc.P1, X0, X1, X2, X3, uA, vA, &z1);
+            e2 = (lt[1 + k].model != LDP_LENS_PINHOLE) ? lens_reproj_err(lt[1 + k], pk.P2, X0, X1, X2, X3, uB_obs, vB_obs, &z2)
+                                                       : reproj_err(pk.P2, X0, X1, X2, X3, uB, vB, &z2);
+        } else {
+            e1 = reproj_err(rc.P1, X0, X1, X2, X3, uA, vA, &z1);
+            e2 = reproj_err(pk.P2, X0, X1, X2, X3, uB, vB, &z2);
+        }
         const float err = (e1 != e1 || e2 != e2) ? __int_as_float(0x7fc00000) : fmaxf(e1, e2);   // np.maximum propagates NaN
         int keep;
         if (P.no_filter) {                                                        // core/pipeline.py:739-743
@@ -624,7 +738,26 @@ __device__ __forceinline__ void load_record(const Workspace& ws, const ldp_param
     craw = P.collect_debug ? ws.dbgm[o].x : 0.f;
 }
 
+// The view's lens table (lens_a, lens_b[]), descriptor -> shared memory, staged like the camera constants: loads first, stores
+// after the caller's other loads are in flight.  Only the LENS instantiations declare and stage it.
+constexpr int LENS_WORDS = (int)(sizeof(ldp_lens) * (LDP_MAX_NN + 1) / 4);
+constexpr int LENS_PER = (LENS_WORDS + K2_THREADS - 1) / K2_THREADS;
+static_assert(offsetof(ldp_ref_desc, lens_b) == offsetof(ldp_ref_desc, lens_a) + sizeof(ldp_lens) && sizeof(ldp_lens) % 8 == 0,
+              "lens table layout");
+struct StagedLens { uint32_t v[LENS_PER]; };
+__device__ __forceinline__ void lens_load(const ldp_ref_desc* rd, int t, StagedLens& sl) {
+    const uint32_t* src = reinterpret_cast<const uint32_t*>(&rd->lens_a);
+#pragma unroll
+    for (int q = 0; q < LENS_PER; ++q) sl.v[q] = (t + q * K2_THREADS < LENS_WORDS) ? __ldg(src + t + q * K2_THREADS) : 0u;
+}
+__device__ __forceinline__ void lens_store(const StagedLens& sl, ldp_lens* dst, int t) {
+    uint32_t* d = reinterpret_cast<uint32_t*>(dst);
+#pragma unroll
+    for (int q = 0; q < LENS_PER; ++q) if (t + q * K2_THREADS < LENS_WORDS) d[t + q * K2_THREADS] = sl.v[q];
+}
+
 // K2b compute: coalesced record in, per-sample result (in place) + per-tile group statistics out.
+template <bool LENS>
 __global__ void __launch_bounds__(K2_THREADS, K2_MIN_BLOCKS)
 ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const Workspace ws, const ldp_outputs out,
                     const GeomArgs ga)
@@ -639,6 +772,9 @@ ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, c
     // indices are requested, one round trip for both; the prefetches are hints (the winner row was written three kernels ago)
     StagedDesc sd;
     stage_load(refs + r, threadIdx.x, K2_THREADS, sd);
+    const ldp_lens* lt = nullptr;
+    StagedLens sl;
+    if constexpr (LENS) lens_load(refs + r, threadIdx.x, sl);
     if (ga.fused && ga.l2_prefetch && ga.have_bestk && threadIdx.x == LDP_MAX_NN + 32)
         l2_prefetch_slice(ws.bestk + (size_t)r * ws.n_pad, (size_t)P.H * P.W, blockIdx.x, gridDim.x);
     if (ga.fused && P.prologue) stage_proview(refs + r, pv, threadIdx.x);
@@ -654,6 +790,11 @@ ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, c
     }
     const int S = out.n_samples[r];
     stage_store(sd, rc, pc, threadIdx.x, K2_THREADS, blockIdx.x, (ga.fused && ga.l2_prefetch) ? (int)gridDim.x : 0);
+    if constexpr (LENS) {
+        __shared__ __align__(8) ldp_lens s_lens[LDP_MAX_NN + 1];
+        lens_store(sl, s_lens, threadIdx.x);
+        lt = s_lens;
+    }
     if (ga.fused && (ga.discard & 1)) {
         const char* row = reinterpret_cast<const char*>(ws.w + (size_t)r * ws.n_pad);
         const int nlines = (int)(ws.n_pad * sizeof(float) / 128);
@@ -676,7 +817,7 @@ ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, c
         else load_record(ws, P, o, rec, craw);
         GCLK_USE(rec.tex[0]); GCLK_USE(rec.tex[2]); GCLK_USE(rec.wv.x); GCLK(2);
         SampleResult s;
-        eval_sample<false>(P, rc, pc, ga, rec, craw, s GCLK_PASS);
+        eval_sample<false, LENS>(P, rc, pc, ga, lt, rec, craw, s GCLK_PASS);
         if (!s.converged && ga.fused) {     // the fix-up reads the record
             ws.pt0[o] = rec.wv;
             ws.pt1[o] = make_float4(__uint_as_float(rec.tex[0]), __uint_as_float(rec.tex[1]), __uint_as_float(rec.tex[2]),
@@ -720,6 +861,7 @@ ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, c
 // output plan, once for all of its pack CTAs: kept points per neighbour group, groups in order of first appearance
 // (reference core/pipeline.py:685-695), and for every 128-sample tile and group the row (relative to the view's first row)
 // at which that tile's kept samples of that group start.
+template <bool LENS>
 __global__ void __launch_bounds__(K2_THREADS)
 ldp_fix_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const Workspace ws, const ldp_outputs out,
                const GeomArgs ga)
@@ -735,6 +877,14 @@ ldp_fix_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const 
     if (n > 0) {
         const int2* fix_list = ws.fix_list + (size_t)ga.ref0 * ws.sel_cap;
         stage_constants(refs + r, rc, pc, tid, K2_THREADS);
+        const ldp_lens* lt = nullptr;
+        if constexpr (LENS) {
+            __shared__ __align__(8) ldp_lens s_lens[LDP_MAX_NN + 1];
+            StagedLens sl;
+            lens_load(refs + r, tid, sl);
+            lens_store(sl, s_lens, tid);
+            lt = s_lens;
+        }
         __syncthreads();
         for (int e = tid; e < n; e += K2_THREADS) {
             const int2 it = fix_list[e];
@@ -746,7 +896,7 @@ ldp_fix_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const 
             load_record(ws, P, o, rec, craw);
             SampleResult s;
             GCLK_DECL
-            eval_sample<true>(P, rc, pc, ga, rec, craw, s GCLK_PASS);
+            eval_sample<true, LENS>(P, rc, pc, ga, lt, rec, craw, s GCLK_PASS);
             store_sample(P, ws, out, o, s);
             if (s.keep) {
                 atomicAdd(&ws.kept[r], 1);
@@ -928,6 +1078,18 @@ ldp_prologue_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, f
     for (int px = blockIdx.x * KP_THREADS + threadIdx.x; px < N; px += gridDim.x * KP_THREADS) {
         const int y = px / P.W;
         o[px] = prologue_cert(__ldcs(c + px), k, px, px - y * P.W, y, P, pv);
+    }
+}
+
+// ldp_undistort_points: the geometry kernels' lens inversion on a list of pixels
+constexpr int KU_THREADS = 256;
+__global__ void __launch_bounds__(KU_THREADS)
+ldp_undistort_kernel(const ldp_lens L, long long n, const float2* __restrict__ in, float2* __restrict__ out) {
+    for (long long i = (long long)blockIdx.x * KU_THREADS + threadIdx.x; i < n; i += (long long)gridDim.x * KU_THREADS) {
+        const float2 p = in[i];
+        float2 q = p;
+        if (L.model != LDP_LENS_PINHOLE) lens_undistort_px(L, p.x, p.y, q.x, q.y);
+        out[i] = q;
     }
 }
 

@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from . import _native as N
-from .core.camera_models import CameraRecord
+from .core.camera_models import CameraRecord, check_lens
 from .core.geometry import fundamental_from_world2cam
 
 # 64-bit word offsets of the pointer fields inside an ldp_ref_desc (patched per call without numpy field lookups)
@@ -25,6 +25,30 @@ _CERT_WORD = N.REF_DESC_DTYPE.fields["cert"][1] // 8
 _WARP_WORD = N.REF_DESC_DTYPE.fields["warp"][1] // 8
 _IMAGE_WORD = N.REF_DESC_DTYPE.fields["image"][1] // 8
 assert N.REF_DESC_DTYPE.itemsize % 8 == 0
+
+_LENS_MODELS = {None: N.LDP_LENS_PINHOLE, "opencv": N.LDP_LENS_OPENCV, "fisheye": N.LDP_LENS_FISHEYE}
+
+
+def lens_of(cam: CameraRecord) -> N.LdpLens:
+    """The ldp_lens of a record: its lens model and coefficients, and the f32 K entries that built its P and F."""
+    check_lens(cam)
+    model = getattr(cam, "lens_model", None)
+    L = N.LdpLens()
+    L.model = _LENS_MODELS[model]
+    K = np.asarray(cam.K, dtype=np.float32)
+    L.fx, L.fy, L.cx, L.cy = float(K[0, 0]), float(K[1, 1]), float(K[0, 2]), float(K[1, 2])
+    if model is not None:
+        for i, c in enumerate(np.asarray(cam.lens_coeffs, dtype=np.float64)):
+            L.k[i] = float(c)
+    return L
+
+
+def _fill_lens(field, cam: CameraRecord) -> None:
+    L = lens_of(cam)
+    field["model"] = L.model
+    field["fx"], field["fy"], field["cx"], field["cy"] = L.fx, L.fy, L.cx, L.cy
+    field["k"] = np.frombuffer(bytes(L.k), dtype=np.float64)
+
 
 SAMPLE_CAP_DEFAULT = 0.9     # matcher.sample_thresh, reference core/matcher.py:92
 BORDER_DEFAULT = 2           # reference core/pipeline.py:646
@@ -99,6 +123,7 @@ class RefBatch:
         self.ref_uids: List[int] = []
         self.force_scalar_loads = False
         self.has_warped_masks = False        # some neighbour mask (mask_b) was registered: the warp planes are read per pixel
+        self.has_lens = False                # some camera carries a lens model: the geometry kernels' lens instantiation runs
         self.pairs = pair_cache or PairConstantCache()
 
     def __len__(self) -> int:
@@ -170,10 +195,16 @@ class RefBatch:
                 t["F"][k] = self.pairs.fundamental(ref_cam, cam).reshape(9)
                 t["sxB"][k], t["syB"][k] = np.float32(cam.width / wm), np.float32(cam.height / hm)
                 t["group"][k] = uids.index(uids[k])          # the reference groups by neighbour uid
+            if any(getattr(c, "lens_model", None) is not None for c in (ref_cam, *nbr_cams)):
+                _fill_lens(t["lens_a"], ref_cam)
+                for k, cam in enumerate(nbr_cams):
+                    _fill_lens(t["lens_b"][k], cam)
             return t
 
         key = (id(ref_cam), tuple(id(c) for c in nbr_cams), self.w_match, self.h_match, iw, ih)
         row1, words = self._new_row(self.pairs.row_template(key, (ref_cam, tuple(nbr_cams)), make_template))
+        if any(getattr(c, "lens_model", None) is not None for c in (ref_cam, *nbr_cams)):
+            self.has_lens = True
         for k in range(nn):
             c = self._check_plane(cert_planes[k], (self.H, self.W), "certainty plane", allow_pinned_host=True)
             w = self._check_plane(warp_planes[k], (self.H, self.W, 4), "warp plane", allow_pinned_host=True)
@@ -312,6 +343,7 @@ class DensifyEngine:
         p.prologue = 0 if cfg.certainty_floor is None else 1
         p.certainty_floor = float(np.float32(cfg.certainty_floor if cfg.certainty_floor is not None else 0.0))
         p.no_warped_masks = 0 if batch.has_warped_masks else 1
+        p.lens = 1 if batch.has_lens else 0
         p.sm_reserve = int(self.sm_reserve)
         p.seed = int(cfg.seed) & 0xFFFFFFFFFFFFFFFF
         p.uniforms_per_ref = int(uniforms_per_ref)
@@ -422,6 +454,22 @@ class DensifyEngine:
         N.check(rc, "ldp_sample_refs")
         torch.cuda.current_stream(dev).synchronize()
         return sel, n_samples, status, used
+
+    def undistort_pixels(self, uv: torch.Tensor, record: CameraRecord) -> torch.Tensor:
+        """``ldp_undistort_points``: the ideal pinhole pixels of the observed pixels ``uv`` (f32 [n, 2] on the engine device)
+        of camera ``record``, NaN where its lens has no valid inverse - the inversion the geometry kernels apply.  Enqueued
+        on the current stream; a record without a lens returns a copy."""
+        if not isinstance(uv, torch.Tensor) or uv.device != self.device or uv.dtype != torch.float32 or uv.dim() != 2 \
+                or uv.shape[1] != 2:
+            raise ValueError(f"uv must be a float32 [n, 2] tensor on {self.device}")
+        uv = uv.contiguous()
+        out = torch.empty_like(uv)
+        L = lens_of(record)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        rc = self.lib.ldp_undistort_points(C.byref(L), int(uv.shape[0]), C.c_void_p(uv.data_ptr()), C.c_void_p(out.data_ptr()),
+                                           C.c_void_p(stream))
+        N.check(rc, "ldp_undistort_points")
+        return out
 
     def alloc_outputs(self, R: int, sel_cap: int, collect_debug: bool = False, taps: bool = False) -> DensifyOutputs:
         """Everything a caller reads back lives in ONE allocation (``packed``): ref_offset | per-view status words | xyz | rgb |
