@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define LDP_ABI_VERSION 13
+#define LDP_ABI_VERSION 14
 #define LDP_MAX_NN 16          /* neighbours per reference view (the panel clamps to 10) */
 #define LDP_MAX_BINS 4096      /* coverage tiles per map: ceil(W/tile)*ceil(H/tile), tile = max(1, W/24) */
 
@@ -91,7 +91,32 @@ typedef struct ldp_params {
     int32_t lens;              /* 1: some camera of the launch has a lens model (ldp_ref_desc.lens_a / lens_b[k] not PINHOLE): the geometry
                                   kernels' lens instantiation runs.  0: the caller guarantees that every camera is pinhole; the lens
                                   fields of the descriptors are not read */
+    int32_t multiview;         /* 1: multi-view refinement of the kept points (see below); needs no_filter = 0 */
+    float multiview_min_cert;  /* multiview: a neighbour's certainty at the sample must be >= this to join, in (0, 1] */
 } ldp_params;
+
+/* Multi-view refinement (ldp_params.multiview = 1).  Not in the reference, which triangulates every sampled pixel from the
+ * reference view and its winning neighbour k alone.  It changes WHERE a kept point is, never WHICH points are kept:
+ *   1. The two-view evaluation (Sampson gate, DLT, reprojection, cheirality, parallax against k) runs unchanged and decides
+ *      keep, group, colour and the debug match.  A sample that is not kept is finished.
+ *   2. Candidates of a kept sample: every neighbour slot q with group[q] == q (a uid listed twice counts once),
+ *      group[q] != group[k], certainty at the pixel >= f32(multiview_min_cert) (after post-processing: with raw planes the
+ *      floor and the masks apply), a finite ideal pixel, and, when sampson_thresh > 0, Sampson(F[q]) < sampson_thresh
+ *      (the two-view gate's f64 decision).  Pixels are decoded and undistorted as in the two-view path; the reference
+ *      pixel is the winner's.
+ *   3. One DLT over the reference, the winner and all candidates: the two-view path's f32 rows, two per view, summed into
+ *      the f64 Gram matrix A^T A and solved by the same null-vector code (inverse iteration; Jacobi in the fix-up).
+ *   4. Trim once: every candidate whose reprojection error (lens-aware) is > reproj_thresh, or whose depth is <= 0, is
+ *      dropped; the winner never is.  If something was dropped and a candidate is left, the DLT is solved again; if none is
+ *      left, the two-view point stands.
+ *   5. The refined point is accepted if in EVERY included view (reference and winner too) its error is <= reproj_thresh and
+ *      its depth > 0, and the reference-winner parallax test passes; otherwise the two-view point stands.
+ *   6. xyz = the accepted point, err = the largest error over the included views, view_mask[point] = bit q for every
+ *      neighbour slot that contributed (the winner's bit always).  A solve that does not converge is redone by the fix-up
+ *      with Jacobi; a converged two-view verdict is never re-evaluated.
+ * sel_idx, sample_flags, group_order, group_count, ref_offset, rgb, the debug outputs and the sample_xyzerr taps (two-view
+ * values) are those of the same launch without multiview; so are xyz and err of every point whose mask is the winner's
+ * bit alone.  ldp_workspace_bytes grows by 20 bytes per sample slot when multiview is set. */
 
 /* Lens model of a camera (COLMAP's models map onto two families; see CameraRecord.from_colmap).  Pixel coordinates are
  * normalised with the record's f32 intrinsics, x = (u - cx) / fx, y = (v - cy) / fy, in f64; with r^2 = x^2 + y^2:
@@ -171,6 +196,8 @@ typedef struct ldp_outputs {
     int32_t* uniforms_used;    /* [n_refs] doubles consumed from the stream */
     int32_t* rounds;           /* [n_refs] rejection rounds of the weighted draw */
     float* weight_sum;         /* [n_refs] the f32 normaliser s actually used */
+    int32_t* view_mask;        /* [capacity] optional, multiview launches only (LDP_ERR_INVALID otherwise): per point, bit q set
+                                  for every neighbour slot q whose match contributed to it; the winner's bit always */
 } ldp_outputs;
 
 /* ---- entry points ------------------------------------------------------------------------------- */
@@ -318,6 +345,14 @@ int ldp_debug_last_cluster(void);          /* cluster size the last draw kernel 
 /* Debug builds (-DLDP_PHASE_CLOCKS) only: copy the draw kernel's per-view phase timestamps [n_refs][32] (SM clocks)
  * to host memory; synchronises.  Release builds return zeros. */
 int ldp_debug_read_clocks(const ldp_params* params, void* workspace, long long* host_out);
+/* Test hooks for the fix-up worklist of the geometry kernels.  ldp_debug_force_fixup: in subsequent MULTIVIEW launches on any
+ * thread (0, 0 restores the default), every sample i (position in its view's sample list) with i % two_view_every == 0 is sent
+ * to the fix-up as if its two-view null-vector iteration had not converged, and every kept sample with i % multiview_every == 0
+ * as if its multi-view solve had not converged (0 = never); the fix-up solves them with Jacobi.  The plain path's kernels do not
+ * read it.  ldp_debug_read_fixups: after a launch (synchronises), host_out[0] = entries of the worklist, host_out[1] = those
+ * that redo only a multi-view solve; params and workspace as given to that launch. */
+int ldp_debug_force_fixup(int two_view_every, int multiview_every);
+int ldp_debug_read_fixups(const ldp_params* params, void* workspace, int32_t* host_out);
 /* Test hook: pipeline a launch over n sub-batches of views on internal streams (1..8; 0 restores the default, which is
  * one batch unless LDP_SUBBATCH is set).  Results do not depend on it. */
 int ldp_debug_set_subbatches(int n);

@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-LDP_ABI_VERSION = 13
+LDP_ABI_VERSION = 14
 LDP_MAX_NN = 16
 LDP_MAX_BINS = 4096
 
@@ -63,6 +63,7 @@ class LdpParams(C.Structure):
         ("certainty_floor", C.c_float), ("no_warped_masks", C.c_int32),
         ("seed", C.c_uint64), ("uniforms_per_ref", C.c_int64),
         ("sm_reserve", C.c_int32), ("lens", C.c_int32),
+        ("multiview", C.c_int32), ("multiview_min_cert", C.c_float),
     ]
 
 
@@ -100,6 +101,7 @@ class LdpOutputs(C.Structure):
         ("dbg_matches", C.c_uint64), ("dbg_cert", C.c_uint64), ("sel_idx", C.c_uint64),
         ("sample_flags", C.c_uint64), ("sample_xyzerr", C.c_uint64),
         ("uniforms_used", C.c_uint64), ("rounds", C.c_uint64), ("weight_sum", C.c_uint64),
+        ("view_mask", C.c_uint64),
     ]
 
 
@@ -111,7 +113,7 @@ EXPORTS = [
     "ldp_struct_size", "ldp_profile_enable", "ldp_profile_read", "ldp_profile_name", "ldp_debug_set_cluster", "ldp_debug_last_cluster", "ldp_debug_set_subbatches", "ldp_debug_read_clocks", "ldp_debug_launch_stream",
     "ldp_pack_ply_records", "ldp_pack_points3d_records", "ldp_rgb_to_uint8", "ldp_gather_points", "ldp_gather_rows", "ldp_concat_points", "ldp_scatter_points",
     "ldp_select_kcenters", "ldp_nearest_neighbors", "ldp_voxel_workspace_bytes", "ldp_voxel_downsample", "ldp_set_sm_reserve",
-    "ldp_undistort_points",
+    "ldp_undistort_points", "ldp_debug_force_fixup", "ldp_debug_read_fixups",
 ]
 
 _lock = threading.Lock()
@@ -205,6 +207,10 @@ def load(build_if_missing: bool = False):
         lib.ldp_set_sm_reserve.argtypes = [C.c_int]
         lib.ldp_undistort_points.restype = C.c_int
         lib.ldp_undistort_points.argtypes = [C.POINTER(LdpLens), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.ldp_debug_force_fixup.restype = C.c_int
+        lib.ldp_debug_force_fixup.argtypes = [C.c_int, C.c_int]
+        lib.ldp_debug_read_fixups.restype = C.c_int
+        lib.ldp_debug_read_fixups.argtypes = [C.POINTER(LdpParams), C.c_void_p, C.POINTER(C.c_int32)]
         if lib.ldp_abi_version() != LDP_ABI_VERSION:
             raise NativeLibraryError(f"ABI version mismatch: library {lib.ldp_abi_version()}, binding {LDP_ABI_VERSION}")
         for which, struct in enumerate((LdpParams, LdpRefDesc, LdpOutputs, LdpLens)):

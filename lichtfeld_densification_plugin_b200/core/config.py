@@ -54,10 +54,17 @@ class DensePipelineConfig:
                                      # memory, cancellation latency and progress granularity are bounded by this); 0 = all in one launch
     viz_every_emission: bool = False # live update: True writes every intermediate PLY the reference would (one per viz_interval
                                      # views, each a rewrite of all points so far); False only the latest one per collected launch
+    multiview: bool = False          # re-triangulate every kept point from all of its confident, consistent neighbours (the
+                                     # reference uses the best neighbour alone); which points are kept does not change
+    multiview_min_certainty: float = 0.5   # multiview: certainty a neighbour's match needs at the pixel to join
 
     def validate(self) -> "DensePipelineConfig":
         if self.matches_per_ref < 0:
             raise ValueError("matches_per_ref must be >= 0")
+        if self.multiview and self.no_filter:
+            raise ValueError("multiview needs the filters: it cannot be combined with no_filter")
+        if not 0.0 < float(self.multiview_min_certainty) <= 1.0:
+            raise ValueError("multiview_min_certainty must lie in (0, 1]")
         if self.rng_mode not in (RNG_PHILOX, RNG_NUMPY_GLOBAL, RNG_EXPLICIT):
             raise ValueError(f"unknown rng_mode {self.rng_mode!r}")
         return self

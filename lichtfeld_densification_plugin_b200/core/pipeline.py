@@ -38,6 +38,7 @@ class PipelineResult:
     err: np.ndarray
     elapsed_seconds: float
     pairs_processed: int
+    n_views: Optional[np.ndarray] = None          # extra, config.multiview: uint8 cameras per point, the reference view included
 
 
 class PipelineCancelled(RuntimeError):
@@ -120,6 +121,7 @@ class _TriangulatedReference:
     debug_matches_by_nbr: Dict[int, np.ndarray]
     debug_cert_by_nbr: Dict[int, np.ndarray]
     ply_records: Optional[np.ndarray] = None      # extra: this view's 15-byte PLY vertex records, packed on the device
+    n_views: Optional[np.ndarray] = None          # extra, config.multiview: uint8 cameras per point, the reference view included
 
 
 def _build_camera_lookup(camera_records: Sequence[CameraRecord]) -> _CameraLookup:
@@ -235,8 +237,11 @@ def _split_reference(out: DensifyOutputs, host: dict, r: int, nbr_uids: List[int
                 dbg_c[nbr_uids[g]] = host["dbg_cert"][pos:pos + cnt]
             pos += cnt
     rec = host["ply"][15 * a:15 * b] if "ply" in host else None
+    n_views = None
+    if "view_mask" in host:
+        n_views = (np.bitwise_count(host["view_mask"][a:b].view(np.uint32)) + 1).astype(np.uint8)
     return _TriangulatedReference(xyz=host["xyz"][a:b], rgb=host["rgb"][a:b], err=host["err"][a:b],
-                                  debug_matches_by_nbr=dbg_m, debug_cert_by_nbr=dbg_c, ply_records=rec)
+                                  debug_matches_by_nbr=dbg_m, debug_cert_by_nbr=dbg_c, ply_records=rec, n_views=n_views)
 
 
 def _download(out: DensifyOutputs, collect_debug: bool, ply_records: bool = False) -> dict:
@@ -273,6 +278,8 @@ def _download(out: DensifyOutputs, collect_debug: bool, ply_records: bool = Fals
     if collect_debug:
         meta["dbg_matches"] = arr("dbg_matches", np.float32, (cap, 4))[:total]
         meta["dbg_cert"] = arr("dbg_cert", np.float32, (cap,))[:total]
+    if "view_mask" in L:
+        meta["view_mask"] = arr("view_mask", np.int32, (cap,))[:total]
     if rec is not None:
         meta["ply"] = rec[:15 * total].cpu().numpy()
     return meta
@@ -595,7 +602,7 @@ def run_dense_pipeline(
                                     w_match=int(w_match), h_match=int(h_match))
     t0 = time.time()
     step = int(getattr(config, "refs_per_launch", 32)) or max(1, len(refs_local))
-    parts_xyz, parts_rgb, parts_err = [], [], []
+    parts_xyz, parts_rgb, parts_err, parts_nv = [], [], [], []
     pairs = 0
     pair_counter = 0
     # live update (core/pipeline.py:296-306,508-532): every viz_interval views the reference re-concatenates and re-packs
@@ -620,6 +627,8 @@ def run_dense_pipeline(
             parts_xyz.append(tri.xyz)
             parts_rgb.append(tri.rgb)
             parts_err.append(tri.err)
+            if tri.n_views is not None:
+                parts_nv.append(tri.n_views)
             pairs += 1
             if tri.debug_matches_by_nbr and debug_state is not None:
                 _emit_debug_previews(mr, tri, debug_state, cameras, total_pairs_est, pair_counter, cancel_requested)
@@ -684,4 +693,5 @@ def run_dense_pipeline(
         raise RuntimeError("No points triangulated. Try adjusting parameters.")
     return PipelineResult(xyz=np.concatenate(parts_xyz, axis=0), rgb=np.concatenate(parts_rgb, axis=0),
                           err=np.concatenate(parts_err, axis=0), elapsed_seconds=time.time() - t0,
-                          pairs_processed=pairs)
+                          pairs_processed=pairs,
+                          n_views=np.concatenate(parts_nv, axis=0) if getattr(config, "multiview", False) else None)

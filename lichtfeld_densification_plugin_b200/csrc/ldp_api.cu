@@ -6,6 +6,7 @@
 #include <cstring>
 #include <string>
 #include <utility>
+#include <vector>
 
 #include "ldp_sample.cu"
 #include "ldp_front.cu"
@@ -89,6 +90,7 @@ int cuda_fail(cudaError_t e, const char* where) {
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 int g_force_cluster = 0;      // test hook (ldp_debug_set_cluster)
+int g_force_fix_two = 0, g_force_fix_mv = 0;   // test hook (ldp_debug_force_fixup)
 int g_sm_reserve = 0;         // ldp_set_sm_reserve
 int g_last_cluster = 0;
 
@@ -284,6 +286,9 @@ int make_plan(const ldp_params* p, void* base, Plan* plan) {
     w.blk_first = reinterpret_cast<int32_t*>(carve(R * plan->nb2 * LDP_MAX_NN * sizeof(int32_t)));
     w.fix_list = reinterpret_cast<int2*>(carve(R * w.sel_cap * sizeof(int2)));
     w.dstat = reinterpret_cast<int32_t*>(carve(R * sizeof(int32_t)));
+    const size_t mv_slots = p->multiview ? R * w.sel_cap : 0;
+    w.vmask = reinterpret_cast<int32_t*>(carve(mv_slots * sizeof(int32_t)));
+    w.mvrec = reinterpret_cast<float4*>(carve(mv_slots * sizeof(float4)));
     // ---- the zero block (one memset per call, clear_launch_state): 8-byte items first
     {
         const size_t z0 = off;
@@ -316,6 +321,10 @@ int check_outputs(const ldp_params* p, const ldp_outputs* o) {
     if (p->collect_debug && (!o->dbg_matches || !o->dbg_cert))
         return fail(LDP_ERR_INVALID, "collect_debug needs dbg_matches and dbg_cert");
     if (o->capacity < 0) return fail(LDP_ERR_INVALID, "negative capacity");
+    if (o->view_mask && !p->multiview) return fail(LDP_ERR_INVALID, "view_mask is written by multiview launches only");
+    if (p->multiview && p->no_filter) return fail(LDP_ERR_INVALID, "multiview needs the filters (no_filter = 0)");
+    if (p->multiview && !(p->multiview_min_cert > 0.0f && p->multiview_min_cert <= 1.0f))
+        return fail(LDP_ERR_INVALID, "multiview_min_cert must lie in (0, 1]");
     return LDP_OK;
 }
 
@@ -583,9 +592,11 @@ ldp::GeomArgs make_geom_args(const ldp_params* p, const Plan& plan, int have_bes
     static const int discard_mode = [] { const char* e = getenv("LDP_DISCARD"); return e ? atoi(e) : 1; }();
     ga.discard = have_bestk ? discard_mode : 0;
     static const int fuse_mode = [] { const char* e = getenv("LDP_FUSE_GATHER"); return e ? atoi(e) : 1; }();
-    ga.fused = fuse_mode;
+    ga.fused = p->multiview ? 1 : fuse_mode;      // the refinement reads the sample index: a multiview launch always gathers itself
     static const int prefetch_mode = [] { const char* e = getenv("LDP_GEOM_PREFETCH"); return e ? atoi(e) : 1; }();
     ga.l2_prefetch = prefetch_mode;
+    ga.force_fix_two = g_force_fix_two;
+    ga.force_fix_mv = g_force_fix_mv;
     return ga;
 }
 
@@ -603,13 +614,15 @@ int launch_geometry(const ldp_params* p, const ldp_ref_desc* refs, const ldp_out
         if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_gather_kernel");
     }
     { KernelTimer kt(st, "ldp_geometry_kernel");
-      if (p->lens) (void)launch_k(ldp::ldp_geometry_kernel<true>, dim3(grid), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga);
-      else (void)launch_k(ldp::ldp_geometry_kernel<false>, dim3(grid), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
+      auto* k2 = p->multiview ? (p->lens ? ldp::ldp_geometry_kernel<true, true> : ldp::ldp_geometry_kernel<false, true>)
+                              : (p->lens ? ldp::ldp_geometry_kernel<true, false> : ldp::ldp_geometry_kernel<false, false>);
+      (void)launch_k(k2, dim3(grid), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
     ++g_launches;
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_geometry_kernel");
     { KernelTimer kt(st, "ldp_fix_kernel");
-      if (p->lens) (void)launch_k(ldp::ldp_fix_kernel<true>, dim3(nsubrefs), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga);
-      else (void)launch_k(ldp::ldp_fix_kernel<false>, dim3(nsubrefs), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
+      auto* kf = p->multiview ? (p->lens ? ldp::ldp_fix_kernel<true, true> : ldp::ldp_fix_kernel<false, true>)
+                              : (p->lens ? ldp::ldp_fix_kernel<true, false> : ldp::ldp_fix_kernel<false, false>);
+      (void)launch_k(kf, dim3(nsubrefs), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
     ++g_launches;
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_fix_kernel");
     return LDP_OK;
@@ -728,6 +741,37 @@ int ldp_debug_read_clocks(const ldp_params* params, void* workspace, long long* 
     if (rc != LDP_OK) return rc;
     cudaError_t e = cudaMemcpy(host_out, plan.ws.dbgclk, (size_t)params->n_refs * 32 * sizeof(long long), cudaMemcpyDeviceToHost);
     if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpy(dbgclk)");
+    return LDP_OK;
+}
+
+int ldp_debug_force_fixup(int two_view_every, int multiview_every) {
+    if (two_view_every < 0 || multiview_every < 0) return fail(LDP_ERR_INVALID, "force_fixup periods must be >= 0");
+    g_force_fix_two = two_view_every;
+    g_force_fix_mv = multiview_every;
+    return LDP_OK;
+}
+
+int ldp_debug_read_fixups(const ldp_params* params, void* workspace, int32_t* host_out) {
+    if (!params || !workspace || !host_out) return fail(LDP_ERR_INVALID, "bad arguments");
+    Plan plan;
+    char* base = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace), 256));
+    int rc = make_plan(params, base, &plan);
+    if (rc != LDP_OK) return rc;
+    host_out[0] = host_out[1] = 0;
+    int32_t counts[ldp::LDP_MAX_SUB];
+    cudaError_t e = cudaMemcpy(counts, plan.ws.fix_count, sizeof(counts), cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpy(fix_count)");
+    const int nsub = choose_subbatches(params->n_refs);
+    std::vector<int2> list;
+    for (int h = 0; h < nsub; ++h) {           // sub-batch h's worklist starts at its first view * sel_cap (launch_geometry)
+        const int lo = (int)(((long long)h * params->n_refs) / nsub);
+        if (counts[h] <= 0) continue;
+        list.resize((size_t)counts[h]);
+        e = cudaMemcpy(list.data(), plan.ws.fix_list + (size_t)lo * plan.ws.sel_cap, list.size() * sizeof(int2), cudaMemcpyDeviceToHost);
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpy(fix_list)");
+        host_out[0] += counts[h];
+        for (const int2& it : list) host_out[1] += (it.y & ldp::MV_FIX) ? 1 : 0;
+    }
     return LDP_OK;
 }
 

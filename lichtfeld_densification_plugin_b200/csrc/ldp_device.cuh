@@ -53,6 +53,10 @@ struct Workspace {
     int32_t* dstat;      // [R] verdict of the first draw round for the rounds that follow: fail code | inexact << 8
     long long* dbgclk;   // [R][32] phase timestamps of the draw kernel (written only with -DLDP_PHASE_CLOCKS)
     size_t n_pad, n_words, found_cap, sel_cap, topk_cap, nchunk_pad, nblk, bins_cap, draw_cmax;
+    // multiview launches only (NULL otherwise)
+    int32_t* vmask;      // [R][sel_cap]  neighbour slots that contributed to the kept sample's point (geometry / fix -> pack)
+    float4* mvrec;       // [R][sel_cap] winner's warp row of a kept sample whose multi-view solve did not converge (its
+                         //   winner slot waits in vmask, its two-view result in pt0 / pt1 for the fix-up to fall back to)
 };
 
 struct SampleGeom {     // launch-constant shape of the sampler

@@ -72,6 +72,9 @@ struct GeomArgs {           // launch-constant extras computed on the host
     int discard;            // 1: drop the dead weight rows from L2 (LDP_DISCARD=0 turns it off)
     int l2_prefetch;        // 1: bulk L2 prefetch of the view's reference image and winner row (LDP_GEOM_PREFETCH=0 turns it off)
     int fused;              // 1: the geometry kernel gathers its own inputs (no gather kernel, no record round trip)
+    // test hook, read by the multiview instantiations only (ldp_debug_force_fixup): n > 0 sends every sample i with i % n == 0
+    // to the fix-up as if its two-view solve (force_fix_two) / its multi-view solve (force_fix_mv) had not converged
+    int force_fix_two, force_fix_mv;
 };
 
 // The workspace rows are dead once their last consumer ran; telling L2 so spares the write-back of lines
@@ -216,16 +219,16 @@ __device__ __forceinline__ double rcp_newton(double v) {
 // (sigma_4/sigma_3)^2 per step: 3-5 steps on consistent matches); returns false if not converged in INVIT_MAX.
 // ROBUST = true : Jacobi.
 constexpr int INVIT_MAX = 24;     // slow convergers are rare; iterating on is far cheaper than the Jacobi fix-up
+struct Gram { double m00, m10, m11, m20, m21, m22, m30, m31, m32, m33; };       // lower triangle of A^T A
+__device__ __forceinline__ void gram_add_row(Gram& g, double a, double b, double c, double d) {
+    g.m00 = fma(a, a, g.m00); g.m10 = fma(b, a, g.m10); g.m11 = fma(b, b, g.m11);
+    g.m20 = fma(c, a, g.m20); g.m21 = fma(c, b, g.m21); g.m22 = fma(c, c, g.m22);
+    g.m30 = fma(d, a, g.m30); g.m31 = fma(d, b, g.m31); g.m32 = fma(d, c, g.m32); g.m33 = fma(d, d, g.m33);
+}
 template <bool ROBUST>
-__device__ __forceinline__ bool null_vector4(const double A[16], double v[4]) {
-    double m00 = 0, m10 = 0, m11 = 0, m20 = 0, m21 = 0, m22 = 0, m30 = 0, m31 = 0, m32 = 0, m33 = 0;
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-        const double a = A[4 * r], b = A[4 * r + 1], c = A[4 * r + 2], d = A[4 * r + 3];
-        m00 = fma(a, a, m00); m10 = fma(b, a, m10); m11 = fma(b, b, m11);
-        m20 = fma(c, a, m20); m21 = fma(c, b, m21); m22 = fma(c, c, m22);
-        m30 = fma(d, a, m30); m31 = fma(d, b, m31); m32 = fma(d, c, m32); m33 = fma(d, d, m33);
-    }
+__device__ __forceinline__ bool null_vector_gram(const Gram& g, double v[4]) {
+    const double m00 = g.m00, m10 = g.m10, m11 = g.m11, m20 = g.m20, m21 = g.m21, m22 = g.m22;
+    const double m30 = g.m30, m31 = g.m31, m32 = g.m32, m33 = g.m33;
     const double tr = m00 + m11 + m22 + m33;
     if (!(tr > 0.0) || !isfinite(tr)) { v[0] = v[1] = v[2] = 0.0; v[3] = 1.0; if (!(tr == tr)) v[0] = tr; return true; }
     if (ROBUST) {
@@ -283,6 +286,13 @@ __device__ __forceinline__ bool null_vector4(const double A[16], double v[4]) {
     }
     v[0] = x0; v[1] = x1; v[2] = x2; v[3] = x3;
     return converged;
+}
+template <bool ROBUST>
+__device__ __forceinline__ bool null_vector4(const double A[16], double v[4]) {
+    Gram g = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+#pragma unroll
+    for (int r = 0; r < 4; ++r) gram_add_row(g, A[4 * r], A[4 * r + 1], A[4 * r + 2], A[4 * r + 3]);
+    return null_vector_gram<ROBUST>(g, v);
 }
 
 // X @ P^T row: the reference's sgemm accumulates the K=4 products with FMAs in index order
@@ -422,6 +432,55 @@ __device__ __forceinline__ float lens_reproj_err(const ldp_lens& L, const float*
     lens_distort(L, ((double)q0 / z - cx) / fx, ((double)q1 / z - cy) / fy, xd, yd);
     const double du = fx * xd + cx - (double)u, dv = fy * yd + cy - (double)v;
     return (float)sqrt(du * du + dv * dv);
+}
+
+// The Sampson gate, the dehomogenisation and the parallax test for the multi-view refinement (mv_refine): the same
+// arithmetic as eval_sample's inline copies, which stay inline because factoring them out changes the two-view kernels'
+// register allocation and spills (DESIGN.md 4.4).
+// Sampson gate in f64: core/geometry.py:133-141, core/pipeline.py:708-727.  se < thr is decided on num^2 vs thr*den outside
+// a 2^-50 band, by the reference's quotient inside it.
+__device__ __forceinline__ int sampson_pass(const float* F, double a0, double a1, double b0, double b1, double thr) {
+    const double l0 = (double)F[0] * a0 + (double)F[1] * a1 + (double)F[2];
+    const double l1 = (double)F[3] * a0 + (double)F[4] * a1 + (double)F[5];
+    const double l2 = (double)F[6] * a0 + (double)F[7] * a1 + (double)F[8];
+    const double m0 = (double)F[0] * b0 + (double)F[3] * b1 + (double)F[6];
+    const double m1 = (double)F[1] * b0 + (double)F[4] * b1 + (double)F[7];
+    const double num = b0 * l0 + b1 * l1 + l2;
+    const double den = l0 * l0 + l1 * l1 + m0 * m0 + m1 * m1 + 1e-12;
+    const double n2 = num * num, td = thr * den;
+    int good;
+    if (n2 < td * (1.0 - 1.0 / 1125899906842624.0)) good = 1;
+    else if (n2 > td * (1.0 + 1.0 / 1125899906842624.0)) good = 0;
+    else good = (__ddiv_rn(n2, den) < thr) ? 1 : 0;
+    if (!(n2 == n2) || !(den == den)) good = 0;                                  // NaN: comparison is False in numpy
+    return good;
+}
+
+// core/geometry.py:85-87: w = where(|Xh3| < 1e-12, 1e-12, Xh3); X = Xh / w
+__device__ __forceinline__ void dehomogenise(const double v[4], float& X0, float& X1, float& X2, float& X3) {
+    const float w32 = (float)v[3];
+    if (fabsf(w32) < 1e-12f) {
+        X0 = __fdiv_rn((float)v[0], 1e-12f); X1 = __fdiv_rn((float)v[1], 1e-12f);
+        X2 = __fdiv_rn((float)v[2], 1e-12f); X3 = __fdiv_rn(w32, 1e-12f);
+    } else {
+        const double iwv = rcp_newton(v[3]);
+        X0 = (float)(v[0] * iwv); X1 = (float)(v[1] * iwv); X2 = (float)(v[2] * iwv); X3 = 1.0f;
+    }
+}
+
+// parallax filter, core/geometry.py:113-119
+__device__ __forceinline__ bool parallax_pass(float X0, float X1, float X2, const float* C1, const float* C2, float par_cos_max) {
+    float a0 = __fsub_rn(X0, C1[0]), a1 = __fsub_rn(X1, C1[1]), a2 = __fsub_rn(X2, C1[2]);
+    float b0 = __fsub_rn(X0, C2[0]), b1 = __fsub_rn(X1, C2[1]), b2 = __fsub_rn(X2, C2[2]);
+    const float na = __fadd_rn(__fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(a0, a0), __fmul_rn(a1, a1)), __fmul_rn(a2, a2))), 1e-12f);
+    const float nb = __fadd_rn(__fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(b0, b0), __fmul_rn(b1, b1)), __fmul_rn(b2, b2))), 1e-12f);
+    a0 = __fdiv_rn(a0, na); a1 = __fdiv_rn(a1, na); a2 = __fdiv_rn(a2, na);
+    b0 = __fdiv_rn(b0, nb); b1 = __fdiv_rn(b1, nb); b2 = __fdiv_rn(b2, nb);
+    float d = __fadd_rn(__fadd_rn(__fmul_rn(a0, b0), __fmul_rn(a1, b1)), __fmul_rn(a2, b2));
+    const bool dnan = (d != d);
+    d = fminf(fmaxf(d, -1.0f), 1.0f);
+    // degrees(arccos(d)) >= min_deg  <=>  d <= par_cos_max (arccos is monotone; threshold found on the host)
+    return !dnan && d <= par_cos_max;
 }
 
 struct SampleResult {
@@ -672,6 +731,131 @@ __device__ __forceinline__ void store_sample(const ldp_params& P, const Workspac
     if (out.sample_xyzerr) reinterpret_cast<float4*>(out.sample_xyzerr)[o] = make_float4(s.X0, s.X1, s.X2, s.err);
 }
 
+// ---- multi-view refinement (ldp_params.multiview; the semantics are stated in include/ldp_b200.h).  Not in the reference.
+// It runs for a KEPT sample only, after its two-view verdict: the candidates' certainty words and warp rows are gathered
+// then, so a launch pays for them at the kept samples alone and the plain path's load chain is untouched.  The candidate
+// set lives in a bit mask; a candidate's pixel is re-decoded (its 8-byte warp half reloaded, from L1) in each pass
+// instead of being kept in registers.
+constexpr int MV_FIX = 1 << 30;     // fix_list entry: only the multi-view solve of a kept sample is to be redone
+
+struct MvPix { float u_obs, v_obs, u, v; };      // observed pixel, ideal pinhole pixel
+
+// neighbour q's pixel at map pixel idx (the xB, yB half of its warp row), decoded like eval_sample decodes the winner's
+template <bool LENS>
+__device__ __forceinline__ MvPix mv_pixel(const ldp_params& P, const PairTable& pc, const ldp_lens* lt, int q, int idx) {
+    const float2 w = __ldg(reinterpret_cast<const float2*>(pc.warp[q] + (size_t)idx * 4 + 2));
+    const float xB = __fmul_rn(__fmul_rn(__fadd_rn(w.x, 1.0f), 0.5f), (float)(P.w_match - 1));
+    const float yB = __fmul_rn(__fmul_rn(__fadd_rn(w.y, 1.0f), 0.5f), (float)(P.h_match - 1));
+    MvPix b;
+    b.u_obs = __fmul_rn(xB, pc.sxB[q]); b.v_obs = __fmul_rn(yB, pc.syB[q]);
+    b.u = b.u_obs; b.v = b.v_obs;
+    if constexpr (LENS) {
+        if (lt[1 + q].model != LDP_LENS_PINHOLE) lens_undistort_px(lt[1 + q], b.u_obs, b.v_obs, b.u, b.v);
+    }
+    return b;
+}
+
+// the two DLT rows of camera Pm at ideal pixel (u, v), f32 like the two-view rows, into the Gram matrix
+__device__ __forceinline__ void gram_add_view(Gram& g, const float* Pm, float u, float v) {
+    double ru[4], rv[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        ru[j] = (double)__fsub_rn(__fmul_rn(u, Pm[8 + j]), Pm[j]);
+        rv[j] = (double)__fsub_rn(__fmul_rn(v, Pm[8 + j]), Pm[4 + j]);
+    }
+    gram_add_row(g, ru[0], ru[1], ru[2], ru[3]);
+    gram_add_row(g, rv[0], rv[1], rv[2], rv[3]);
+}
+
+// reprojection error of one view (lens-aware like eval_sample's) and its depth
+template <bool LENS>
+__device__ __forceinline__ float mv_view_err(const ldp_lens* L, const float* Pm, float X0, float X1, float X2, float X3,
+                                             const MvPix& b, float* z) {
+    if constexpr (LENS) {
+        if (L->model != LDP_LENS_PINHOLE) return lens_reproj_err(*L, Pm, X0, X1, X2, X3, b.u_obs, b.v_obs, z);
+    }
+    return reproj_err(Pm, X0, X1, X2, X3, b.u, b.v, z);
+}
+
+// Refines the kept two-view point (X, err) of the sample at map pixel idx, winner k, winner warp row wv.  On return X / err
+// hold the point to emit and mask its view mask.  ROBUST = false: returns false if a solve did not converge (nothing is
+// changed; the fix-up repeats the refinement with ROBUST = true, which always converges).
+template <bool ROBUST, bool LENS>
+__device__ bool mv_refine(const ldp_params& P, const RefConst& rc, const PairTable& pc, const ProView& pv, const GeomArgs& ga,
+                          const ldp_lens* lt, int idx, int k, float4 wv, float& X0, float& X1, float& X2, float& err, int& mask) {
+    mask = 1 << k;
+    const float wm1 = (float)(P.w_match - 1), hm1 = (float)(P.h_match - 1);
+    MvPix a, bk;
+    {
+        const float xA = __fmul_rn(__fmul_rn(__fadd_rn(wv.x, 1.0f), 0.5f), wm1);
+        const float yA = __fmul_rn(__fmul_rn(__fadd_rn(wv.y, 1.0f), 0.5f), hm1);
+        const float xB = __fmul_rn(__fmul_rn(__fadd_rn(wv.z, 1.0f), 0.5f), wm1);
+        const float yB = __fmul_rn(__fmul_rn(__fadd_rn(wv.w, 1.0f), 0.5f), hm1);
+        a.u_obs = __fmul_rn(xA, rc.sxA); a.v_obs = __fmul_rn(yA, rc.syA);
+        bk.u_obs = __fmul_rn(xB, pc.sxB[k]); bk.v_obs = __fmul_rn(yB, pc.syB[k]);
+        a.u = a.u_obs; a.v = a.v_obs; bk.u = bk.u_obs; bk.v = bk.v_obs;
+        if constexpr (LENS) {
+            if (lt[0].model != LDP_LENS_PINHOLE) lens_undistort_px(lt[0], a.u_obs, a.v_obs, a.u, a.v);
+            if (lt[1 + k].model != LDP_LENS_PINHOLE) lens_undistort_px(lt[1 + k], bk.u_obs, bk.v_obs, bk.u, bk.v);
+        }
+    }
+    // ---- candidates: one slot per neighbour uid, not the winner's, confident, finite, through the Sampson gate
+    const int gk = pc.group[k];
+    unsigned cand = 0;
+    Gram g = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    gram_add_view(g, rc.P1, a.u, a.v);
+    gram_add_view(g, pc.P2[k], bk.u, bk.v);
+    const Gram g2v = g;
+    for (int q = 0; q < rc.nn; ++q) {
+        if (pc.group[q] != q || q == gk) continue;             // (also excludes k: group[k] == k means q == gk)
+        if (!(cert_at(P, pc, pv, q, idx) >= P.multiview_min_cert)) continue;
+        const MvPix b = mv_pixel<LENS>(P, pc, lt, q, idx);
+        if (!isfinite(b.u) || !isfinite(b.v)) continue;
+        if (P.sampson_thresh > 0.0 && !sampson_pass(pc.F[q], a.u, a.v, b.u, b.v, P.sampson_thresh)) continue;
+        cand |= 1u << q;
+        gram_add_view(g, pc.P2[q], b.u, b.v);
+    }
+    if (!cand) return true;
+    // ---- solve, trim once, solve again if something was dropped
+    double v[4];
+    if (!null_vector_gram<ROBUST>(g, v)) return false;
+    float Y0, Y1, Y2, Y3;
+    dehomogenise(v, Y0, Y1, Y2, Y3);
+    const float thr = P.reproj_thresh;
+    unsigned used = cand;
+    g = g2v;
+    for (unsigned m = cand; m; m &= m - 1) {
+        const int q = __ffs(m) - 1;
+        const MvPix b = mv_pixel<LENS>(P, pc, lt, q, idx);
+        float z;
+        const float e = mv_view_err<LENS>(lt + 1 + q, pc.P2[q], Y0, Y1, Y2, Y3, b, &z);
+        if (!(e <= thr) || !(z > 0.0f)) used &= ~(1u << q);
+        else gram_add_view(g, pc.P2[q], b.u, b.v);
+    }
+    if (!used) return true;                                    // nothing left beside the winner: the two-view point stands
+    if (used != cand) {
+        if (!null_vector_gram<ROBUST>(g, v)) return false;
+        dehomogenise(v, Y0, Y1, Y2, Y3);
+    }
+    // ---- accept: every included view within the threshold and in front, the reference-winner parallax still met
+    float zA, zB;
+    const float eA = mv_view_err<LENS>(lt, rc.P1, Y0, Y1, Y2, Y3, a, &zA);
+    const float eB = mv_view_err<LENS>(lt + 1 + k, pc.P2[k], Y0, Y1, Y2, Y3, bk, &zB);
+    bool ok = eA <= thr && zA > 0.0f && eB <= thr && zB > 0.0f;
+    float emax = fmaxf(eA, eB);
+    for (unsigned m = used; m && ok; m &= m - 1) {
+        const int q = __ffs(m) - 1;
+        const MvPix b = mv_pixel<LENS>(P, pc, lt, q, idx);
+        float z;
+        const float e = mv_view_err<LENS>(lt + 1 + q, pc.P2[q], Y0, Y1, Y2, Y3, b, &z);
+        ok = e <= thr && z > 0.0f;
+        emax = fmaxf(emax, e);
+    }
+    if (ok && P.min_parallax_deg > 0.0f) ok = parallax_pass(Y0, Y1, Y2, rc.C1, pc.C2[k], ga.par_cos_max);
+    if (ok) { X0 = Y0; X1 = Y1; X2 = Y2; err = emax; mask |= (int)used; }
+    return true;
+}
+
 // K2a gather: one thread per sample, few registers, full occupancy: the dependent chain of scattered loads
 // (sample index -> winning neighbour -> warp row -> texels) is what bounds this stage, so it runs with as many
 // threads in flight as the SM holds and leaves a 32-byte record per sample for the arithmetic kernel.
@@ -757,7 +941,8 @@ __device__ __forceinline__ void lens_store(const StagedLens& sl, ldp_lens* dst, 
 }
 
 // K2b compute: coalesced record in, per-sample result (in place) + per-tile group statistics out.
-template <bool LENS>
+// MV: multiview launch (always fused): a kept sample's point is refined from its other confident neighbours (mv_refine).
+template <bool LENS, bool MV>
 __global__ void __launch_bounds__(K2_THREADS, K2_MIN_BLOCKS)
 ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const Workspace ws, const ldp_outputs out,
                     const GeomArgs ga)
@@ -818,6 +1003,9 @@ ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, c
         GCLK_USE(rec.tex[0]); GCLK_USE(rec.tex[2]); GCLK_USE(rec.wv.x); GCLK(2);
         SampleResult s;
         eval_sample<false, LENS>(P, rc, pc, ga, lt, rec, craw, s GCLK_PASS);
+        if constexpr (MV) {
+            if (ga.force_fix_two > 0 && i % ga.force_fix_two == 0) s.converged = false;
+        }
         if (!s.converged && ga.fused) {     // the fix-up reads the record
             ws.pt0[o] = rec.wv;
             ws.pt1[o] = make_float4(__uint_as_float(rec.tex[0]), __uint_as_float(rec.tex[1]), __uint_as_float(rec.tex[2]),
@@ -831,6 +1019,23 @@ ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, c
             s.keep = 0;
         } else {
             store_sample(P, ws, out, o, s);
+            if constexpr (MV) {
+                if (s.keep) {               // the verdict is final; only the point moves
+                    float X0 = s.X0, X1 = s.X1, X2 = s.X2, err = s.err;
+                    int mask;
+                    const int k = (int)(rec.k_cert & 0xffu);
+                    const bool conv = mv_refine<false, LENS>(P, rc, pc, pv, ga, lt, idx_f, k, rec.wv, X0, X1, X2, err, mask);
+                    if (conv && !(ga.force_fix_mv > 0 && i % ga.force_fix_mv == 0)) {
+                        ws.pt0[o] = make_float4(X0, X1, X2, err);
+                        ws.vmask[o] = mask;
+                    } else {                // rare: the fix-up redoes the multi-view solve from the winner's warp row and slot
+                        ws.mvrec[o] = rec.wv;           //   (vmask holds the slot until then); pt0 is the fallback
+                        ws.vmask[o] = k;
+                        const int slot = atomicAdd(ws.fix_count + ga.sub, 1);
+                        ws.fix_list[(size_t)ga.ref0 * ws.sel_cap + slot] = make_int2(r, i | MV_FIX);
+                    }
+                }
+            }
         }
         keep = s.keep;
         grp = s.grp;
@@ -861,7 +1066,7 @@ ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, c
 // output plan, once for all of its pack CTAs: kept points per neighbour group, groups in order of first appearance
 // (reference core/pipeline.py:685-695), and for every 128-sample tile and group the row (relative to the view's first row)
 // at which that tile's kept samples of that group start.
-template <bool LENS>
+template <bool LENS, bool MV>
 __global__ void __launch_bounds__(K2_THREADS)
 ldp_fix_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const Workspace ws, const ldp_outputs out,
                const GeomArgs ga)
@@ -885,12 +1090,29 @@ ldp_fix_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const 
             lens_store(sl, s_lens, tid);
             lt = s_lens;
         }
+        const ProView* pv = nullptr;
+        if constexpr (MV) {
+            __shared__ ProView s_pv;
+            if (P.prologue) stage_proview(refs + r, s_pv, tid);
+            pv = &s_pv;
+        }
         __syncthreads();
         for (int e = tid; e < n; e += K2_THREADS) {
             const int2 it = fix_list[e];
             if (it.x != r) continue;
-            const int i = it.y;
+            const int i = MV ? (it.y & ~MV_FIX) : it.y;
             const size_t o = (size_t)r * ws.sel_cap + i;
+            int idx = 0;
+            if constexpr (MV) idx = ((out.sel_idx ? out.sel_idx : ws.sel) + (size_t)r * ws.sel_cap)[i];
+            if (MV && (it.y & MV_FIX)) {    // kept, two-view result final (pt0): redo the multi-view solve alone
+                const float4 x = ws.pt0[o];
+                float X0 = x.x, X1 = x.y, X2 = x.z, err = x.w;
+                int mask;
+                mv_refine<true, LENS>(P, rc, pc, *pv, ga, lt, idx, ws.vmask[o], ws.mvrec[o], X0, X1, X2, err, mask);
+                ws.pt0[o] = make_float4(X0, X1, X2, err);
+                ws.vmask[o] = mask;
+                continue;
+            }
             SampleRec rec;
             float craw;
             load_record(ws, P, o, rec, craw);
@@ -898,6 +1120,15 @@ ldp_fix_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const 
             GCLK_DECL
             eval_sample<true, LENS>(P, rc, pc, ga, lt, rec, craw, s GCLK_PASS);
             store_sample(P, ws, out, o, s);
+            if constexpr (MV) {
+                if (s.keep) {
+                    float X0 = s.X0, X1 = s.X1, X2 = s.X2, err = s.err;
+                    int mask;
+                    mv_refine<true, LENS>(P, rc, pc, *pv, ga, lt, idx, (int)(rec.k_cert & 0xffu), rec.wv, X0, X1, X2, err, mask);
+                    ws.pt0[o] = make_float4(X0, X1, X2, err);
+                    ws.vmask[o] = mask;
+                }
+            }
             if (s.keep) {
                 atomicAdd(&ws.kept[r], 1);
                 atomicAdd(&ws.blk_cnt[((size_t)r * ga.nb2 + i / K2_THREADS) * LDP_MAX_NN + s.grp], 1);
@@ -1011,6 +1242,9 @@ ldp_pack_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const
     float4 pa = make_float4(0.f, 0.f, 0.f, 0.f), pc4 = pa, pd = pa;
     if (in_row) { pa = __ldcg(ws.pt0 + o); pc4 = __ldcg(ws.pt1 + o); }
     if (in_row && P.collect_debug && out.dbg_matches) pd = __ldcg(ws.dbgm + o);
+    const bool mv_out = P.multiview && out.view_mask;
+    int vm = 0;
+    if (in_row && mv_out) vm = __ldcg(ws.vmask + o);
     int start_g = 0;
     if (tid < LDP_MAX_NN) start_g = __ldcg(ws.blk_first + ((size_t)r * ga.nb2 + b) * LDP_MAX_NN + tid);
     long long partk = 0;
@@ -1049,6 +1283,7 @@ ldp_pack_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const
             out.xyz[dst * 3 + 0] = pa.x; out.xyz[dst * 3 + 1] = pa.y; out.xyz[dst * 3 + 2] = pa.z;
             out.rgb[dst * 3 + 0] = pc4.x; out.rgb[dst * 3 + 1] = pc4.y; out.rgb[dst * 3 + 2] = pc4.z;
             out.err[dst] = pa.w;
+            if (mv_out) out.view_mask[dst] = vm;
             if (P.collect_debug && out.dbg_matches) {
                 reinterpret_cast<float4*>(out.dbg_matches)[dst] = pd;
                 if (out.dbg_cert) out.dbg_cert[dst] = pc4.w;

@@ -71,12 +71,26 @@ class PathConfig:
     # A float: the planes are RAW matcher outputs and the kernels apply clamp(min=certainty_floor) and the masks
     # registered with RefBatch.add on the fly (reference core/pipeline.py:405-430, config.certainty_thresh).
     certainty_floor: Optional[float] = None
+    # Multi-view refinement (include/ldp_b200.h): a kept point is re-triangulated from every other neighbour whose certainty at
+    # the pixel is >= multiview_min_certainty and whose match agrees; which points are kept does not change.
+    multiview: bool = False
+    multiview_min_certainty: float = 0.5
 
     @classmethod
     def from_pipeline_config(cls, cfg, sample_cap: float = SAMPLE_CAP_DEFAULT) -> "PathConfig":
         return cls(matches_per_ref=int(cfg.matches_per_ref), reproj_thresh=float(cfg.reproj_thresh),
                    sampson_thresh=float(cfg.sampson_thresh), min_parallax_deg=float(cfg.min_parallax_deg),
-                   no_filter=bool(cfg.no_filter), sample_cap=float(sample_cap), seed=int(getattr(cfg, "seed", 0)))
+                   no_filter=bool(cfg.no_filter), sample_cap=float(sample_cap), seed=int(getattr(cfg, "seed", 0)),
+                   multiview=bool(getattr(cfg, "multiview", False)),
+                   multiview_min_certainty=float(getattr(cfg, "multiview_min_certainty", 0.5)))
+
+    def check_multiview(self) -> None:
+        if not self.multiview:
+            return
+        if self.no_filter:
+            raise ValueError("multiview needs the filters: it cannot be combined with no_filter")
+        if not 0.0 < float(self.multiview_min_certainty) <= 1.0:
+            raise ValueError("multiview_min_certainty must lie in (0, 1]")
 
 
 class PairConstantCache:
@@ -296,6 +310,7 @@ class DensifyOutputs:
     weight_sum: torch.Tensor
     dbg_matches: Optional[torch.Tensor] = None
     dbg_cert: Optional[torch.Tensor] = None
+    view_mask: Optional[torch.Tensor] = None   # int32 [capacity], multiview launches: neighbour slots behind each point
     sel_idx: Optional[torch.Tensor] = None
     sample_flags: Optional[torch.Tensor] = None
     sample_xyzerr: Optional[torch.Tensor] = None
@@ -344,6 +359,9 @@ class DensifyEngine:
         p.certainty_floor = float(np.float32(cfg.certainty_floor if cfg.certainty_floor is not None else 0.0))
         p.no_warped_masks = 0 if batch.has_warped_masks else 1
         p.lens = 1 if batch.has_lens else 0
+        cfg.check_multiview()
+        p.multiview = 1 if cfg.multiview else 0
+        p.multiview_min_cert = float(np.float32(cfg.multiview_min_certainty))
         p.sm_reserve = int(self.sm_reserve)
         p.seed = int(cfg.seed) & 0xFFFFFFFFFFFFFFFF
         p.uniforms_per_ref = int(uniforms_per_ref)
@@ -384,7 +402,9 @@ class DensifyEngine:
         params = self._params(batch, cfg, collect_debug, rng_mode, upr)
         ws = self._ensure_workspace(params)
         sel_cap = self.sel_capacity(cfg.matches_per_ref)
-        out = outputs if outputs is not None else self.alloc_outputs(R, sel_cap, collect_debug, taps)
+        out = outputs if outputs is not None else self.alloc_outputs(R, sel_cap, collect_debug, taps, multiview=cfg.multiview)
+        if cfg.multiview and out.view_mask is None:
+            raise ValueError("a multiview launch needs outputs allocated with multiview=True")
         if descs_dev is None:
             descs_dev = self.upload_descs(batch)
         o = N.LdpOutputs()
@@ -395,6 +415,8 @@ class DensifyEngine:
         o.uniforms_used, o.rounds, o.weight_sum = out.uniforms_used.data_ptr(), out.rounds.data_ptr(), out.weight_sum.data_ptr()
         if out.dbg_matches is not None:
             o.dbg_matches, o.dbg_cert = out.dbg_matches.data_ptr(), out.dbg_cert.data_ptr()
+        if cfg.multiview:
+            o.view_mask = out.view_mask.data_ptr()
         if out.sel_idx is not None:
             o.sel_idx = out.sel_idx.data_ptr()
         if out.sample_flags is not None:
@@ -471,9 +493,10 @@ class DensifyEngine:
         N.check(rc, "ldp_undistort_points")
         return out
 
-    def alloc_outputs(self, R: int, sel_cap: int, collect_debug: bool = False, taps: bool = False) -> DensifyOutputs:
+    def alloc_outputs(self, R: int, sel_cap: int, collect_debug: bool = False, taps: bool = False,
+                      multiview: bool = False) -> DensifyOutputs:
         """Everything a caller reads back lives in ONE allocation (``packed``): ref_offset | per-view status words | xyz | rgb |
-        err [| debug matches | debug certainties] - a rank hands its whole result to a single collective
+        err [| debug matches | debug certainties] [| view masks] - a rank hands its whole result to a single collective
         (``distributed`` / bench.py) and the drop-in path reads it back with a single device->host copy."""
         dev = self.device
         cap = max(1, R * sel_cap)
@@ -484,6 +507,8 @@ class DensifyEngine:
                  ("xyz", 12 * cap), ("rgb", 12 * cap), ("err", 4 * cap)]
         if collect_debug:
             sizes += [("dbg_matches", 16 * cap), ("dbg_cert", 4 * cap)]
+        if multiview:
+            sizes += [("view_mask", 4 * cap)]
         off, layout = 0, {}
         for name, nbytes in sizes:
             off = (off + 15) // 16 * 16
@@ -510,6 +535,8 @@ class DensifyEngine:
         if collect_debug:
             out.dbg_matches = view("dbg_matches", torch.float32, (cap, 4))
             out.dbg_cert = view("dbg_cert", torch.float32, (cap,))
+        if multiview:
+            out.view_mask = view("view_mask", torch.int32, (cap,))
         if taps:
             out.sel_idx = torch.zeros((R, sel_cap), **i32)
             out.sample_flags = torch.zeros((R, sel_cap), dtype=torch.uint8, device=dev)
