@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define LDP_ABI_VERSION 14
+#define LDP_ABI_VERSION 15
 #define LDP_MAX_NN 16          /* neighbours per reference view (the panel clamps to 10) */
 #define LDP_MAX_BINS 4096      /* coverage tiles per map: ceil(W/tile)*ceil(H/tile), tile = max(1, W/24) */
 
@@ -320,6 +320,36 @@ int ldp_nearest_neighbors(const float* flat_poses, int32_t n, int32_t k, int64_t
 int ldp_voxel_workspace_bytes(int64_t n, size_t* bytes_out);
 int ldp_voxel_downsample(const float* xyz, const float* rgb, int64_t n, double voxel_size, float* xyz_out, float* rgb_out,
                          int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- statistical outlier removal ------------------------------------------------------------------------------------
+ * Open3D's PointCloud::RemoveStatisticalOutliers(nb_neighbors, std_ratio), restated from its published source.  PARITY
+ * UNPINNED: Open3D is not in the reference tree nor in this image.  Inputs: xyz [n,3] f32 device, k = nb_neighbors in
+ * [1, 64], std_ratio > 0; k_eff = min(k, n).
+ *   1. For every point i, the k_eff nearest points of the cloud, the point itself included (at distance 0), by
+ *      d^2 = (dx*dx + dy*dy) + dz*dz in f64 with dx = f64(x_j) - f64(x_i), no FMA contraction; d = sqrt(d^2).
+ *   2. m_i = (sum of those k_eff distances in ascending order, added sequentially in f64) / k_eff.
+ *   3. V = n; mean = (sum over m_i > 0 of m_i) / V; Q = sum over m_i > 0 of (m_i - mean)^2; std = sqrt(Q / (V - 1));
+ *      threshold = mean + std_ratio * std (no FMA).
+ *   4. Point i is kept iff m_i > 0 && m_i < threshold; kept_idx_out lists the kept points in ascending index.
+ * Open3D's quirks are kept: a point whose k nearest are all exact duplicates has m_i = 0 and is dropped (and left out of the
+ * sums but not out of V); n = 1 gives std = NaN and keeps nothing; k = 1 keeps nothing.
+ * Order of the two sums of step 3 (Open3D adds in index order; ours differs from it only for points within a few ulps of
+ * the threshold): (a) partial p = sequential sum over points [256 p, 256 p + 256) in index order; (b) t = 0..1023: v_t =
+ * sequential sum of partials t, t + 1024, t + 2048, ...; (c) for s = 512, 256, ..., 1: v_t = v_t + v_{t+s} for t < s; the
+ * sum is v_0.  The terms of points with m_i <= 0 are skipped.  Nothing depends on the grid, the launch configuration or
+ * the stream; m_i is exact (bit-identical to the rule) whatever the density: the k-NN search stops only on a conservative
+ * bound (DESIGN.md §4.5).
+ * kept_idx_out: int64 [n] device, the first status_out[1] entries are written; mean_dist_out: f64 [n] device (m_i) or NULL;
+ * stats_out: f64 [3] device = {mean, std, threshold} or NULL; status_out: int32 [3] device = {1 if a coordinate is not
+ * finite (then nothing else is written), kept count, points whose search left the finest grid}.  n = 0 zeroes status_out
+ * and writes nothing else.  Synchronises the stream once (the finest cell size follows from a trial grid's cell count). */
+int ldp_outlier_workspace_bytes(int64_t n, int32_t nb_neighbors, size_t* bytes_out);
+int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, double std_ratio,
+                             int64_t* kept_idx_out, double* mean_dist_out, double* stats_out, int32_t* status_out,
+                             void* workspace, size_t workspace_bytes, void* stream);
+/* Test hook: R, the shells of cells searched per grid level before a point moves to the next coarser level (0 restores the
+ * default, 2).  Results do not depend on it. */
+int ldp_debug_outlier_max_shells(int shells);
 
 /* SMs the one-CTA-per-SM first draw kernel leaves free when ldp_params.sm_reserve is -1 (process-wide default, initially 0; the
  * environment variable LDP_SM_RESERVE, when set, wins over both).  With several launches in flight on different streams (engine.DensifyRing) or a

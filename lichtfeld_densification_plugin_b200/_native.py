@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-LDP_ABI_VERSION = 14
+LDP_ABI_VERSION = 15
 LDP_MAX_NN = 16
 LDP_MAX_BINS = 4096
 
@@ -114,6 +114,7 @@ EXPORTS = [
     "ldp_pack_ply_records", "ldp_pack_points3d_records", "ldp_rgb_to_uint8", "ldp_gather_points", "ldp_gather_rows", "ldp_concat_points", "ldp_scatter_points",
     "ldp_select_kcenters", "ldp_nearest_neighbors", "ldp_voxel_workspace_bytes", "ldp_voxel_downsample", "ldp_set_sm_reserve",
     "ldp_undistort_points", "ldp_debug_force_fixup", "ldp_debug_read_fixups",
+    "ldp_outlier_workspace_bytes", "ldp_statistical_outliers", "ldp_debug_outlier_max_shells",
 ]
 
 _lock = threading.Lock()
@@ -211,6 +212,13 @@ def load(build_if_missing: bool = False):
         lib.ldp_debug_force_fixup.argtypes = [C.c_int, C.c_int]
         lib.ldp_debug_read_fixups.restype = C.c_int
         lib.ldp_debug_read_fixups.argtypes = [C.POINTER(LdpParams), C.c_void_p, C.POINTER(C.c_int32)]
+        lib.ldp_outlier_workspace_bytes.restype = C.c_int
+        lib.ldp_outlier_workspace_bytes.argtypes = [C.c_int64, C.c_int32, C.POINTER(C.c_size_t)]
+        lib.ldp_statistical_outliers.restype = C.c_int
+        lib.ldp_statistical_outliers.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
+        lib.ldp_debug_outlier_max_shells.restype = C.c_int
+        lib.ldp_debug_outlier_max_shells.argtypes = [C.c_int]
         if lib.ldp_abi_version() != LDP_ABI_VERSION:
             raise NativeLibraryError(f"ABI version mismatch: library {lib.ldp_abi_version()}, binding {LDP_ABI_VERSION}")
         for which, struct in enumerate((LdpParams, LdpRefDesc, LdpOutputs, LdpLens)):

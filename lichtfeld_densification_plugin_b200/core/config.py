@@ -57,6 +57,9 @@ class DensePipelineConfig:
     multiview: bool = False          # re-triangulate every kept point from all of its confident, consistent neighbours (the
                                      # reference uses the best neighbour alone); which points are kept does not change
     multiview_min_certainty: float = 0.5   # multiview: certainty a neighbour's match needs at the pixel to join
+    outlier_neighbors: int = 0       # > 0: drop statistical outliers (floaters) from the final cloud, Open3D's
+                                     # remove_statistical_outlier(nb_neighbors = this, std_ratio); 0 = off
+    outlier_std_ratio: float = 2.0
 
     def validate(self) -> "DensePipelineConfig":
         if self.matches_per_ref < 0:
@@ -65,6 +68,10 @@ class DensePipelineConfig:
             raise ValueError("multiview needs the filters: it cannot be combined with no_filter")
         if not 0.0 < float(self.multiview_min_certainty) <= 1.0:
             raise ValueError("multiview_min_certainty must lie in (0, 1]")
+        if not 0 <= int(self.outlier_neighbors) <= 64:
+            raise ValueError("outlier_neighbors must lie in [0, 64] (0 = off)")
+        if not float(self.outlier_std_ratio) > 0.0:
+            raise ValueError("outlier_std_ratio must be positive")
         if self.rng_mode not in (RNG_PHILOX, RNG_NUMPY_GLOBAL, RNG_EXPLICIT):
             raise ValueError(f"unknown rng_mode {self.rng_mode!r}")
         return self

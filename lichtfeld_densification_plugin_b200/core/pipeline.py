@@ -691,7 +691,20 @@ def run_dense_pipeline(
         progress_callback(90.0, "Finalizing triangulation...")
     if not parts_xyz:
         raise RuntimeError("No points triangulated. Try adjusting parameters.")
-    return PipelineResult(xyz=np.concatenate(parts_xyz, axis=0), rgb=np.concatenate(parts_rgb, axis=0),
-                          err=np.concatenate(parts_err, axis=0), elapsed_seconds=time.time() - t0,
-                          pairs_processed=pairs,
-                          n_views=np.concatenate(parts_nv, axis=0) if getattr(config, "multiview", False) else None)
+    xyz, rgb, err = np.concatenate(parts_xyz, axis=0), np.concatenate(parts_rgb, axis=0), np.concatenate(parts_err, axis=0)
+    n_views = np.concatenate(parts_nv, axis=0) if getattr(config, "multiview", False) else None
+    k_out = int(getattr(config, "outlier_neighbors", 0))
+    if k_out > 0:
+        # floaters: the whole cloud at once (neighbours cross views); the intermediate PLYs above stay unfiltered
+        if progress_callback:
+            progress_callback(95.0, "Removing outliers...")
+        from ..output import remove_statistical_outliers
+        dev = torch.device("cuda", torch.cuda.current_device())
+        xyz_dev = torch.from_numpy(np.ascontiguousarray(xyz, dtype=np.float32)).to(dev)
+        # xyz stands in for rgb: only kept_idx is used, and it is applied to every per-point array on the host
+        res = remove_statistical_outliers(xyz_dev, xyz_dev, nb_neighbors=k_out, std_ratio=float(config.outlier_std_ratio))
+        keep = res.kept_idx.cpu().numpy()
+        xyz, rgb, err = xyz[keep], rgb[keep], err[keep]
+        if n_views is not None:
+            n_views = n_views[keep]
+    return PipelineResult(xyz=xyz, rgb=rgb, err=err, elapsed_seconds=time.time() - t0, pairs_processed=pairs, n_views=n_views)

@@ -14,6 +14,7 @@
 #include "ldp_output.cu"
 #include "ldp_select.cu"
 #include "ldp_voxel.cu"
+#include "ldp_outlier.cu"
 
 namespace {
 
@@ -969,7 +970,7 @@ static int voxel_plan(int64_t n, void* base, ldp::VoxelWs* ws, size_t* bytes) {
     size_t off = 0;
     auto carve = [&](size_t b) { void* p = base ? static_cast<char*>(base) + off : nullptr; off += align_up(b, 256); return p; };
     ws->bounds = reinterpret_cast<double*>(carve(8 * sizeof(double)));
-    ws->bounds_u = reinterpret_cast<unsigned int*>(carve(4 * sizeof(unsigned int)));
+    ws->bounds_u = reinterpret_cast<unsigned int*>(carve(8 * sizeof(unsigned int)));
     ws->keys = reinterpret_cast<unsigned long long*>(carve(cap * sizeof(unsigned long long)));
     ws->first = reinterpret_cast<int*>(carve(cap * sizeof(int)));
     ws->slot = reinterpret_cast<int*>(carve(N * sizeof(int)));
@@ -1030,7 +1031,7 @@ int ldp_voxel_downsample(const float* xyz, const float* rgb, int64_t n, double v
     const unsigned grid = (unsigned)((n + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
     const unsigned rgrid = (unsigned)std::min<long long>(grid, (long long)sm_count() * 8);
     (void)launch_k(ldp::ldp_voxel_bounds_kernel, dim3(rgrid), dim3(ldp::KV_THREADS), 0, st, xyz, rgb, (long long)n, ws);
-    (void)launch_k(ldp::ldp_voxel_insert_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, xyz, (long long)n, voxel_size, ws);
+    (void)launch_k(ldp::ldp_voxel_insert_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, xyz, (long long)n, voxel_size, (const double*)nullptr, ws);
     (void)launch_k(ldp::ldp_voxel_flag_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws);
     g_launches += 3;
     scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, ws.status + 1, st);
@@ -1042,6 +1043,206 @@ int ldp_voxel_downsample(const float* xyz, const float* rgb, int64_t n, double v
     (void)launch_k(ldp::ldp_voxel_large_kernel, dim3((unsigned)sm_count()), dim3(ldp::SC_THREADS), 0, st, xyz, rgb, ws, (const int*)ws.seg, xyz_out, rgb_out);
     g_launches += 3;
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "voxel downsample kernels");
+    return LDP_OK;
+}
+
+// ---- statistical outlier removal (ldp_outlier.cu)
+static int g_outlier_shells = 0;           // ldp_debug_outlier_max_shells; 0 = ldp::OL_DEFAULT_SHELLS
+
+struct OutlierPlan {
+    ldp::VoxelWs vws;                      // grid-building scratch, shared by the trial grid and every level
+    int* vstat;                            // [2] status of the voxel kernels: overflow flag, cell count
+    double* h_trial;                       // [1] trial cell size
+    double* stats;                         // [3] used when the caller passes no stats_out
+    double* m;                             // [n] used when the caller passes no mean_dist_out
+    double* part;                          // [ceil(n / KS_CHUNK)] first-stage partial sums
+    ldp::OutlierLevel* levels;             // [KS_MAX_LEVELS] level descriptors for the k-NN kernel
+    unsigned long long* keys[ldp::OL_MAX_LEVELS];
+    int2* cell[ldp::OL_MAX_LEVELS];
+    float4* pts[ldp::OL_MAX_LEVELS];
+};
+
+static int outlier_plan(int64_t n, void* base, OutlierPlan* pl, size_t* bytes) {
+    if (n < 0 || n > 500000000ll) return fail(LDP_ERR_INVALID, "statistical outliers: bad point count");
+    size_t off = 0;
+    int rc = voxel_plan(n, base, &pl->vws, &off);
+    if (rc != LDP_OK) return rc;
+    const size_t cap = voxel_cap(n), N = (size_t)std::max<int64_t>(n, 1);
+    auto carve = [&](size_t b) { void* p = base ? static_cast<char*>(base) + off : nullptr; off += align_up(b, 256); return p; };
+    pl->vstat = reinterpret_cast<int*>(carve(2 * sizeof(int)));
+    pl->h_trial = reinterpret_cast<double*>(carve(sizeof(double)));
+    pl->stats = reinterpret_cast<double*>(carve(3 * sizeof(double)));
+    pl->m = reinterpret_cast<double*>(carve(N * sizeof(double)));
+    pl->part = reinterpret_cast<double*>(carve((N / ldp::OL_CHUNK + 1) * sizeof(double)));
+    pl->levels = reinterpret_cast<ldp::OutlierLevel*>(carve(ldp::OL_MAX_LEVELS * sizeof(ldp::OutlierLevel)));
+    for (int l = 0; l < ldp::OL_MAX_LEVELS; ++l) {
+        pl->keys[l] = reinterpret_cast<unsigned long long*>(carve(cap * sizeof(unsigned long long)));
+        pl->cell[l] = reinterpret_cast<int2*>(carve(cap * sizeof(int2)));
+        pl->pts[l] = reinterpret_cast<float4*>(carve(N * sizeof(float4)));
+    }
+    *bytes = off;
+    return LDP_OK;
+}
+
+int ldp_outlier_workspace_bytes(int64_t n, int32_t nb_neighbors, size_t* bytes_out) {
+    if (!bytes_out) return fail(LDP_ERR_INVALID, "null bytes_out");
+    if (nb_neighbors < 1 || nb_neighbors > ldp::OL_MAX_K) return fail(LDP_ERR_INVALID, "nb_neighbors must lie in [1, 64]");
+    OutlierPlan pl;
+    return outlier_plan(n, nullptr, &pl, bytes_out);
+}
+
+int ldp_debug_outlier_max_shells(int shells) {
+    if (shells < 0) return fail(LDP_ERR_INVALID, "shells must be >= 0");
+    g_outlier_shells = shells;
+    return LDP_OK;
+}
+
+static float host_f32_unordered(unsigned int k) {          // ldp::f32_unordered on the host
+    const unsigned int b = (k & 0x80000000u) ? (k & 0x7fffffffu) : ~k;
+    float f;
+    std::memcpy(&f, &b, sizeof(f));
+    return f;
+}
+
+// hash insert, first-of-cell flags, ranks: the cells of a grid of size h (or *h_dev) in pl.vws.keys
+static void outlier_insert(const float* xyz, int64_t n, double h, const double* h_dev, OutlierPlan& pl, unsigned grid, cudaStream_t st,
+                           int* cells_out) {
+    ldp::VoxelWs& ws = pl.vws;
+    const size_t cap = (size_t)ws.cap_mask + 1;
+    (void)cudaMemsetAsync(ws.keys, 0xFF, cap * sizeof(unsigned long long), st);
+    (void)cudaMemsetAsync(ws.first, 0x7F, cap * sizeof(int), st);
+    (void)launch_k(ldp::ldp_voxel_insert_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, xyz, (long long)n, h, h_dev, ws);
+    (void)launch_k(ldp::ldp_voxel_flag_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws);
+    g_launches += 2;
+    scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, cells_out, st);
+}
+
+int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, double std_ratio, int64_t* kept_idx_out,
+                             double* mean_dist_out, double* stats_out, int32_t* status_out, void* workspace, size_t workspace_bytes,
+                             void* stream) {
+    g_launches = 0;
+    if (nb_neighbors < 1 || nb_neighbors > ldp::OL_MAX_K) return fail(LDP_ERR_INVALID, "nb_neighbors must lie in [1, 64]");
+    if (!(std_ratio > 0.0)) return fail(LDP_ERR_INVALID, "std_ratio must be positive");
+    if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    cudaError_t e = cudaMemsetAsync(status_out, 0, 3 * sizeof(int32_t), st);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(status)");
+    if (n == 0) return LDP_OK;
+    if (!xyz || !kept_idx_out || !workspace) return fail(LDP_ERR_INVALID, "null pointer");
+    OutlierPlan pl;
+    size_t need = 0;
+    int rc = outlier_plan(n, workspace, &pl, &need);
+    if (rc != LDP_OK) return rc;
+    if (workspace_bytes < need) return fail(LDP_ERR_WORKSPACE, "outlier workspace too small");
+    const int k = (int)std::min<int64_t>(nb_neighbors, n);
+    ldp::VoxelWs& ws = pl.vws;
+    ws.status = pl.vstat;
+    const unsigned grid = (unsigned)((n + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
+    const unsigned rgrid = (unsigned)std::min<long long>(grid, (long long)sm_count() * 8);
+    const size_t cap = (size_t)ws.cap_mask + 1;
+    const unsigned cgrid = (unsigned)((cap + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
+
+    // 1. bounds and a trial grid; its cell count sets the level-0 cell size (the one host synchronisation)
+    unsigned int bu[8];
+    double h_trial = 0.0;
+    {
+        KernelTimer kt(st, "ldp_outlier_trial_grid");
+        e = cudaMemsetAsync(ws.bounds_u, 0xFF, 3 * sizeof(unsigned int), st);
+        if (e == cudaSuccess) e = cudaMemsetAsync(ws.bounds_u + 3, 0, 5 * sizeof(unsigned int), st);
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(outlier bounds)");
+        (void)launch_k(ldp::ldp_voxel_bounds_kernel, dim3(rgrid), dim3(ldp::KV_THREADS), 0, st, xyz, (const float*)nullptr, (long long)n, ws);
+        (void)launch_k(ldp::ldp_outlier_trial_size_kernel, dim3(1), dim3(1), 0, st, (const unsigned int*)ws.bounds_u, (long long)n, k, pl.h_trial);
+        g_launches += 2;
+        outlier_insert(xyz, n, 0.0, pl.h_trial, pl, grid, st, reinterpret_cast<int*>(ws.bounds_u + 7));
+    }
+    e = cudaMemcpyAsync(bu, ws.bounds_u, sizeof(bu), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&h_trial, pl.h_trial, sizeof(double), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return cuda_fail(e, "outlier trial grid");
+    double mn[3], mx[3], ext = 0.0;
+    bool finite = true;
+    for (int c = 0; c < 3; ++c) {
+        mn[c] = (double)host_f32_unordered(bu[c]);
+        mx[c] = (double)host_f32_unordered(bu[4 + c]);
+        finite = finite && std::isfinite(mn[c]) && std::isfinite(mx[c]);
+        ext = std::max(ext, mx[c] - mn[c]);
+    }
+    if (!finite) {                                      // status_out[0] = 1 (little-endian int32, zeroed above)
+        e = cudaMemsetAsync(status_out, 1, 1, st);
+        return e == cudaSuccess ? LDP_OK : cuda_fail(e, "cudaMemsetAsync(status)");
+    }
+    const double trial_cells = (double)std::max(1u, bu[7]);
+    double h = 1.0;
+    if (ext > 0.0) h = std::max(h_trial * std::sqrt(0.5 * k * trial_cells / (double)n), ext / 1048576.0);
+
+    // 2. the pyramid: h_l = h0 * 8^l up to the first level with at most 3 cells per axis
+    ldp::OutlierGrid lv;
+    int n_levels = 0;
+    {
+        KernelTimer kt(st, "ldp_outlier_pyramid");
+        for (;;) {
+            ldp::OutlierLevel& L = lv.lv[n_levels];
+            L.keys = pl.keys[n_levels]; L.cell = pl.cell[n_levels]; L.pts = pl.pts[n_levels];
+            L.cap_mask = ws.cap_mask; L.h = h; L.pad = 0;
+            for (int c = 0; c < 3; ++c) {
+                L.vmin[c] = mn[c] - h * 0.5;                                  // ldp_voxel_insert_kernel's expression
+                L.gmax[c] = (int)std::floor((mx[c] - L.vmin[c]) / h);
+            }
+            ws.keys = pl.keys[n_levels];
+            e = cudaMemsetAsync(ws.count, 0, ((size_t)n + 1) * sizeof(int), st);
+            if (e == cudaSuccess) e = cudaMemsetAsync(ws.cursor, 0, (size_t)n * sizeof(int), st);
+            if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(outlier level)");
+            outlier_insert(xyz, n, h, nullptr, pl, grid, st, pl.vstat + 1);
+            (void)launch_k(ldp::ldp_voxel_count_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws);
+            ++g_launches;
+            scan_exclusive(ws.count, ws.seg, n, ws.block_tot, nullptr, st);
+            (void)launch_k(ldp::ldp_voxel_group_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws, (const int*)ws.seg);
+            (void)launch_k(ldp::ldp_outlier_cells_kernel, dim3(cgrid), dim3(ldp::KV_THREADS), 0, st, ws, pl.cell[n_levels]);
+            (void)launch_k(ldp::ldp_outlier_pack_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, xyz, (long long)n,
+                           (const int*)ws.members, pl.pts[n_levels]);
+            g_launches += 3;
+            ++n_levels;
+            if (n_levels == ldp::OL_MAX_LEVELS || !(ext / h > 2.0)) break;
+            h *= 8.0;
+        }
+    }
+    (void)launch_k(ldp::ldp_outlier_levels_kernel, dim3(1), dim3(1), 0, st, lv, n_levels, pl.levels);
+    ++g_launches;
+
+    // 3. k nearest, per-point mean distance
+    double* m = mean_dist_out ? mean_dist_out : pl.m;
+    double* stats = stats_out ? stats_out : pl.stats;
+    {
+        KernelTimer kt(st, "ldp_outlier_knn_kernel");
+        const unsigned kgrid = (unsigned)((n + ldp::OL_THREADS - 1) / ldp::OL_THREADS);
+        (void)launch_k(ldp::ldp_outlier_knn_kernel, dim3(kgrid), dim3(ldp::OL_THREADS), (size_t)k * ldp::OL_THREADS * sizeof(double), st,
+                       (const ldp::OutlierLevel*)pl.levels, n_levels, (long long)n, k,
+                       g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, m, (int*)status_out);
+        ++g_launches;
+    }
+
+    // 4. threshold, keep flags, kept indices
+    {
+        KernelTimer kt(st, "ldp_outlier_threshold");
+        const long long n_part = (n + ldp::OL_CHUNK - 1) / ldp::OL_CHUNK;
+        const unsigned pgrid = (unsigned)((n_part + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
+        (void)launch_k(ldp::ldp_outlier_partial_kernel, dim3(pgrid), dim3(ldp::KV_THREADS), 0, st, (const double*)m, (long long)n,
+                       (const double*)nullptr, pl.part);
+        (void)launch_k(ldp::ldp_outlier_stats_kernel, dim3(1), dim3(ldp::OL_FINAL), 0, st, (const double*)pl.part, n_part, (long long)n,
+                       std_ratio, 0, stats);
+        (void)launch_k(ldp::ldp_outlier_partial_kernel, dim3(pgrid), dim3(ldp::KV_THREADS), 0, st, (const double*)m, (long long)n,
+                       (const double*)stats, pl.part);
+        (void)launch_k(ldp::ldp_outlier_stats_kernel, dim3(1), dim3(ldp::OL_FINAL), 0, st, (const double*)pl.part, n_part, (long long)n,
+                       std_ratio, 1, stats);
+        (void)launch_k(ldp::ldp_outlier_flag_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (const double*)m, (long long)n,
+                       (const double*)stats, ws.flag);
+        g_launches += 5;
+        scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, (int*)status_out + 1, st);
+        (void)launch_k(ldp::ldp_outlier_kept_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (const int*)ws.flag, (const int*)ws.rank,
+                       (long long)n, reinterpret_cast<long long*>(kept_idx_out));
+        ++g_launches;
+    }
+    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "statistical outlier kernels");
     return LDP_OK;
 }
 

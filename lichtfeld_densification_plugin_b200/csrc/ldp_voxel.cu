@@ -16,7 +16,7 @@ constexpr unsigned long long VX_EMPTY = 0xFFFFFFFFFFFFFFFFull;
 
 struct VoxelWs {
     double* bounds;                 // [8] min x,y,z (as doubles after the reduction), max colour, scratch
-    unsigned int* bounds_u;         // [4] ordered-uint encodings while reducing: min x,y,z, max rgb
+    unsigned int* bounds_u;         // [8] ordered-uint encodings while reducing: min x,y,z, max rgb, max x,y,z; [7] scratch
     unsigned long long* keys;       // [cap] voxel key per slot (VX_EMPTY = free)
     int* first;                     // [cap] smallest point index in the slot's voxel
     int* slot;                      // [n]   slot of each point
@@ -44,24 +44,30 @@ __global__ void __launch_bounds__(KV_THREADS)
 ldp_voxel_bounds_kernel(const float* __restrict__ xyz, const float* __restrict__ rgb, long long n, VoxelWs ws)
 {
     grid_dependency_sync();
-    unsigned int mn[3] = {0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu}, mx = 0u;
+    // rgb == nullptr (outlier filter): bounds_u[4 + c] = max of coordinate c instead of bounds_u[3] = max colour.  Both
+    // maxima also catch a NaN with the sign bit clear; the minima catch one with it set.
+    unsigned int mn[3] = {0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu}, mx[3] = {0u, 0u, 0u};
     for (long long i = (long long)blockIdx.x * KV_THREADS + threadIdx.x; i < n; i += (long long)gridDim.x * KV_THREADS) {
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             mn[c] = min(mn[c], f32_ordered(xyz[3 * i + c]));
-            mx = max(mx, f32_ordered(rgb[3 * i + c]));
+            if (rgb) mx[0] = max(mx[0], f32_ordered(rgb[3 * i + c]));
+            else mx[c] = max(mx[c], f32_ordered(xyz[3 * i + c]));
         }
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
 #pragma unroll
-        for (int c = 0; c < 3; ++c) mn[c] = min(mn[c], __shfl_xor_sync(0xffffffffu, mn[c], o));
-        mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+        for (int c = 0; c < 3; ++c) {
+            mn[c] = min(mn[c], __shfl_xor_sync(0xffffffffu, mn[c], o));
+            mx[c] = max(mx[c], __shfl_xor_sync(0xffffffffu, mx[c], o));
+        }
     }
     if ((threadIdx.x & 31) == 0) {
 #pragma unroll
         for (int c = 0; c < 3; ++c) atomicMin(&ws.bounds_u[c], mn[c]);
-        atomicMax(&ws.bounds_u[3], mx);
+        if (rgb) atomicMax(&ws.bounds_u[3], mx[0]);
+        else for (int c = 0; c < 3; ++c) atomicMax(&ws.bounds_u[4 + c], mx[c]);
     }
 }
 
@@ -70,13 +76,14 @@ __device__ __forceinline__ unsigned long long vx_hash(unsigned long long k) {
     return k;
 }
 
-// voxel index of every point, hash insert, smallest point index per voxel
+// voxel index of every point, hash insert, smallest point index per voxel (the size is read from size_dev when given)
 __global__ void __launch_bounds__(KV_THREADS)
-ldp_voxel_insert_kernel(const float* __restrict__ xyz, long long n, double voxel_size, VoxelWs ws)
+ldp_voxel_insert_kernel(const float* __restrict__ xyz, long long n, double voxel_size, const double* __restrict__ size_dev, VoxelWs ws)
 {
     grid_dependency_sync();
     const long long i = (long long)blockIdx.x * KV_THREADS + threadIdx.x;
     if (i >= n) return;
+    if (size_dev) voxel_size = *size_dev;
     unsigned long long key = 0ull;
     bool bad = false;
 #pragma unroll

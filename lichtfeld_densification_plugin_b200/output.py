@@ -6,6 +6,7 @@ Mirrors, on tensors that stay on the GPU (SURVEY.md 8a row a15, 8f rows 2 and 4)
 * ``write_ply`` / ``write_points3D_bin``   reference core/writers.py:15-46 (files byte-identical; the records are built by
   ``ldp_pack_ply_records`` / ``ldp_pack_points3d_records`` and reach the host as one copy of 15 / 43 bytes per point)
 * ``voxel_downsample``                 reference densify.py:29-50 (Open3D voxel grid mean; parity unpinned, see the function)
+* ``remove_statistical_outliers``      not in the reference: Open3D's ``remove_statistical_outlier`` (parity unpinned)
 * ``apply_point_cap``                  reference densify.py:110-120 (the indices are numpy's own
   ``default_rng(seed).choice`` on the host - PCG64 + a sequential shuffle, microseconds; only the gather is device work)
 * ``subsample_preview_matches``        reference core/pipeline.py:573-582 (debug preview subsample of the kept matches)
@@ -18,6 +19,7 @@ No CPU fallback: every function needs the CUDA library (``NativeLibraryError`` o
 from __future__ import annotations
 
 import ctypes as C
+from dataclasses import dataclass
 from typing import Optional, Tuple
 
 import numpy as np
@@ -241,6 +243,64 @@ def voxel_downsample(xyz: torch.Tensor, rgb: torch.Tensor, voxel_size: float) ->
     if bad:
         raise ValueError("voxel_size is too small for the extent of the cloud (or a coordinate is not finite)")
     return o_xyz[:nv], o_rgb[:nv]
+
+
+@dataclass
+class OutlierResult:
+    """What ``remove_statistical_outliers`` returns: the kept rows and the filter's statistics."""
+    xyz: torch.Tensor               # [m, 3] f32, kept rows in input order
+    rgb: torch.Tensor               # [m, 3] f32
+    err: Optional[torch.Tensor]     # [m] f32, None when no err was given
+    kept_idx: torch.Tensor          # [m] int64 device, ascending
+    mean_dist: torch.Tensor         # [n] f64 device: mean distance of every point to its k nearest (itself included)
+    cloud_mean: float
+    std_dev: float
+    threshold: float
+
+
+def remove_statistical_outliers(xyz: torch.Tensor, rgb: torch.Tensor, err: Optional[torch.Tensor] = None, *,
+                                nb_neighbors: int, std_ratio: float) -> OutlierResult:
+    """Open3D's ``remove_statistical_outlier(nb_neighbors, std_ratio)`` on device tensors: a point is kept iff the mean
+    distance to its ``nb_neighbors`` nearest points (itself included) is positive and below ``mean + std_ratio * std`` of
+    those means over the cloud.  The k-nearest-neighbour search is exact (f64 distances).  PARITY UNPINNED (Open3D is not
+    installed here; the rule and the order of its sums are in include/ldp_b200.h).  Synchronises twice: once inside the
+    call (the finest grid cell size follows from a trial grid's cell count) and once to learn the kept count."""
+    if not 1 <= int(nb_neighbors) <= 64:
+        raise ValueError("nb_neighbors must lie in [1, 64]")
+    if not float(std_ratio) > 0.0:
+        raise ValueError("std_ratio must be positive")
+    xyz, rgb = _f32c(xyz, "xyz"), _f32c(rgb, "rgb")
+    if err is not None:
+        err = _f32c(err, "err")
+    lib, stream = _lib_and_stream(xyz)
+    dev, n = xyz.device, int(xyz.shape[0])
+    need = C.c_size_t(0)
+    N.check(lib.ldp_outlier_workspace_bytes(n, int(nb_neighbors), C.byref(need)), "ldp_outlier_workspace_bytes")
+    ws = torch.empty((max(1, need.value),), dtype=torch.uint8, device=dev)
+    kept = torch.empty((n,), dtype=torch.int64, device=dev)
+    mean_dist = torch.empty((n,), dtype=torch.float64, device=dev)
+    stats = torch.full((3,), float("nan"), dtype=torch.float64, device=dev)
+    status = torch.zeros((3,), dtype=torch.int32, device=dev)
+    N.check(lib.ldp_statistical_outliers(C.c_void_p(xyz.data_ptr()), n, int(nb_neighbors), C.c_double(float(std_ratio)),
+                                         C.c_void_p(kept.data_ptr()), C.c_void_p(mean_dist.data_ptr()), C.c_void_p(stats.data_ptr()),
+                                         C.c_void_p(status.data_ptr()), C.c_void_p(ws.data_ptr()), C.c_size_t(need.value),
+                                         C.c_void_p(stream)), "ldp_statistical_outliers")
+    status_h, stats_h = status.to("cpu", non_blocking=True), stats.to("cpu", non_blocking=True)
+    torch.cuda.current_stream(dev).synchronize()
+    bad, m = int(status_h[0]), int(status_h[1])
+    if bad:
+        raise ValueError("a coordinate is not finite")
+    kept = kept[:m]
+    o_xyz = torch.empty((m, 3), dtype=torch.float32, device=dev)
+    o_rgb = torch.empty((m, 3), dtype=torch.float32, device=dev)
+    o_err = torch.empty((m,), dtype=torch.float32, device=dev) if err is not None else None
+    N.check(lib.ldp_gather_points(C.c_void_p(xyz.data_ptr()), C.c_void_p(rgb.data_ptr()),
+                                  C.c_void_p(err.data_ptr() if err is not None else 0), C.c_void_p(kept.data_ptr()), m, n,
+                                  C.c_void_p(o_xyz.data_ptr()), C.c_void_p(o_rgb.data_ptr()),
+                                  C.c_void_p(o_err.data_ptr() if o_err is not None else 0), C.c_void_p(0), C.c_void_p(stream)),
+            "ldp_gather_points")
+    mu, sd, thr = (float(v) for v in stats_h.tolist())
+    return OutlierResult(xyz=o_xyz, rgb=o_rgb, err=o_err, kept_idx=kept, mean_dist=mean_dist, cloud_mean=mu, std_dev=sd, threshold=thr)
 
 
 PREVIEW_MAX_MATCHES = 10000       # reference core/pipeline.py:50 _PREVIEW_MAX_MATCHES
