@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define LDP_ABI_VERSION 15
+#define LDP_ABI_VERSION 16
 #define LDP_MAX_NN 16          /* neighbours per reference view (the panel clamps to 10) */
 #define LDP_MAX_BINS 4096      /* coverage tiles per map: ceil(W/tile)*ceil(H/tile), tile = max(1, W/24) */
 
@@ -248,6 +248,8 @@ int ldp_postprocess_certainty(const ldp_params* params, const ldp_ref_desc* refs
  * to the actual point count (then n is an upper bound that sizes the launch and min(n, *n_dev) records are written:
  * no host synchronisation between the path and the packing); records_out: device, n * 15 / n * 43 bytes.
  *   ldp_pack_ply_records       per vertex  <fff xyz, BBB rgb                           core/writers.py:44-45
+ *   ldp_pack_ply_normal_records  per vertex  <fff xyz, <fff normal, BBB rgb (27 bytes; not in the reference: the
+ *                              PLY of core/writers.py write_ply(..., normals=), nx ny nz between z and red)
  *   ldp_pack_points3d_records  per point   <Q first_id + i, <ddd xyz, <BBB rgb, <d err  core/writers.py:23-26
  *                              (first_id = 1 for a whole file; a rank writing rows [a, b) passes a + 1)
  *   ldp_rgb_to_uint8           to_uint8_rgb on n_values floats                         core/image_utils.py:24-26
@@ -256,6 +258,8 @@ int ldp_postprocess_certainty(const ldp_params* params, const ldp_ref_desc* refs
  *                              negative indices wrap like numpy's; an index outside [-n, n) sets *bad_index_flag
  *                              (device int32, may be NULL) and leaves the row unwritten. */
 int ldp_pack_ply_records(const float* xyz, const float* rgb, int64_t n, const int64_t* n_dev, uint8_t* records_out, void* stream);
+int ldp_pack_ply_normal_records(const float* xyz, const float* rgb, const float* normals, int64_t n, const int64_t* n_dev,
+                                uint8_t* records_out, void* stream);
 int ldp_pack_points3d_records(const float* xyz, const float* rgb, const float* err, int64_t n, const int64_t* n_dev,
                               uint64_t first_id, uint8_t* records_out, void* stream);
 int ldp_rgb_to_uint8(const float* rgb, int64_t n_values, uint8_t* out, void* stream);
@@ -350,6 +354,33 @@ int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, 
 /* Test hook: R, the shells of cells searched per grid level before a point moves to the next coarser level (0 restores the
  * default, 2).  Results do not depend on it. */
 int ldp_debug_outlier_max_shells(int shells);
+
+/* ---- oriented point normals (not in the reference) ------------------------------------------------------------------
+ * Inputs: xyz [n,3] f32 device, k in [3, 64]; k_eff = min(k, n).
+ *   1. Neighbourhood of point i: the k_eff points j with the smallest (d^2, j), compared lexicographically, with d^2 the
+ *      outlier rule's (dx*dx + dy*dy) + dz*dz in f64 without FMA and j the row index; i itself is a candidate at d^2 = 0.
+ *      The index breaks ties, so the set is unique (on a lattice, tied neighbours would change the normal).
+ *   2. In f64, over the neighbourhood in ascending (d^2, j) order, added sequentially, no FMA: mu = (sum x_j) / k_eff;
+ *      C = (sum (x_j - mu)(x_j - mu)^T) / k_eff (upper triangle; each entry its own sequential sum).
+ *   3. Eigenvalues l0 <= l1 <= l2 of C by cyclic Jacobi in f64 (to convergence).  The normal is the unit eigenvector of
+ *      l0; curvature (surface variation) = l0 / ((l0 + l1) + l2).
+ *   4. Undefined when k_eff < 3, trace(C) = 0 (all duplicates) or l1 <= 1e-12 * l2 (a line): normal (0, 0, 0),
+ *      curvature NaN, counted in status_out[1].
+ *   5. Sign: first canonical (the component of largest magnitude positive, the lowest axis on ties); then, when the point
+ *      has a centre c, flipped iff n . (c - x) < 0, in f64.  A point triangulated from a camera faces that camera.
+ * Steps 1 and 2 are bit-exact: the k-NN search stops only on a conservative bound (DESIGN.md §4.6); step 3 matches
+ * numpy.linalg.eigh within eigenvector conditioning.  Parity with Open3D's estimate_normals is not claimed.
+ * centers: f32 [n_centers,3] device or NULL (no orientation step); center_idx: int32 [n] device, the centre of every point,
+ * or NULL for centers[0] (needs centers).  normals_out f32 [n,3] device; curvature_out f32 [n] device or NULL; knn_idx_out
+ * int32 [n,k_eff] device or NULL (row i: the neighbourhood of step 1, ascending).  status_out: int32 [3] device = {bit mask:
+ * 1 a coordinate is not finite (then nothing else is written), 2 a centre index is out of range (that point keeps its
+ * canonical sign); undefined normals; points whose search left the finest grid}.  n = 0 zeroes status_out and writes
+ * nothing else.  Synchronises the stream once (the trial grid, as ldp_statistical_outliers); ldp_debug_outlier_max_shells
+ * applies.  Results do not depend on the grid, the launch or the stream. */
+int ldp_normals_workspace_bytes(int64_t n, int32_t k, size_t* bytes_out);
+int ldp_estimate_normals(const float* xyz, int64_t n, int32_t k, const float* centers, int32_t n_centers, const int32_t* center_idx,
+                         float* normals_out, float* curvature_out, int32_t* knn_idx_out, int32_t* status_out, void* workspace,
+                         size_t workspace_bytes, void* stream);
 
 /* SMs the one-CTA-per-SM first draw kernel leaves free when ldp_params.sm_reserve is -1 (process-wide default, initially 0; the
  * environment variable LDP_SM_RESERVE, when set, wins over both).  With several launches in flight on different streams (engine.DensifyRing) or a

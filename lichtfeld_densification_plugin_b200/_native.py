@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-LDP_ABI_VERSION = 15
+LDP_ABI_VERSION = 16
 LDP_MAX_NN = 16
 LDP_MAX_BINS = 4096
 
@@ -115,6 +115,7 @@ EXPORTS = [
     "ldp_select_kcenters", "ldp_nearest_neighbors", "ldp_voxel_workspace_bytes", "ldp_voxel_downsample", "ldp_set_sm_reserve",
     "ldp_undistort_points", "ldp_debug_force_fixup", "ldp_debug_read_fixups",
     "ldp_outlier_workspace_bytes", "ldp_statistical_outliers", "ldp_debug_outlier_max_shells",
+    "ldp_normals_workspace_bytes", "ldp_estimate_normals", "ldp_pack_ply_normal_records",
 ]
 
 _lock = threading.Lock()
@@ -219,6 +220,14 @@ def load(build_if_missing: bool = False):
                                                  C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
         lib.ldp_debug_outlier_max_shells.restype = C.c_int
         lib.ldp_debug_outlier_max_shells.argtypes = [C.c_int]
+        lib.ldp_normals_workspace_bytes.restype = C.c_int
+        lib.ldp_normals_workspace_bytes.argtypes = [C.c_int64, C.c_int32, C.POINTER(C.c_size_t)]
+        lib.ldp_estimate_normals.restype = C.c_int
+        lib.ldp_estimate_normals.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
+        lib.ldp_pack_ply_normal_records.restype = C.c_int
+        lib.ldp_pack_ply_normal_records.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                                    C.c_void_p]
         if lib.ldp_abi_version() != LDP_ABI_VERSION:
             raise NativeLibraryError(f"ABI version mismatch: library {lib.ldp_abi_version()}, binding {LDP_ABI_VERSION}")
         for which, struct in enumerate((LdpParams, LdpRefDesc, LdpOutputs, LdpLens)):

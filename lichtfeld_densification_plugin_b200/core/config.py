@@ -60,6 +60,8 @@ class DensePipelineConfig:
     outlier_neighbors: int = 0       # > 0: drop statistical outliers (floaters) from the final cloud, Open3D's
                                      # remove_statistical_outlier(nb_neighbors = this, std_ratio); 0 = off
     outlier_std_ratio: float = 2.0
+    normal_neighbors: int = 0        # > 0: PipelineResult.normals, PCA over this many nearest points, each normal facing
+                                     # the camera that triangulated its point; 0 = off
 
     def validate(self) -> "DensePipelineConfig":
         if self.matches_per_ref < 0:
@@ -72,6 +74,8 @@ class DensePipelineConfig:
             raise ValueError("outlier_neighbors must lie in [0, 64] (0 = off)")
         if not float(self.outlier_std_ratio) > 0.0:
             raise ValueError("outlier_std_ratio must be positive")
+        if not (int(self.normal_neighbors) == 0 or 3 <= int(self.normal_neighbors) <= 64):
+            raise ValueError("normal_neighbors must be 0 (off) or lie in [3, 64]")
         if self.rng_mode not in (RNG_PHILOX, RNG_NUMPY_GLOBAL, RNG_EXPLICIT):
             raise ValueError(f"unknown rng_mode {self.rng_mode!r}")
         return self

@@ -39,6 +39,8 @@ class PipelineResult:
     elapsed_seconds: float
     pairs_processed: int
     n_views: Optional[np.ndarray] = None          # extra, config.multiview: uint8 cameras per point, the reference view included
+    normals: Optional[np.ndarray] = None          # extra, config.normal_neighbors: f32 [n,3] unit normals facing each point's
+                                                  # reference camera; (0, 0, 0) where undefined
 
 
 class PipelineCancelled(RuntimeError):
@@ -602,7 +604,7 @@ def run_dense_pipeline(
                                     w_match=int(w_match), h_match=int(h_match))
     t0 = time.time()
     step = int(getattr(config, "refs_per_launch", 32)) or max(1, len(refs_local))
-    parts_xyz, parts_rgb, parts_err, parts_nv = [], [], [], []
+    parts_xyz, parts_rgb, parts_err, parts_nv, parts_ref = [], [], [], [], []
     pairs = 0
     pair_counter = 0
     # live update (core/pipeline.py:296-306,508-532): every viz_interval views the reference re-concatenates and re-packs
@@ -627,6 +629,7 @@ def run_dense_pipeline(
             parts_xyz.append(tri.xyz)
             parts_rgb.append(tri.rgb)
             parts_err.append(tri.err)
+            parts_ref.append(np.full((int(tri.xyz.shape[0]),), int(mr.packed.ref_id), np.int64))   # each point's reference view
             if tri.n_views is not None:
                 parts_nv.append(tri.n_views)
             pairs += 1
@@ -693,18 +696,34 @@ def run_dense_pipeline(
         raise RuntimeError("No points triangulated. Try adjusting parameters.")
     xyz, rgb, err = np.concatenate(parts_xyz, axis=0), np.concatenate(parts_rgb, axis=0), np.concatenate(parts_err, axis=0)
     n_views = np.concatenate(parts_nv, axis=0) if getattr(config, "multiview", False) else None
+    ref_uid = np.concatenate(parts_ref, axis=0)
     k_out = int(getattr(config, "outlier_neighbors", 0))
+    k_nrm = int(getattr(config, "normal_neighbors", 0))
+    normals = None
+    if k_out > 0 or k_nrm > 0:
+        dev = torch.device("cuda", torch.cuda.current_device())
+        xyz_dev = torch.from_numpy(np.ascontiguousarray(xyz, dtype=np.float32)).to(dev)
     if k_out > 0:
         # floaters: the whole cloud at once (neighbours cross views); the intermediate PLYs above stay unfiltered
         if progress_callback:
             progress_callback(95.0, "Removing outliers...")
         from ..output import remove_statistical_outliers
-        dev = torch.device("cuda", torch.cuda.current_device())
-        xyz_dev = torch.from_numpy(np.ascontiguousarray(xyz, dtype=np.float32)).to(dev)
         # xyz stands in for rgb: only kept_idx is used, and it is applied to every per-point array on the host
         res = remove_statistical_outliers(xyz_dev, xyz_dev, nb_neighbors=k_out, std_ratio=float(config.outlier_std_ratio))
         keep = res.kept_idx.cpu().numpy()
-        xyz, rgb, err = xyz[keep], rgb[keep], err[keep]
+        xyz, rgb, err, ref_uid = xyz[keep], rgb[keep], err[keep], ref_uid[keep]
+        xyz_dev = res.xyz
         if n_views is not None:
             n_views = n_views[keep]
-    return PipelineResult(xyz=xyz, rgb=rgb, err=err, elapsed_seconds=time.time() - t0, pairs_processed=pairs, n_views=n_views)
+    if k_nrm > 0:
+        # every point faces the camera it was triangulated from (its reference view, a contributing view in every mode)
+        if progress_callback:
+            progress_callback(97.0, "Estimating normals...")
+        from ..output import estimate_normals
+        uids, center_idx = np.unique(ref_uid, return_inverse=True)
+        centers = np.stack([np.asarray(cameras.C_by[int(u)], np.float64).reshape(3) for u in uids]).astype(np.float32)
+        nres = estimate_normals(xyz_dev, nb_neighbors=k_nrm, centers=torch.from_numpy(centers).to(dev),
+                                center_idx=torch.from_numpy(center_idx.astype(np.int32)).to(dev))
+        normals = nres.normals.cpu().numpy()
+    return PipelineResult(xyz=xyz, rgb=rgb, err=err, elapsed_seconds=time.time() - t0, pairs_processed=pairs, n_views=n_views,
+                          normals=normals)

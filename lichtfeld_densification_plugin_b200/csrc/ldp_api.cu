@@ -785,6 +785,7 @@ int ldp_debug_set_cluster(int csize) {
 const char* ldp_profile_name(int i) { return (i >= 0 && i < g_prof_n) ? g_prof_name[i] : ""; }
 
 // ---- output contract on the device (ldp_output.cu)
+// format 2 takes the normals [n,3] in place of err
 static int pack_records(int format, const float* xyz, const float* rgb, const float* err, int64_t n, const int64_t* n_dev,
                         uint64_t first_id, uint8_t* out, void* stream) {
     if (n < 0) return fail(LDP_ERR_INVALID, "negative point count");
@@ -796,10 +797,13 @@ static int pack_records(int format, const float* xyz, const float* rgb, const fl
     const int aligned = (reinterpret_cast<uintptr_t>(out) & 15u) == 0;
     if (format == 0)
         (void)launch_k(ldp::ldp_records_kernel<0>, dim3(grid), dim3(ldp::KO_THREADS), 0, st, xyz, rgb, err, (long long)n,
-                       reinterpret_cast<const long long*>(n_dev), (unsigned long long)first_id, out, aligned);
-    else
+                       reinterpret_cast<const long long*>(n_dev), (unsigned long long)first_id, out, aligned, (const float*)nullptr);
+    else if (format == 1)
         (void)launch_k(ldp::ldp_records_kernel<1>, dim3(grid), dim3(ldp::KO_THREADS), 0, st, xyz, rgb, err, (long long)n,
-                       reinterpret_cast<const long long*>(n_dev), (unsigned long long)first_id, out, aligned);
+                       reinterpret_cast<const long long*>(n_dev), (unsigned long long)first_id, out, aligned, (const float*)nullptr);
+    else
+        (void)launch_k(ldp::ldp_records_kernel<2>, dim3(grid), dim3(ldp::KO_THREADS), 0, st, xyz, rgb, (const float*)nullptr,
+                       (long long)n, reinterpret_cast<const long long*>(n_dev), 0ull, out, aligned, err);
     ++g_launches;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "ldp_records_kernel");
@@ -808,6 +812,12 @@ static int pack_records(int format, const float* xyz, const float* rgb, const fl
 
 int ldp_pack_ply_records(const float* xyz, const float* rgb, int64_t n, const int64_t* n_dev, uint8_t* records_out, void* stream) {
     return pack_records(0, xyz, rgb, nullptr, n, n_dev, 0, records_out, stream);
+}
+
+int ldp_pack_ply_normal_records(const float* xyz, const float* rgb, const float* normals, int64_t n, const int64_t* n_dev,
+                                uint8_t* records_out, void* stream) {
+    if (n > 0 && !normals) return fail(LDP_ERR_INVALID, "null normals");
+    return pack_records(2, xyz, rgb, normals, n, n_dev, 0, records_out, stream);
 }
 
 int ldp_pack_points3d_records(const float* xyz, const float* rgb, const float* err, int64_t n, const int64_t* n_dev,
@@ -1062,8 +1072,9 @@ struct OutlierPlan {
     float4* pts[ldp::OL_MAX_LEVELS];
 };
 
-static int outlier_plan(int64_t n, void* base, OutlierPlan* pl, size_t* bytes) {
-    if (n < 0 || n > 500000000ll) return fail(LDP_ERR_INVALID, "statistical outliers: bad point count");
+// with_stats = false (the normal call) leaves out the per-point means and the partial sums
+static int outlier_plan(int64_t n, void* base, OutlierPlan* pl, size_t* bytes, bool with_stats = true) {
+    if (n < 0 || n > 500000000ll) return fail(LDP_ERR_INVALID, "k-NN search: bad point count");
     size_t off = 0;
     int rc = voxel_plan(n, base, &pl->vws, &off);
     if (rc != LDP_OK) return rc;
@@ -1072,8 +1083,8 @@ static int outlier_plan(int64_t n, void* base, OutlierPlan* pl, size_t* bytes) {
     pl->vstat = reinterpret_cast<int*>(carve(2 * sizeof(int)));
     pl->h_trial = reinterpret_cast<double*>(carve(sizeof(double)));
     pl->stats = reinterpret_cast<double*>(carve(3 * sizeof(double)));
-    pl->m = reinterpret_cast<double*>(carve(N * sizeof(double)));
-    pl->part = reinterpret_cast<double*>(carve((N / ldp::OL_CHUNK + 1) * sizeof(double)));
+    pl->m = reinterpret_cast<double*>(carve(with_stats ? N * sizeof(double) : 0));
+    pl->part = reinterpret_cast<double*>(carve(with_stats ? (N / ldp::OL_CHUNK + 1) * sizeof(double) : 0));
     pl->levels = reinterpret_cast<ldp::OutlierLevel*>(carve(ldp::OL_MAX_LEVELS * sizeof(ldp::OutlierLevel)));
     for (int l = 0; l < ldp::OL_MAX_LEVELS; ++l) {
         pl->keys[l] = reinterpret_cast<unsigned long long*>(carve(cap * sizeof(unsigned long long)));
@@ -1117,24 +1128,12 @@ static void outlier_insert(const float* xyz, int64_t n, double h, const double* 
     scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, cells_out, st);
 }
 
-int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, double std_ratio, int64_t* kept_idx_out,
-                             double* mean_dist_out, double* stats_out, int32_t* status_out, void* workspace, size_t workspace_bytes,
-                             void* stream) {
-    g_launches = 0;
-    if (nb_neighbors < 1 || nb_neighbors > ldp::OL_MAX_K) return fail(LDP_ERR_INVALID, "nb_neighbors must lie in [1, 64]");
-    if (!(std_ratio > 0.0)) return fail(LDP_ERR_INVALID, "std_ratio must be positive");
-    if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    cudaError_t e = cudaMemsetAsync(status_out, 0, 3 * sizeof(int32_t), st);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(status)");
-    if (n == 0) return LDP_OK;
-    if (!xyz || !kept_idx_out || !workspace) return fail(LDP_ERR_INVALID, "null pointer");
-    OutlierPlan pl;
-    size_t need = 0;
-    int rc = outlier_plan(n, workspace, &pl, &need);
-    if (rc != LDP_OK) return rc;
-    if (workspace_bytes < need) return fail(LDP_ERR_WORKSPACE, "outlier workspace too small");
-    const int k = (int)std::min<int64_t>(nb_neighbors, n);
+// Steps 1 and 2 of the k-NN search, shared by ldp_statistical_outliers and ldp_estimate_normals: bounds and a trial grid,
+// whose cell count sets the level-0 cell size (the one host synchronisation), then the pyramid and its level descriptors
+// in pl.levels.  A coordinate that is not finite sets status_out[0] = 1 and leaves *n_levels_out = 0.
+static int knn_pyramid(const float* xyz, int64_t n, int k, OutlierPlan& pl, cudaStream_t st, int32_t* status_out, int* n_levels_out) {
+    *n_levels_out = 0;
+    cudaError_t e;
     ldp::VoxelWs& ws = pl.vws;
     ws.status = pl.vstat;
     const unsigned grid = (unsigned)((n + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
@@ -1167,7 +1166,7 @@ int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, 
         finite = finite && std::isfinite(mn[c]) && std::isfinite(mx[c]);
         ext = std::max(ext, mx[c] - mn[c]);
     }
-    if (!finite) {                                      // status_out[0] = 1 (little-endian int32, zeroed above)
+    if (!finite) {                                      // status_out[0] = 1 (little-endian int32, zeroed by the caller)
         e = cudaMemsetAsync(status_out, 1, 1, st);
         return e == cudaSuccess ? LDP_OK : cuda_fail(e, "cudaMemsetAsync(status)");
     }
@@ -1208,6 +1207,32 @@ int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, 
     }
     (void)launch_k(ldp::ldp_outlier_levels_kernel, dim3(1), dim3(1), 0, st, lv, n_levels, pl.levels);
     ++g_launches;
+    *n_levels_out = n_levels;
+    return LDP_OK;
+}
+
+int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, double std_ratio, int64_t* kept_idx_out,
+                             double* mean_dist_out, double* stats_out, int32_t* status_out, void* workspace, size_t workspace_bytes,
+                             void* stream) {
+    g_launches = 0;
+    if (nb_neighbors < 1 || nb_neighbors > ldp::OL_MAX_K) return fail(LDP_ERR_INVALID, "nb_neighbors must lie in [1, 64]");
+    if (!(std_ratio > 0.0)) return fail(LDP_ERR_INVALID, "std_ratio must be positive");
+    if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    cudaError_t e = cudaMemsetAsync(status_out, 0, 3 * sizeof(int32_t), st);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(status)");
+    if (n == 0) return LDP_OK;
+    if (!xyz || !kept_idx_out || !workspace) return fail(LDP_ERR_INVALID, "null pointer");
+    OutlierPlan pl;
+    size_t need = 0;
+    int rc = outlier_plan(n, workspace, &pl, &need);
+    if (rc != LDP_OK) return rc;
+    if (workspace_bytes < need) return fail(LDP_ERR_WORKSPACE, "outlier workspace too small");
+    const int k = (int)std::min<int64_t>(nb_neighbors, n);
+    int n_levels = 0;
+    if ((rc = knn_pyramid(xyz, n, k, pl, st, status_out, &n_levels)) != LDP_OK || n_levels == 0) return rc;
+    ldp::VoxelWs& ws = pl.vws;
+    const unsigned grid = (unsigned)((n + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
 
     // 3. k nearest, per-point mean distance
     double* m = mean_dist_out ? mean_dist_out : pl.m;
@@ -1215,9 +1240,9 @@ int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, 
     {
         KernelTimer kt(st, "ldp_outlier_knn_kernel");
         const unsigned kgrid = (unsigned)((n + ldp::OL_THREADS - 1) / ldp::OL_THREADS);
-        (void)launch_k(ldp::ldp_outlier_knn_kernel, dim3(kgrid), dim3(ldp::OL_THREADS), (size_t)k * ldp::OL_THREADS * sizeof(double), st,
+        (void)launch_k(ldp::ldp_outlier_knn_kernel<false>, dim3(kgrid), dim3(ldp::OL_THREADS), (size_t)k * ldp::OL_THREADS * sizeof(double), st,
                        (const ldp::OutlierLevel*)pl.levels, n_levels, (long long)n, k,
-                       g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, m, (int*)status_out);
+                       g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, m, (int*)status_out, ldp::NormalArgs{});
         ++g_launches;
     }
 
@@ -1243,6 +1268,49 @@ int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, 
         ++g_launches;
     }
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "statistical outlier kernels");
+    return LDP_OK;
+}
+
+// ---- oriented normals (ldp_outlier.cu: ldp_outlier_knn_kernel<true> and its epilogue)
+int ldp_normals_workspace_bytes(int64_t n, int32_t k, size_t* bytes_out) {
+    if (!bytes_out) return fail(LDP_ERR_INVALID, "null bytes_out");
+    if (k < 3 || k > ldp::OL_MAX_K) return fail(LDP_ERR_INVALID, "k must lie in [3, 64]");
+    OutlierPlan pl;
+    return outlier_plan(n, nullptr, &pl, bytes_out, false);
+}
+
+int ldp_estimate_normals(const float* xyz, int64_t n, int32_t k, const float* centers, int32_t n_centers, const int32_t* center_idx,
+                         float* normals_out, float* curvature_out, int32_t* knn_idx_out, int32_t* status_out, void* workspace,
+                         size_t workspace_bytes, void* stream) {
+    g_launches = 0;
+    if (k < 3 || k > ldp::OL_MAX_K) return fail(LDP_ERR_INVALID, "k must lie in [3, 64]");
+    if (center_idx && !centers) return fail(LDP_ERR_INVALID, "center_idx needs centers");
+    if (centers && n_centers < 1) return fail(LDP_ERR_INVALID, "n_centers must be >= 1 when centers are given");
+    if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    cudaError_t e = cudaMemsetAsync(status_out, 0, 3 * sizeof(int32_t), st);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(status)");
+    if (n == 0) return LDP_OK;
+    if (!xyz || !normals_out || !workspace) return fail(LDP_ERR_INVALID, "null pointer");
+    OutlierPlan pl;
+    size_t need = 0;
+    int rc = outlier_plan(n, workspace, &pl, &need, false);
+    if (rc != LDP_OK) return rc;
+    if (workspace_bytes < need) return fail(LDP_ERR_WORKSPACE, "normals workspace too small");
+    const int k_eff = (int)std::min<int64_t>(k, n);
+    int n_levels = 0;
+    if ((rc = knn_pyramid(xyz, n, k_eff, pl, st, status_out, &n_levels)) != LDP_OK || n_levels == 0) return rc;
+    {
+        KernelTimer kt(st, "ldp_normals_knn_kernel");
+        ldp::NormalArgs na{xyz, centers, center_idx, normals_out, curvature_out, knn_idx_out, centers ? n_centers : 0, 0};
+        const unsigned kgrid = (unsigned)((n + ldp::OL_THREADS - 1) / ldp::OL_THREADS);
+        (void)launch_k(ldp::ldp_outlier_knn_kernel<true>, dim3(kgrid), dim3(ldp::OL_THREADS),
+                       (size_t)k_eff * ldp::OL_THREADS * (sizeof(double) + sizeof(int)), st,
+                       (const ldp::OutlierLevel*)pl.levels, n_levels, (long long)n, k_eff,
+                       g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, (double*)nullptr, (int*)status_out, na);
+        ++g_launches;
+    }
+    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "normal kernels");
     return LDP_OK;
 }
 

@@ -1,6 +1,6 @@
 // Output contract on the device (SURVEY 8a row a15, 8f row 2): the reference turns the path's float colours into
 // uint8 (core/image_utils.py:24-26) and writes one struct.pack per point (core/writers.py:15-46).  Here the records
-// are built where the points are - 15 bytes per vertex for the binary PLY, 43 bytes per point for COLMAP's
+// are built where the points are - 15 bytes per vertex for the binary PLY (27 with a normal), 43 bytes per point for COLMAP's
 // points3D.bin - so a caller copies n * 15 bytes to the host and appends them to the header with one write; and the
 // rows a point cap keeps (densify.py:110-120; the indices stay numpy's default_rng(seed).choice on the host) are
 // gathered on the device.  Included by ldp_api.cu (unity build).
@@ -8,7 +8,7 @@
 
 namespace ldp {
 
-constexpr int KO_THREADS = 256;       // points per CTA: 256 * 15 and 256 * 43 bytes are multiples of 16
+constexpr int KO_THREADS = 256;       // points per CTA: 256 * 15, 256 * 27 and 256 * 43 bytes are multiples of 16
 
 // np.clip(np.round(c * 255.0), 0, 255).astype(np.uint8) on a float32 colour: the product stays float32 (NEP 50),
 // np.round is half-to-even
@@ -38,13 +38,14 @@ __device__ __forceinline__ void flush_records(const uint8_t* smem, uint8_t* out,
 
 // FORMAT 0: PLY vertex  <fff BBB            (core/writers.py:44-45)
 // FORMAT 1: points3D    <Q id <ddd <BBB <d  (core/writers.py:23-26; ids are first_id + i, first_id = 1 for a whole file)
+// FORMAT 2: PLY vertex with a normal  <fff xyz <fff nxyz BBB (core/writers.py write_ply(..., normals=))
 template <int FORMAT>
 __global__ void __launch_bounds__(KO_THREADS)
 ldp_records_kernel(const float* __restrict__ xyz, const float* __restrict__ rgb, const float* __restrict__ err,
                    long long n_max, const long long* __restrict__ n_dev, unsigned long long first_id,
-                   uint8_t* __restrict__ out, int aligned)
+                   uint8_t* __restrict__ out, int aligned, const float* __restrict__ nrm)
 {
-    constexpr int REC = (FORMAT == 0) ? 15 : 43;
+    constexpr int REC = (FORMAT == 0) ? 15 : (FORMAT == 1) ? 43 : 27;
     __shared__ __align__(16) uint8_t rec[KO_THREADS * REC];
     grid_dependency_sync();
     long long n = n_max;
@@ -60,6 +61,11 @@ ldp_records_kernel(const float* __restrict__ xyz, const float* __restrict__ rgb,
         if (FORMAT == 0) {
             put_bytes(d, &x, 4); put_bytes(d + 4, &y, 4); put_bytes(d + 8, &z, 4);
             d[12] = r8; d[13] = g8; d[14] = b8;
+        } else if (FORMAT == 2) {
+            const float nx = nrm[3 * i], ny = nrm[3 * i + 1], nz = nrm[3 * i + 2];
+            put_bytes(d, &x, 4); put_bytes(d + 4, &y, 4); put_bytes(d + 8, &z, 4);
+            put_bytes(d + 12, &nx, 4); put_bytes(d + 16, &ny, 4); put_bytes(d + 20, &nz, 4);
+            d[24] = r8; d[25] = g8; d[26] = b8;
         } else {
             const unsigned long long id = first_id + (unsigned long long)i;
             const double xd = (double)x, yd = (double)y, zd = (double)z, ed = err ? (double)err[i] : 0.0;

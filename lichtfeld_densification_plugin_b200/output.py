@@ -7,6 +7,7 @@ Mirrors, on tensors that stay on the GPU (SURVEY.md 8a row a15, 8f rows 2 and 4)
   ``ldp_pack_ply_records`` / ``ldp_pack_points3d_records`` and reach the host as one copy of 15 / 43 bytes per point)
 * ``voxel_downsample``                 reference densify.py:29-50 (Open3D voxel grid mean; parity unpinned, see the function)
 * ``remove_statistical_outliers``      not in the reference: Open3D's ``remove_statistical_outlier`` (parity unpinned)
+* ``estimate_normals``                 not in the reference: oriented normals by PCA over the exact k nearest neighbours
 * ``apply_point_cap``                  reference densify.py:110-120 (the indices are numpy's own
   ``default_rng(seed).choice`` on the host - PCG64 + a sequential shuffle, microseconds; only the gather is device work)
 * ``subsample_preview_matches``        reference core/pipeline.py:573-582 (debug preview subsample of the kept matches)
@@ -29,6 +30,7 @@ from . import _native as N
 from .core.writers import ply_header
 
 PLY_RECORD_BYTES = 15
+PLY_NORMAL_RECORD_BYTES = 27
 POINTS3D_RECORD_BYTES = 43
 
 
@@ -134,19 +136,29 @@ def to_uint8_rgb(rgb: torch.Tensor) -> torch.Tensor:
 
 
 def ply_records(xyz: torch.Tensor, rgb: torch.Tensor, n: Optional[int] = None, n_dev: Optional[torch.Tensor] = None,
-                out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """uint8 [n * 15] device tensor of PLY vertex records (``<fff`` xyz, ``BBB`` to_uint8_rgb(rgb)).
+                out: Optional[torch.Tensor] = None, normals: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """uint8 [n * 15] device tensor of PLY vertex records (``<fff`` xyz, ``BBB`` to_uint8_rgb(rgb)); with ``normals``
+    [n,3] f32, [n * 27] records (``<fff`` xyz, ``<fff`` normal, ``BBB``).
 
     ``n`` defaults to all rows.  With ``n_dev`` (an int64 device scalar, e.g. ``outputs.ref_offset[-1:]``) only
     ``min(n, n_dev)`` records are written and nothing synchronises with the host."""
     xyz, rgb = _f32c(xyz, "xyz"), _f32c(rgb, "rgb")
     lib, stream = _lib_and_stream(xyz)
     n = int(xyz.shape[0]) if n is None else int(n)
+    rec_bytes = PLY_RECORD_BYTES if normals is None else PLY_NORMAL_RECORD_BYTES
     if out is None:
-        out = torch.empty((n * PLY_RECORD_BYTES,), dtype=torch.uint8, device=xyz.device)
-    N.check(lib.ldp_pack_ply_records(C.c_void_p(xyz.data_ptr()), C.c_void_p(rgb.data_ptr()), n,
-                                     C.c_void_p(n_dev.data_ptr() if n_dev is not None else 0),
-                                     C.c_void_p(out.data_ptr()), C.c_void_p(stream)), "ldp_pack_ply_records")
+        out = torch.empty((n * rec_bytes,), dtype=torch.uint8, device=xyz.device)
+    n_dev_p = C.c_void_p(n_dev.data_ptr() if n_dev is not None else 0)
+    if normals is None:
+        N.check(lib.ldp_pack_ply_records(C.c_void_p(xyz.data_ptr()), C.c_void_p(rgb.data_ptr()), n, n_dev_p,
+                                         C.c_void_p(out.data_ptr()), C.c_void_p(stream)), "ldp_pack_ply_records")
+    else:
+        normals = _f32c(normals, "normals")
+        if tuple(normals.shape) != tuple(xyz.shape):
+            raise ValueError("normals must have the shape of xyz")
+        N.check(lib.ldp_pack_ply_normal_records(C.c_void_p(xyz.data_ptr()), C.c_void_p(rgb.data_ptr()),
+                                                C.c_void_p(normals.data_ptr()), n, n_dev_p, C.c_void_p(out.data_ptr()),
+                                                C.c_void_p(stream)), "ldp_pack_ply_normal_records")
     return out
 
 
@@ -166,12 +178,13 @@ def points3d_records(xyz: torch.Tensor, rgb: torch.Tensor, err: Optional[torch.T
     return out
 
 
-def write_ply(path_out: str, xyz: torch.Tensor, rgb: torch.Tensor) -> None:
-    """The reference's ``write_ply(path, xyz, to_uint8_rgb(rgb))`` for device tensors: same bytes."""
+def write_ply(path_out: str, xyz: torch.Tensor, rgb: torch.Tensor, normals: Optional[torch.Tensor] = None) -> None:
+    """The reference's ``write_ply(path, xyz, to_uint8_rgb(rgb))`` for device tensors: same bytes.  ``normals`` [n,3] f32
+    (``estimate_normals``) adds nx / ny / nz: the bytes of ``core.writers.write_ply(..., normals=)``."""
     n = int(xyz.shape[0])
-    rec = ply_records(xyz, rgb).cpu().numpy() if n else np.zeros((0,), np.uint8)
+    rec = ply_records(xyz, rgb, normals=normals).cpu().numpy() if n else np.zeros((0,), np.uint8)
     with open(path_out, "wb") as f:
-        f.write(ply_header(n))
+        f.write(ply_header(n, normals is not None))
         rec.tofile(f)
 
 
@@ -301,6 +314,59 @@ def remove_statistical_outliers(xyz: torch.Tensor, rgb: torch.Tensor, err: Optio
             "ldp_gather_points")
     mu, sd, thr = (float(v) for v in stats_h.tolist())
     return OutlierResult(xyz=o_xyz, rgb=o_rgb, err=o_err, kept_idx=kept, mean_dist=mean_dist, cloud_mean=mu, std_dev=sd, threshold=thr)
+
+
+@dataclass
+class NormalResult:
+    """What ``estimate_normals`` returns (device tensors, rows in input order)."""
+    normals: torch.Tensor               # [n, 3] f32 unit normals; (0, 0, 0) where undefined
+    curvature: torch.Tensor             # [n] f32 surface variation l0 / (l0 + l1 + l2); NaN where undefined
+    neighbors: Optional[torch.Tensor]   # [n, k_eff] int32 neighbourhoods, ascending (d^2, index); None unless asked for
+    undefined: int                      # points whose normal is undefined (fewer than 3 points, duplicates, a line)
+
+
+def estimate_normals(xyz: torch.Tensor, *, nb_neighbors: int, centers: Optional[torch.Tensor] = None,
+                     center_idx: Optional[torch.Tensor] = None, return_neighbors: bool = False) -> NormalResult:
+    """Oriented normals of a device cloud: PCA over the exact ``nb_neighbors`` nearest points of every point (itself
+    included, ties by index), the eigenvector of the smallest eigenvalue of their f64 covariance.  ``centers`` [c,3]
+    (e.g. camera centres) orients every normal toward ``centers[center_idx[i]]`` (``centers[0]`` without ``center_idx``);
+    without ``centers`` the sign is canonical (largest component positive).  The rule is in include/ldp_b200.h.
+    Synchronises twice: once inside the call (the grid's cell size) and once to read the status."""
+    if not 3 <= int(nb_neighbors) <= 64:
+        raise ValueError("nb_neighbors must lie in [3, 64]")
+    if center_idx is not None and centers is None:
+        raise ValueError("center_idx needs centers")
+    xyz = _f32c(xyz, "xyz")
+    lib, stream = _lib_and_stream(xyz)
+    dev, n = xyz.device, int(xyz.shape[0])
+    k_eff = min(int(nb_neighbors), n)
+    n_centers = 0
+    if centers is not None:
+        centers = _f32c(centers, "centers").to(dev)
+        if centers.dim() != 2 or centers.shape[1] != 3 or centers.shape[0] < 1:
+            raise ValueError("centers must be a [c, 3] float32 tensor with c >= 1")
+        n_centers = int(centers.shape[0])
+    if center_idx is not None:
+        center_idx = center_idx.to(device=dev, dtype=torch.int32).contiguous()
+        if center_idx.shape != (n,):
+            raise ValueError("center_idx must hold one index per point")
+    need = C.c_size_t(0)
+    N.check(lib.ldp_normals_workspace_bytes(n, int(nb_neighbors), C.byref(need)), "ldp_normals_workspace_bytes")
+    ws = torch.empty((max(1, need.value),), dtype=torch.uint8, device=dev)
+    normals = torch.empty((n, 3), dtype=torch.float32, device=dev)
+    curvature = torch.empty((n,), dtype=torch.float32, device=dev)
+    nbrs = torch.empty((n, k_eff), dtype=torch.int32, device=dev) if return_neighbors else None
+    status = torch.zeros((3,), dtype=torch.int32, device=dev)
+    ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)          # noqa: E731
+    N.check(lib.ldp_estimate_normals(ptr(xyz), n, int(nb_neighbors), ptr(centers), n_centers, ptr(center_idx), ptr(normals),
+                                     ptr(curvature), ptr(nbrs), ptr(status), ptr(ws), C.c_size_t(need.value),
+                                     C.c_void_p(stream)), "ldp_estimate_normals")
+    bad, undefined, _ = (int(v) for v in status.cpu().tolist())
+    if bad & 1:
+        raise ValueError("a coordinate is not finite")
+    if bad & 2:
+        raise ValueError("a centre index is out of range")
+    return NormalResult(normals=normals, curvature=curvature, neighbors=nbrs, undefined=undefined)
 
 
 PREVIEW_MAX_MATCHES = 10000       # reference core/pipeline.py:50 _PREVIEW_MAX_MATCHES
