@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define LDP_ABI_VERSION 16
+#define LDP_ABI_VERSION 17
 #define LDP_MAX_NN 16          /* neighbours per reference view (the panel clamps to 10) */
 #define LDP_MAX_BINS 4096      /* coverage tiles per map: ceil(W/tile)*ceil(H/tile), tile = max(1, W/24) */
 
@@ -81,8 +81,8 @@ typedef struct ldp_params {
     float certainty_floor;     /* f32(config.certainty_thresh), core/pipeline.py:407; read only if prologue */
     int32_t no_warped_masks;   /* prologue only.  1: the caller guarantees that every ldp_ref_desc.mask_b[k] of the launch is NULL
                                   (no neighbour masks to sample through the warp): the first kernel's instantiation that reads
-                                  no warp row runs, with the plain kernel's registers and occupancy (and the experimental fused
-                                  front kernel may take raw planes); 0: unknown -- the instantiation that reads the warp planes */
+                                  no warp row runs, with the plain kernel's registers and occupancy; 0: unknown -- the
+                                  instantiation that reads the warp planes */
     uint64_t seed;             /* Philox key */
     int64_t uniforms_per_ref;  /* explicit mode: doubles available per reference view */
     int32_t sm_reserve;        /* SMs the one-CTA-per-SM first draw kernel leaves to kernels of OTHER launches in flight on other
@@ -382,10 +382,9 @@ int ldp_estimate_normals(const float* xyz, int64_t n, int32_t k, const float* ce
                          float* normals_out, float* curvature_out, int32_t* knn_idx_out, int32_t* status_out, void* workspace,
                          size_t workspace_bytes, void* stream);
 
-/* SMs the one-CTA-per-SM first draw kernel leaves free when ldp_params.sm_reserve is -1 (process-wide default, initially 0; the
- * environment variable LDP_SM_RESERVE, when set, wins over both).  With several launches in flight on different streams (engine.DensifyRing) or a
- * collective running beside the path, the free SMs let the other kernels make progress: measured 0.1445 -> 0.1420 ms per
- * step at 3 launches in flight with 16. */
+/* SMs the one-CTA-per-SM first draw kernel leaves free when ldp_params.sm_reserve is -1 (process-wide default, initially 0).
+ * With several launches in flight on different streams (engine.DensifyRing) or a collective running beside the path, the
+ * free SMs let the other kernels make progress: measured 0.1445 -> 0.1420 ms per step at 3 launches in flight with 16. */
 int ldp_set_sm_reserve(int n_sms);
 
 /* Kernel launches enqueued by the last ldp_* call on this thread (for bench.py's gpu_launches). */
@@ -414,9 +413,6 @@ int ldp_debug_read_clocks(const ldp_params* params, void* workspace, long long* 
  * that redo only a multi-view solve; params and workspace as given to that launch. */
 int ldp_debug_force_fixup(int two_view_every, int multiview_every);
 int ldp_debug_read_fixups(const ldp_params* params, void* workspace, int32_t* host_out);
-/* Test hook: pipeline a launch over n sub-batches of views on internal streams (1..8; 0 restores the default, which is
- * one batch unless LDP_SUBBATCH is set).  Results do not depend on it. */
-int ldp_debug_set_subbatches(int n);
 
 /* Measurement hook: enqueue `reps` back-to-back launches of the path's first (dominant, HBM-bound) kernel alone on
  * `stream`, so that bench.py can time its average launch duration with two CUDA events instead of bracketing every

@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-LDP_ABI_VERSION = 16
+LDP_ABI_VERSION = 17
 LDP_MAX_NN = 16
 LDP_MAX_BINS = 4096
 
@@ -110,7 +110,7 @@ REF_DESC_DTYPE = np.dtype(LdpRefDesc)
 EXPORTS = [
     "ldp_abi_version", "ldp_last_error_string", "ldp_sel_capacity", "ldp_workspace_bytes",
     "ldp_densify_refs", "ldp_sample_refs", "ldp_triangulate_samples", "ldp_postprocess_certainty", "ldp_last_launch_count",
-    "ldp_struct_size", "ldp_profile_enable", "ldp_profile_read", "ldp_profile_name", "ldp_debug_set_cluster", "ldp_debug_last_cluster", "ldp_debug_set_subbatches", "ldp_debug_read_clocks", "ldp_debug_launch_stream",
+    "ldp_struct_size", "ldp_profile_enable", "ldp_profile_read", "ldp_profile_name", "ldp_debug_set_cluster", "ldp_debug_last_cluster", "ldp_debug_read_clocks", "ldp_debug_launch_stream",
     "ldp_pack_ply_records", "ldp_pack_points3d_records", "ldp_rgb_to_uint8", "ldp_gather_points", "ldp_gather_rows", "ldp_concat_points", "ldp_scatter_points",
     "ldp_select_kcenters", "ldp_nearest_neighbors", "ldp_voxel_workspace_bytes", "ldp_voxel_downsample", "ldp_set_sm_reserve",
     "ldp_undistort_points", "ldp_debug_force_fixup", "ldp_debug_read_fixups",

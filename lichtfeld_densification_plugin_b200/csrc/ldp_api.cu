@@ -1,7 +1,6 @@
 // C ABI of the densification path (include/ldp_b200.h).  Unity build: the kernels live in the two
 // included translation units; this file carves the workspace, picks launch geometry and enqueues.
 #include <cstdio>
-#include <cstdlib>
 #include <cmath>
 #include <cstring>
 #include <string>
@@ -9,7 +8,6 @@
 #include <vector>
 
 #include "ldp_sample.cu"
-#include "ldp_front.cu"
 #include "ldp_geometry.cu"
 #include "ldp_output.cu"
 #include "ldp_select.cu"
@@ -110,21 +108,29 @@ constexpr size_t K1_SMEM_BUDGET = 200 * 1024;
 
 // Every kernel is launched with programmatic dependent launch allowed: its CTAs may be scheduled while the previous
 // kernel of the stream drains, and block in griddepcontrol.wait (ldp_device.cuh:grid_dependency_sync) until that kernel's
-// memory is visible.  Hides the launch latency at each of the 6 kernel boundaries of a step.  LDP_PDL=0 turns it off.
+// memory is visible.  Hides the launch latency at each of the 6 kernel boundaries of a step.
+// cluster > 0: the grid is launched as thread-block clusters of that many CTAs along x.
 template <typename... KArgs, typename... Args>
-cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-    static const int pdl = [] { const char* e = getenv("LDP_PDL"); return e ? atoi(e) : 1; }();
+cudaError_t launch_k(int cluster, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = block;
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
-    cudaLaunchAttribute attr[1];
+    cudaLaunchAttribute attr[2];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pdl;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    attr[1].id = cudaLaunchAttributeClusterDimension;
+    attr[1].val.clusterDim.x = (unsigned)cluster;
+    attr[1].val.clusterDim.y = 1;
+    attr[1].val.clusterDim.z = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = 1;
+    cfg.numAttrs = cluster > 0 ? 2 : 1;
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+}
+template <typename... KArgs, typename... Args>
+cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+    return launch_k(0, kernel, grid, block, smem, st, std::forward<Args>(args)...);
 }
 
 struct Plan {
@@ -136,28 +142,7 @@ struct Plan {
     int nb2;
     void* zero_base;        // launch state that every call clears with ONE memset: counters, per-view statistics, coverage
     size_t zero_bytes;      //   keys, tile partial slots
-    int use_front;          // the fused persistent front kernel replaces stream + prep
-    int front_grid;
-    size_t front_smem;
 };
-
-// CTAs of the front kernel that are resident at once (2 per SM for up to 4 neighbour planes per stage, else 1)
-int front_grid_size(int nn_stage, size_t smem) {
-    (void)nn_stage;
-    const size_t per_sm = 227 * 1024;
-    int per = (int)(per_sm / (smem + 2048));
-    if (per > 2) per = 2;
-    if (per < 1) per = 1;
-    return per * sm_count();
-}
-
-int choose_subbatches(int n_refs);
-
-int next_epoch() {
-    static int epoch = 0;
-    epoch = (epoch % 0x3fffffff) + 1;      // never 0: the counters are cleared to 0 at the start of every call
-    return epoch;
-}
 
 int64_t sel_capacity(int32_t M) {
     const int64_t m_main = (int64_t)((double)M * 0.85);      // int(M * 0.85), reference core/sampling.py:31
@@ -239,29 +224,7 @@ int make_plan(const ldp_params* p, void* base, Plan* plan) {
         g.prep_lb_cap = (int)align_up((size_t)lb, 4);
     }
     plan->prep_smem = (size_t)g.prep_lb_cap * 8;
-    // ---- which first stage: the fused persistent front kernel (ldp_front.cu) needs the vector path (16-byte aligned rows of
-    //      W % 4 == 0 pixels), coverage tiles wider than a pixel, a known neighbour count <= 8 per view, no warped masks,
-    //      and few enough tiles per view that the resident CTAs can park a whole view (see the deadlock note there)
-    //      MEASURED SLOWER than the two kernels it replaces and therefore OFF unless LDP_FRONT=1 (profiles/r02_summary.md):
-    //      131-140 us against 41 + 27 us at the bench shape.  With one quad per thread and tile every per-tile step (stage
-    //      selection, block reductions, announcement, barriers) is paid per quad: 84 M warp instructions against 25 M.
-    static const int front_mode = [] { const char* e = getenv("LDP_FRONT"); return e ? atoi(e) : 0; }();
-    g.front_nn = p->nn_max;
-    g.front_cache = 0;
-    plan->use_front = 0;
-    plan->front_grid = 0;
-    plan->front_smem = 0;
-    if (front_mode && !p->no_filter && p->W % 4 == 0 && p->scalar_loads == 0 && g.prep_lean && p->nn_max >= 1 && p->nn_max <= 8 &&
-        (!p->prologue || p->no_warped_masks) && choose_subbatches(p->n_refs) == 1 && plan->prep_smem <= 16 * 1024) {
-        size_t smem = ((size_t)ldp::KF_STAGES * g.front_nn + ldp::KF_PARK) * ldp::KF_TILE * sizeof(float) + plan->prep_smem;
-        const size_t cache = (size_t)p->n_refs * ((size_t)g.front_nn * sizeof(void*) + sizeof(int));
-        g.front_cache = (cache <= 12 * 1024) ? 1 : 0;        // what is left of the SM's shared memory beside two CTAs' rings
-        if (g.front_cache) smem += cache;
-        const int grid = front_grid_size(g.front_nn, smem);
-        const size_t tpv = ((size_t)N + ldp::KF_TILE - 1) / ldp::KF_TILE;
-        if (smem <= 200 * 1024 && tpv <= (size_t)3 * grid) { plan->use_front = 1; plan->front_grid = grid; plan->front_smem = smem; }
-    }
-    w.nblk = plan->use_front ? ((size_t)N + ldp::KF_TILE - 1) / ldp::KF_TILE : ((size_t)N + ldp::KS_SPAN - 1) / ldp::KS_SPAN;
+    w.nblk = ((size_t)N + ldp::KS_SPAN - 1) / ldp::KS_SPAN;
 
     size_t off = 0;
     char* b = static_cast<char*>(base);
@@ -294,15 +257,12 @@ int make_plan(const ldp_params* p, void* base, Plan* plan) {
     {
         const size_t z0 = off;
         auto sub = [&](size_t bytes) { char* q = b ? b + off : nullptr; off += align_up(bytes, 8); return q; };
-        w.vword = reinterpret_cast<unsigned long long*>(sub(R * sizeof(unsigned long long)));
         w.gbins = reinterpret_cast<unsigned long long*>(sub(R * w.bins_cap * sizeof(unsigned long long)));
         w.partial = reinterpret_cast<double*>(sub(R * w.nblk * sizeof(double)));
         w.rstat = reinterpret_cast<ldp::RefStat*>(sub(R * sizeof(ldp::RefStat)));
         w.bflags = reinterpret_cast<int32_t*>(sub(R * w.nblk * sizeof(int32_t)));
         w.kept = reinterpret_cast<int32_t*>(sub(R * sizeof(int32_t)));
-        w.fix_count = reinterpret_cast<int32_t*>(sub(ldp::LDP_MAX_SUB * sizeof(int32_t)));
-        w.arrive = reinterpret_cast<int32_t*>(sub(R * sizeof(int32_t)));
-        w.ticket = reinterpret_cast<int32_t*>(sub(8 * sizeof(int32_t)));
+        w.fix_count = reinterpret_cast<int32_t*>(sub(sizeof(int32_t)));
         plan->zero_base = b ? b + z0 : nullptr;
         plan->zero_bytes = off - z0;
         off = align_up(off, 256);
@@ -331,27 +291,9 @@ int check_outputs(const ldp_params* p, const ldp_outputs* o) {
 
 static int vec_ok_for(const ldp_params* p) { return (p->W % 4 == 0 && p->scalar_loads == 0) ? 1 : 0; }
 
-// the fused first stage (ldp_front.cu): persistent CTAs, TMA ring, stream + normalise
-cudaError_t launch_front(const ldp_params* p, const ldp_ref_desc* refs, const ldp_outputs* out, Plan& plan, cudaStream_t st) {
-    static bool configured_dev[MAX_DEVICES] = {};
-        bool& configured = configured_dev[current_device()];
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(ldp::ldp_front_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ldp::ldp_front_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        configured = true;
-    }
-    plan.geom.epoch = next_epoch();
-    const long long total = (long long)plan.ws.nblk * p->n_refs;
-    const unsigned grid = (unsigned)std::min<long long>(plan.front_grid, total);
-    if (p->prologue)
-        return launch_k(ldp::ldp_front_kernel<true>, dim3(grid), dim3(ldp::KF_THREADS), plan.front_smem, st, *p, refs, plan.ws, *out, plan.geom);
-    return launch_k(ldp::ldp_front_kernel<false>, dim3(grid), dim3(ldp::KF_THREADS), plan.front_smem, st, *p, refs, plan.ws, *out, plan.geom);
-}
-
 // the first kernel of the path (also launched alone by ldp_debug_launch_stream for the roofline measurement)
-void launch_stream(const ldp_params* p, const ldp_ref_desc* refs, Plan& plan, cudaStream_t st, int nsubrefs) {
-    const dim3 grid((unsigned)plan.ws.nblk, (unsigned)nsubrefs);
+void launch_stream(const ldp_params* p, const ldp_ref_desc* refs, Plan& plan, cudaStream_t st) {
+    const dim3 grid((unsigned)plan.ws.nblk, (unsigned)p->n_refs);
     if (p->prologue && !p->no_warped_masks) switch (p->nn_max) {      // raw matcher planes: post-processing fused into the read
           case 1: (void)launch_k(ldp::ldp_stream_kernel<1, 2>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
           case 2: (void)launch_k(ldp::ldp_stream_kernel<2, 2>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
@@ -378,9 +320,8 @@ void launch_stream(const ldp_params* p, const ldp_ref_desc* refs, Plan& plan, cu
 }
 
 int launch_sample(const ldp_params* p, const ldp_ref_desc* refs, const double* uniforms, const ldp_outputs* out,
-                  Plan& plan, int vec_ok, cudaStream_t st, int ref0, int nsubrefs) {
+                  Plan& plan, int vec_ok, cudaStream_t st) {
     plan.geom.vec = vec_ok;
-    plan.geom.ref0 = ref0;
     static bool configured_dev[MAX_DEVICES] = {};
         bool& configured = configured_dev[current_device()];
     if (!configured) {
@@ -401,24 +342,13 @@ int launch_sample(const ldp_params* p, const ldp_ref_desc* refs, const double* u
         configured = true;
     }
     if (plan.prep_smem > 64 * 1024) return fail(LDP_ERR_INVALID, "map too wide for the prep kernel tables");
-    const dim3 grid((unsigned)plan.ws.nblk, (unsigned)nsubrefs);
+    const int R = p->n_refs;
+    const dim3 grid((unsigned)plan.ws.nblk, (unsigned)R);
     cudaError_t e;
-    if (plan.use_front) {
-        if (plan.geom.chunk_shift > 7) {      // chunk sums are accumulated with atomics: start from zero
-            e = cudaMemsetAsync(plan.ws.csum, 0, (size_t)nsubrefs * plan.ws.nchunk_pad * sizeof(double), st);
-            if (e == cudaSuccess) e = cudaMemsetAsync(plan.ws.csum0, 0, (size_t)nsubrefs * plan.ws.nchunk_pad * sizeof(double), st);
-            if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(csum)");
-        }
-        { KernelTimer kt(st, "ldp_front_kernel");
-          e = launch_front(p, refs, out, plan, st); }
-        ++g_launches;
-        if (e != cudaSuccess || (e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_front_kernel");
-    } else {
     { KernelTimer kt(st, "ldp_stream_kernel");
-      launch_stream(p, refs, plan, st, nsubrefs); }
+      launch_stream(p, refs, plan, st); }
     ++g_launches;
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_stream_kernel");
-    }
     if (p->no_filter) {
         { KernelTimer kt(st, "ldp_topm_kernel");
           size_t n2 = 1;
@@ -437,53 +367,34 @@ int launch_sample(const ldp_params* p, const ldp_ref_desc* refs, const double* u
               const size_t per = (((n4 + c - 1) / c) + 31) & ~(size_t)31;
               return (c > 1 ? 2 : 1) * keys_cap * 8 + (per / 32) * 4;
           };
-          if (topm_smem(1) <= K1_SMEM_BUDGET && !getenv("LDP_TOPM_GENERIC")) {
+          if (topm_smem(1) <= K1_SMEM_BUDGET) {
               // one cluster of C CTAs per view: the largest C that keeps every view's cluster in one wave (one CTA per SM)
               int csize = 1;
               for (int c = 8; c > 1; c >>= 1)
-                  if ((long long)nsubrefs * c <= sm_count() && (size_t)c * 1024 <= n2) { csize = c; break; }
-              static const int env_c = [] { const char* e = getenv("LDP_TOPM_CLUSTER"); return e ? atoi(e) : 0; }();
-              if ((env_c == 1 || env_c == 2 || env_c == 4 || env_c == 8) && (size_t)env_c <= n2) csize = env_c;
+                  if ((long long)R * c <= sm_count() && (size_t)c * 1024 <= n2) { csize = c; break; }
               const int fc = g_force_cluster;              // test hook
               if ((fc == 1 || fc == 2 || fc == 4 || fc == 8) && (size_t)fc <= n2) csize = fc;
               while (csize > 1 && topm_smem(csize) > K1_SMEM_BUDGET) csize >>= 1;
-              static const int pdl = [] { const char* e = getenv("LDP_PDL"); return e ? atoi(e) : 1; }();
               for (;;) {
-                  cudaLaunchConfig_t cfg = {};
-                  cfg.gridDim = dim3((unsigned)(nsubrefs * csize));
-                  cfg.blockDim = dim3(ldp::K1_THREADS);
-                  cfg.dynamicSmemBytes = topm_smem(csize);
-                  cfg.stream = st;
-                  cudaLaunchAttribute attr[2];
-                  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-                  attr[0].val.programmaticStreamSerializationAllowed = pdl;
-                  attr[1].id = cudaLaunchAttributeClusterDimension;
-                  attr[1].val.clusterDim.x = (unsigned)csize;
-                  attr[1].val.clusterDim.y = 1;
-                  attr[1].val.clusterDim.z = 1;
-                  cfg.attrs = attr;
-                  cfg.numAttrs = csize > 1 ? 2 : 1;
-                  if (cudaLaunchKernelEx(&cfg, ldp::ldp_topm_kernel, *p, refs, plan.ws, *out, plan.geom, csize) == cudaSuccess || csize == 1) break;
+                  if (launch_k(csize > 1 ? csize : 0, ldp::ldp_topm_kernel, dim3((unsigned)(R * csize)), dim3(ldp::K1_THREADS),
+                               topm_smem(csize), st, *p, refs, plan.ws, *out, plan.geom, csize) == cudaSuccess || csize == 1) break;
                   (void)cudaGetLastError();
                   csize >>= 1;                             // cluster not schedulable: smaller one
               }
               g_last_cluster = csize;
           } else
-              (void)launch_k(ldp::ldp_topm_generic_kernel, dim3(nsubrefs), dim3(ldp::K1_THREADS), 0, st, *p, refs, plan.ws, *out, plan.geom); }
+              (void)launch_k(ldp::ldp_topm_generic_kernel, dim3(R), dim3(ldp::K1_THREADS), 0, st, *p, refs, plan.ws, *out, plan.geom); }
         ++g_launches;
         if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_topm_kernel");
         return LDP_OK;
     }
-    if (!plan.use_front) {
     if (plan.geom.chunk_shift > 7) {      // chunk sums are accumulated with atomics: start from zero
-        e = cudaMemsetAsync(plan.ws.csum + (size_t)ref0 * plan.ws.nchunk_pad, 0, (size_t)nsubrefs * plan.ws.nchunk_pad * sizeof(double), st);
-        if (e == cudaSuccess)
-            e = cudaMemsetAsync(plan.ws.csum0 + (size_t)ref0 * plan.ws.nchunk_pad, 0, (size_t)nsubrefs * plan.ws.nchunk_pad * sizeof(double), st);
+        e = cudaMemsetAsync(plan.ws.csum, 0, (size_t)R * plan.ws.nchunk_pad * sizeof(double), st);
+        if (e == cudaSuccess) e = cudaMemsetAsync(plan.ws.csum0, 0, (size_t)R * plan.ws.nchunk_pad * sizeof(double), st);
         if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(csum)");
     }
     { KernelTimer kt(st, "ldp_prep_kernel");
-      static const bool force_generic = getenv("LDP_PREP_GENERIC") != nullptr;
-      if (vec_ok && plan.geom.prep_lean && !force_generic) {
+      if (vec_ok && plan.geom.prep_lean) {
           const bool xc = plan.geom.step_dx == 0;       // W divides the pass stride: a thread stays in one pixel column
 #define LDP_PREP_LAUNCH(CSV) \
           do { if (xc) (void)launch_k(ldp::ldp_prep_kernel<CSV, true>, dim3(grid), dim3(ldp::KS_THREADS), plan.prep_smem, st, *p, refs, plan.ws, *out, plan.geom); \
@@ -500,16 +411,15 @@ int launch_sample(const ldp_params* p, const ldp_ref_desc* refs, const double* u
       } }
     ++g_launches;
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_prep_kernel");
-    }
-    // ---- round 1: independent CTAs, as many per view as the device has SMs for (one CTA per SM: the table fills it)
-    static const int env_reserve = [] { const char* e = getenv("LDP_SM_RESERVE"); return e ? atoi(e) : -1; }();   // SMs left to concurrent
-    const int sm_reserve = env_reserve >= 0 ? env_reserve : (p->sm_reserve >= 0 ? p->sm_reserve : g_sm_reserve);                                             // kernels (other launches in
-    int c_first = (sm_count() - sm_reserve) / nsubrefs;                                                            // flight, communication)
+    // ---- round 1: independent CTAs, as many per view as the device has SMs for (one CTA per SM: the table fills it), less
+    //      the SMs left to concurrent kernels (other launches in flight, communication)
+    const int sm_reserve = p->sm_reserve >= 0 ? p->sm_reserve : g_sm_reserve;
+    int c_first = (sm_count() - sm_reserve) / R;
     if (c_first < 1) c_first = 1;
     if (c_first > (int)plan.ws.draw_cmax) c_first = (int)plan.ws.draw_cmax;
     if (g_force_cluster > 0) c_first = g_force_cluster;
     { KernelTimer kt(st, "ldp_draw_kernel");
-      (void)launch_k(ldp::ldp_draw_kernel<1>, dim3((unsigned)(nsubrefs * c_first)), dim3(ldp::KD_THREADS), plan.k1_smem, st,
+      (void)launch_k(ldp::ldp_draw_kernel<1>, dim3((unsigned)(R * c_first)), dim3(ldp::KD_THREADS), plan.k1_smem, st,
                      *p, refs, uniforms, plan.ws, *out, plan.geom, c_first); }
     ++g_launches;
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_draw_kernel<1>");
@@ -524,30 +434,14 @@ int launch_sample(const ldp_params* p, const ldp_ref_desc* refs, const double* u
         while (want < 8 && (long long)want * (1 << 18) < (long long)plan.geom.N) want <<= 1;
         int csize = 1;
         for (int c = want; c > 1; c >>= 1) {
-            if ((long long)nsubrefs * c > sm_count()) continue;
-            if (max_active_clusters(c, plan.k1_smem) >= nsubrefs) { csize = c; break; }
+            if ((long long)R * c > sm_count()) continue;
+            if (max_active_clusters(c, plan.k1_smem) >= R) { csize = c; break; }
         }
         if (g_force_cluster > 0) csize = g_force_cluster;
-        static const int env_c = [] { const char* e = getenv("LDP_RESUME_CLUSTER"); return e ? atoi(e) : 0; }();
-        if (env_c > 0) csize = env_c;
         KernelTimer kt(st, "ldp_resume_kernel");
         for (;;) {
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3((unsigned)(nsubrefs * csize));
-            cfg.blockDim = dim3(ldp::KD_THREADS);
-            cfg.dynamicSmemBytes = plan.k1_smem;
-            cfg.stream = st;
-            static const int pdl = [] { const char* e = getenv("LDP_PDL"); return e ? atoi(e) : 1; }();
-            cudaLaunchAttribute attr[2];
-            attr[0].id = cudaLaunchAttributeClusterDimension;
-            attr[0].val.clusterDim.x = (unsigned)csize;
-            attr[0].val.clusterDim.y = 1;
-            attr[0].val.clusterDim.z = 1;
-            attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            attr[1].val.programmaticStreamSerializationAllowed = pdl;
-            cfg.attrs = attr;
-            cfg.numAttrs = 2;
-            e = cudaLaunchKernelEx(&cfg, ldp::ldp_draw_kernel<2>, *p, refs, uniforms, plan.ws, *out, plan.geom, c_first);
+            e = launch_k(csize, ldp::ldp_draw_kernel<2>, dim3((unsigned)(R * csize)), dim3(ldp::KD_THREADS), plan.k1_smem, st,
+                         *p, refs, uniforms, plan.ws, *out, plan.geom, c_first);
             if (e == cudaSuccess) break;
             (void)cudaGetLastError();
             if (csize == 1) return cuda_fail(e, "ldp_draw_kernel<2>");
@@ -581,39 +475,24 @@ float parallax_cos_threshold(float min_deg) {
     return unord(lo);
 }
 
-ldp::GeomArgs make_geom_args(const ldp_params* p, const Plan& plan, int have_bestk, int ref0, int sub) {
+ldp::GeomArgs make_geom_args(const ldp_params* p, const Plan& plan, int have_bestk) {
     thread_local float cached_deg = -1.f, cached_cos = 1.f;
     if (p->min_parallax_deg != cached_deg) { cached_cos = parallax_cos_threshold(p->min_parallax_deg); cached_deg = p->min_parallax_deg; }
     ldp::GeomArgs ga;
     ga.par_cos_max = cached_cos;
     ga.have_bestk = have_bestk;
     ga.nb2 = plan.nb2;
-    ga.ref0 = ref0;
-    ga.sub = sub;
-    static const int discard_mode = [] { const char* e = getenv("LDP_DISCARD"); return e ? atoi(e) : 1; }();
-    ga.discard = have_bestk ? discard_mode : 0;
-    static const int fuse_mode = [] { const char* e = getenv("LDP_FUSE_GATHER"); return e ? atoi(e) : 1; }();
-    ga.fused = p->multiview ? 1 : fuse_mode;      // the refinement reads the sample index: a multiview launch always gathers itself
-    static const int prefetch_mode = [] { const char* e = getenv("LDP_GEOM_PREFETCH"); return e ? atoi(e) : 1; }();
-    ga.l2_prefetch = prefetch_mode;
     ga.force_fix_two = g_force_fix_two;
     ga.force_fix_mv = g_force_fix_mv;
     return ga;
 }
 
-// gather -> compute -> fix+plan for views [ref0, ref0 + nsubrefs)
+// gather + compute -> fix + plan
 int launch_geometry(const ldp_params* p, const ldp_ref_desc* refs, const ldp_outputs* out, Plan& plan,
-                    int have_bestk, cudaStream_t st, int ref0, int nsubrefs, int sub) {
-    const ldp::GeomArgs ga = make_geom_args(p, plan, have_bestk, ref0, sub);
-    const dim3 grid((unsigned)plan.nb2, (unsigned)nsubrefs);
-    const dim3 ggrid((unsigned)((plan.ws.sel_cap + ldp::KG_THREADS * KG_SPT - 1) / (ldp::KG_THREADS * KG_SPT)), (unsigned)nsubrefs);
+                    int have_bestk, cudaStream_t st) {
+    const ldp::GeomArgs ga = make_geom_args(p, plan, have_bestk);
+    const dim3 grid((unsigned)plan.nb2, (unsigned)p->n_refs);
     cudaError_t e;
-    if (!ga.fused) {
-        { KernelTimer kt(st, "ldp_gather_kernel");
-          (void)launch_k(ldp::ldp_gather_kernel, dim3(ggrid), dim3(ldp::KG_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
-        ++g_launches;
-        if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_gather_kernel");
-    }
     { KernelTimer kt(st, "ldp_geometry_kernel");
       auto* k2 = p->multiview ? (p->lens ? ldp::ldp_geometry_kernel<true, true> : ldp::ldp_geometry_kernel<false, true>)
                               : (p->lens ? ldp::ldp_geometry_kernel<true, false> : ldp::ldp_geometry_kernel<false, false>);
@@ -623,7 +502,7 @@ int launch_geometry(const ldp_params* p, const ldp_ref_desc* refs, const ldp_out
     { KernelTimer kt(st, "ldp_fix_kernel");
       auto* kf = p->multiview ? (p->lens ? ldp::ldp_fix_kernel<true, true> : ldp::ldp_fix_kernel<false, true>)
                               : (p->lens ? ldp::ldp_fix_kernel<true, false> : ldp::ldp_fix_kernel<false, false>);
-      (void)launch_k(kf, dim3(nsubrefs), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
+      (void)launch_k(kf, dim3(p->n_refs), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
     ++g_launches;
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_fix_kernel");
     return LDP_OK;
@@ -631,7 +510,7 @@ int launch_geometry(const ldp_params* p, const ldp_ref_desc* refs, const ldp_out
 
 // ordered scatter of all views of the launch (needs every view's kept count)
 int launch_pack(const ldp_params* p, const ldp_ref_desc* refs, const ldp_outputs* out, Plan& plan, cudaStream_t st) {
-    const ldp::GeomArgs ga = make_geom_args(p, plan, 1, 0, 0);
+    const ldp::GeomArgs ga = make_geom_args(p, plan, 1);
     const dim3 grid((unsigned)plan.nb2, (unsigned)p->n_refs);
     { KernelTimer kt(st, "ldp_pack_kernel");
       (void)launch_k(ldp::ldp_pack_kernel, dim3(grid), dim3(ldp::K3_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
@@ -639,41 +518,6 @@ int launch_pack(const ldp_params* p, const ldp_ref_desc* refs, const ldp_outputs
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "ldp_pack_kernel");
     return LDP_OK;
-}
-
-// Internal streams for pipelining a launch over sub-batches of views: the kernels of the path stress different
-// resources (HBM stream, issue-bound prep, latency-bound draw, DRAM-latency gather, FP64 geometry), so the kernels of
-// one sub-batch overlap those of the next.  Fork/join with events keeps the call stream-ordered for the caller.
-struct SubStreams {
-    cudaStream_t s[ldp::LDP_MAX_SUB];
-    cudaEvent_t start, done[ldp::LDP_MAX_SUB];
-    bool ok = false;
-};
-SubStreams& substreams() {
-    static thread_local SubStreams ss;
-    if (!ss.ok) {
-        bool good = cudaEventCreateWithFlags(&ss.start, cudaEventDisableTiming) == cudaSuccess;
-        for (int i = 0; i < ldp::LDP_MAX_SUB && good; ++i) {
-            good = cudaStreamCreateWithFlags(&ss.s[i], cudaStreamNonBlocking) == cudaSuccess &&
-                   cudaEventCreateWithFlags(&ss.done[i], cudaEventDisableTiming) == cudaSuccess;
-        }
-        ss.ok = good;
-    }
-    return ss;
-}
-
-int g_force_sub = -1;      // ldp_debug_set_subbatches; -1 = environment / default
-int choose_subbatches(int n_refs) {
-    int n = g_force_sub;
-    if (n < 0) {
-        static int env_n = -2;
-        if (env_n == -2) { const char* e = getenv("LDP_SUBBATCH"); env_n = e ? atoi(e) : 0; }
-        n = env_n;
-    }
-    if (n <= 0) n = 1;
-    if (n > ldp::LDP_MAX_SUB) n = ldp::LDP_MAX_SUB;
-    while (n > 1 && n_refs < 2 * n) --n;
-    return n;
 }
 
 }  // namespace
@@ -704,12 +548,6 @@ int ldp_profile_read(float* ms_out, int max_n) {
 
 int ldp_debug_last_cluster(void) { return g_last_cluster; }
 
-int ldp_debug_set_subbatches(int n) {
-    if (n < -1 || n > ldp::LDP_MAX_SUB) return fail(LDP_ERR_INVALID, "sub-batches must be -1 (default) .. 8");
-    g_force_sub = n;
-    return LDP_OK;
-}
-
 int ldp_debug_launch_stream(const ldp_params* params, const ldp_ref_desc* refs, void* workspace, size_t workspace_bytes,
                             void* stream, int reps) {
     if (!params || !refs || !workspace || reps < 1) return fail(LDP_ERR_INVALID, "bad arguments");
@@ -719,18 +557,9 @@ int ldp_debug_launch_stream(const ldp_params* params, const ldp_ref_desc* refs, 
     if (rc != LDP_OK) return rc;
     if (plan.bytes + (size_t)(base - static_cast<char*>(workspace)) > workspace_bytes) return fail(LDP_ERR_WORKSPACE, "workspace too small");
     plan.geom.vec = vec_ok_for(params);
-    plan.geom.ref0 = 0;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cudaError_t e;
-    if (plan.use_front) {      // the fused front kernel is the first stage on this shape (it cleans its own counters up)
-        ldp_outputs none = {};
-        e = clear_launch_state(plan, st);
-        for (int i = 0; i < reps && e == cudaSuccess; ++i) e = launch_front(params, refs, &none, plan, st);
-        if (e != cudaSuccess) return cuda_fail(e, "ldp_front_kernel");
-    } else {
-        for (int i = 0; i < reps; ++i) launch_stream(params, refs, plan, st, params->n_refs);
-    }
-    e = cudaGetLastError();
+    for (int i = 0; i < reps; ++i) launch_stream(params, refs, plan, st);
+    cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "ldp_stream_kernel");
     return LDP_OK;
 }
@@ -759,20 +588,15 @@ int ldp_debug_read_fixups(const ldp_params* params, void* workspace, int32_t* ho
     int rc = make_plan(params, base, &plan);
     if (rc != LDP_OK) return rc;
     host_out[0] = host_out[1] = 0;
-    int32_t counts[ldp::LDP_MAX_SUB];
-    cudaError_t e = cudaMemcpy(counts, plan.ws.fix_count, sizeof(counts), cudaMemcpyDeviceToHost);
+    int32_t count = 0;
+    cudaError_t e = cudaMemcpy(&count, plan.ws.fix_count, sizeof(count), cudaMemcpyDeviceToHost);
     if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpy(fix_count)");
-    const int nsub = choose_subbatches(params->n_refs);
-    std::vector<int2> list;
-    for (int h = 0; h < nsub; ++h) {           // sub-batch h's worklist starts at its first view * sel_cap (launch_geometry)
-        const int lo = (int)(((long long)h * params->n_refs) / nsub);
-        if (counts[h] <= 0) continue;
-        list.resize((size_t)counts[h]);
-        e = cudaMemcpy(list.data(), plan.ws.fix_list + (size_t)lo * plan.ws.sel_cap, list.size() * sizeof(int2), cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpy(fix_list)");
-        host_out[0] += counts[h];
-        for (const int2& it : list) host_out[1] += (it.y & ldp::MV_FIX) ? 1 : 0;
-    }
+    if (count <= 0) return LDP_OK;
+    std::vector<int2> list((size_t)count);
+    e = cudaMemcpy(list.data(), plan.ws.fix_list, list.size() * sizeof(int2), cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpy(fix_list)");
+    host_out[0] = count;
+    for (const int2& it : list) host_out[1] += (it.y & ldp::MV_FIX) ? 1 : 0;
     return LDP_OK;
 }
 
@@ -1343,49 +1167,6 @@ int ldp_workspace_bytes(const ldp_params* params, size_t* bytes_out) {
 // addresses live in device memory, so alignment cannot be checked here without a copy.  Callers that
 // cannot guarantee it set params->scalar_loads = 1 to force the scalar load path.
 
-// L2 residency for the inter-kernel workspace (weights / p, winning neighbour, sample records): the path re-reads
-// them from several kernels of the same call while ~0.2 GB of certainty planes stream through the 126 MB L2.
-// An access-policy window marks the hot prefix of the workspace as persisting for the kernels of this call.
-struct L2Window {
-    cudaStream_t st;
-    bool active;
-    L2Window(cudaStream_t s, void* base, size_t bytes) : st(s), active(false) {
-        static int mode = -1;          // -1 unknown, 0 off, 1 on
-        static size_t max_window = 0, persist_bytes = 0;
-        if (mode < 0) {
-            const char* env = getenv("LDP_L2_PERSIST");
-            mode = (env && env[0] == '1') ? 1 : 0;
-            if (mode) {
-                int dev = 0;
-                cudaDeviceProp prop;
-                if (cudaGetDevice(&dev) != cudaSuccess || cudaGetDeviceProperties(&prop, dev) != cudaSuccess ||
-                    prop.persistingL2CacheMaxSize <= 0) { mode = 0; }
-                else {
-                    persist_bytes = (size_t)prop.persistingL2CacheMaxSize;
-                    max_window = (size_t)prop.accessPolicyMaxWindowSize;
-                    if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, persist_bytes) != cudaSuccess) { (void)cudaGetLastError(); mode = 0; }
-                }
-            }
-        }
-        if (mode != 1 || bytes == 0) return;
-        cudaStreamAttrValue v = {};
-        v.accessPolicyWindow.base_ptr = base;
-        v.accessPolicyWindow.num_bytes = bytes < max_window ? bytes : max_window;
-        const double ratio = (double)persist_bytes / (double)v.accessPolicyWindow.num_bytes;
-        v.accessPolicyWindow.hitRatio = ratio >= 1.0 ? 1.0f : (float)ratio;
-        v.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        v.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        if (cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &v) == cudaSuccess) active = true;
-        else (void)cudaGetLastError();
-    }
-    ~L2Window() {
-        if (!active) return;
-        cudaStreamAttrValue v = {};
-        v.accessPolicyWindow.num_bytes = 0;
-        (void)cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &v);
-    }
-};
-
 int ldp_densify_refs(const ldp_params* params, const ldp_ref_desc* refs, const double* uniforms,
                      const ldp_outputs* out, void* workspace, size_t workspace_bytes, void* stream) {
     g_launches = 0;
@@ -1402,32 +1183,12 @@ int ldp_densify_refs(const ldp_params* params, const ldp_ref_desc* refs, const d
     if (rc != LDP_OK) return rc;
     if (plan.bytes + (size_t)(base - static_cast<char*>(workspace)) > workspace_bytes) return fail(LDP_ERR_WORKSPACE, "workspace too small");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    // the winning-neighbour plane is written by the first kernel and gathered (1 byte per sample, random) by the fifth
-    L2Window l2(st, plan.ws.bestk, (size_t)params->n_refs * plan.ws.n_pad);      // winning-neighbour plane (1 B / px)
     cudaError_t e = clear_launch_state(plan, st);
     if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(launch state)");
-    const int nsub = choose_subbatches(params->n_refs);
-    if (nsub == 1) {
-        rc = launch_sample(params, refs, uniforms, out, plan, vec_ok_for(params), st, 0, params->n_refs);
-        if (rc != LDP_OK) return rc;
-        rc = launch_geometry(params, refs, out, plan, 1, st, 0, params->n_refs, 0);
-        if (rc != LDP_OK) return rc;
-        return launch_pack(params, refs, out, plan, st);
-    }
-    SubStreams& ss = substreams();
-    if (!ss.ok) return fail(LDP_ERR_CUDA, "cannot create internal streams");
-    if ((e = cudaEventRecord(ss.start, st)) != cudaSuccess) return cuda_fail(e, "cudaEventRecord(start)");
-    for (int h = 0; h < nsub; ++h) {
-        const int lo = (int)(((long long)h * params->n_refs) / nsub), hi = (int)(((long long)(h + 1) * params->n_refs) / nsub);
-        cudaStream_t sh = ss.s[h];
-        if ((e = cudaStreamWaitEvent(sh, ss.start, 0)) != cudaSuccess) return cuda_fail(e, "cudaStreamWaitEvent(start)");
-        rc = launch_sample(params, refs, uniforms, out, plan, vec_ok_for(params), sh, lo, hi - lo);
-        if (rc != LDP_OK) return rc;
-        rc = launch_geometry(params, refs, out, plan, 1, sh, lo, hi - lo, h);
-        if (rc != LDP_OK) return rc;
-        if ((e = cudaEventRecord(ss.done[h], sh)) != cudaSuccess) return cuda_fail(e, "cudaEventRecord(done)");
-        if ((e = cudaStreamWaitEvent(st, ss.done[h], 0)) != cudaSuccess) return cuda_fail(e, "cudaStreamWaitEvent(done)");
-    }
+    rc = launch_sample(params, refs, uniforms, out, plan, vec_ok_for(params), st);
+    if (rc != LDP_OK) return rc;
+    rc = launch_geometry(params, refs, out, plan, 1, st);
+    if (rc != LDP_OK) return rc;
     return launch_pack(params, refs, out, plan, st);
 }
 
@@ -1447,7 +1208,7 @@ int ldp_sample_refs(const ldp_params* params, const ldp_ref_desc* refs, const do
     if (plan.bytes + (size_t)(base - static_cast<char*>(workspace)) > workspace_bytes) return fail(LDP_ERR_WORKSPACE, "workspace too small");
     cudaError_t e = clear_launch_state(plan, static_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(launch state)");
-    return launch_sample(params, refs, uniforms, out, plan, vec_ok_for(params), static_cast<cudaStream_t>(stream), 0, params->n_refs);
+    return launch_sample(params, refs, uniforms, out, plan, vec_ok_for(params), static_cast<cudaStream_t>(stream));
 }
 
 int ldp_triangulate_samples(const ldp_params* params, const ldp_ref_desc* refs, const ldp_outputs* out,
@@ -1467,7 +1228,7 @@ int ldp_triangulate_samples(const ldp_params* params, const ldp_ref_desc* refs, 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     cudaError_t e = clear_launch_state(plan, st);
     if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(launch state)");
-    rc = launch_geometry(params, refs, out, plan, 0, st, 0, params->n_refs, 0);
+    rc = launch_geometry(params, refs, out, plan, 0, st);
     if (rc != LDP_OK) return rc;
     return launch_pack(params, refs, out, plan, st);
 }

@@ -6,8 +6,6 @@
 
 namespace ldp {
 
-constexpr int LDP_MAX_SUB = 8;      // sub-batches a launch may be pipelined over
-
 // ---------------------------------------------------------------------------------------------
 // Workspace carved by the host (ldp_api.cu).  Everything is per reference view r; rows are padded so
 // that float4 / 16-byte accesses stay aligned.
@@ -45,11 +43,7 @@ struct Workspace {
     int32_t* blk_cnt;    // [R][nb2][LDP_MAX_NN] kept samples per 128-sample tile and group (geometry -> pack)
     int32_t* blk_first;  // [R][nb2][LDP_MAX_NN] first sample position per tile and group
     int2* fix_list;      // [R*sel_cap] (view, sample) pairs whose null-vector iteration did not converge
-    int32_t* fix_count;  // [LDP_MAX_SUB] one counter per sub-batch (its list starts at ref0 * sel_cap)
-    int32_t* arrive;     // [R] front kernel: tiles of the view announced so far (zeroed with fix_count)
-    unsigned long long* vword;   // [R] front kernel: (launch epoch << 34 | bad flags << 32 | bits of the f32 normaliser s), one 64-bit
-                         //     store by the CTA that completes the view; 0 until then
-    int32_t* ticket;     // [2] front kernel: next tile ticket, CTAs that have left
+    int32_t* fix_count;  // [1]          entries in fix_list
     int32_t* dstat;      // [R] verdict of the first draw round for the rounds that follow: fail code | inexact << 8
     long long* dbgclk;   // [R][32] phase timestamps of the draw kernel (written only with -DLDP_PHASE_CLOCKS)
     size_t n_pad, n_words, found_cap, sel_cap, topk_cap, nchunk_pad, nblk, bins_cap, draw_cmax;
@@ -74,14 +68,10 @@ struct SampleGeom {     // launch-constant shape of the sampler
     uint32_t t_magic32;           // ceil(2^32 / tile): floor(n / tile) = umulhi(n, t_magic32) for n * tile < 2^32
     int step_dx, step_dy;         // (KS_THREADS * 4) % W, (KS_THREADS * 4) / W: pixel step of the full-grid passes
     int prep_lean;                // the lean prep kernel applies (vector path, W <= 8192)
-    int ref0;           // first view of this sub-launch (views are indexed blockIdx + ref0)
     int draw_ept;       // draw kernel: chunk-table entries per thread (multiple of 8)
     int draw_pre_cap;   // draw kernel: doubles in the padded prefix table
     int draw_ng;        // draw kernel: guide-table buckets
     int draw_smem_bytes; // draw kernel: dynamic shared memory of the launch
-    int front_nn;       // front kernel: neighbour planes a TMA stage holds (max neighbours of the launch)
-    int epoch;          // front kernel: value that marks a view's flag as raised in THIS launch
-    int front_cache;    // front kernel: per-view plane pointers / neighbour counts are cached in shared memory
 };
 
 // ---------------------------------------------------------------------------------------------

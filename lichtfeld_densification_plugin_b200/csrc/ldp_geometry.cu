@@ -67,11 +67,6 @@ struct GeomArgs {           // launch-constant extras computed on the host
     float par_cos_max;      // parallax: keep iff clip(cos) <= par_cos_max  (== f32 arccos/degrees test, see ldp_api.cu)
     int have_bestk;
     int nb2;                // 128-sample tiles per view
-    int ref0;               // first view of this sub-launch
-    int sub;                // sub-batch index (selects the fix-up counter)
-    int discard;            // 1: drop the dead weight rows from L2 (LDP_DISCARD=0 turns it off)
-    int l2_prefetch;        // 1: bulk L2 prefetch of the view's reference image and winner row (LDP_GEOM_PREFETCH=0 turns it off)
-    int fused;              // 1: the geometry kernel gathers its own inputs (no gather kernel, no record round trip)
     // test hook, read by the multiview instantiations only (ldp_debug_force_fixup): n > 0 sends every sample i with i % n == 0
     // to the fix-up as if its two-view solve (force_fix_two) / its multi-view solve (force_fix_mv) had not converged
     int force_fix_two, force_fix_mv;
@@ -510,7 +505,7 @@ __device__ __forceinline__ void gclk_use(uint32_t x) { asm volatile("" :: "r"(x)
 #define GCLK_FLUSH do { } while (0)
 #endif
 
-// Compact per-sample record written by the gather kernel and consumed (coalesced) by the compute kernel.
+// Per-sample inputs gathered by the geometry kernel; stored (pt0 / pt1) for the samples the fix-up re-evaluates.
 struct SampleRec {
     float4 wv;              // winning neighbour's warp row: xA, yA, xB, yB in [-1, 1]
     uint32_t tex[3];        // the four bilinear texels, 3 bytes each: t00 t01 t10 t11
@@ -856,72 +851,6 @@ __device__ bool mv_refine(const ldp_params& P, const RefConst& rc, const PairTab
     return true;
 }
 
-// K2a gather: one thread per sample, few registers, full occupancy: the dependent chain of scattered loads
-// (sample index -> winning neighbour -> warp row -> texels) is what bounds this stage, so it runs with as many
-// threads in flight as the SM holds and leaves a 32-byte record per sample for the arithmetic kernel.
-constexpr int KG_THREADS = 256;
-#ifndef KG_SPT
-#define KG_SPT 2                    // samples per thread: their dependent load chains overlap, and the grid is one wave
-#endif
-#ifndef KG_MIN_BLOCKS
-#define KG_MIN_BLOCKS 6
-#endif
-__global__ void __launch_bounds__(KG_THREADS, KG_MIN_BLOCKS)
-ldp_gather_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const Workspace ws, const ldp_outputs out,
-                  const GeomArgs ga)
-{
-    __shared__ RefConst rc;
-    __shared__ PairTable pc;
-    __shared__ ProView pv;
-    const int r = blockIdx.y + ga.ref0;
-    const int i0 = blockIdx.x * (KG_THREADS * KG_SPT);
-    stage_constants(refs + r, rc, pc, threadIdx.x, KG_THREADS);          // host-written descriptors: no kernel produces them
-    if (P.prologue) stage_proview(refs + r, pv, threadIdx.x);
-    grid_dependency_sync();
-    const int32_t* sel = (out.sel_idx ? out.sel_idx : ws.sel) + (size_t)r * ws.sel_cap;
-    // the sample indices do not depend on anything staged below: fetch them first (rows are sel_cap long, always readable)
-    int idx[KG_SPT];
-#pragma unroll
-    for (int q = 0; q < KG_SPT; ++q) {
-        const int i = i0 + q * KG_THREADS + threadIdx.x;
-        idx[q] = (i < (int)ws.sel_cap) ? __ldg(sel + i) : 0;
-    }
-    const int S = out.n_samples[r];
-    if (ga.discard & 1) {          // the draw kernel was the last reader of this view's p row
-        const char* row = reinterpret_cast<const char*>(ws.w + (size_t)r * ws.n_pad);
-        const int nlines = (int)(ws.n_pad * sizeof(float) / 128);
-        for (int l = blockIdx.x * KG_THREADS + threadIdx.x; l < nlines; l += gridDim.x * KG_THREADS) l2_discard_line(row + (size_t)l * 128);
-    }
-    if (i0 >= S) return;
-    __syncthreads();
-    SampleRec rec[KG_SPT];
-    float craw[KG_SPT];
-#pragma unroll
-    for (int q = 0; q < KG_SPT; ++q) {
-        const int i = i0 + q * KG_THREADS + threadIdx.x;
-        if (i < S) gather_sample(P, rc, pc, pv, ga, ga.have_bestk ? (int)ws.bestk[(size_t)r * ws.n_pad + idx[q]] : 0, idx[q], rec[q], craw[q]);
-    }
-#pragma unroll
-    for (int q = 0; q < KG_SPT; ++q) {
-        const int i = i0 + q * KG_THREADS + threadIdx.x;
-        if (i < S) {
-            const size_t o = (size_t)r * ws.sel_cap + i;
-            ws.pt0[o] = rec[q].wv;                                                                   // record, part 1
-            ws.pt1[o] = make_float4(__uint_as_float(rec[q].tex[0]), __uint_as_float(rec[q].tex[1]), __uint_as_float(rec[q].tex[2]),
-                                    __uint_as_float(rec[q].k_cert));                                 // record, part 2
-            if (P.collect_debug) ws.dbgm[o].x = craw[q];
-        }
-    }
-}
-
-__device__ __forceinline__ void load_record(const Workspace& ws, const ldp_params& P, size_t o, SampleRec& rec, float& craw) {
-    rec.wv = ws.pt0[o];
-    const float4 b = ws.pt1[o];
-    rec.tex[0] = __float_as_uint(b.x); rec.tex[1] = __float_as_uint(b.y); rec.tex[2] = __float_as_uint(b.z);
-    rec.k_cert = __float_as_uint(b.w);
-    craw = P.collect_debug ? ws.dbgm[o].x : 0.f;
-}
-
 // The view's lens table (lens_a, lens_b[]), descriptor -> shared memory, staged like the camera constants: loads first, stores
 // after the caller's other loads are in flight.  Only the LENS instantiations declare and stage it.
 constexpr int LENS_WORDS = (int)(sizeof(ldp_lens) * (LDP_MAX_NN + 1) / 4);
@@ -940,8 +869,8 @@ __device__ __forceinline__ void lens_store(const StagedLens& sl, ldp_lens* dst, 
     for (int q = 0; q < LENS_PER; ++q) if (t + q * K2_THREADS < LENS_WORDS) d[t + q * K2_THREADS] = sl.v[q];
 }
 
-// K2b compute: coalesced record in, per-sample result (in place) + per-tile group statistics out.
-// MV: multiview launch (always fused): a kept sample's point is refined from its other confident neighbours (mv_refine).
+// K2b compute: gathers each sample's inputs, per-sample result (in place) + per-tile group statistics out.
+// MV: multiview launch: a kept sample's point is refined from its other confident neighbours (mv_refine).
 template <bool LENS, bool MV>
 __global__ void __launch_bounds__(K2_THREADS, K2_MIN_BLOCKS)
 ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const Workspace ws, const ldp_outputs out,
@@ -951,7 +880,7 @@ ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, c
     __shared__ PairTable pc;
     __shared__ int s_cnt[LDP_MAX_NN], s_first[LDP_MAX_NN];
     __shared__ ProView pv;
-    const int r = blockIdx.y + ga.ref0;
+    const int r = blockIdx.y;
     GCLK_DECL
     // host-written descriptors, no kernel produces them: their loads are put in flight first and collected after the sample
     // indices are requested, one round trip for both; the prefetches are hints (the winner row was written three kernels ago)
@@ -960,61 +889,54 @@ ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, c
     const ldp_lens* lt = nullptr;
     StagedLens sl;
     if constexpr (LENS) lens_load(refs + r, threadIdx.x, sl);
-    if (ga.fused && ga.l2_prefetch && ga.have_bestk && threadIdx.x == LDP_MAX_NN + 32)
+    if (ga.have_bestk && threadIdx.x == LDP_MAX_NN + 32)
         l2_prefetch_slice(ws.bestk + (size_t)r * ws.n_pad, (size_t)P.H * P.W, blockIdx.x, gridDim.x);
-    if (ga.fused && P.prologue) stage_proview(refs + r, pv, threadIdx.x);
+    if (P.prologue) stage_proview(refs + r, pv, threadIdx.x);
     GCLK(0);
     grid_dependency_sync();
     GCLK(10);
     const int i0 = blockIdx.x * K2_THREADS;
-    int idx_f = 0;
-    if (ga.fused) {
-        const int32_t* sel = (out.sel_idx ? out.sel_idx : ws.sel) + (size_t)r * ws.sel_cap;
-        const int i_ = i0 + threadIdx.x;
-        idx_f = (i_ < (int)ws.sel_cap) ? __ldg(sel + i_) : 0;
-    }
+    const int32_t* sel = (out.sel_idx ? out.sel_idx : ws.sel) + (size_t)r * ws.sel_cap;
+    const int i = i0 + threadIdx.x;
+    const int idx_f = (i < (int)ws.sel_cap) ? __ldg(sel + i) : 0;
     const int S = out.n_samples[r];
-    stage_store(sd, rc, pc, threadIdx.x, K2_THREADS, blockIdx.x, (ga.fused && ga.l2_prefetch) ? (int)gridDim.x : 0);
+    stage_store(sd, rc, pc, threadIdx.x, K2_THREADS, blockIdx.x, (int)gridDim.x);
     if constexpr (LENS) {
         __shared__ __align__(8) ldp_lens s_lens[LDP_MAX_NN + 1];
         lens_store(sl, s_lens, threadIdx.x);
         lt = s_lens;
     }
-    if (ga.fused && (ga.discard & 1)) {
+    if (ga.have_bestk) {                    // the draw kernel of this launch was the last reader of the view's p row
         const char* row = reinterpret_cast<const char*>(ws.w + (size_t)r * ws.n_pad);
         const int nlines = (int)(ws.n_pad * sizeof(float) / 128);
         for (int l = i0 + threadIdx.x; l < nlines; l += gridDim.x * K2_THREADS) l2_discard_line(row + (size_t)l * 128);
     }
     if (i0 >= S) return;
     int k_pre = 0;                          // needs no staged constant: requested before the barrier
-    if (ga.fused && ga.have_bestk && i0 + (int)threadIdx.x < S) k_pre = ws.bestk[(size_t)r * ws.n_pad + idx_f];
+    if (ga.have_bestk && i0 + (int)threadIdx.x < S) k_pre = ws.bestk[(size_t)r * ws.n_pad + idx_f];
     if (threadIdx.x < LDP_MAX_NN) { s_cnt[threadIdx.x] = 0; s_first[threadIdx.x] = 0x7fffffff; }
     __syncthreads();
     GCLK_USE(idx_f); GCLK(1);
-    const int i = i0 + threadIdx.x;
     const int lane = threadIdx.x & 31;
     int keep = 0, grp = -1;
     if (i < S) {
         const size_t o = (size_t)r * ws.sel_cap + i;
         SampleRec rec;
         float craw;
-        if (ga.fused) gather_sample(P, rc, pc, pv, ga, k_pre, idx_f, rec, craw);
-        else load_record(ws, P, o, rec, craw);
+        gather_sample(P, rc, pc, pv, ga, k_pre, idx_f, rec, craw);
         GCLK_USE(rec.tex[0]); GCLK_USE(rec.tex[2]); GCLK_USE(rec.wv.x); GCLK(2);
         SampleResult s;
         eval_sample<false, LENS>(P, rc, pc, ga, lt, rec, craw, s GCLK_PASS);
         if constexpr (MV) {
             if (ga.force_fix_two > 0 && i % ga.force_fix_two == 0) s.converged = false;
         }
-        if (!s.converged && ga.fused) {     // the fix-up reads the record
+        if (!s.converged) {                 // rare: store the record for the fix-up (flag bit 7), keep = 0 for now
             ws.pt0[o] = rec.wv;
             ws.pt1[o] = make_float4(__uint_as_float(rec.tex[0]), __uint_as_float(rec.tex[1]), __uint_as_float(rec.tex[2]),
                                     __uint_as_float(rec.k_cert));
             if (P.collect_debug) ws.dbgm[o].x = craw;
-        }
-        if (!s.converged) {                 // rare: leave the record in place for the fix-up (flag bit 7), keep = 0 for now
-            const int slot = atomicAdd(ws.fix_count + ga.sub, 1);
-            ws.fix_list[(size_t)ga.ref0 * ws.sel_cap + slot] = make_int2(r, i);
+            const int slot = atomicAdd(ws.fix_count, 1);
+            ws.fix_list[slot] = make_int2(r, i);
             ws.flags[o] = (uint8_t)(0x80 | (s.grp << 2));
             s.keep = 0;
         } else {
@@ -1031,8 +953,8 @@ ldp_geometry_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, c
                     } else {                // rare: the fix-up redoes the multi-view solve from the winner's warp row and slot
                         ws.mvrec[o] = rec.wv;           //   (vmask holds the slot until then); pt0 is the fallback
                         ws.vmask[o] = k;
-                        const int slot = atomicAdd(ws.fix_count + ga.sub, 1);
-                        ws.fix_list[(size_t)ga.ref0 * ws.sel_cap + slot] = make_int2(r, i | MV_FIX);
+                        const int slot = atomicAdd(ws.fix_count, 1);
+                        ws.fix_list[slot] = make_int2(r, i | MV_FIX);
                     }
                 }
             }
@@ -1077,10 +999,9 @@ ldp_fix_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const 
     constexpr int TB = 128;                                 // tiles staged per block step
     __shared__ int s_c[TB * LDP_MAX_NN], s_f[TB * LDP_MAX_NN];
     grid_dependency_sync();
-    const int r = blockIdx.x + ga.ref0, tid = threadIdx.x;
-    const int n = ws.fix_count[ga.sub];
+    const int r = blockIdx.x, tid = threadIdx.x;
+    const int n = *ws.fix_count;
     if (n > 0) {
-        const int2* fix_list = ws.fix_list + (size_t)ga.ref0 * ws.sel_cap;
         stage_constants(refs + r, rc, pc, tid, K2_THREADS);
         const ldp_lens* lt = nullptr;
         if constexpr (LENS) {
@@ -1098,7 +1019,7 @@ ldp_fix_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const 
         }
         __syncthreads();
         for (int e = tid; e < n; e += K2_THREADS) {
-            const int2 it = fix_list[e];
+            const int2 it = ws.fix_list[e];
             if (it.x != r) continue;
             const int i = MV ? (it.y & ~MV_FIX) : it.y;
             const size_t o = (size_t)r * ws.sel_cap + i;
@@ -1113,9 +1034,12 @@ ldp_fix_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const 
                 ws.vmask[o] = mask;
                 continue;
             }
-            SampleRec rec;
-            float craw;
-            load_record(ws, P, o, rec, craw);
+            SampleRec rec;                  // the record the geometry kernel stored
+            rec.wv = ws.pt0[o];
+            const float4 b = ws.pt1[o];
+            rec.tex[0] = __float_as_uint(b.x); rec.tex[1] = __float_as_uint(b.y); rec.tex[2] = __float_as_uint(b.z);
+            rec.k_cert = __float_as_uint(b.w);
+            const float craw = P.collect_debug ? ws.dbgm[o].x : 0.f;
             SampleResult s;
             GCLK_DECL
             eval_sample<true, LENS>(P, rc, pc, ga, lt, rec, craw, s GCLK_PASS);

@@ -117,7 +117,7 @@ ldp_stream_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, con
     __shared__ double red_d[32];
     __shared__ float red_f[32];
     __shared__ ProView s_pv;
-    const int r = blockIdx.y + G.ref0, blk = blockIdx.x, tid = threadIdx.x;
+    const int r = blockIdx.y, blk = blockIdx.x, tid = threadIdx.x;
     const int N = G.N;
     const ldp_ref_desc* rd = refs + r;
     const int nn = rd->nn;
@@ -317,14 +317,14 @@ ldp_prep_generic_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ ref
 {
     grid_dependency_sync();
     {   // the draw kernels' selection bitmap: cleared here, one kernel ahead of its first use
-        uint32_t* bm = ws.bitmap + (size_t)(blockIdx.y + G.ref0) * ws.n_words;
+        uint32_t* bm = ws.bitmap + (size_t)blockIdx.y * ws.n_words;
         for (int i = blockIdx.x * KS_THREADS + threadIdx.x; i < (int)ws.n_words; i += gridDim.x * KS_THREADS) bm[i] = 0u;
     }
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ int red_i[32];
     __shared__ float s_s;
     __shared__ int s_bad;
-    const int r = blockIdx.y + G.ref0, blk = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+    const int r = blockIdx.y, blk = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
     const int N = G.N, W = P.W;
     const ldp_ref_desc* rd = refs + r;
     // ---- s: fixed-order reduction of the per-CTA partials (every CTA of the view computes the same value)
@@ -484,7 +484,7 @@ ldp_prep_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const
 {
     grid_dependency_sync();
     {   // the draw kernels' selection bitmap: cleared here, one kernel ahead of its first use
-        uint32_t* bm = ws.bitmap + (size_t)(blockIdx.y + G.ref0) * ws.n_words;
+        uint32_t* bm = ws.bitmap + (size_t)blockIdx.y * ws.n_words;
         for (int i = blockIdx.x * KS_THREADS + threadIdx.x; i < (int)ws.n_words; i += gridDim.x * KS_THREADS) bm[i] = 0u;
     }
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -493,7 +493,7 @@ ldp_prep_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const
     __shared__ int s_bad;
     constexpr int NIT = KS_SPAN / (KS_THREADS * 4);
     constexpr int STEP = KS_THREADS * 4;
-    const int r = blockIdx.y + G.ref0, blk = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+    const int r = blockIdx.y, blk = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
     const int N = G.N, W = P.W;
     const ldp_ref_desc* rd = refs + r;
     LDP_PCLK(0);
@@ -722,7 +722,7 @@ ldp_draw_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const
 
     const int C = (MODE == 1) ? c_first : (int)cluster.num_blocks();
     const int crank = (MODE == 1) ? (int)(blockIdx.x % (unsigned)C) : (int)cluster.block_rank();
-    const int r = blockIdx.x / C + G.ref0;
+    const int r = blockIdx.x / C;
     const int tid = threadIdx.x, lane = tid & 31;
     const int T = blockDim.x;
     const int gtid = crank * T + tid, GT = C * T;
@@ -1262,7 +1262,7 @@ ldp_topm_generic_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ ref
     __shared__ int red_i[32];
     __shared__ uint32_t s_prefix;
     __shared__ int s_remaining;
-    const int r = blockIdx.x + G.ref0, tid = threadIdx.x, T = blockDim.x, N = G.N;
+    const int r = blockIdx.x, tid = threadIdx.x, T = blockDim.x, N = G.N;
     const float* __restrict__ w = ws.w + (size_t)r * ws.n_pad;
     int32_t* __restrict__ sel = (out.sel_idx ? out.sel_idx : ws.sel) + (size_t)r * ws.sel_cap;
     unsigned long long* keys = ws.topk_keys + (size_t)r * ws.topk_cap;
@@ -1503,7 +1503,7 @@ ldp_topm_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const
     __shared__ int s_cnt, s_tot;
     grid_dependency_sync();
     const int rank = (C > 1) ? (int)cl.block_rank() : 0;
-    const int r = (int)(blockIdx.x / (unsigned)C) + G.ref0, tid = threadIdx.x, T = blockDim.x, N = G.N, lane = tid & 31;
+    const int r = (int)(blockIdx.x / (unsigned)C), tid = threadIdx.x, T = blockDim.x, N = G.N, lane = tid & 31;
     const float* __restrict__ w = ws.w + (size_t)r * ws.n_pad;
     int32_t* __restrict__ sel = (out.sel_idx ? out.sel_idx : ws.sel) + (size_t)r * ws.sel_cap;
     const int M = min(P.matches_per_ref, N);

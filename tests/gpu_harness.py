@@ -1,12 +1,14 @@
 """Test infrastructure: run the CUDA path and the oracle on the same inputs and compare stage by stage."""
 from __future__ import annotations
 
+import ctypes as C
 from dataclasses import dataclass, field
 from typing import Dict, List, Optional
 
 import numpy as np
 import torch
 
+from lichtfeld_densification_plugin_b200 import _native as N
 from lichtfeld_densification_plugin_b200.engine import DensifyEngine, PathConfig
 from oracle import densify_oracle as O
 from tests.helpers import oracle_cam
@@ -58,6 +60,7 @@ class GpuRun:
     dbg_matches: Optional[List[np.ndarray]] = None
     dbg_cert: Optional[List[np.ndarray]] = None
     launches: int = 0
+    fixups: int = 0                      # entries of the launch's fix-up worklist (ldp_debug_read_fixups)
 
 
 def run_gpu(engine: DensifyEngine, scene, inputs: List[dict], cfg: PathConfig, uniforms: Optional[np.ndarray] = None,
@@ -78,8 +81,11 @@ def run_gpu(engine: DensifyEngine, scene, inputs: List[dict], cfg: PathConfig, u
                   mask_a=to_dev(inp.get("mask_a")),
                   masks_b=[to_dev(m) for m in inp["masks_b"]] if inp.get("masks_b") is not None else None)
     u = torch.from_numpy(np.ascontiguousarray(uniforms)).to(dev) if uniforms is not None else None
-    out = engine.densify(batch, cfg, uniforms=u, collect_debug=collect_debug, taps=True)
+    pl = engine.prepare(batch, cfg, uniforms=u, collect_debug=collect_debug, taps=True)
+    out = pl.launch()
     torch.cuda.synchronize()
+    fx = (C.c_int32 * 2)()
+    N.check(engine.lib.ldp_debug_read_fixups(C.byref(pl.params), C.c_void_p(pl.workspace.data_ptr()), fx), "ldp_debug_read_fixups")
     off = out.ref_offset.cpu().numpy()
     S = out.n_samples.cpu().numpy()
     R = len(inputs)
@@ -92,7 +98,7 @@ def run_gpu(engine: DensifyEngine, scene, inputs: List[dict], cfg: PathConfig, u
         err=[out.err[off[r]:off[r + 1]].cpu().numpy() for r in range(R)],
         status=out.status.cpu().numpy(), uniforms_used=out.uniforms_used.cpu().numpy(), rounds=out.rounds.cpu().numpy(),
         weight_sum=out.weight_sum.cpu().numpy(), group_order=out.group_order.cpu().numpy(),
-        group_count=out.group_count.cpu().numpy(), launches=out.launches,
+        group_count=out.group_count.cpu().numpy(), launches=out.launches, fixups=int(fx[0]),
     )
     if collect_debug:
         g.dbg_matches = [out.dbg_matches[off[r]:off[r + 1]].cpu().numpy() for r in range(R)]

@@ -245,27 +245,6 @@ def test_select_samples_with_coverage_drop_in(engine):
     assert np.array_equal(top, O.select_samples(cert, 500, no_filter=True))
 
 
-def test_subbatch_pipelining_does_not_change_results(engine, fast_scene):
-    """A launch may be pipelined over sub-batches of views on internal streams: outputs are identical."""
-    scene, inputs = fast_scene
-    c = dict(M=10000, no_filter=False, wm=scene.w_match, hm=scene.h_match)
-    lib = engine.lib
-    base = None
-    try:
-        for nsub in (1, 2, 3, 4):
-            assert lib.ldp_debug_set_subbatches(nsub) == 0
-            g = G.run_gpu(engine, scene, inputs, G.path_cfg(c, seed=5))
-            if base is None:
-                base = g
-                continue
-            for r in range(len(inputs)):
-                assert np.array_equal(base.sel_idx[r], g.sel_idx[r]), (nsub, r)
-                assert np.array_equal(base.xyz[r], g.xyz[r]) and np.array_equal(base.rgb[r], g.rgb[r])
-                assert np.array_equal(base.err[r], g.err[r])
-    finally:
-        lib.ldp_debug_set_subbatches(-1)
-
-
 def _colliding_weight_map(H=90, W=120, seed=11):
     """f32 map, distinct values, in which 49 tiles hold an adjacent-float pair (smaller weight at the lower index) whose
     quotients by s = f32(sum of the border-masked weights) round to the same f32."""
