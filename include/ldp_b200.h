@@ -421,7 +421,7 @@ int ldp_debug_launch_stream(const ldp_params* params, const ldp_ref_desc* refs, 
                             void* stream, int reps);
 
 /* sizeof() of the ABI structs as this library was compiled: which = 0 ldp_params, 1 ldp_ref_desc,
- * 2 ldp_outputs.  Bindings check these against their own struct definitions at load time. */
+ * 2 ldp_outputs, 3 ldp_lens.  Bindings check these against their own struct definitions at load time. */
 int64_t ldp_struct_size(int which);
 
 #ifdef __cplusplus

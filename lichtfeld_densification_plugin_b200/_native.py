@@ -107,16 +107,51 @@ class LdpOutputs(C.Structure):
 
 REF_DESC_DTYPE = np.dtype(LdpRefDesc)
 
-EXPORTS = [
-    "ldp_abi_version", "ldp_last_error_string", "ldp_sel_capacity", "ldp_workspace_bytes",
-    "ldp_densify_refs", "ldp_sample_refs", "ldp_triangulate_samples", "ldp_postprocess_certainty", "ldp_last_launch_count",
-    "ldp_struct_size", "ldp_profile_enable", "ldp_profile_read", "ldp_profile_name", "ldp_debug_set_cluster", "ldp_debug_last_cluster", "ldp_debug_read_clocks", "ldp_debug_launch_stream",
-    "ldp_pack_ply_records", "ldp_pack_points3d_records", "ldp_rgb_to_uint8", "ldp_gather_points", "ldp_gather_rows", "ldp_concat_points", "ldp_scatter_points",
-    "ldp_select_kcenters", "ldp_nearest_neighbors", "ldp_voxel_workspace_bytes", "ldp_voxel_downsample", "ldp_set_sm_reserve",
-    "ldp_undistort_points", "ldp_debug_force_fixup", "ldp_debug_read_fixups",
-    "ldp_outlier_workspace_bytes", "ldp_statistical_outliers", "ldp_debug_outlier_max_shells",
-    "ldp_normals_workspace_bytes", "ldp_estimate_normals", "ldp_pack_ply_normal_records",
-]
+_P, _I32, _I64, _SZ = C.c_void_p, C.c_int32, C.c_int64, C.c_size_t
+_PARAMS, _OUTPUTS, _SZ_OUT = C.POINTER(LdpParams), C.POINTER(LdpOutputs), C.POINTER(C.c_size_t)
+
+# The C ABI, in include/ldp_b200.h's order: name -> (restype, argtypes).  Device pointers and streams are c_void_p.
+SIGNATURES = {
+    "ldp_abi_version": (C.c_int, []),
+    "ldp_last_error_string": (C.c_char_p, []),
+    "ldp_sel_capacity": (_I64, [_I32]),
+    "ldp_workspace_bytes": (C.c_int, [_PARAMS, _SZ_OUT]),
+    "ldp_densify_refs": (C.c_int, [_PARAMS, _P, _P, _OUTPUTS, _P, _SZ, _P]),
+    "ldp_sample_refs": (C.c_int, [_PARAMS, _P, _P, _OUTPUTS, _P, _SZ, _P]),
+    "ldp_triangulate_samples": (C.c_int, [_PARAMS, _P, _OUTPUTS, _P, _SZ, _P]),
+    "ldp_undistort_points": (C.c_int, [C.POINTER(LdpLens), _I64, _P, _P, _P]),
+    "ldp_postprocess_certainty": (C.c_int, [_PARAMS, _P, _P, _SZ, _SZ, _P]),
+    "ldp_pack_ply_records": (C.c_int, [_P, _P, _I64, _P, _P, _P]),
+    "ldp_pack_ply_normal_records": (C.c_int, [_P, _P, _P, _I64, _P, _P, _P]),
+    "ldp_pack_points3d_records": (C.c_int, [_P, _P, _P, _I64, _P, C.c_uint64, _P, _P]),
+    "ldp_rgb_to_uint8": (C.c_int, [_P, _I64, _P, _P]),
+    "ldp_gather_points": (C.c_int, [_P, _P, _P, _P, _I64, _I64, _P, _P, _P, _P, _P]),
+    "ldp_gather_rows": (C.c_int, [_P, _I32, _P, _I64, _I64, _P, _P, _P]),
+    "ldp_concat_points": (C.c_int, [_P, _P, _P, _P, _I32, _I64, _P, _P, _P, _I64, _P, _P, _P]),
+    "ldp_scatter_points": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _I64, _P, _P, _P, _I64, _P, _P, _P]),
+    "ldp_select_kcenters": (C.c_int, [_P, _I32, _I32, _P, _P, _P, _P]),
+    "ldp_nearest_neighbors": (C.c_int, [_P, _I32, _I32, _P, _P]),
+    "ldp_voxel_workspace_bytes": (C.c_int, [_I64, _SZ_OUT]),
+    "ldp_voxel_downsample": (C.c_int, [_P, _P, _I64, C.c_double, _P, _P, _P, _P, _SZ, _P]),
+    "ldp_outlier_workspace_bytes": (C.c_int, [_I64, _I32, _SZ_OUT]),
+    "ldp_statistical_outliers": (C.c_int, [_P, _I64, _I32, C.c_double, _P, _P, _P, _P, _P, _SZ, _P]),
+    "ldp_debug_outlier_max_shells": (C.c_int, [C.c_int]),
+    "ldp_normals_workspace_bytes": (C.c_int, [_I64, _I32, _SZ_OUT]),
+    "ldp_estimate_normals": (C.c_int, [_P, _I64, _I32, _P, _I32, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "ldp_set_sm_reserve": (C.c_int, [C.c_int]),
+    "ldp_last_launch_count": (C.c_int, []),
+    "ldp_profile_enable": (C.c_int, [C.c_int]),
+    "ldp_profile_read": (C.c_int, [C.POINTER(C.c_float), C.c_int]),
+    "ldp_profile_name": (C.c_char_p, [C.c_int]),
+    "ldp_debug_set_cluster": (C.c_int, [C.c_int]),
+    "ldp_debug_last_cluster": (C.c_int, []),
+    "ldp_debug_read_clocks": (C.c_int, [_PARAMS, _P, C.POINTER(C.c_longlong)]),
+    "ldp_debug_force_fixup": (C.c_int, [C.c_int, C.c_int]),
+    "ldp_debug_read_fixups": (C.c_int, [_PARAMS, _P, C.POINTER(C.c_int32)]),
+    "ldp_debug_launch_stream": (C.c_int, [_PARAMS, _P, _P, _SZ, _P, C.c_int]),
+    "ldp_struct_size": (_I64, [C.c_int]),
+}
+EXPORTS = list(SIGNATURES)
 
 _lock = threading.Lock()
 _lib = None
@@ -146,88 +181,11 @@ def load(build_if_missing: bool = False):
             lib = C.CDLL(path)
         except OSError as exc:
             raise NativeLibraryError(f"cannot load {path}: {exc}") from exc
-        for name in EXPORTS:
+        for name, (restype, argtypes) in SIGNATURES.items():
             if not hasattr(lib, name):
                 raise NativeLibraryError(f"{path} does not export {name}")
-        lib.ldp_abi_version.restype = C.c_int
-        lib.ldp_last_error_string.restype = C.c_char_p
-        lib.ldp_sel_capacity.restype = C.c_int64
-        lib.ldp_sel_capacity.argtypes = [C.c_int32]
-        lib.ldp_struct_size.restype = C.c_int64
-        lib.ldp_struct_size.argtypes = [C.c_int]
-        lib.ldp_last_launch_count.restype = C.c_int
-        lib.ldp_profile_enable.restype = C.c_int
-        lib.ldp_profile_enable.argtypes = [C.c_int]
-        lib.ldp_profile_read.restype = C.c_int
-        lib.ldp_debug_last_cluster.restype = C.c_int
-        lib.ldp_debug_set_cluster.restype = C.c_int
-        lib.ldp_debug_set_cluster.argtypes = [C.c_int]
-        lib.ldp_profile_name.restype = C.c_char_p
-        lib.ldp_profile_name.argtypes = [C.c_int]
-        lib.ldp_profile_read.argtypes = [C.POINTER(C.c_float), C.c_int]
-        lib.ldp_workspace_bytes.restype = C.c_int
-        lib.ldp_workspace_bytes.argtypes = [C.POINTER(LdpParams), C.POINTER(C.c_size_t)]
-        for fn in (lib.ldp_densify_refs, lib.ldp_sample_refs):
-            fn.restype = C.c_int
-            fn.argtypes = [C.POINTER(LdpParams), C.c_void_p, C.c_void_p, C.POINTER(LdpOutputs), C.c_void_p,
-                           C.c_size_t, C.c_void_p]
-        lib.ldp_triangulate_samples.restype = C.c_int
-        lib.ldp_triangulate_samples.argtypes = [C.POINTER(LdpParams), C.c_void_p, C.POINTER(LdpOutputs), C.c_void_p,
-                                                C.c_size_t, C.c_void_p]
-        lib.ldp_debug_launch_stream.restype = C.c_int
-        lib.ldp_debug_launch_stream.argtypes = [C.POINTER(LdpParams), C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int]
-        lib.ldp_postprocess_certainty.restype = C.c_int
-        lib.ldp_postprocess_certainty.argtypes = [C.POINTER(LdpParams), C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p]
-        lib.ldp_pack_ply_records.restype = C.c_int
-        lib.ldp_pack_ply_records.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
-        lib.ldp_pack_points3d_records.restype = C.c_int
-        lib.ldp_pack_points3d_records.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_uint64,
-                                                  C.c_void_p, C.c_void_p]
-        lib.ldp_rgb_to_uint8.restype = C.c_int
-        lib.ldp_rgb_to_uint8.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
-        lib.ldp_gather_points.restype = C.c_int
-        lib.ldp_gather_points.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
-                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
-        lib.ldp_gather_rows.restype = C.c_int
-        lib.ldp_gather_rows.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
-        lib.ldp_concat_points.restype = C.c_int
-        lib.ldp_concat_points.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p,
-                                          C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
-        lib.ldp_scatter_points.restype = C.c_int
-        lib.ldp_scatter_points.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int64,
-                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
-        lib.ldp_select_kcenters.restype = C.c_int
-        lib.ldp_select_kcenters.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
-        lib.ldp_nearest_neighbors.restype = C.c_int
-        lib.ldp_nearest_neighbors.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
-        lib.ldp_voxel_workspace_bytes.restype = C.c_int
-        lib.ldp_voxel_workspace_bytes.argtypes = [C.c_int64, C.POINTER(C.c_size_t)]
-        lib.ldp_voxel_downsample.restype = C.c_int
-        lib.ldp_voxel_downsample.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p,
-                                             C.c_void_p, C.c_size_t, C.c_void_p]
-        lib.ldp_set_sm_reserve.restype = C.c_int
-        lib.ldp_set_sm_reserve.argtypes = [C.c_int]
-        lib.ldp_undistort_points.restype = C.c_int
-        lib.ldp_undistort_points.argtypes = [C.POINTER(LdpLens), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
-        lib.ldp_debug_force_fixup.restype = C.c_int
-        lib.ldp_debug_force_fixup.argtypes = [C.c_int, C.c_int]
-        lib.ldp_debug_read_fixups.restype = C.c_int
-        lib.ldp_debug_read_fixups.argtypes = [C.POINTER(LdpParams), C.c_void_p, C.POINTER(C.c_int32)]
-        lib.ldp_outlier_workspace_bytes.restype = C.c_int
-        lib.ldp_outlier_workspace_bytes.argtypes = [C.c_int64, C.c_int32, C.POINTER(C.c_size_t)]
-        lib.ldp_statistical_outliers.restype = C.c_int
-        lib.ldp_statistical_outliers.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p,
-                                                 C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
-        lib.ldp_debug_outlier_max_shells.restype = C.c_int
-        lib.ldp_debug_outlier_max_shells.argtypes = [C.c_int]
-        lib.ldp_normals_workspace_bytes.restype = C.c_int
-        lib.ldp_normals_workspace_bytes.argtypes = [C.c_int64, C.c_int32, C.POINTER(C.c_size_t)]
-        lib.ldp_estimate_normals.restype = C.c_int
-        lib.ldp_estimate_normals.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
-                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
-        lib.ldp_pack_ply_normal_records.restype = C.c_int
-        lib.ldp_pack_ply_normal_records.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
-                                                    C.c_void_p]
+            fn = getattr(lib, name)
+            fn.restype, fn.argtypes = restype, argtypes
         if lib.ldp_abi_version() != LDP_ABI_VERSION:
             raise NativeLibraryError(f"ABI version mismatch: library {lib.ldp_abi_version()}, binding {LDP_ABI_VERSION}")
         for which, struct in enumerate((LdpParams, LdpRefDesc, LdpOutputs, LdpLens)):

@@ -3,6 +3,7 @@
 #include <cstdio>
 #include <cmath>
 #include <cstring>
+#include <mutex>
 #include <string>
 #include <utility>
 #include <vector>
@@ -44,10 +45,30 @@ struct KernelTimer {
     ~KernelTimer() { if (slot >= 0) cudaEventRecord(g_prof_ev[2 * slot + 1], st); }
 };
 
+// First statement of every entry point that enqueues work: ldp_last_launch_count and the profile describe that call alone.
+void begin_call() {
+    g_launches = 0;
+    g_prof_n = 0;
+}
+
+int fail(int code, const char* what) {
+    g_last_error = what ? what : "";
+    return code;
+}
+// Drops the error a failed runtime call left in this thread's last-error slot, so that a later, unrelated check (the
+// caller's own, e.g. torch's after its next launch) does not report it again.
+void clear_last_error() { (void)cudaGetLastError(); }
+int cuda_fail(cudaError_t e, const char* where) {
+    clear_last_error();
+    g_last_error = std::string(where) + ": " + cudaGetErrorString(e);
+    return LDP_ERR_CUDA;
+}
+int check(cudaError_t e, const char* where) { return e == cudaSuccess ? LDP_OK : cuda_fail(e, where); }
+
 constexpr int MAX_DEVICES = 64;
 int current_device() {
     int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) { (void)cudaGetLastError(); dev = 0; }
+    if (cudaGetDevice(&dev) != cudaSuccess) { clear_last_error(); dev = 0; }
     return (dev >= 0 && dev < MAX_DEVICES) ? dev : 0;
 }
 
@@ -72,18 +93,9 @@ int max_active_clusters(int csize, size_t smem) {
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     int n = 0;
-    if (cudaOccupancyMaxActiveClusters(&n, ldp::ldp_draw_kernel<2>, &cfg) != cudaSuccess) { (void)cudaGetLastError(); n = 0; }
+    if (cudaOccupancyMaxActiveClusters(&n, ldp::ldp_draw_kernel<2>, &cfg) != cudaSuccess) { clear_last_error(); n = 0; }
     cache[csize] = n > 0 ? n : -1;
     return cache[csize];
-}
-
-int fail(int code, const char* what) {
-    g_last_error = what ? what : "";
-    return code;
-}
-int cuda_fail(cudaError_t e, const char* where) {
-    g_last_error = std::string(where) + ": " + cudaGetErrorString(e);
-    return LDP_ERR_CUDA;
 }
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
@@ -99,12 +111,13 @@ int sm_count() {          // of the CURRENT device
     if (cached[dev] == 0) {
         int n = 0;
         if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) cached[dev] = n;
-        else { (void)cudaGetLastError(); cached[dev] = 148; }
+        else { clear_last_error(); cached[dev] = 148; }
     }
     return cached[dev];
 }
 
 constexpr size_t K1_SMEM_BUDGET = 200 * 1024;
+constexpr size_t PREP_SMEM_MAX = 64 * 1024;
 
 // Every kernel is launched with programmatic dependent launch allowed: its CTAs may be scheduled while the previous
 // kernel of the stream drains, and block in griddepcontrol.wait (ldp_device.cuh:grid_dependency_sync) until that kernel's
@@ -128,10 +141,91 @@ cudaError_t launch_k(int cluster, void (*kernel)(KArgs...), dim3 grid, dim3 bloc
     cfg.numAttrs = cluster > 0 ? 2 : 1;
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
-template <typename... KArgs, typename... Args>
-cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-    return launch_k(0, kernel, grid, block, smem, st, std::forward<Args>(args)...);
+
+// What the launch returned, counted in ldp_last_launch_count; a failure is reported under the kernel's name.
+int launched(cudaError_t e, const char* name) {
+    ++g_launches;
+    return check(e, name);
 }
+template <typename... KArgs, typename... Args>
+int launch(const char* name, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+    return launched(launch_k(0, kernel, grid, block, smem, st, std::forward<Args>(args)...), name);
+}
+
+// A kernel launched as thread-block clusters: launch_at(c) enqueues it with clusters of c CTAs.  A size the device cannot
+// schedule (odd sizes may not be) falls back to the largest power of two below it.  The size launched is what
+// ldp_debug_last_cluster reports.
+template <typename LaunchAt>
+int launch_cluster(const char* name, int csize, LaunchAt launch_at) {
+    cudaError_t e;
+    while ((e = launch_at(csize)) != cudaSuccess && csize > 1) {
+        clear_last_error();
+        csize = csize > 4 ? 4 : (csize > 2 ? 2 : 1);
+    }
+    g_last_cluster = csize;
+    return launched(e, name);
+}
+
+// ---- instantiations the host picks from
+// [prologue mode][nn_max].  Mode 0: processed certainty planes; 1: raw matcher planes and no neighbour mask anywhere (no
+// warp row is read); 2: raw planes whose post-processing samples the neighbour masks through the warp.  An nn_max outside
+// the unrolled ones (0 = unknown) takes the generic <0, mode>.
+using StreamKernel = decltype(&ldp::ldp_stream_kernel<0, 0>);
+const StreamKernel k_stream[3][9] = {
+    {ldp::ldp_stream_kernel<0, 0>, ldp::ldp_stream_kernel<1, 0>, ldp::ldp_stream_kernel<2, 0>, ldp::ldp_stream_kernel<3, 0>,
+     ldp::ldp_stream_kernel<4, 0>, ldp::ldp_stream_kernel<5, 0>, ldp::ldp_stream_kernel<6, 0>, ldp::ldp_stream_kernel<7, 0>,
+     ldp::ldp_stream_kernel<8, 0>},
+    {ldp::ldp_stream_kernel<0, 1>, ldp::ldp_stream_kernel<1, 1>, ldp::ldp_stream_kernel<2, 1>, ldp::ldp_stream_kernel<3, 1>,
+     ldp::ldp_stream_kernel<4, 1>, ldp::ldp_stream_kernel<0, 1>, ldp::ldp_stream_kernel<0, 1>, ldp::ldp_stream_kernel<0, 1>,
+     ldp::ldp_stream_kernel<0, 1>},
+    {ldp::ldp_stream_kernel<0, 2>, ldp::ldp_stream_kernel<1, 2>, ldp::ldp_stream_kernel<2, 2>, ldp::ldp_stream_kernel<3, 2>,
+     ldp::ldp_stream_kernel<4, 2>, ldp::ldp_stream_kernel<0, 2>, ldp::ldp_stream_kernel<0, 2>, ldp::ldp_stream_kernel<0, 2>,
+     ldp::ldp_stream_kernel<0, 2>},
+};
+// [chunk_shift 5, 6, 7, other][W divides the pass stride: a thread stays in one pixel column]
+using PrepKernel = decltype(&ldp::ldp_prep_generic_kernel);
+const PrepKernel k_prep[4][2] = {
+    {ldp::ldp_prep_kernel<5, false>, ldp::ldp_prep_kernel<5, true>},
+    {ldp::ldp_prep_kernel<6, false>, ldp::ldp_prep_kernel<6, true>},
+    {ldp::ldp_prep_kernel<7, false>, ldp::ldp_prep_kernel<7, true>},
+    {ldp::ldp_prep_kernel<0, false>, ldp::ldp_prep_kernel<0, true>},
+};
+
+// Raises the dynamic shared memory limit of every kernel that takes more than the default 48 KB, once per device (a
+// process may drive several).  Threads that make their first call at the same time wait for one configuration.
+int configure_device() {
+    static std::once_flag once[MAX_DEVICES];
+    static cudaError_t result[MAX_DEVICES];
+    const int dev = current_device();
+    std::call_once(once[dev], [dev] {
+        cudaError_t e = cudaSuccess;
+        auto raise = [&e](const void* kernel, size_t bytes) {
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+        };
+        raise((const void*)ldp::ldp_draw_kernel<1>, K1_SMEM_BUDGET);
+        raise((const void*)ldp::ldp_draw_kernel<2>, K1_SMEM_BUDGET);
+        raise((const void*)ldp::ldp_prep_generic_kernel, PREP_SMEM_MAX);
+        for (const auto& row : k_prep)
+            for (PrepKernel k : row) raise((const void*)k, PREP_SMEM_MAX);
+        raise((const void*)ldp::ldp_topm_kernel, K1_SMEM_BUDGET);
+        raise((const void*)ldp::ldp_kcenters_kernel<true>, K1_SMEM_BUDGET);
+        result[dev] = e;
+    });
+    return check(result[dev], "cudaFuncSetAttribute");
+}
+
+// Bump allocator over a workspace: consecutive blocks, the offset rounded up to `align` bytes after each; base = nullptr
+// only measures.
+struct Carver {
+    char* base;
+    size_t off = 0;
+    template <typename T>
+    T* take(size_t count, size_t align = 256) {
+        T* q = base ? reinterpret_cast<T*>(base + off) : nullptr;
+        off = align_up(off + count * sizeof(T), align);
+        return q;
+    }
+};
 
 struct Plan {
     ldp::Workspace ws;
@@ -226,53 +320,47 @@ int make_plan(const ldp_params* p, void* base, Plan* plan) {
     plan->prep_smem = (size_t)g.prep_lb_cap * 8;
     w.nblk = ((size_t)N + ldp::KS_SPAN - 1) / ldp::KS_SPAN;
 
-    size_t off = 0;
-    char* b = static_cast<char*>(base);
-    auto carve = [&](size_t bytes) { char* q = b ? b + off : nullptr; off = align_up(off + bytes, 256); return q; };
-    w.w = reinterpret_cast<float*>(carve(R * w.n_pad * sizeof(float)));
-    w.bestk = reinterpret_cast<uint8_t*>(carve(R * w.n_pad));
-    w.bitmap = reinterpret_cast<uint32_t*>(carve(R * w.n_words * sizeof(uint32_t)));
-    w.gone = reinterpret_cast<uint32_t*>(carve(R * w.n_words * sizeof(uint32_t)));
+    Carver c{static_cast<char*>(base)};
+    w.w = c.take<float>(R * w.n_pad);
+    w.bestk = c.take<uint8_t>(R * w.n_pad);
+    w.bitmap = c.take<uint32_t>(R * w.n_words);
+    w.gone = c.take<uint32_t>(R * w.n_words);
     w.draw_cmax = 8;
-    w.found = reinterpret_cast<int32_t*>(carve(R * w.draw_cmax * w.found_cap * sizeof(int32_t)));
-    w.fcnt = reinterpret_cast<int32_t*>(carve(R * w.draw_cmax * sizeof(int32_t)));
-    w.sel = reinterpret_cast<int32_t*>(carve(R * w.sel_cap * sizeof(int32_t)));
-    w.pt0 = reinterpret_cast<float4*>(carve(R * w.sel_cap * sizeof(float4)));
-    w.pt1 = reinterpret_cast<float4*>(carve(R * w.sel_cap * sizeof(float4)));
-    w.dbgm = reinterpret_cast<float4*>(carve(p->collect_debug ? R * w.sel_cap * sizeof(float4) : 0));
-    w.flags = reinterpret_cast<uint8_t*>(carve(R * w.sel_cap));
-    w.topk_keys = reinterpret_cast<unsigned long long*>(carve(R * w.topk_cap * sizeof(unsigned long long)));
-    w.csum = reinterpret_cast<double*>(carve(R * w.nchunk_pad * sizeof(double)));
-    w.csum0 = reinterpret_cast<double*>(carve(R * w.nchunk_pad * sizeof(double)));
-    w.dbgclk = reinterpret_cast<long long*>(carve(R * 32 * sizeof(long long)));
+    w.found = c.take<int32_t>(R * w.draw_cmax * w.found_cap);
+    w.fcnt = c.take<int32_t>(R * w.draw_cmax);
+    w.sel = c.take<int32_t>(R * w.sel_cap);
+    w.pt0 = c.take<float4>(R * w.sel_cap);
+    w.pt1 = c.take<float4>(R * w.sel_cap);
+    w.dbgm = c.take<float4>(p->collect_debug ? R * w.sel_cap : 0);
+    w.flags = c.take<uint8_t>(R * w.sel_cap);
+    w.topk_keys = c.take<unsigned long long>(R * w.topk_cap);
+    w.csum = c.take<double>(R * w.nchunk_pad);
+    w.csum0 = c.take<double>(R * w.nchunk_pad);
+    w.dbgclk = c.take<long long>(R * 32);
     plan->nb2 = (int)((w.sel_cap + ldp::K2_THREADS - 1) / ldp::K2_THREADS);
-    w.blk_cnt = reinterpret_cast<int32_t*>(carve(R * plan->nb2 * LDP_MAX_NN * sizeof(int32_t)));
-    w.blk_first = reinterpret_cast<int32_t*>(carve(R * plan->nb2 * LDP_MAX_NN * sizeof(int32_t)));
-    w.fix_list = reinterpret_cast<int2*>(carve(R * w.sel_cap * sizeof(int2)));
-    w.dstat = reinterpret_cast<int32_t*>(carve(R * sizeof(int32_t)));
+    w.blk_cnt = c.take<int32_t>(R * plan->nb2 * LDP_MAX_NN);
+    w.blk_first = c.take<int32_t>(R * plan->nb2 * LDP_MAX_NN);
+    w.fix_list = c.take<int2>(R * w.sel_cap);
+    w.dstat = c.take<int32_t>(R);
     const size_t mv_slots = p->multiview ? R * w.sel_cap : 0;
-    w.vmask = reinterpret_cast<int32_t*>(carve(mv_slots * sizeof(int32_t)));
-    w.mvrec = reinterpret_cast<float4*>(carve(mv_slots * sizeof(float4)));
-    // ---- the zero block (one memset per call, clear_launch_state): 8-byte items first
-    {
-        const size_t z0 = off;
-        auto sub = [&](size_t bytes) { char* q = b ? b + off : nullptr; off += align_up(bytes, 8); return q; };
-        w.gbins = reinterpret_cast<unsigned long long*>(sub(R * w.bins_cap * sizeof(unsigned long long)));
-        w.partial = reinterpret_cast<double*>(sub(R * w.nblk * sizeof(double)));
-        w.rstat = reinterpret_cast<ldp::RefStat*>(sub(R * sizeof(ldp::RefStat)));
-        w.bflags = reinterpret_cast<int32_t*>(sub(R * w.nblk * sizeof(int32_t)));
-        w.kept = reinterpret_cast<int32_t*>(sub(R * sizeof(int32_t)));
-        w.fix_count = reinterpret_cast<int32_t*>(sub(sizeof(int32_t)));
-        plan->zero_base = b ? b + z0 : nullptr;
-        plan->zero_bytes = off - z0;
-        off = align_up(off, 256);
-    }
-    plan->bytes = off;
+    w.vmask = c.take<int32_t>(mv_slots);
+    w.mvrec = c.take<float4>(mv_slots);
+    // ---- the zero block (one memset per call, clear_launch_state): 8-byte items first, packed on 8 bytes
+    const size_t z0 = c.off;
+    w.gbins = c.take<unsigned long long>(R * w.bins_cap, 8);
+    w.partial = c.take<double>(R * w.nblk, 8);
+    w.rstat = c.take<ldp::RefStat>(R, 8);
+    w.bflags = c.take<int32_t>(R * w.nblk, 8);
+    w.kept = c.take<int32_t>(R, 8);
+    w.fix_count = c.take<int32_t>(1, 8);
+    plan->zero_base = base ? static_cast<char*>(base) + z0 : nullptr;
+    plan->zero_bytes = c.off - z0;
+    plan->bytes = align_up(c.off, 256);
     return LDP_OK;
 }
 
-cudaError_t clear_launch_state(const Plan& plan, cudaStream_t st) {
-    return cudaMemsetAsync(plan.zero_base, 0, plan.zero_bytes, st);
+int clear_launch_state(const Plan& plan, cudaStream_t st) {
+    return check(cudaMemsetAsync(plan.zero_base, 0, plan.zero_bytes, st), "cudaMemsetAsync(launch state)");
 }
 
 int check_outputs(const ldp_params* p, const ldp_outputs* o) {
@@ -289,128 +377,79 @@ int check_outputs(const ldp_params* p, const ldp_outputs* o) {
     return LDP_OK;
 }
 
-static int vec_ok_for(const ldp_params* p) { return (p->W % 4 == 0 && p->scalar_loads == 0) ? 1 : 0; }
+// The sample kernels' vector loads: the host wrapper guarantees 16-byte aligned certainty planes when W % 4 == 0; the planes'
+// addresses live in device memory, so alignment cannot be checked here without a copy.  Callers that cannot guarantee it
+// set params->scalar_loads = 1 to force the scalar load path.
+int vec_ok_for(const ldp_params* p) { return (p->W % 4 == 0 && p->scalar_loads == 0) ? 1 : 0; }
+
+// The plan of `p` laid over the caller's workspace from its first 256-byte boundary, checked to fit in workspace_bytes (the
+// read-back hooks, which reuse a launch's workspace, pass SIZE_MAX).
+int bind_plan(const ldp_params* p, void* workspace, size_t workspace_bytes, Plan* plan) {
+    if (!workspace) return fail(LDP_ERR_INVALID, "null workspace");
+    char* base = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace), 256));
+    const int rc = make_plan(p, base, plan);
+    if (rc != LDP_OK) return rc;
+    if (plan->bytes + (size_t)(base - static_cast<char*>(workspace)) > workspace_bytes) return fail(LDP_ERR_WORKSPACE, "workspace too small");
+    plan->geom.vec = vec_ok_for(p);
+    return LDP_OK;
+}
 
 // the first kernel of the path (also launched alone by ldp_debug_launch_stream for the roofline measurement)
-void launch_stream(const ldp_params* p, const ldp_ref_desc* refs, Plan& plan, cudaStream_t st) {
-    const dim3 grid((unsigned)plan.ws.nblk, (unsigned)p->n_refs);
-    if (p->prologue && !p->no_warped_masks) switch (p->nn_max) {      // raw matcher planes: post-processing fused into the read
-          case 1: (void)launch_k(ldp::ldp_stream_kernel<1, 2>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 2: (void)launch_k(ldp::ldp_stream_kernel<2, 2>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 3: (void)launch_k(ldp::ldp_stream_kernel<3, 2>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 4: (void)launch_k(ldp::ldp_stream_kernel<4, 2>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          default: (void)launch_k(ldp::ldp_stream_kernel<0, 2>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-    } else if (p->prologue) switch (p->nn_max) {                      // ... and no neighbour mask anywhere: no warp row is read
-          case 1: (void)launch_k(ldp::ldp_stream_kernel<1, 1>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 2: (void)launch_k(ldp::ldp_stream_kernel<2, 1>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 3: (void)launch_k(ldp::ldp_stream_kernel<3, 1>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 4: (void)launch_k(ldp::ldp_stream_kernel<4, 1>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          default: (void)launch_k(ldp::ldp_stream_kernel<0, 1>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-    } else switch (p->nn_max) {
-          case 1: (void)launch_k(ldp::ldp_stream_kernel<1, 0>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 2: (void)launch_k(ldp::ldp_stream_kernel<2, 0>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 3: (void)launch_k(ldp::ldp_stream_kernel<3, 0>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 4: (void)launch_k(ldp::ldp_stream_kernel<4, 0>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 5: (void)launch_k(ldp::ldp_stream_kernel<5, 0>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 6: (void)launch_k(ldp::ldp_stream_kernel<6, 0>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 7: (void)launch_k(ldp::ldp_stream_kernel<7, 0>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          case 8: (void)launch_k(ldp::ldp_stream_kernel<8, 0>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-          default: (void)launch_k(ldp::ldp_stream_kernel<0, 0>, dim3(grid), dim3(ldp::KS_THREADS), 0, st, *p, refs, plan.ws, plan.geom); break;
-      }
+int launch_stream(const ldp_params* p, const ldp_ref_desc* refs, const Plan& plan, cudaStream_t st) {
+    const int mode = p->prologue ? (p->no_warped_masks ? 1 : 2) : 0;
+    const int nn = (p->nn_max >= 1 && p->nn_max <= 8) ? p->nn_max : 0;
+    return launch("ldp_stream_kernel", k_stream[mode][nn], dim3((unsigned)plan.ws.nblk, (unsigned)p->n_refs), dim3(ldp::KS_THREADS),
+                  0, st, *p, refs, plan.ws, plan.geom);
 }
 
 int launch_sample(const ldp_params* p, const ldp_ref_desc* refs, const double* uniforms, const ldp_outputs* out,
-                  Plan& plan, int vec_ok, cudaStream_t st) {
-    plan.geom.vec = vec_ok;
-    static bool configured_dev[MAX_DEVICES] = {};
-        bool& configured = configured_dev[current_device()];
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(ldp::ldp_draw_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K1_SMEM_BUDGET);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ldp::ldp_draw_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K1_SMEM_BUDGET);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(draw)");
-        e = cudaFuncSetAttribute(ldp::ldp_prep_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(prep)");
-        e = cudaFuncSetAttribute(ldp::ldp_prep_kernel<5, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ldp::ldp_prep_kernel<6, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ldp::ldp_prep_kernel<7, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ldp::ldp_prep_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ldp::ldp_prep_kernel<5, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ldp::ldp_prep_kernel<6, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ldp::ldp_prep_kernel<7, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ldp::ldp_prep_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(prep lean)");
-        configured = true;
-    }
-    if (plan.prep_smem > 64 * 1024) return fail(LDP_ERR_INVALID, "map too wide for the prep kernel tables");
+                  const Plan& plan, cudaStream_t st) {
+    int rc = configure_device();
+    if (rc != LDP_OK) return rc;
+    if (plan.prep_smem > PREP_SMEM_MAX) return fail(LDP_ERR_INVALID, "map too wide for the prep kernel tables");
     const int R = p->n_refs;
     const dim3 grid((unsigned)plan.ws.nblk, (unsigned)R);
-    cudaError_t e;
     { KernelTimer kt(st, "ldp_stream_kernel");
-      launch_stream(p, refs, plan, st); }
-    ++g_launches;
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_stream_kernel");
+      if ((rc = launch_stream(p, refs, plan, st)) != LDP_OK) return rc; }
     if (p->no_filter) {
-        { KernelTimer kt(st, "ldp_topm_kernel");
-          size_t n2 = 1;
-          const size_t Mn = (size_t)std::min((long long)p->matches_per_ref, (long long)plan.geom.N);
-          while (n2 < Mn) n2 <<= 1;
-          static bool topm_configured_dev[MAX_DEVICES] = {};
-        bool& topm_configured = topm_configured_dev[current_device()];
-          if (!topm_configured) {
-              (void)cudaFuncSetAttribute(ldp::ldp_topm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K1_SMEM_BUDGET);
-              topm_configured = true;
-          }
-          // dynamic shared memory of a CTA: its sort buffer(s) + one tie count per 128-pixel row of its slice
-          const size_t n4 = plan.ws.n_pad / 4;
-          auto topm_smem = [&](int c) {
-              const size_t keys_cap = std::max(n2 / (size_t)c, std::min(n2, (size_t)1024));
-              const size_t per = (((n4 + c - 1) / c) + 31) & ~(size_t)31;
-              return (c > 1 ? 2 : 1) * keys_cap * 8 + (per / 32) * 4;
-          };
-          if (topm_smem(1) <= K1_SMEM_BUDGET) {
-              // one cluster of C CTAs per view: the largest C that keeps every view's cluster in one wave (one CTA per SM)
-              int csize = 1;
-              for (int c = 8; c > 1; c >>= 1)
-                  if ((long long)R * c <= sm_count() && (size_t)c * 1024 <= n2) { csize = c; break; }
-              const int fc = g_force_cluster;              // test hook
-              if ((fc == 1 || fc == 2 || fc == 4 || fc == 8) && (size_t)fc <= n2) csize = fc;
-              while (csize > 1 && topm_smem(csize) > K1_SMEM_BUDGET) csize >>= 1;
-              for (;;) {
-                  if (launch_k(csize > 1 ? csize : 0, ldp::ldp_topm_kernel, dim3((unsigned)(R * csize)), dim3(ldp::K1_THREADS),
-                               topm_smem(csize), st, *p, refs, plan.ws, *out, plan.geom, csize) == cudaSuccess || csize == 1) break;
-                  (void)cudaGetLastError();
-                  csize >>= 1;                             // cluster not schedulable: smaller one
-              }
-              g_last_cluster = csize;
-          } else
-              (void)launch_k(ldp::ldp_topm_generic_kernel, dim3(R), dim3(ldp::K1_THREADS), 0, st, *p, refs, plan.ws, *out, plan.geom); }
-        ++g_launches;
-        if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_topm_kernel");
-        return LDP_OK;
+        KernelTimer kt(st, "ldp_topm_kernel");
+        size_t n2 = 1;
+        const size_t Mn = (size_t)std::min((long long)p->matches_per_ref, (long long)plan.geom.N);
+        while (n2 < Mn) n2 <<= 1;
+        // dynamic shared memory of a CTA: its sort buffer(s) + one tie count per 128-pixel row of its slice
+        const size_t n4 = plan.ws.n_pad / 4;
+        auto topm_smem = [&](int c) {
+            const size_t keys_cap = std::max(n2 / (size_t)c, std::min(n2, (size_t)1024));
+            const size_t per = (((n4 + c - 1) / c) + 31) & ~(size_t)31;
+            return (c > 1 ? 2 : 1) * keys_cap * 8 + (per / 32) * 4;
+        };
+        if (topm_smem(1) > K1_SMEM_BUDGET)
+            return launch("ldp_topm_generic_kernel", ldp::ldp_topm_generic_kernel, dim3(R), dim3(ldp::K1_THREADS), 0, st, *p, refs,
+                          plan.ws, *out, plan.geom);
+        // one cluster of C CTAs per view: the largest C that keeps every view's cluster in one wave (one CTA per SM)
+        int csize = 1;
+        for (int c = 8; c > 1; c >>= 1)
+            if ((long long)R * c <= sm_count() && (size_t)c * 1024 <= n2) { csize = c; break; }
+        const int fc = g_force_cluster;              // test hook
+        if ((fc == 1 || fc == 2 || fc == 4 || fc == 8) && (size_t)fc <= n2) csize = fc;
+        while (csize > 1 && topm_smem(csize) > K1_SMEM_BUDGET) csize >>= 1;
+        return launch_cluster("ldp_topm_kernel", csize, [&](int c) {
+            return launch_k(c > 1 ? c : 0, ldp::ldp_topm_kernel, dim3((unsigned)(R * c)), dim3(ldp::K1_THREADS), topm_smem(c), st,
+                            *p, refs, plan.ws, *out, plan.geom, c);
+        });
     }
     if (plan.geom.chunk_shift > 7) {      // chunk sums are accumulated with atomics: start from zero
-        e = cudaMemsetAsync(plan.ws.csum, 0, (size_t)R * plan.ws.nchunk_pad * sizeof(double), st);
-        if (e == cudaSuccess) e = cudaMemsetAsync(plan.ws.csum0, 0, (size_t)R * plan.ws.nchunk_pad * sizeof(double), st);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(csum)");
+        const size_t bytes = (size_t)R * plan.ws.nchunk_pad * sizeof(double);
+        if ((rc = check(cudaMemsetAsync(plan.ws.csum, 0, bytes, st), "cudaMemsetAsync(csum)")) != LDP_OK) return rc;
+        if ((rc = check(cudaMemsetAsync(plan.ws.csum0, 0, bytes, st), "cudaMemsetAsync(csum0)")) != LDP_OK) return rc;
     }
     { KernelTimer kt(st, "ldp_prep_kernel");
-      if (vec_ok && plan.geom.prep_lean) {
-          const bool xc = plan.geom.step_dx == 0;       // W divides the pass stride: a thread stays in one pixel column
-#define LDP_PREP_LAUNCH(CSV) \
-          do { if (xc) (void)launch_k(ldp::ldp_prep_kernel<CSV, true>, dim3(grid), dim3(ldp::KS_THREADS), plan.prep_smem, st, *p, refs, plan.ws, *out, plan.geom); \
-               else (void)launch_k(ldp::ldp_prep_kernel<CSV, false>, dim3(grid), dim3(ldp::KS_THREADS), plan.prep_smem, st, *p, refs, plan.ws, *out, plan.geom); } while (0)
-          switch (plan.geom.chunk_shift) {
-              case 5: LDP_PREP_LAUNCH(5); break;
-              case 6: LDP_PREP_LAUNCH(6); break;
-              case 7: LDP_PREP_LAUNCH(7); break;
-              default: LDP_PREP_LAUNCH(0); break;
-          }
-#undef LDP_PREP_LAUNCH
-      } else {
-          (void)launch_k(ldp::ldp_prep_generic_kernel, dim3(grid), dim3(ldp::KS_THREADS), plan.prep_smem, st, *p, refs, plan.ws, *out, plan.geom);
-      } }
-    ++g_launches;
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_prep_kernel");
+      const int cs = plan.geom.chunk_shift;
+      const bool xc = plan.geom.step_dx == 0;       // W divides the pass stride: a thread stays in one pixel column
+      const PrepKernel kp = (plan.geom.vec && plan.geom.prep_lean) ? k_prep[(cs >= 5 && cs <= 7) ? cs - 5 : 3][xc]
+                                                                   : ldp::ldp_prep_generic_kernel;
+      if ((rc = launch("ldp_prep_kernel", kp, grid, dim3(ldp::KS_THREADS), plan.prep_smem, st, *p, refs, plan.ws, *out, plan.geom)) != LDP_OK)
+          return rc; }
     // ---- round 1: independent CTAs, as many per view as the device has SMs for (one CTA per SM: the table fills it), less
     //      the SMs left to concurrent kernels (other launches in flight, communication)
     const int sm_reserve = p->sm_reserve >= 0 ? p->sm_reserve : g_sm_reserve;
@@ -419,39 +458,28 @@ int launch_sample(const ldp_params* p, const ldp_ref_desc* refs, const double* u
     if (c_first > (int)plan.ws.draw_cmax) c_first = (int)plan.ws.draw_cmax;
     if (g_force_cluster > 0) c_first = g_force_cluster;
     { KernelTimer kt(st, "ldp_draw_kernel");
-      (void)launch_k(ldp::ldp_draw_kernel<1>, dim3((unsigned)(R * c_first)), dim3(ldp::KD_THREADS), plan.k1_smem, st,
-                     *p, refs, uniforms, plan.ws, *out, plan.geom, c_first); }
-    ++g_launches;
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_draw_kernel<1>");
-    {
-        // ---- rounds 2.., coverage, compaction: one cluster per view.  The kernel is a chain of latency-bound phases (table
-        // rebuild, a few hundred draws per round, bitmap compaction): one CTA per 2^18 pixels is as fast as more of them
-        // (measured: 46 views at 512^2, 1 vs 2 vs 4 CTAs: 24.9 / 24.9 / 37 us) and leaves the other SMs to the launches in
-        // flight beside this one (3 in flight: 0.143 -> 0.136 ms per step; 640^2, 32 views: 4 -> 2 CTAs 1.33 -> 1.28 ms per
-        // 250 views).  Capped by what is resident at once (GPC boundaries make that smaller than sm_count / n_refs: ask the
-        // occupancy API).
-        int want = 1;
-        while (want < 8 && (long long)want * (1 << 18) < (long long)plan.geom.N) want <<= 1;
-        int csize = 1;
-        for (int c = want; c > 1; c >>= 1) {
-            if ((long long)R * c > sm_count()) continue;
-            if (max_active_clusters(c, plan.k1_smem) >= R) { csize = c; break; }
-        }
-        if (g_force_cluster > 0) csize = g_force_cluster;
-        KernelTimer kt(st, "ldp_resume_kernel");
-        for (;;) {
-            e = launch_k(csize, ldp::ldp_draw_kernel<2>, dim3((unsigned)(R * csize)), dim3(ldp::KD_THREADS), plan.k1_smem, st,
-                         *p, refs, uniforms, plan.ws, *out, plan.geom, c_first);
-            if (e == cudaSuccess) break;
-            (void)cudaGetLastError();
-            if (csize == 1) return cuda_fail(e, "ldp_draw_kernel<2>");
-            csize = (csize > 4) ? 4 : (csize > 2 ? 2 : 1);      // odd sizes may not be schedulable: fall back
-        }
-        g_last_cluster = csize;
+      if ((rc = launch("ldp_draw_kernel<1>", ldp::ldp_draw_kernel<1>, dim3((unsigned)(R * c_first)), dim3(ldp::KD_THREADS), plan.k1_smem,
+                       st, *p, refs, uniforms, plan.ws, *out, plan.geom, c_first)) != LDP_OK)
+          return rc; }
+    // ---- rounds 2.., coverage, compaction: one cluster per view.  The kernel is a chain of latency-bound phases (table
+    // rebuild, a few hundred draws per round, bitmap compaction): one CTA per 2^18 pixels is as fast as more of them
+    // (measured: 46 views at 512^2, 1 vs 2 vs 4 CTAs: 24.9 / 24.9 / 37 us) and leaves the other SMs to the launches in
+    // flight beside this one (3 in flight: 0.143 -> 0.136 ms per step; 640^2, 32 views: 4 -> 2 CTAs 1.33 -> 1.28 ms per
+    // 250 views).  Capped by what is resident at once (GPC boundaries make that smaller than sm_count / n_refs: ask the
+    // occupancy API).
+    int want = 1;
+    while (want < 8 && (long long)want * (1 << 18) < (long long)plan.geom.N) want <<= 1;
+    int csize = 1;
+    for (int c = want; c > 1; c >>= 1) {
+        if ((long long)R * c > sm_count()) continue;
+        if (max_active_clusters(c, plan.k1_smem) >= R) { csize = c; break; }
     }
-    ++g_launches;
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_draw_kernel");
-    return LDP_OK;
+    if (g_force_cluster > 0) csize = g_force_cluster;
+    KernelTimer kt(st, "ldp_resume_kernel");
+    return launch_cluster("ldp_draw_kernel<2>", csize, [&](int c) {
+        return launch_k(c, ldp::ldp_draw_kernel<2>, dim3((unsigned)(R * c)), dim3(ldp::KD_THREADS), plan.k1_smem, st,
+                        *p, refs, uniforms, plan.ws, *out, plan.geom, c_first);
+    });
 }
 
 // Largest f32 cosine d for which the reference's parallax test passes, i.e. for which
@@ -487,37 +515,25 @@ ldp::GeomArgs make_geom_args(const ldp_params* p, const Plan& plan, int have_bes
     return ga;
 }
 
-// gather + compute -> fix + plan
-int launch_geometry(const ldp_params* p, const ldp_ref_desc* refs, const ldp_outputs* out, Plan& plan,
-                    int have_bestk, cudaStream_t st) {
-    const ldp::GeomArgs ga = make_geom_args(p, plan, have_bestk);
+// gather + compute -> fix + plan, then the ordered scatter of all views of the launch (needs every view's kept count)
+int launch_triangulate(const ldp_params* p, const ldp_ref_desc* refs, const ldp_outputs* out, const Plan& plan,
+                       int have_bestk, cudaStream_t st) {
+    ldp::GeomArgs ga = make_geom_args(p, plan, have_bestk);
     const dim3 grid((unsigned)plan.nb2, (unsigned)p->n_refs);
-    cudaError_t e;
+    int rc;
+    // The order in which these instantiations are first named here steers the device compiler's inlining: as a [lens][mv]
+    // table, ldp_fix_kernel<true, true> compiles to different code (166 instead of 158 registers, 272 bytes of stack).
     { KernelTimer kt(st, "ldp_geometry_kernel");
-      auto* k2 = p->multiview ? (p->lens ? ldp::ldp_geometry_kernel<true, true> : ldp::ldp_geometry_kernel<false, true>)
+      auto* k2 =p->multiview ? (p->lens ? ldp::ldp_geometry_kernel<true, true> : ldp::ldp_geometry_kernel<false, true>)
                               : (p->lens ? ldp::ldp_geometry_kernel<true, false> : ldp::ldp_geometry_kernel<false, false>);
-      (void)launch_k(k2, dim3(grid), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
-    ++g_launches;
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_geometry_kernel");
+      if ((rc = launch("ldp_geometry_kernel", k2, grid, dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga)) != LDP_OK) return rc; }
     { KernelTimer kt(st, "ldp_fix_kernel");
       auto* kf = p->multiview ? (p->lens ? ldp::ldp_fix_kernel<true, true> : ldp::ldp_fix_kernel<false, true>)
                               : (p->lens ? ldp::ldp_fix_kernel<true, false> : ldp::ldp_fix_kernel<false, false>);
-      (void)launch_k(kf, dim3(p->n_refs), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
-    ++g_launches;
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ldp_fix_kernel");
-    return LDP_OK;
-}
-
-// ordered scatter of all views of the launch (needs every view's kept count)
-int launch_pack(const ldp_params* p, const ldp_ref_desc* refs, const ldp_outputs* out, Plan& plan, cudaStream_t st) {
-    const ldp::GeomArgs ga = make_geom_args(p, plan, 1);
-    const dim3 grid((unsigned)plan.nb2, (unsigned)p->n_refs);
-    { KernelTimer kt(st, "ldp_pack_kernel");
-      (void)launch_k(ldp::ldp_pack_kernel, dim3(grid), dim3(ldp::K3_THREADS), 0, st, *p, refs, plan.ws, *out, ga); }
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_pack_kernel");
-    return LDP_OK;
+      if ((rc = launch("ldp_fix_kernel", kf, dim3(p->n_refs), dim3(ldp::K2_THREADS), 0, st, *p, refs, plan.ws, *out, ga)) != LDP_OK) return rc; }
+    ga.have_bestk = 1;
+    KernelTimer kt(st, "ldp_pack_kernel");
+    return launch("ldp_pack_kernel", ldp::ldp_pack_kernel, grid, dim3(ldp::K3_THREADS), 0, st, *p, refs, plan.ws, *out, ga);
 }
 
 }  // namespace
@@ -550,28 +566,21 @@ int ldp_debug_last_cluster(void) { return g_last_cluster; }
 
 int ldp_debug_launch_stream(const ldp_params* params, const ldp_ref_desc* refs, void* workspace, size_t workspace_bytes,
                             void* stream, int reps) {
+    begin_call();
     if (!params || !refs || !workspace || reps < 1) return fail(LDP_ERR_INVALID, "bad arguments");
     Plan plan;
-    char* base = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace), 256));
-    int rc = make_plan(params, base, &plan);
-    if (rc != LDP_OK) return rc;
-    if (plan.bytes + (size_t)(base - static_cast<char*>(workspace)) > workspace_bytes) return fail(LDP_ERR_WORKSPACE, "workspace too small");
-    plan.geom.vec = vec_ok_for(params);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    for (int i = 0; i < reps; ++i) launch_stream(params, refs, plan, st);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_stream_kernel");
-    return LDP_OK;
+    int rc = bind_plan(params, workspace, workspace_bytes, &plan);
+    for (int i = 0; i < reps && rc == LDP_OK; ++i) rc = launch_stream(params, refs, plan, static_cast<cudaStream_t>(stream));
+    return rc;
 }
 
 int ldp_debug_read_clocks(const ldp_params* params, void* workspace, long long* host_out) {
+    if (!params || !workspace || !host_out) return fail(LDP_ERR_INVALID, "bad arguments");
     Plan plan;
-    char* base = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace), 256));
-    int rc = make_plan(params, base, &plan);
+    const int rc = bind_plan(params, workspace, SIZE_MAX, &plan);
     if (rc != LDP_OK) return rc;
-    cudaError_t e = cudaMemcpy(host_out, plan.ws.dbgclk, (size_t)params->n_refs * 32 * sizeof(long long), cudaMemcpyDeviceToHost);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpy(dbgclk)");
-    return LDP_OK;
+    return check(cudaMemcpy(host_out, plan.ws.dbgclk, (size_t)params->n_refs * 32 * sizeof(long long), cudaMemcpyDeviceToHost),
+                 "cudaMemcpy(dbgclk)");
 }
 
 int ldp_debug_force_fixup(int two_view_every, int multiview_every) {
@@ -584,17 +593,17 @@ int ldp_debug_force_fixup(int two_view_every, int multiview_every) {
 int ldp_debug_read_fixups(const ldp_params* params, void* workspace, int32_t* host_out) {
     if (!params || !workspace || !host_out) return fail(LDP_ERR_INVALID, "bad arguments");
     Plan plan;
-    char* base = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace), 256));
-    int rc = make_plan(params, base, &plan);
+    int rc = bind_plan(params, workspace, SIZE_MAX, &plan);
     if (rc != LDP_OK) return rc;
     host_out[0] = host_out[1] = 0;
     int32_t count = 0;
-    cudaError_t e = cudaMemcpy(&count, plan.ws.fix_count, sizeof(count), cudaMemcpyDeviceToHost);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpy(fix_count)");
+    if ((rc = check(cudaMemcpy(&count, plan.ws.fix_count, sizeof(count), cudaMemcpyDeviceToHost), "cudaMemcpy(fix_count)")) != LDP_OK)
+        return rc;
     if (count <= 0) return LDP_OK;
     std::vector<int2> list((size_t)count);
-    e = cudaMemcpy(list.data(), plan.ws.fix_list, list.size() * sizeof(int2), cudaMemcpyDeviceToHost);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpy(fix_list)");
+    if ((rc = check(cudaMemcpy(list.data(), plan.ws.fix_list, list.size() * sizeof(int2), cudaMemcpyDeviceToHost),
+                    "cudaMemcpy(fix_list)")) != LDP_OK)
+        return rc;
     host_out[0] = count;
     for (const int2& it : list) host_out[1] += (it.y & ldp::MV_FIX) ? 1 : 0;
     return LDP_OK;
@@ -609,113 +618,92 @@ int ldp_debug_set_cluster(int csize) {
 const char* ldp_profile_name(int i) { return (i >= 0 && i < g_prof_n) ? g_prof_name[i] : ""; }
 
 // ---- output contract on the device (ldp_output.cu)
-// format 2 takes the normals [n,3] in place of err
-static int pack_records(int format, const float* xyz, const float* rgb, const float* err, int64_t n, const int64_t* n_dev,
-                        uint64_t first_id, uint8_t* out, void* stream) {
+// format 0: PLY, 1: points3D (err, first_id), 2: PLY with normals
+static int pack_records(int format, const float* xyz, const float* rgb, const float* err, const float* normals, int64_t n,
+                        const int64_t* n_dev, uint64_t first_id, uint8_t* out, void* stream) {
+    begin_call();
     if (n < 0) return fail(LDP_ERR_INVALID, "negative point count");
-    g_launches = 0;
     if (n == 0) return LDP_OK;
+    if (format == 2 && !normals) return fail(LDP_ERR_INVALID, "null normals");
     if (!xyz || !rgb || !out) return fail(LDP_ERR_INVALID, "null pointer");
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    static const decltype(&ldp::ldp_records_kernel<0>) k_records[3] = {ldp::ldp_records_kernel<0>, ldp::ldp_records_kernel<1>,
+                                                                        ldp::ldp_records_kernel<2>};
     const unsigned grid = (unsigned)((n + ldp::KO_THREADS - 1) / ldp::KO_THREADS);
     const int aligned = (reinterpret_cast<uintptr_t>(out) & 15u) == 0;
-    if (format == 0)
-        (void)launch_k(ldp::ldp_records_kernel<0>, dim3(grid), dim3(ldp::KO_THREADS), 0, st, xyz, rgb, err, (long long)n,
-                       reinterpret_cast<const long long*>(n_dev), (unsigned long long)first_id, out, aligned, (const float*)nullptr);
-    else if (format == 1)
-        (void)launch_k(ldp::ldp_records_kernel<1>, dim3(grid), dim3(ldp::KO_THREADS), 0, st, xyz, rgb, err, (long long)n,
-                       reinterpret_cast<const long long*>(n_dev), (unsigned long long)first_id, out, aligned, (const float*)nullptr);
-    else
-        (void)launch_k(ldp::ldp_records_kernel<2>, dim3(grid), dim3(ldp::KO_THREADS), 0, st, xyz, rgb, (const float*)nullptr,
-                       (long long)n, reinterpret_cast<const long long*>(n_dev), 0ull, out, aligned, err);
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_records_kernel");
-    return LDP_OK;
+    return launch("ldp_records_kernel", k_records[format], dim3(grid), dim3(ldp::KO_THREADS), 0, reinterpret_cast<cudaStream_t>(stream),
+                  xyz, rgb, err, (long long)n, reinterpret_cast<const long long*>(n_dev), (unsigned long long)first_id, out, aligned,
+                  normals);
 }
 
 int ldp_pack_ply_records(const float* xyz, const float* rgb, int64_t n, const int64_t* n_dev, uint8_t* records_out, void* stream) {
-    return pack_records(0, xyz, rgb, nullptr, n, n_dev, 0, records_out, stream);
+    return pack_records(0, xyz, rgb, nullptr, nullptr, n, n_dev, 0, records_out, stream);
 }
 
 int ldp_pack_ply_normal_records(const float* xyz, const float* rgb, const float* normals, int64_t n, const int64_t* n_dev,
                                 uint8_t* records_out, void* stream) {
-    if (n > 0 && !normals) return fail(LDP_ERR_INVALID, "null normals");
-    return pack_records(2, xyz, rgb, normals, n, n_dev, 0, records_out, stream);
+    return pack_records(2, xyz, rgb, nullptr, normals, n, n_dev, 0, records_out, stream);
 }
 
 int ldp_pack_points3d_records(const float* xyz, const float* rgb, const float* err, int64_t n, const int64_t* n_dev,
                               uint64_t first_id, uint8_t* records_out, void* stream) {
-    return pack_records(1, xyz, rgb, err, n, n_dev, first_id, records_out, stream);
+    return pack_records(1, xyz, rgb, err, nullptr, n, n_dev, first_id, records_out, stream);
 }
 
 int ldp_undistort_points(const ldp_lens* lens, int64_t n, const float* uv_in, float* uv_out, void* stream) {
+    begin_call();
     if (!lens || n < 0) return fail(LDP_ERR_INVALID, "bad arguments");
     if (lens->model < LDP_LENS_PINHOLE || lens->model > LDP_LENS_FISHEYE) return fail(LDP_ERR_INVALID, "unknown lens model");
-    g_launches = 0;
     if (n == 0) return LDP_OK;
     if (!uv_in || !uv_out) return fail(LDP_ERR_INVALID, "null pointer");
     if ((reinterpret_cast<size_t>(uv_in) | reinterpret_cast<size_t>(uv_out)) & 7) return fail(LDP_ERR_INVALID, "uv arrays must be 8-byte aligned");
     const long long blocks = (n + ldp::KU_THREADS - 1) / ldp::KU_THREADS;
     const unsigned grid = (unsigned)std::min<long long>(blocks, (long long)sm_count() * 16);
-    (void)launch_k(ldp::ldp_undistort_kernel, dim3(grid), dim3(ldp::KU_THREADS), 0, reinterpret_cast<cudaStream_t>(stream), *lens,
-                   (long long)n, reinterpret_cast<const float2*>(uv_in), reinterpret_cast<float2*>(uv_out));
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_undistort_kernel");
-    return LDP_OK;
+    return launch("ldp_undistort_kernel", ldp::ldp_undistort_kernel, dim3(grid), dim3(ldp::KU_THREADS), 0,
+                  reinterpret_cast<cudaStream_t>(stream), *lens, (long long)n, reinterpret_cast<const float2*>(uv_in),
+                  reinterpret_cast<float2*>(uv_out));
 }
 
 int ldp_rgb_to_uint8(const float* rgb, int64_t n_values, uint8_t* out, void* stream) {
+    begin_call();
     if (n_values < 0) return fail(LDP_ERR_INVALID, "negative count");
-    g_launches = 0;
     if (n_values == 0) return LDP_OK;
     if (!rgb || !out) return fail(LDP_ERR_INVALID, "null pointer");
     const long long blocks = (n_values + ldp::KO_THREADS - 1) / ldp::KO_THREADS;
     const unsigned grid = (unsigned)std::min<long long>(blocks, (long long)sm_count() * 16);
-    (void)launch_k(ldp::ldp_rgb_u8_kernel, dim3(grid), dim3(ldp::KO_THREADS), 0, reinterpret_cast<cudaStream_t>(stream), rgb, (long long)n_values, out);
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_rgb_u8_kernel");
-    return LDP_OK;
+    return launch("ldp_rgb_u8_kernel", ldp::ldp_rgb_u8_kernel, dim3(grid), dim3(ldp::KO_THREADS), 0, reinterpret_cast<cudaStream_t>(stream),
+                  rgb, (long long)n_values, out);
 }
 
 int ldp_gather_points(const float* xyz, const float* rgb, const float* err, const int64_t* sel, int64_t m, int64_t n,
                       float* xyz_out, float* rgb_out, float* err_out, int32_t* bad_index_flag, void* stream) {
+    begin_call();
     if (m < 0 || n < 0) return fail(LDP_ERR_INVALID, "negative count");
-    g_launches = 0;
     if (m == 0) return LDP_OK;
     if (!xyz || !rgb || !sel || !xyz_out || !rgb_out) return fail(LDP_ERR_INVALID, "null pointer");
     const unsigned grid = (unsigned)((m + ldp::KO_THREADS - 1) / ldp::KO_THREADS);
-    (void)launch_k(ldp::ldp_gather_rows_kernel, dim3(grid), dim3(ldp::KO_THREADS), 0, reinterpret_cast<cudaStream_t>(stream), xyz, rgb, err,
-                   reinterpret_cast<const long long*>(sel), (long long)m, (long long)n, xyz_out, rgb_out, err_out, (int*)bad_index_flag);
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_gather_rows_kernel");
-    return LDP_OK;
+    return launch("ldp_gather_rows_kernel", ldp::ldp_gather_rows_kernel, dim3(grid), dim3(ldp::KO_THREADS), 0,
+                  reinterpret_cast<cudaStream_t>(stream), xyz, rgb, err, reinterpret_cast<const long long*>(sel), (long long)m,
+                  (long long)n, xyz_out, rgb_out, err_out, (int*)bad_index_flag);
 }
 
 int ldp_gather_rows(const float* src, int32_t row_floats, const int64_t* sel, int64_t m, int64_t n, float* out,
                     int32_t* bad_index_flag, void* stream) {
+    begin_call();
     if (m < 0 || n < 0 || row_floats <= 0) return fail(LDP_ERR_INVALID, "bad row gather shape");
-    g_launches = 0;
     if (m == 0) return LDP_OK;
     if (!src || !sel || !out) return fail(LDP_ERR_INVALID, "null pointer");
     const long long blocks = (m * row_floats + ldp::KO_THREADS - 1) / ldp::KO_THREADS;
     const unsigned grid = (unsigned)std::min<long long>(blocks, (long long)sm_count() * 16);
-    (void)launch_k(ldp::ldp_gather_f32_rows_kernel, dim3(grid), dim3(ldp::KO_THREADS), 0, reinterpret_cast<cudaStream_t>(stream), src,
-                   (int)row_floats, reinterpret_cast<const long long*>(sel), (long long)m, (long long)n, out, (int*)bad_index_flag);
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_gather_f32_rows_kernel");
-    return LDP_OK;
+    return launch("ldp_gather_f32_rows_kernel", ldp::ldp_gather_f32_rows_kernel, dim3(grid), dim3(ldp::KO_THREADS), 0,
+                  reinterpret_cast<cudaStream_t>(stream), src, (int)row_floats, reinterpret_cast<const long long*>(sel), (long long)m,
+                  (long long)n, out, (int*)bad_index_flag);
 }
 
 int ldp_concat_points(const float* const* xyz_src, const float* const* rgb_src, const float* const* err_src,
                       const int64_t* const* count_src, int32_t n_seg, int64_t seg_cap, float* xyz_out, float* rgb_out,
                       float* err_out, int64_t out_capacity, int64_t* seg_offset_out, int64_t* total_out, void* stream) {
+    begin_call();
     if (n_seg < 0 || seg_cap < 0 || out_capacity < 0) return fail(LDP_ERR_INVALID, "negative size");
-    g_launches = 0;
     if (n_seg == 0) return LDP_OK;
     if (!xyz_src || !rgb_src || !err_src || !count_src || !xyz_out || !rgb_out || !err_out) return fail(LDP_ERR_INVALID, "null pointer");
     if (n_seg > 65535) return fail(LDP_ERR_INVALID, "too many segments");
@@ -723,73 +711,53 @@ int ldp_concat_points(const float* const* xyz_src, const float* const* rgb_src, 
     // enough CTAs to keep a few MB of (possibly remote) reads in flight: about four waves of CTAs over all segments
     const long long per_seg = std::max<long long>(64, (long long)sm_count() * 8 * 4 / std::max(1, n_seg));
     const unsigned gx = (unsigned)std::max<long long>(1, std::min<long long>(blocks, per_seg));
-    (void)launch_k(ldp::ldp_concat_points_kernel, dim3(gx, (unsigned)n_seg), dim3(ldp::KO_THREADS), 0, reinterpret_cast<cudaStream_t>(stream),
-                   xyz_src, rgb_src, err_src, reinterpret_cast<const long long* const*>(count_src), (int)n_seg, (long long)seg_cap,
-                   xyz_out, rgb_out, err_out, (long long)out_capacity, reinterpret_cast<long long*>(seg_offset_out),
-                   reinterpret_cast<long long*>(total_out));
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_concat_points_kernel");
-    return LDP_OK;
+    return launch("ldp_concat_points_kernel", ldp::ldp_concat_points_kernel, dim3(gx, (unsigned)n_seg), dim3(ldp::KO_THREADS), 0,
+                  reinterpret_cast<cudaStream_t>(stream), xyz_src, rgb_src, err_src, reinterpret_cast<const long long* const*>(count_src),
+                  (int)n_seg, (long long)seg_cap, xyz_out, rgb_out, err_out, (long long)out_capacity,
+                  reinterpret_cast<long long*>(seg_offset_out), reinterpret_cast<long long*>(total_out));
 }
 
 int ldp_scatter_points(const float* xyz, const float* rgb, const float* err, const int64_t* const* count_src, int32_t rank,
                        int32_t world, int64_t seg_cap, float* const* xyz_dst, float* const* rgb_dst, float* const* err_dst,
                        int64_t out_capacity, int64_t* seg_offset_out, int64_t* total_out, void* stream) {
+    begin_call();
     if (world < 1 || world > 64 || rank < 0 || rank >= world || seg_cap < 0 || out_capacity < 0) return fail(LDP_ERR_INVALID, "bad rank / world / size");
-    g_launches = 0;
     if (!xyz || !rgb || !err || !count_src || !xyz_dst || !rgb_dst || !err_dst) return fail(LDP_ERR_INVALID, "null pointer");
     const long long blocks = (seg_cap * 3 + ldp::KO_THREADS * 4 - 1) / (ldp::KO_THREADS * 4);
     const long long per_dst = std::max<long long>(32, (long long)sm_count() * 8 * 2 / world);
     const unsigned gx = (unsigned)std::max<long long>(1, std::min<long long>(blocks, per_dst));
-    (void)launch_k(ldp::ldp_scatter_points_kernel, dim3(gx, (unsigned)world), dim3(ldp::KO_THREADS), 0, reinterpret_cast<cudaStream_t>(stream),
-                   xyz, rgb, err, reinterpret_cast<const long long* const*>(count_src), (int)rank, (int)world, (long long)seg_cap,
-                   xyz_dst, rgb_dst, err_dst, (long long)out_capacity, reinterpret_cast<long long*>(seg_offset_out),
-                   reinterpret_cast<long long*>(total_out));
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_scatter_points_kernel");
-    return LDP_OK;
+    return launch("ldp_scatter_points_kernel", ldp::ldp_scatter_points_kernel, dim3(gx, (unsigned)world), dim3(ldp::KO_THREADS), 0,
+                  reinterpret_cast<cudaStream_t>(stream), xyz, rgb, err, reinterpret_cast<const long long* const*>(count_src), (int)rank,
+                  (int)world, (long long)seg_cap, xyz_dst, rgb_dst, err_dst, (long long)out_capacity,
+                  reinterpret_cast<long long*>(seg_offset_out), reinterpret_cast<long long*>(total_out));
 }
 
 // ---- pair generation on the device (ldp_select.cu)
 int ldp_select_kcenters(const float* flat_poses, int32_t n, int32_t k, float* scratch, int32_t* centers_sorted,
                         int32_t* centers_order, void* stream) {
-    g_launches = 0;
+    begin_call();
     if (n <= 0 || k <= 0 || k > n) return fail(LDP_ERR_INVALID, "k-centres needs 1 <= k <= n");
     if (n > ldp::KC_THREADS * ldp::KC_MAX_PER_THREAD) return fail(LDP_ERR_INVALID, "k-centres: more than 8192 views");
     if (!flat_poses || !scratch || !centers_sorted || !centers_order) return fail(LDP_ERR_INVALID, "null pointer");
     const size_t smem = (size_t)n * ldp::KC_PAD * sizeof(float);
-    if (smem <= K1_SMEM_BUDGET) {                        // the poses fit in shared memory (n <= 3011)
-        static bool configured_dev[MAX_DEVICES] = {};
-        bool& configured = configured_dev[current_device()];
-        if (!configured) {
-            (void)cudaFuncSetAttribute(ldp::ldp_kcenters_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K1_SMEM_BUDGET);
-            configured = true;
-        }
-        (void)launch_k(ldp::ldp_kcenters_kernel<true>, dim3(1), dim3(ldp::KC_THREADS), smem, reinterpret_cast<cudaStream_t>(stream),
-                       flat_poses, (int)n, (int)k, scratch, centers_sorted, centers_order);
-    } else
-        (void)launch_k(ldp::ldp_kcenters_kernel<false>, dim3(1), dim3(ldp::KC_THREADS), 0, reinterpret_cast<cudaStream_t>(stream),
-                       flat_poses, (int)n, (int)k, scratch, centers_sorted, centers_order);
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_kcenters_kernel");
-    return LDP_OK;
+    const bool in_smem = smem <= K1_SMEM_BUDGET;         // the poses fit in shared memory (n <= 3011)
+    if (in_smem) {
+        const int rc = configure_device();
+        if (rc != LDP_OK) return rc;
+    }
+    return launch("ldp_kcenters_kernel", in_smem ? ldp::ldp_kcenters_kernel<true> : ldp::ldp_kcenters_kernel<false>, dim3(1),
+                  dim3(ldp::KC_THREADS), in_smem ? smem : 0, reinterpret_cast<cudaStream_t>(stream), flat_poses, (int)n, (int)k, scratch,
+                  centers_sorted, centers_order);
 }
 
 int ldp_nearest_neighbors(const float* flat_poses, int32_t n, int32_t k, int64_t* idx_out, void* stream) {
-    g_launches = 0;
+    begin_call();
     if (n < 0 || k < 0) return fail(LDP_ERR_INVALID, "negative size");
     if (n <= 1 || k == 0) return LDP_OK;
     if (k > n - 1 || k > ldp::KNN_MAX_K) return fail(LDP_ERR_INVALID, "nearest neighbours needs k <= min(n - 1, 16)");
     if (!flat_poses || !idx_out) return fail(LDP_ERR_INVALID, "null pointer");
-    (void)launch_k(ldp::ldp_knn_kernel, dim3((unsigned)n), dim3(ldp::KNN_THREADS), 0, reinterpret_cast<cudaStream_t>(stream), flat_poses,
-                   (int)n, (int)k, reinterpret_cast<long long*>(idx_out));
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_knn_kernel");
-    return LDP_OK;
+    return launch("ldp_knn_kernel", ldp::ldp_knn_kernel, dim3((unsigned)n), dim3(ldp::KNN_THREADS), 0, reinterpret_cast<cudaStream_t>(stream),
+                  flat_poses, (int)n, (int)k, reinterpret_cast<long long*>(idx_out));
 }
 
 // ---- voxel-grid downsample (ldp_voxel.cu)
@@ -801,24 +769,23 @@ static size_t voxel_cap(int64_t n) {
 static int voxel_plan(int64_t n, void* base, ldp::VoxelWs* ws, size_t* bytes) {
     if (n < 0 || n > 500000000ll) return fail(LDP_ERR_INVALID, "voxel downsample: bad point count");
     const size_t cap = voxel_cap(n), N = (size_t)std::max<int64_t>(n, 1);
-    size_t off = 0;
-    auto carve = [&](size_t b) { void* p = base ? static_cast<char*>(base) + off : nullptr; off += align_up(b, 256); return p; };
-    ws->bounds = reinterpret_cast<double*>(carve(8 * sizeof(double)));
-    ws->bounds_u = reinterpret_cast<unsigned int*>(carve(8 * sizeof(unsigned int)));
-    ws->keys = reinterpret_cast<unsigned long long*>(carve(cap * sizeof(unsigned long long)));
-    ws->first = reinterpret_cast<int*>(carve(cap * sizeof(int)));
-    ws->slot = reinterpret_cast<int*>(carve(N * sizeof(int)));
-    ws->flag = reinterpret_cast<int*>(carve(N * sizeof(int)));
-    ws->rank = reinterpret_cast<int*>(carve(N * sizeof(int)));
-    ws->count = reinterpret_cast<int*>(carve((N + 1) * sizeof(int)));
-    ws->cursor = reinterpret_cast<int*>(carve(N * sizeof(int)));
-    ws->seg = reinterpret_cast<int*>(carve(N * sizeof(int)));
-    ws->members = reinterpret_cast<int*>(carve(N * sizeof(int)));
-    ws->block_tot = reinterpret_cast<int*>(carve((N / ldp::SC_THREADS + 2) * sizeof(int)));
-    ws->large = reinterpret_cast<int*>(carve((N + 2) * sizeof(int)));
+    Carver c{static_cast<char*>(base)};
+    ws->bounds = c.take<double>(8);
+    ws->bounds_u = c.take<unsigned int>(8);
+    ws->keys = c.take<unsigned long long>(cap);
+    ws->first = c.take<int>(cap);
+    ws->slot = c.take<int>(N);
+    ws->flag = c.take<int>(N);
+    ws->rank = c.take<int>(N);
+    ws->count = c.take<int>(N + 1);
+    ws->cursor = c.take<int>(N);
+    ws->seg = c.take<int>(N);
+    ws->members = c.take<int>(N);
+    ws->block_tot = c.take<int>(N / ldp::SC_THREADS + 2);
+    ws->large = c.take<int>(N + 2);
     ws->status = nullptr;
     ws->cap_mask = cap - 1;
-    *bytes = off;
+    *bytes = c.off;
     return LDP_OK;
 }
 
@@ -830,54 +797,63 @@ int ldp_voxel_workspace_bytes(int64_t n, size_t* bytes_out) {
 
 static int scan_exclusive(const int* in, int* out, int64_t n, int* block_tot, int* grand_total, cudaStream_t st) {
     const int nblocks = (int)((n + ldp::SC_THREADS - 1) / ldp::SC_THREADS);
-    (void)launch_k(ldp::ldp_scan_blocks_kernel, dim3(nblocks), dim3(ldp::SC_THREADS), 0, st, in, out, (long long)n, block_tot);
-    (void)launch_k(ldp::ldp_scan_totals_kernel, dim3(1), dim3(ldp::SC_THREADS), 0, st, block_tot, nblocks, grand_total);
-    (void)launch_k(ldp::ldp_scan_add_kernel, dim3(nblocks), dim3(ldp::SC_THREADS), 0, st, out, (long long)n, (const int*)block_tot);
-    g_launches += 3;
-    return LDP_OK;
+    int rc = launch("ldp_scan_blocks_kernel", ldp::ldp_scan_blocks_kernel, dim3(nblocks), dim3(ldp::SC_THREADS), 0, st, in, out,
+                    (long long)n, block_tot);
+    if (rc == LDP_OK)
+        rc = launch("ldp_scan_totals_kernel", ldp::ldp_scan_totals_kernel, dim3(1), dim3(ldp::SC_THREADS), 0, st, block_tot, nblocks,
+                    grand_total);
+    if (rc == LDP_OK)
+        rc = launch("ldp_scan_add_kernel", ldp::ldp_scan_add_kernel, dim3(nblocks), dim3(ldp::SC_THREADS), 0, st, out, (long long)n,
+                    (const int*)block_tot);
+    return rc;
 }
 
 int ldp_voxel_downsample(const float* xyz, const float* rgb, int64_t n, double voxel_size, float* xyz_out, float* rgb_out,
                          int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream) {
-    g_launches = 0;
+    begin_call();
     if (!(voxel_size > 0.0)) return fail(LDP_ERR_INVALID, "voxel_size must be positive");       // Open3D: "voxel_size <= 0."
     if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    cudaError_t e = cudaMemsetAsync(status_out, 0, 2 * sizeof(int32_t), st);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(status)");
-    if (n == 0) return LDP_OK;
+    int rc = check(cudaMemsetAsync(status_out, 0, 2 * sizeof(int32_t), st), "cudaMemsetAsync(status)");
+    if (rc != LDP_OK || n == 0) return rc;
     if (!xyz || !rgb || !xyz_out || !rgb_out || !workspace) return fail(LDP_ERR_INVALID, "null pointer");
     ldp::VoxelWs ws;
     size_t need = 0;
-    int rc = voxel_plan(n, workspace, &ws, &need);
-    if (rc != LDP_OK) return rc;
+    if ((rc = voxel_plan(n, workspace, &ws, &need)) != LDP_OK) return rc;
     if (workspace_bytes < need) return fail(LDP_ERR_INVALID, "voxel workspace too small");
     ws.status = status_out;
     const size_t cap = (size_t)ws.cap_mask + 1;
-    e = cudaMemsetAsync(ws.bounds_u, 0xFF, 3 * sizeof(unsigned int), st);
+    cudaError_t e = cudaMemsetAsync(ws.bounds_u, 0xFF, 3 * sizeof(unsigned int), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(ws.bounds_u + 3, 0, sizeof(unsigned int), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(ws.keys, 0xFF, cap * sizeof(unsigned long long), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(ws.first, 0x7F, cap * sizeof(int), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(ws.count, 0, ((size_t)n + 1) * sizeof(int), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(ws.cursor, 0, (size_t)n * sizeof(int), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(ws.large, 0, 2 * sizeof(int), st);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(voxel workspace)");
+    if ((rc = check(e, "cudaMemsetAsync(voxel workspace)")) != LDP_OK) return rc;
     const unsigned grid = (unsigned)((n + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
     const unsigned rgrid = (unsigned)std::min<long long>(grid, (long long)sm_count() * 8);
-    (void)launch_k(ldp::ldp_voxel_bounds_kernel, dim3(rgrid), dim3(ldp::KV_THREADS), 0, st, xyz, rgb, (long long)n, ws);
-    (void)launch_k(ldp::ldp_voxel_insert_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, xyz, (long long)n, voxel_size, (const double*)nullptr, ws);
-    (void)launch_k(ldp::ldp_voxel_flag_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws);
-    g_launches += 3;
-    scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, ws.status + 1, st);
-    (void)launch_k(ldp::ldp_voxel_count_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws);
-    ++g_launches;
-    scan_exclusive(ws.count, ws.seg, n, ws.block_tot, nullptr, st);
-    (void)launch_k(ldp::ldp_voxel_group_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws, (const int*)ws.seg);
-    (void)launch_k(ldp::ldp_voxel_mean_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, xyz, rgb, ws, (const int*)ws.seg, xyz_out, rgb_out);
-    (void)launch_k(ldp::ldp_voxel_large_kernel, dim3((unsigned)sm_count()), dim3(ldp::SC_THREADS), 0, st, xyz, rgb, ws, (const int*)ws.seg, xyz_out, rgb_out);
-    g_launches += 3;
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "voxel downsample kernels");
-    return LDP_OK;
+    const dim3 block(ldp::KV_THREADS);
+    rc = launch("ldp_voxel_bounds_kernel", ldp::ldp_voxel_bounds_kernel, dim3(rgrid), block, 0, st, xyz, rgb, (long long)n, ws);
+    if (rc != LDP_OK) return rc;
+    rc = launch("ldp_voxel_insert_kernel", ldp::ldp_voxel_insert_kernel, dim3(grid), block, 0, st, xyz, (long long)n, voxel_size,
+                (const double*)nullptr, ws);
+    if (rc != LDP_OK) return rc;
+    rc = launch("ldp_voxel_flag_kernel", ldp::ldp_voxel_flag_kernel, dim3(grid), block, 0, st, (long long)n, ws);
+    if (rc != LDP_OK) return rc;
+    rc = scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, ws.status + 1, st);
+    if (rc != LDP_OK) return rc;
+    rc = launch("ldp_voxel_count_kernel", ldp::ldp_voxel_count_kernel, dim3(grid), block, 0, st, (long long)n, ws);
+    if (rc != LDP_OK) return rc;
+    rc = scan_exclusive(ws.count, ws.seg, n, ws.block_tot, nullptr, st);
+    if (rc != LDP_OK) return rc;
+    rc = launch("ldp_voxel_group_kernel", ldp::ldp_voxel_group_kernel, dim3(grid), block, 0, st, (long long)n, ws, (const int*)ws.seg);
+    if (rc != LDP_OK) return rc;
+    rc = launch("ldp_voxel_mean_kernel", ldp::ldp_voxel_mean_kernel, dim3(grid), block, 0, st, xyz, rgb, ws, (const int*)ws.seg,
+                xyz_out, rgb_out);
+    if (rc != LDP_OK) return rc;
+    return launch("ldp_voxel_large_kernel", ldp::ldp_voxel_large_kernel, dim3((unsigned)sm_count()), dim3(ldp::SC_THREADS), 0, st, xyz,
+                  rgb, ws, (const int*)ws.seg, xyz_out, rgb_out);
 }
 
 // ---- statistical outlier removal (ldp_outlier.cu)
@@ -899,23 +875,22 @@ struct OutlierPlan {
 // with_stats = false (the normal call) leaves out the per-point means and the partial sums
 static int outlier_plan(int64_t n, void* base, OutlierPlan* pl, size_t* bytes, bool with_stats = true) {
     if (n < 0 || n > 500000000ll) return fail(LDP_ERR_INVALID, "k-NN search: bad point count");
-    size_t off = 0;
-    int rc = voxel_plan(n, base, &pl->vws, &off);
+    Carver c{static_cast<char*>(base)};
+    int rc = voxel_plan(n, base, &pl->vws, &c.off);
     if (rc != LDP_OK) return rc;
     const size_t cap = voxel_cap(n), N = (size_t)std::max<int64_t>(n, 1);
-    auto carve = [&](size_t b) { void* p = base ? static_cast<char*>(base) + off : nullptr; off += align_up(b, 256); return p; };
-    pl->vstat = reinterpret_cast<int*>(carve(2 * sizeof(int)));
-    pl->h_trial = reinterpret_cast<double*>(carve(sizeof(double)));
-    pl->stats = reinterpret_cast<double*>(carve(3 * sizeof(double)));
-    pl->m = reinterpret_cast<double*>(carve(with_stats ? N * sizeof(double) : 0));
-    pl->part = reinterpret_cast<double*>(carve(with_stats ? (N / ldp::OL_CHUNK + 1) * sizeof(double) : 0));
-    pl->levels = reinterpret_cast<ldp::OutlierLevel*>(carve(ldp::OL_MAX_LEVELS * sizeof(ldp::OutlierLevel)));
+    pl->vstat = c.take<int>(2);
+    pl->h_trial = c.take<double>(1);
+    pl->stats = c.take<double>(3);
+    pl->m = c.take<double>(with_stats ? N : 0);
+    pl->part = c.take<double>(with_stats ? N / ldp::OL_CHUNK + 1 : 0);
+    pl->levels = c.take<ldp::OutlierLevel>(ldp::OL_MAX_LEVELS);
     for (int l = 0; l < ldp::OL_MAX_LEVELS; ++l) {
-        pl->keys[l] = reinterpret_cast<unsigned long long*>(carve(cap * sizeof(unsigned long long)));
-        pl->cell[l] = reinterpret_cast<int2*>(carve(cap * sizeof(int2)));
-        pl->pts[l] = reinterpret_cast<float4*>(carve(N * sizeof(float4)));
+        pl->keys[l] = c.take<unsigned long long>(cap);
+        pl->cell[l] = c.take<int2>(cap);
+        pl->pts[l] = c.take<float4>(N);
     }
-    *bytes = off;
+    *bytes = c.off;
     return LDP_OK;
 }
 
@@ -940,24 +915,30 @@ static float host_f32_unordered(unsigned int k) {          // ldp::f32_unordered
 }
 
 // hash insert, first-of-cell flags, ranks: the cells of a grid of size h (or *h_dev) in pl.vws.keys
-static void outlier_insert(const float* xyz, int64_t n, double h, const double* h_dev, OutlierPlan& pl, unsigned grid, cudaStream_t st,
-                           int* cells_out) {
+static int outlier_insert(const float* xyz, int64_t n, double h, const double* h_dev, OutlierPlan& pl, unsigned grid, cudaStream_t st,
+                          int* cells_out) {
     ldp::VoxelWs& ws = pl.vws;
     const size_t cap = (size_t)ws.cap_mask + 1;
-    (void)cudaMemsetAsync(ws.keys, 0xFF, cap * sizeof(unsigned long long), st);
-    (void)cudaMemsetAsync(ws.first, 0x7F, cap * sizeof(int), st);
-    (void)launch_k(ldp::ldp_voxel_insert_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, xyz, (long long)n, h, h_dev, ws);
-    (void)launch_k(ldp::ldp_voxel_flag_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws);
-    g_launches += 2;
-    scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, cells_out, st);
+    cudaError_t e = cudaMemsetAsync(ws.keys, 0xFF, cap * sizeof(unsigned long long), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(ws.first, 0x7F, cap * sizeof(int), st);
+    int rc = check(e, "cudaMemsetAsync(outlier grid)");
+    if (rc != LDP_OK) return rc;
+    rc = launch("ldp_voxel_insert_kernel", ldp::ldp_voxel_insert_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, xyz, (long long)n, h,
+                h_dev, ws);
+    if (rc != LDP_OK) return rc;
+    rc = launch("ldp_voxel_flag_kernel", ldp::ldp_voxel_flag_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws);
+    if (rc != LDP_OK) return rc;
+    return scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, cells_out, st);
 }
 
 // Steps 1 and 2 of the k-NN search, shared by ldp_statistical_outliers and ldp_estimate_normals: bounds and a trial grid,
 // whose cell count sets the level-0 cell size (the one host synchronisation), then the pyramid and its level descriptors
-// in pl.levels.  A coordinate that is not finite sets status_out[0] = 1 and leaves *n_levels_out = 0.
+// in pl.levels.  A coordinate that is not finite sets status_out[0] = 1 and leaves *n_levels_out = 0 (and returns LDP_OK);
+// any CUDA failure returns LDP_ERR_CUDA.
 static int knn_pyramid(const float* xyz, int64_t n, int k, OutlierPlan& pl, cudaStream_t st, int32_t* status_out, int* n_levels_out) {
     *n_levels_out = 0;
     cudaError_t e;
+    int rc;
     ldp::VoxelWs& ws = pl.vws;
     ws.status = pl.vstat;
     const unsigned grid = (unsigned)((n + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
@@ -972,16 +953,20 @@ static int knn_pyramid(const float* xyz, int64_t n, int k, OutlierPlan& pl, cuda
         KernelTimer kt(st, "ldp_outlier_trial_grid");
         e = cudaMemsetAsync(ws.bounds_u, 0xFF, 3 * sizeof(unsigned int), st);
         if (e == cudaSuccess) e = cudaMemsetAsync(ws.bounds_u + 3, 0, 5 * sizeof(unsigned int), st);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(outlier bounds)");
-        (void)launch_k(ldp::ldp_voxel_bounds_kernel, dim3(rgrid), dim3(ldp::KV_THREADS), 0, st, xyz, (const float*)nullptr, (long long)n, ws);
-        (void)launch_k(ldp::ldp_outlier_trial_size_kernel, dim3(1), dim3(1), 0, st, (const unsigned int*)ws.bounds_u, (long long)n, k, pl.h_trial);
-        g_launches += 2;
-        outlier_insert(xyz, n, 0.0, pl.h_trial, pl, grid, st, reinterpret_cast<int*>(ws.bounds_u + 7));
+        if ((rc = check(e, "cudaMemsetAsync(outlier bounds)")) != LDP_OK) return rc;
+        rc = launch("ldp_voxel_bounds_kernel", ldp::ldp_voxel_bounds_kernel, dim3(rgrid), dim3(ldp::KV_THREADS), 0, st, xyz,
+                    (const float*)nullptr, (long long)n, ws);
+        if (rc != LDP_OK) return rc;
+        rc = launch("ldp_outlier_trial_size_kernel", ldp::ldp_outlier_trial_size_kernel, dim3(1), dim3(1), 0, st,
+                    (const unsigned int*)ws.bounds_u, (long long)n, k, pl.h_trial);
+        if (rc != LDP_OK) return rc;
+        rc = outlier_insert(xyz, n, 0.0, pl.h_trial, pl, grid, st, reinterpret_cast<int*>(ws.bounds_u + 7));
+        if (rc != LDP_OK) return rc;
     }
     e = cudaMemcpyAsync(bu, ws.bounds_u, sizeof(bu), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(&h_trial, pl.h_trial, sizeof(double), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) return cuda_fail(e, "outlier trial grid");
+    if ((rc = check(e, "outlier trial grid")) != LDP_OK) return rc;
     double mn[3], mx[3], ext = 0.0;
     bool finite = true;
     for (int c = 0; c < 3; ++c) {
@@ -990,10 +975,8 @@ static int knn_pyramid(const float* xyz, int64_t n, int k, OutlierPlan& pl, cuda
         finite = finite && std::isfinite(mn[c]) && std::isfinite(mx[c]);
         ext = std::max(ext, mx[c] - mn[c]);
     }
-    if (!finite) {                                      // status_out[0] = 1 (little-endian int32, zeroed by the caller)
-        e = cudaMemsetAsync(status_out, 1, 1, st);
-        return e == cudaSuccess ? LDP_OK : cuda_fail(e, "cudaMemsetAsync(status)");
-    }
+    if (!finite)                                        // status_out[0] = 1 (little-endian int32, zeroed by the caller)
+        return check(cudaMemsetAsync(status_out, 1, 1, st), "cudaMemsetAsync(status)");
     const double trial_cells = (double)std::max(1u, bu[7]);
     double h = 1.0;
     if (ext > 0.0) h = std::max(h_trial * std::sqrt(0.5 * k * trial_cells / (double)n), ext / 1048576.0);
@@ -1014,23 +997,27 @@ static int knn_pyramid(const float* xyz, int64_t n, int k, OutlierPlan& pl, cuda
             ws.keys = pl.keys[n_levels];
             e = cudaMemsetAsync(ws.count, 0, ((size_t)n + 1) * sizeof(int), st);
             if (e == cudaSuccess) e = cudaMemsetAsync(ws.cursor, 0, (size_t)n * sizeof(int), st);
-            if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(outlier level)");
-            outlier_insert(xyz, n, h, nullptr, pl, grid, st, pl.vstat + 1);
-            (void)launch_k(ldp::ldp_voxel_count_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws);
-            ++g_launches;
-            scan_exclusive(ws.count, ws.seg, n, ws.block_tot, nullptr, st);
-            (void)launch_k(ldp::ldp_voxel_group_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws, (const int*)ws.seg);
-            (void)launch_k(ldp::ldp_outlier_cells_kernel, dim3(cgrid), dim3(ldp::KV_THREADS), 0, st, ws, pl.cell[n_levels]);
-            (void)launch_k(ldp::ldp_outlier_pack_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, xyz, (long long)n,
-                           (const int*)ws.members, pl.pts[n_levels]);
-            g_launches += 3;
+            if ((rc = check(e, "cudaMemsetAsync(outlier level)")) != LDP_OK) return rc;
+            if ((rc = outlier_insert(xyz, n, h, nullptr, pl, grid, st, pl.vstat + 1)) != LDP_OK) return rc;
+            rc = launch("ldp_voxel_count_kernel", ldp::ldp_voxel_count_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws);
+            if (rc != LDP_OK) return rc;
+            if ((rc = scan_exclusive(ws.count, ws.seg, n, ws.block_tot, nullptr, st)) != LDP_OK) return rc;
+            rc = launch("ldp_voxel_group_kernel", ldp::ldp_voxel_group_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (long long)n, ws,
+                        (const int*)ws.seg);
+            if (rc != LDP_OK) return rc;
+            rc = launch("ldp_outlier_cells_kernel", ldp::ldp_outlier_cells_kernel, dim3(cgrid), dim3(ldp::KV_THREADS), 0, st, ws,
+                        pl.cell[n_levels]);
+            if (rc != LDP_OK) return rc;
+            rc = launch("ldp_outlier_pack_kernel", ldp::ldp_outlier_pack_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, xyz,
+                        (long long)n, (const int*)ws.members, pl.pts[n_levels]);
+            if (rc != LDP_OK) return rc;
             ++n_levels;
             if (n_levels == ldp::OL_MAX_LEVELS || !(ext / h > 2.0)) break;
             h *= 8.0;
         }
     }
-    (void)launch_k(ldp::ldp_outlier_levels_kernel, dim3(1), dim3(1), 0, st, lv, n_levels, pl.levels);
-    ++g_launches;
+    rc = launch("ldp_outlier_levels_kernel", ldp::ldp_outlier_levels_kernel, dim3(1), dim3(1), 0, st, lv, n_levels, pl.levels);
+    if (rc != LDP_OK) return rc;
     *n_levels_out = n_levels;
     return LDP_OK;
 }
@@ -1038,19 +1025,17 @@ static int knn_pyramid(const float* xyz, int64_t n, int k, OutlierPlan& pl, cuda
 int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, double std_ratio, int64_t* kept_idx_out,
                              double* mean_dist_out, double* stats_out, int32_t* status_out, void* workspace, size_t workspace_bytes,
                              void* stream) {
-    g_launches = 0;
+    begin_call();
     if (nb_neighbors < 1 || nb_neighbors > ldp::OL_MAX_K) return fail(LDP_ERR_INVALID, "nb_neighbors must lie in [1, 64]");
     if (!(std_ratio > 0.0)) return fail(LDP_ERR_INVALID, "std_ratio must be positive");
     if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    cudaError_t e = cudaMemsetAsync(status_out, 0, 3 * sizeof(int32_t), st);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(status)");
-    if (n == 0) return LDP_OK;
+    int rc = check(cudaMemsetAsync(status_out, 0, 3 * sizeof(int32_t), st), "cudaMemsetAsync(status)");
+    if (rc != LDP_OK || n == 0) return rc;
     if (!xyz || !kept_idx_out || !workspace) return fail(LDP_ERR_INVALID, "null pointer");
     OutlierPlan pl;
     size_t need = 0;
-    int rc = outlier_plan(n, workspace, &pl, &need);
-    if (rc != LDP_OK) return rc;
+    if ((rc = outlier_plan(n, workspace, &pl, &need)) != LDP_OK) return rc;
     if (workspace_bytes < need) return fail(LDP_ERR_WORKSPACE, "outlier workspace too small");
     const int k = (int)std::min<int64_t>(nb_neighbors, n);
     int n_levels = 0;
@@ -1064,35 +1049,30 @@ int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, 
     {
         KernelTimer kt(st, "ldp_outlier_knn_kernel");
         const unsigned kgrid = (unsigned)((n + ldp::OL_THREADS - 1) / ldp::OL_THREADS);
-        (void)launch_k(ldp::ldp_outlier_knn_kernel<false>, dim3(kgrid), dim3(ldp::OL_THREADS), (size_t)k * ldp::OL_THREADS * sizeof(double), st,
-                       (const ldp::OutlierLevel*)pl.levels, n_levels, (long long)n, k,
-                       g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, m, (int*)status_out, ldp::NormalArgs{});
-        ++g_launches;
+        rc = launch("ldp_outlier_knn_kernel", ldp::ldp_outlier_knn_kernel<false>, dim3(kgrid), dim3(ldp::OL_THREADS),
+                    (size_t)k * ldp::OL_THREADS * sizeof(double), st, (const ldp::OutlierLevel*)pl.levels, n_levels, (long long)n, k,
+                    g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, m, (int*)status_out, ldp::NormalArgs{});
+        if (rc != LDP_OK) return rc;
     }
 
-    // 4. threshold, keep flags, kept indices
-    {
-        KernelTimer kt(st, "ldp_outlier_threshold");
-        const long long n_part = (n + ldp::OL_CHUNK - 1) / ldp::OL_CHUNK;
-        const unsigned pgrid = (unsigned)((n_part + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
-        (void)launch_k(ldp::ldp_outlier_partial_kernel, dim3(pgrid), dim3(ldp::KV_THREADS), 0, st, (const double*)m, (long long)n,
-                       (const double*)nullptr, pl.part);
-        (void)launch_k(ldp::ldp_outlier_stats_kernel, dim3(1), dim3(ldp::OL_FINAL), 0, st, (const double*)pl.part, n_part, (long long)n,
-                       std_ratio, 0, stats);
-        (void)launch_k(ldp::ldp_outlier_partial_kernel, dim3(pgrid), dim3(ldp::KV_THREADS), 0, st, (const double*)m, (long long)n,
-                       (const double*)stats, pl.part);
-        (void)launch_k(ldp::ldp_outlier_stats_kernel, dim3(1), dim3(ldp::OL_FINAL), 0, st, (const double*)pl.part, n_part, (long long)n,
-                       std_ratio, 1, stats);
-        (void)launch_k(ldp::ldp_outlier_flag_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (const double*)m, (long long)n,
-                       (const double*)stats, ws.flag);
-        g_launches += 5;
-        scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, (int*)status_out + 1, st);
-        (void)launch_k(ldp::ldp_outlier_kept_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (const int*)ws.flag, (const int*)ws.rank,
-                       (long long)n, reinterpret_cast<long long*>(kept_idx_out));
-        ++g_launches;
+    // 4. threshold (first pass: the mean; second: the spread around it, std and threshold), keep flags, kept indices
+    KernelTimer kt(st, "ldp_outlier_threshold");
+    const long long n_part = (n + ldp::OL_CHUNK - 1) / ldp::OL_CHUNK;
+    const unsigned pgrid = (unsigned)((n_part + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
+    for (int second = 0; second < 2; ++second) {
+        rc = launch("ldp_outlier_partial_kernel", ldp::ldp_outlier_partial_kernel, dim3(pgrid), dim3(ldp::KV_THREADS), 0, st,
+                    (const double*)m, (long long)n, second ? (const double*)stats : nullptr, pl.part);
+        if (rc != LDP_OK) return rc;
+        rc = launch("ldp_outlier_stats_kernel", ldp::ldp_outlier_stats_kernel, dim3(1), dim3(ldp::OL_FINAL), 0, st, (const double*)pl.part,
+                    n_part, (long long)n, std_ratio, second, stats);
+        if (rc != LDP_OK) return rc;
     }
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "statistical outlier kernels");
-    return LDP_OK;
+    rc = launch("ldp_outlier_flag_kernel", ldp::ldp_outlier_flag_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (const double*)m,
+                (long long)n, (const double*)stats, ws.flag);
+    if (rc != LDP_OK) return rc;
+    if ((rc = scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, (int*)status_out + 1, st)) != LDP_OK) return rc;
+    return launch("ldp_outlier_kept_kernel", ldp::ldp_outlier_kept_kernel, dim3(grid), dim3(ldp::KV_THREADS), 0, st, (const int*)ws.flag,
+                  (const int*)ws.rank, (long long)n, reinterpret_cast<long long*>(kept_idx_out));
 }
 
 // ---- oriented normals (ldp_outlier.cu: ldp_outlier_knn_kernel<true> and its epilogue)
@@ -1106,36 +1086,29 @@ int ldp_normals_workspace_bytes(int64_t n, int32_t k, size_t* bytes_out) {
 int ldp_estimate_normals(const float* xyz, int64_t n, int32_t k, const float* centers, int32_t n_centers, const int32_t* center_idx,
                          float* normals_out, float* curvature_out, int32_t* knn_idx_out, int32_t* status_out, void* workspace,
                          size_t workspace_bytes, void* stream) {
-    g_launches = 0;
+    begin_call();
     if (k < 3 || k > ldp::OL_MAX_K) return fail(LDP_ERR_INVALID, "k must lie in [3, 64]");
     if (center_idx && !centers) return fail(LDP_ERR_INVALID, "center_idx needs centers");
     if (centers && n_centers < 1) return fail(LDP_ERR_INVALID, "n_centers must be >= 1 when centers are given");
     if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    cudaError_t e = cudaMemsetAsync(status_out, 0, 3 * sizeof(int32_t), st);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(status)");
-    if (n == 0) return LDP_OK;
+    int rc = check(cudaMemsetAsync(status_out, 0, 3 * sizeof(int32_t), st), "cudaMemsetAsync(status)");
+    if (rc != LDP_OK || n == 0) return rc;
     if (!xyz || !normals_out || !workspace) return fail(LDP_ERR_INVALID, "null pointer");
     OutlierPlan pl;
     size_t need = 0;
-    int rc = outlier_plan(n, workspace, &pl, &need, false);
-    if (rc != LDP_OK) return rc;
+    if ((rc = outlier_plan(n, workspace, &pl, &need, false)) != LDP_OK) return rc;
     if (workspace_bytes < need) return fail(LDP_ERR_WORKSPACE, "normals workspace too small");
     const int k_eff = (int)std::min<int64_t>(k, n);
     int n_levels = 0;
     if ((rc = knn_pyramid(xyz, n, k_eff, pl, st, status_out, &n_levels)) != LDP_OK || n_levels == 0) return rc;
-    {
-        KernelTimer kt(st, "ldp_normals_knn_kernel");
-        ldp::NormalArgs na{xyz, centers, center_idx, normals_out, curvature_out, knn_idx_out, centers ? n_centers : 0, 0};
-        const unsigned kgrid = (unsigned)((n + ldp::OL_THREADS - 1) / ldp::OL_THREADS);
-        (void)launch_k(ldp::ldp_outlier_knn_kernel<true>, dim3(kgrid), dim3(ldp::OL_THREADS),
-                       (size_t)k_eff * ldp::OL_THREADS * (sizeof(double) + sizeof(int)), st,
-                       (const ldp::OutlierLevel*)pl.levels, n_levels, (long long)n, k_eff,
-                       g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, (double*)nullptr, (int*)status_out, na);
-        ++g_launches;
-    }
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "normal kernels");
-    return LDP_OK;
+    KernelTimer kt(st, "ldp_normals_knn_kernel");
+    const ldp::NormalArgs na{xyz, centers, center_idx, normals_out, curvature_out, knn_idx_out, centers ? n_centers : 0, 0};
+    const unsigned kgrid = (unsigned)((n + ldp::OL_THREADS - 1) / ldp::OL_THREADS);
+    return launch("ldp_outlier_knn_kernel", ldp::ldp_outlier_knn_kernel<true>, dim3(kgrid), dim3(ldp::OL_THREADS),
+                  (size_t)k_eff * ldp::OL_THREADS * (sizeof(double) + sizeof(int)), st, (const ldp::OutlierLevel*)pl.levels, n_levels,
+                  (long long)n, k_eff, g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, (double*)nullptr,
+                  (int*)status_out, na);
 }
 
 int ldp_set_sm_reserve(int n_sms) {
@@ -1163,14 +1136,9 @@ int ldp_workspace_bytes(const ldp_params* params, size_t* bytes_out) {
     return LDP_OK;
 }
 
-// vec_hint: the host wrapper guarantees 16-byte aligned certainty planes when W % 4 == 0; the planes'
-// addresses live in device memory, so alignment cannot be checked here without a copy.  Callers that
-// cannot guarantee it set params->scalar_loads = 1 to force the scalar load path.
-
 int ldp_densify_refs(const ldp_params* params, const ldp_ref_desc* refs, const double* uniforms,
                      const ldp_outputs* out, void* workspace, size_t workspace_bytes, void* stream) {
-    g_launches = 0;
-    g_prof_n = 0;
+    begin_call();
     int rc = check_outputs(params, out);
     if (rc != LDP_OK) return rc;
     if (params->n_refs == 0) return LDP_OK;
@@ -1178,65 +1146,47 @@ int ldp_densify_refs(const ldp_params* params, const ldp_ref_desc* refs, const d
     if (params->rng_mode == LDP_RNG_EXPLICIT && !params->no_filter && !uniforms)
         return fail(LDP_ERR_INVALID, "explicit rng mode needs a uniform stream");
     Plan plan;
-    char* base = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace), 256));
-    rc = make_plan(params, base, &plan);
-    if (rc != LDP_OK) return rc;
-    if (plan.bytes + (size_t)(base - static_cast<char*>(workspace)) > workspace_bytes) return fail(LDP_ERR_WORKSPACE, "workspace too small");
+    if ((rc = bind_plan(params, workspace, workspace_bytes, &plan)) != LDP_OK) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cudaError_t e = clear_launch_state(plan, st);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(launch state)");
-    rc = launch_sample(params, refs, uniforms, out, plan, vec_ok_for(params), st);
-    if (rc != LDP_OK) return rc;
-    rc = launch_geometry(params, refs, out, plan, 1, st);
-    if (rc != LDP_OK) return rc;
-    return launch_pack(params, refs, out, plan, st);
+    if ((rc = clear_launch_state(plan, st)) != LDP_OK) return rc;
+    if ((rc = launch_sample(params, refs, uniforms, out, plan, st)) != LDP_OK) return rc;
+    return launch_triangulate(params, refs, out, plan, 1, st);
 }
 
 int ldp_sample_refs(const ldp_params* params, const ldp_ref_desc* refs, const double* uniforms,
                     const ldp_outputs* out, void* workspace, size_t workspace_bytes, void* stream) {
-    g_launches = 0;
-    g_prof_n = 0;
+    begin_call();
     if (!params || !out || !out->status || !out->n_samples || !out->sel_idx) return fail(LDP_ERR_INVALID, "sample stage needs status, n_samples, sel_idx");
     if (params->n_refs == 0) return LDP_OK;
     if (!refs || !workspace) return fail(LDP_ERR_INVALID, "null refs/workspace");
     if (params->rng_mode == LDP_RNG_EXPLICIT && !params->no_filter && !uniforms)
         return fail(LDP_ERR_INVALID, "explicit rng mode needs a uniform stream");
     Plan plan;
-    char* base = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace), 256));
-    int rc = make_plan(params, base, &plan);
+    int rc = bind_plan(params, workspace, workspace_bytes, &plan);
     if (rc != LDP_OK) return rc;
-    if (plan.bytes + (size_t)(base - static_cast<char*>(workspace)) > workspace_bytes) return fail(LDP_ERR_WORKSPACE, "workspace too small");
-    cudaError_t e = clear_launch_state(plan, static_cast<cudaStream_t>(stream));
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(launch state)");
-    return launch_sample(params, refs, uniforms, out, plan, vec_ok_for(params), static_cast<cudaStream_t>(stream));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if ((rc = clear_launch_state(plan, st)) != LDP_OK) return rc;
+    return launch_sample(params, refs, uniforms, out, plan, st);
 }
 
 int ldp_triangulate_samples(const ldp_params* params, const ldp_ref_desc* refs, const ldp_outputs* out,
                             void* workspace, size_t workspace_bytes, void* stream) {
-    g_launches = 0;
-    g_prof_n = 0;
+    begin_call();
     int rc = check_outputs(params, out);
     if (rc != LDP_OK) return rc;
     if (!out->sel_idx) return fail(LDP_ERR_INVALID, "triangulate stage reads out->sel_idx / out->n_samples");
     if (params->n_refs == 0) return LDP_OK;
     if (!refs || !workspace) return fail(LDP_ERR_INVALID, "null refs/workspace");
     Plan plan;
-    char* base = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace), 256));
-    rc = make_plan(params, base, &plan);
-    if (rc != LDP_OK) return rc;
-    if (plan.bytes + (size_t)(base - static_cast<char*>(workspace)) > workspace_bytes) return fail(LDP_ERR_WORKSPACE, "workspace too small");
+    if ((rc = bind_plan(params, workspace, workspace_bytes, &plan)) != LDP_OK) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cudaError_t e = clear_launch_state(plan, st);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(launch state)");
-    rc = launch_geometry(params, refs, out, plan, 0, st);
-    if (rc != LDP_OK) return rc;
-    return launch_pack(params, refs, out, plan, st);
+    if ((rc = clear_launch_state(plan, st)) != LDP_OK) return rc;
+    return launch_triangulate(params, refs, out, plan, 0, st);
 }
 
 int ldp_postprocess_certainty(const ldp_params* params, const ldp_ref_desc* refs, float* outp,
                               size_t ref_stride, size_t plane_stride, void* stream) {
-    g_launches = 0;
-    g_prof_n = 0;
+    begin_call();
     if (!params || params->n_refs < 0 || params->H <= 0 || params->W <= 0) return fail(LDP_ERR_INVALID, "bad shape");
     if (params->n_refs == 0) return LDP_OK;
     if (!refs || !outp) return fail(LDP_ERR_INVALID, "null refs/out");
@@ -1245,12 +1195,9 @@ int ldp_postprocess_certainty(const ldp_params* params, const ldp_ref_desc* refs
     const int N = params->H * params->W;
     const int bx = std::min((N + ldp::KP_THREADS - 1) / ldp::KP_THREADS, 4 * sm_count());
     const dim3 grid((unsigned)bx, LDP_MAX_NN, (unsigned)params->n_refs);
-    { KernelTimer kt(st, "ldp_prologue_kernel");
-      (void)launch_k(ldp::ldp_prologue_kernel, dim3(grid), dim3(ldp::KP_THREADS), 0, st, *params, refs, outp, ref_stride, plane_stride); }
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "ldp_prologue_kernel");
-    return LDP_OK;
+    KernelTimer kt(st, "ldp_prologue_kernel");
+    return launch("ldp_prologue_kernel", ldp::ldp_prologue_kernel, grid, dim3(ldp::KP_THREADS), 0, st, *params, refs, outp, ref_stride,
+                  plane_stride);
 }
 
 }  // extern "C"

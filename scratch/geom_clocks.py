@@ -7,7 +7,7 @@ B.NVCC_FLAGS.append("-DLDP_GEOM_CLOCKS")
 for f in sys.argv[1:]:
     B.NVCC_FLAGS.append(f)
 B.build(force=True)
-from lichtfeld_densification_plugin_b200 import synth, _native as N
+from lichtfeld_densification_plugin_b200 import synth
 from lichtfeld_densification_plugin_b200.engine import DensifyEngine, PathConfig
 dev = torch.device("cuda", 0)
 scene = synth.make_scene(185, "fast", 0.25, 4)
@@ -30,7 +30,6 @@ for _ in range(NRUN):
 torch.cuda.synchronize()
 params = eng._params(batch, cfg, False, 0, 0)
 host = (C.c_longlong * (len(batch) * 32))()
-eng.lib.ldp_debug_read_clocks.argtypes = [C.POINTER(N.LdpParams), C.c_void_p, C.POINTER(C.c_longlong)]
 rc = eng.lib.ldp_debug_read_clocks(C.byref(params), C.c_void_p(eng._workspace.data_ptr()), host)
 clk = np.array(host[:], dtype=np.float64).reshape(len(batch), 32)[:, :36 if False else 32]
 names = {0: "stage constants", 10: "grid dependency sync", 1: "idx, S, barrier", 2: "gather (k, warp row, texels)", 3: "coords, Sampson, colour", 4: "DLT rows",

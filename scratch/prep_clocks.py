@@ -5,7 +5,7 @@ import numpy as np, torch
 from lichtfeld_densification_plugin_b200 import build as B
 B.NVCC_FLAGS.append("-DLDP_PHASE_CLOCKS")
 B.build(force=True)
-from lichtfeld_densification_plugin_b200 import synth, _native as N
+from lichtfeld_densification_plugin_b200 import synth
 from lichtfeld_densification_plugin_b200.engine import DensifyEngine, PathConfig
 dev = torch.device("cuda", 0)
 scene = synth.make_scene(185, "fast", 0.25, 4)
@@ -24,7 +24,6 @@ for _ in range(4):
 torch.cuda.synchronize()
 params = eng._params(batch, cfg, False, 0, 0)
 host = (C.c_longlong * (len(batch) * 32))()
-eng.lib.ldp_debug_read_clocks.argtypes = [C.POINTER(N.LdpParams), C.c_void_p, C.POINTER(C.c_longlong)]
 eng.lib.ldp_debug_read_clocks(C.byref(params), C.c_void_p(eng._workspace.data_ptr()), host)
 clk = np.array(host[:]).reshape(len(batch), 32)
 t0 = clk[:, 16].min()

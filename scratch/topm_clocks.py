@@ -3,7 +3,7 @@ sys.path.insert(0, "/root/repo")
 import numpy as np, torch
 from lichtfeld_densification_plugin_b200 import build as B
 B.NVCC_FLAGS.append("-DLDP_PHASE_CLOCKS"); B.build(force=True)
-from lichtfeld_densification_plugin_b200 import synth, _native as N
+from lichtfeld_densification_plugin_b200 import synth
 from lichtfeld_densification_plugin_b200.engine import DensifyEngine, PathConfig
 dev = torch.device("cuda", 0)
 FAM = sys.argv[1] if len(sys.argv) > 1 else "R"
@@ -17,7 +17,6 @@ for _ in range(3): out = eng.densify(b, cfg)
 torch.cuda.synchronize()
 params = eng._params(b, cfg, False, 0, 0)
 host = (C.c_longlong * (len(b) * 32))()
-eng.lib.ldp_debug_read_clocks.argtypes = [C.POINTER(N.LdpParams), C.c_void_p, C.POINTER(C.c_longlong)]
 eng.lib.ldp_debug_read_clocks(C.byref(params), C.c_void_p(eng._workspace.data_ptr()), host)
 clk = np.array(host[:]).reshape(len(b), 32)
 for a, bb, nm in ((0, 1, "cap count (+ radix select)"), (1, 2, "tie rows"), (2, 3, "gather / ordered emit"), (3, 4, "sort"),):

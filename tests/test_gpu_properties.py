@@ -481,3 +481,33 @@ def test_launches_in_flight_with_late_starting_draw_ctas(engine):
         ns, uu, off, xyz = want[c]
         assert torch.equal(o.n_samples, ns) and torch.equal(o.uniforms_used, uu), (c, (o.uniforms_used != uu).nonzero().flatten().tolist())
         assert torch.equal(o.ref_offset, off) and torch.equal(o.xyz[:int(off[-1])], xyz), c
+
+
+@pytest.mark.parametrize("no_filter, kernels", [
+    (False, ["ldp_stream_kernel", "ldp_prep_kernel", "ldp_draw_kernel", "ldp_resume_kernel", "ldp_geometry_kernel", "ldp_fix_kernel",
+             "ldp_pack_kernel"]),
+    (True, ["ldp_stream_kernel", "ldp_topm_kernel", "ldp_geometry_kernel", "ldp_fix_kernel", "ldp_pack_kernel"]),
+])
+def test_profile_names_and_launch_count(engine, fast_scene, no_filter, kernels):
+    """One call's profile lists its kernels in launch order under the names bench.py's per-kernel report keys on, and
+    ldp_last_launch_count (bench.py's gpu_launches) counts exactly those launches."""
+    import ctypes as C
+    from lichtfeld_densification_plugin_b200.engine import PathConfig
+    scene, inputs = fast_scene
+    dev = engine.device
+    b = engine.new_batch(scene.H, scene.W, scene.w_match, scene.h_match)
+    for rp in range(2):
+        inp = inputs[rp]
+        k = len(inp["nbr_indices"])
+        b.add([inp["cert"][q].to(dev) for q in range(k)], [inp["warp"][q].to(dev) for q in range(k)], inp["image"].to(dev),
+              scene.cameras[inp["ref_index"]], [scene.cameras[j] for j in inp["nbr_indices"]], rng_stream=rp)
+    lib = engine.lib
+    assert lib.ldp_profile_enable(1) == 0
+    try:
+        engine.densify(b, PathConfig(matches_per_ref=10000, no_filter=no_filter, seed=3))
+        assert lib.ldp_last_launch_count() == len(kernels)
+        ms = (C.c_float * 64)()
+        assert lib.ldp_profile_read(ms, 64) == len(kernels)
+        assert [lib.ldp_profile_name(i).decode() for i in range(len(kernels))] == kernels
+    finally:
+        lib.ldp_profile_enable(0)

@@ -24,12 +24,35 @@ def test_header_symbols_exported(lib):
         assert hasattr(lib, name), name
 
 
+SCALARS = {"int": ctypes.c_int, "int32_t": ctypes.c_int32, "int64_t": ctypes.c_int64, "uint64_t": ctypes.c_uint64,
+           "size_t": ctypes.c_size_t, "double": ctypes.c_double, "const char*": ctypes.c_char_p}
+
+
+def test_binding_signatures_match_the_header(lib):
+    """Every prototype's return type and parameter list against the binding's restype / argtypes (a missing argtypes lets
+    ctypes pass a Python int as a 32-bit C int, which truncates a pointer)."""
+    header = open(os.path.join(ROOT, "include", "ldp_b200.h")).read()
+    protos = re.findall(r"^\s*(int|int64_t|const char\*)\s+(ldp_[a-z_0-9]+)\s*\(([^)]*)\)\s*;", header, flags=re.M)
+    assert [name for _, name, _ in protos] == list(_native.SIGNATURES)
+    for ret, name, params in protos:
+        fn = getattr(lib, name)
+        assert fn.restype is SCALARS[ret], name
+        params = [] if params.strip() == "void" else [" ".join(p.split()) for p in params.split(",")]
+        assert fn.argtypes is not None and len(fn.argtypes) == len(params), name
+        for decl, t in zip(params, fn.argtypes):
+            if "*" in decl:
+                assert t is ctypes.c_void_p or issubclass(t, ctypes._Pointer), (name, decl, t)
+            else:
+                assert t is SCALARS[decl.rsplit(" ", 1)[0]], (name, decl, t)
+
+
 def test_abi_version_and_struct_layout(lib):
     header = open(os.path.join(ROOT, "include", "ldp_b200.h")).read()
     assert int(re.search(r"#define LDP_ABI_VERSION (\d+)", header).group(1)) == lib.ldp_abi_version() == _native.LDP_ABI_VERSION
     assert int(re.search(r"#define LDP_MAX_NN (\d+)", header).group(1)) == _native.LDP_MAX_NN
-    for which, struct in enumerate((_native.LdpParams, _native.LdpRefDesc, _native.LdpOutputs)):
+    for which, struct in enumerate((_native.LdpParams, _native.LdpRefDesc, _native.LdpOutputs, _native.LdpLens)):
         assert lib.ldp_struct_size(which) == ctypes.sizeof(struct)
+    assert lib.ldp_struct_size(4) == -1
     assert _native.REF_DESC_DTYPE.itemsize == ctypes.sizeof(_native.LdpRefDesc)
 
 
