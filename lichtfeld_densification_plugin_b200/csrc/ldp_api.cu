@@ -182,13 +182,14 @@ const StreamKernel k_stream[3][9] = {
      ldp::ldp_stream_kernel<4, 2>, ldp::ldp_stream_kernel<0, 2>, ldp::ldp_stream_kernel<0, 2>, ldp::ldp_stream_kernel<0, 2>,
      ldp::ldp_stream_kernel<0, 2>},
 };
-// [chunk_shift 5, 6, 7, other][W divides the pass stride: a thread stays in one pixel column]
-using PrepKernel = decltype(&ldp::ldp_prep_generic_kernel);
-const PrepKernel k_prep[4][2] = {
-    {ldp::ldp_prep_kernel<5, false>, ldp::ldp_prep_kernel<5, true>},
-    {ldp::ldp_prep_kernel<6, false>, ldp::ldp_prep_kernel<6, true>},
-    {ldp::ldp_prep_kernel<7, false>, ldp::ldp_prep_kernel<7, true>},
-    {ldp::ldp_prep_kernel<0, false>, ldp::ldp_prep_kernel<0, true>},
+// [chunk_shift 5, 6, 7, other][PrepCols]
+using ldp::PrepCols;
+using PrepKernel = decltype(&ldp::ldp_prep_kernel<5, PrepCols::CONST>);
+const PrepKernel k_prep[4][3] = {
+    {ldp::ldp_prep_kernel<5, PrepCols::CONST>, ldp::ldp_prep_kernel<5, PrepCols::QUAD>, ldp::ldp_prep_kernel<5, PrepCols::PIXEL>},
+    {ldp::ldp_prep_kernel<6, PrepCols::CONST>, ldp::ldp_prep_kernel<6, PrepCols::QUAD>, ldp::ldp_prep_kernel<6, PrepCols::PIXEL>},
+    {ldp::ldp_prep_kernel<7, PrepCols::CONST>, ldp::ldp_prep_kernel<7, PrepCols::QUAD>, ldp::ldp_prep_kernel<7, PrepCols::PIXEL>},
+    {ldp::ldp_prep_kernel<0, PrepCols::CONST>, ldp::ldp_prep_kernel<0, PrepCols::QUAD>, ldp::ldp_prep_kernel<0, PrepCols::PIXEL>},
 };
 
 // Raises the dynamic shared memory limit of every kernel that takes more than the default 48 KB, once per device (a
@@ -204,7 +205,6 @@ int configure_device() {
         };
         raise((const void*)ldp::ldp_draw_kernel<1>, K1_SMEM_BUDGET);
         raise((const void*)ldp::ldp_draw_kernel<2>, K1_SMEM_BUDGET);
-        raise((const void*)ldp::ldp_prep_generic_kernel, PREP_SMEM_MAX);
         for (const auto& row : k_prep)
             for (PrepKernel k : row) raise((const void*)k, PREP_SMEM_MAX);
         raise((const void*)ldp::ldp_topm_kernel, K1_SMEM_BUDGET);
@@ -271,7 +271,6 @@ int make_plan(const ldp_params* p, void* base, Plan* plan) {
     g.t_magic32 = (g.tile > 1) ? (uint32_t)(((1ull << 32) + (unsigned long long)g.tile - 1) / (unsigned long long)g.tile) : 0u;
     g.step_dx = (ldp::KS_THREADS * 4) % p->W;
     g.step_dy = (ldp::KS_THREADS * 4) / p->W;
-    g.prep_lean = (p->W <= 8192 && p->H <= 8192 && g.tile > 1) ? 1 : 0;
     int cs = 5;
     for (;; ++cs) {
         const size_t nchunk = ((size_t)N + ((size_t)1 << cs) - 1) >> cs;
@@ -444,10 +443,14 @@ int launch_sample(const ldp_params* p, const ldp_ref_desc* refs, const double* u
         if ((rc = check(cudaMemsetAsync(plan.ws.csum0, 0, bytes, st), "cudaMemsetAsync(csum0)")) != LDP_OK) return rc;
     }
     { KernelTimer kt(st, "ldp_prep_kernel");
-      const int cs = plan.geom.chunk_shift;
-      const bool xc = plan.geom.step_dx == 0;       // W divides the pass stride: a thread stays in one pixel column
-      const PrepKernel kp = (plan.geom.vec && plan.geom.prep_lean) ? k_prep[(cs >= 5 && cs <= 7) ? cs - 5 : 3][xc]
-                                                                   : ldp::ldp_prep_generic_kernel;
+      const ldp::SampleGeom& g = plan.geom;
+      // QUAD needs every quad in one image row (W % 4 == 0) and in at most two tiles (tiles wider than one pixel), and
+      // umulhi(x, t_magic32) exact for every column: (W - 1) * tile < 2^32.  CONST is the QUAD case in which W divides the
+      // pass stride (step_dx == 0), so that a thread stays in one pixel column.  Every other map takes PIXEL.
+      const bool quad = p->W % 4 == 0 && g.tile > 1 && (unsigned long long)(p->W - 1) * g.tile < (1ull << 32);
+      const PrepCols cols = !quad ? PrepCols::PIXEL : g.step_dx == 0 ? PrepCols::CONST : PrepCols::QUAD;
+      const int cs = g.chunk_shift;
+      const PrepKernel kp = k_prep[(cs >= 5 && cs <= 7) ? cs - 5 : 3][(int)cols];
       if ((rc = launch("ldp_prep_kernel", kp, grid, dim3(ldp::KS_THREADS), plan.prep_smem, st, *p, refs, plan.ws, *out, plan.geom)) != LDP_OK)
           return rc; }
     // ---- round 1: independent CTAs, as many per view as the device has SMs for (one CTA per SM: the table fills it), less

@@ -65,9 +65,8 @@ struct SampleGeom {     // launch-constant shape of the sampler
     int prep_lb_cap;    // local tile bins per CTA of the prep kernel
     unsigned long long w_magic;   // ceil(2^40 / W): floor(n / W) = (n * w_magic) >> 40 for n < 2^21 * ...
     unsigned long long t_magic;   // ceil(2^40 / tile)
-    uint32_t t_magic32;           // ceil(2^32 / tile): floor(n / tile) = umulhi(n, t_magic32) for n * tile < 2^32
+    uint32_t t_magic32;           // ceil(2^32 / tile) (0 for tile 1): floor(n / tile) = umulhi(n, t_magic32) for n * tile < 2^32
     int step_dx, step_dy;         // (KS_THREADS * 4) % W, (KS_THREADS * 4) / W: pixel step of the full-grid passes
-    int prep_lean;                // the lean prep kernel applies (vector path, W <= 8192)
     int draw_ept;       // draw kernel: chunk-table entries per thread (multiple of 8)
     int draw_pre_cap;   // draw kernel: doubles in the padded prefix table
     int draw_ng;        // draw kernel: guide-table buckets

@@ -306,155 +306,17 @@ ldp_stream_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, con
 // =============================================================================================
 // K1b  prep: same grid.  s = f32(sum of the f64 partials) (or the caller's override); p = fl32(w / s) is
 //      written back IN PLACE over w (so the draw kernel never divides); f64 sums of p per chunk go to the
-//      global chunk table; per-tile arg-max of p (the coverage picks) via shared-memory then global 64-bit
-//      atomicMax on (p bits, ~index); number of positive p and their smallest exponent (exactness test).
+//      global chunk table; per-tile arg-max of p (the coverage picks); number of positive p and their smallest
+//      exponent (exactness test); clears the selection bitmap.
 //      reference core/sampling.py:26-29 (normalise), :34-50 (coverage walk == per-tile arg-max)
-//      Issue-bound: per quad one tile lookup (quads that straddle a tile edge take the per-pixel path).
-// =============================================================================================
-__global__ void __launch_bounds__(KS_THREADS)
-ldp_prep_generic_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const Workspace ws, const ldp_outputs out,
-                        const SampleGeom G)
-{
-    grid_dependency_sync();
-    {   // the draw kernels' selection bitmap: cleared here, one kernel ahead of its first use
-        uint32_t* bm = ws.bitmap + (size_t)blockIdx.y * ws.n_words;
-        for (int i = blockIdx.x * KS_THREADS + threadIdx.x; i < (int)ws.n_words; i += gridDim.x * KS_THREADS) bm[i] = 0u;
-    }
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    __shared__ int red_i[32];
-    __shared__ float s_s;
-    __shared__ int s_bad;
-    const int r = blockIdx.y, blk = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
-    const int N = G.N, W = P.W;
-    const ldp_ref_desc* rd = refs + r;
-    // ---- s: fixed-order reduction of the per-CTA partials (every CTA of the view computes the same value)
-    if (tid < 32) {
-        double a = 0.0;
-        int f = 0;
-        for (int i = lane; i < (int)ws.nblk; i += 32) {
-            a += ws.partial[(size_t)r * ws.nblk + i];
-            f |= ws.bflags[(size_t)r * ws.nblk + i];
-        }
-        a = warp_sum(a);
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) f |= __shfl_xor_sync(0xffffffffu, f, o);
-        if (lane == 0) {
-            float s = (float)a;
-            if (rd->weight_sum_override > 0.f) s = rd->weight_sum_override;
-            s_s = s;
-            s_bad = f;
-            if (blk == 0) {
-                ws.rstat[r].s = s;
-                ws.rstat[r].bad = f;
-                if (out.weight_sum) out.weight_sum[r] = s;
-            }
-        }
-    }
-    __syncthreads();
-    const float s = s_s;
-    if (s_bad || !(s > 0.f)) return;       // the draw kernel reports the status
-
-    // ---- local tile bins of the rows this CTA covers
-    const int base = blk * KS_SPAN;
-    const int end = min(base + KS_SPAN, N);
-    const int y_first = (int)div_magic((uint32_t)base, G.w_magic), y_last = (int)div_magic((uint32_t)(end - 1), G.w_magic);
-    const int ty0 = (int)div_magic((uint32_t)y_first, G.t_magic), ty1 = (int)div_magic((uint32_t)y_last, G.t_magic);
-    const int nlb = (ty1 - ty0 + 1) * G.nbx;
-    unsigned long long* lb = reinterpret_cast<unsigned long long*>(smem_raw);            // [nlb]
-    for (int i = tid; i < nlb; i += KS_THREADS) lb[i] = 0ull;
-    __syncthreads();
-
-    float* __restrict__ w = ws.w + (size_t)r * ws.n_pad;
-    double* __restrict__ csum = ws.csum + (size_t)r * ws.nchunk_pad;
-    double* __restrict__ csum0 = ws.csum0 + (size_t)r * ws.nchunk_pad;      // the copy the first draw round searches (see Workspace)
-    const int cs = G.chunk_shift;
-    const int gl = min(32, (1 << cs) >> 2);            // lanes that share one chunk
-    int lpos = 0;
-    uint32_t lminbits = 0x7fffffffu;                   // smallest positive p (bit pattern orders like the value)
-#pragma unroll 2
-    for (int it = 0; it < KS_SPAN / (KS_THREADS * 4); ++it) {
-        const int px = base + (it * KS_THREADS + tid) * 4;     // warp-uniform trip count: whole warps drop out together
-        double a = 0.0;
-        if (px < N) {
-            const float4 v = *reinterpret_cast<const float4*>(w + px);
-            float pv[4];
-            pv[0] = __fdiv_rn(v.x, s); pv[1] = __fdiv_rn(v.y, s);              // core/sampling.py:29 (f32 division)
-            pv[2] = __fdiv_rn(v.z, s); pv[3] = __fdiv_rn(v.w, s);
-            *reinterpret_cast<float4*>(w + px) = make_float4(pv[0], pv[1], pv[2], pv[3]);
-            a = (widen_f32(pv[0]) + widen_f32(pv[1])) + (widen_f32(pv[2]) + widen_f32(pv[3]));
-            // positives, smallest positive
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const uint32_t b = __float_as_uint(pv[j]);
-                lpos += (pv[j] > 0.f) ? 1 : 0;
-                lminbits = min(lminbits, (pv[j] > 0.f) ? b : 0x7fffffffu);
-            }
-            // per-tile arg-max.  A quad lies in one image row (W % 4 == 0 on this path) and touches at most two tiles:
-            // pixels [0, nsplit) belong to tile tx0, the rest to tx0 + 1.  Both halves are handled without divergence.
-            const int y = (int)div_magic((uint32_t)px, G.w_magic), x = px - y * W;
-            if (G.vec && G.tile > 1) {         // (tiles one pixel wide - maps narrower than 48 px - put four tiles under a quad: per pixel)
-                const int tx0 = (int)div_magic((uint32_t)x, G.t_magic);
-                const int nsplit = min(4, (tx0 + 1) * G.tile - x);
-                const int brow = ((int)div_magic((uint32_t)y, G.t_magic) - ty0) * G.nbx + tx0;
-                float pm0 = 0.f, pm1 = 0.f;
-                int j0 = 0, j1 = 0;
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {                      // strict > keeps the lowest index on ties
-                    if (j < nsplit) { if (pv[j] > pm0) { pm0 = pv[j]; j0 = j; } }
-                    else            { if (pv[j] > pm1) { pm1 = pv[j]; j1 = j; } }
-                }
-                if (pm0 > 0.f) {
-                    const unsigned long long key = cov_key(pm0, px + j0);
-                    if (lb[brow] < key) atomicMax(&lb[brow], key);
-                }
-                if (pm1 > 0.f) {
-                    const unsigned long long key = cov_key(pm1, px + j1);
-                    if (lb[brow + 1] < key) atomicMax(&lb[brow + 1], key);
-                }
-            } else {
-                int yy = y, xx = x;
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    if (pv[j] > 0.f && px + j < N) {
-                        const int b = ((int)div_magic((uint32_t)yy, G.t_magic) - ty0) * G.nbx + (int)div_magic((uint32_t)xx, G.t_magic);
-                        const unsigned long long key = cov_key(pv[j], px + j);
-                        if (lb[b] < key) atomicMax(&lb[b], key);
-                    }
-                    if (++xx == W) { xx = 0; ++yy; }
-                }
-            }
-        }
-        for (int o = 1; o < gl; o <<= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-        if (px < N && (lane & (gl - 1)) == 0) {
-            if (cs <= 7) { csum[px >> cs] = a; csum0[px >> cs] = a; }
-            else { atomicAdd(&csum[px >> cs], a); atomicAdd(&csum0[px >> cs], a); }      // chunks wider than a warp-row (zeroed by the host memset)
-        }
-    }
-    const int npos = block_sum(lpos, red_i);
-    const int eminbits = block_min((int)lminbits, red_i);
-    if (tid == 0) {
-        if (npos) atomicAdd(&ws.rstat[r].npos, npos);
-        if (eminbits != 0x7fffffff) atomicMax(&ws.rstat[r].emin_inv, 255 - ((eminbits >> 23) & 0xff));
-    }
-    __syncthreads();
-    unsigned long long* gb = ws.gbins + (size_t)r * ws.bins_cap;
-    for (int i = tid; i < nlb; i += KS_THREADS) {
-        const unsigned long long key = lb[i];
-        if (key) atomicMax(&gb[(ty0 + i / G.nbx) * G.nbx + (i % G.nbx)], key);
-    }
-}
-
-// =============================================================================================
-// K1b' prep, lean variant for the vector path (W % 4 == 0, 16-byte aligned rows, W <= 8192): same outputs as
-//      ldp_prep_generic_kernel with ~4x fewer instructions per pixel (the generic kernel is issue-bound):
+//      Issue-bound, so the per-pixel work is kept small:
 //        * p = fl32(w / s) with the correctly rounded reciprocal of s hoisted out of the loop and two FMA residual
 //          corrections per value (div_by); zeros and tiny quotients take the IEEE division.
 //        * positives / smallest positive exponent from the quad minimum; zeros (border, masked) take a side path;
-//        * per-tile arg-max of p in two phases with native 32-bit shared atomics: (A) tile maximum of the value,
-//          (B) after a CTA barrier, lowest pixel index among the pixels that reach it -- only quads whose maximum
-//          equals their tile's maximum look at single pixels.  One 64-bit key per tile and CTA goes to the global
-//          table, as before.
+//        * per-tile arg-max as one 64-bit key (p bits << 32 | ~index) per tile in shared memory, raised by atomicMax
+//          behind an exact pre-filter; one key per tile and CTA then goes to the global table.
 //      CS = chunk_shift (5..7: chunk sums by shuffles inside a warp row of 128 pixels; 0: wider chunks, atomics).
+//      COLS = how a quad's coverage tiles are found (PrepCols; launch_sample states when each mode applies).
 // =============================================================================================
 // fl32(a / b) for b > 0 with y = RN(1/b) hoisted: two residual corrections on the FMA pipe.  q1 is a faithful quotient
 // (error <= 1/2 ulp + 2^-23 ulp), so by Markstein's theorem (y correctly rounded, residual exact) the second correction
@@ -477,7 +339,13 @@ __device__ __forceinline__ long long gtimer() { long long t; asm volatile("mov.u
 #ifndef KP_MIN_BLOCKS
 #define KP_MIN_BLOCKS 5
 #endif
-template <int CS, bool XCONST>
+// How the prep kernel finds the coverage tiles of a quad's pixels.
+enum class PrepCols {
+    CONST,      // as QUAD, and a thread's quads all start in one pixel column: its tile split is computed once
+    QUAD,       // a quad lies in one image row and in at most two tiles, whose columns umulhi(x, t_magic32) finds
+    PIXEL,      // any map: a tile per pixel, through the 40-bit magic
+};
+template <int CS, PrepCols COLS>
 __global__ void __launch_bounds__(KS_THREADS, KP_MIN_BLOCKS)
 ldp_prep_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const Workspace ws, const ldp_outputs out,
                 const SampleGeom G)
@@ -528,7 +396,9 @@ ldp_prep_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const
 
     const int end = min(base + KS_SPAN, N);
     const int y_first = (int)div_magic((uint32_t)base, G.w_magic), y_last = (int)div_magic((uint32_t)(end - 1), G.w_magic);
-    const int ty0 = (int)__umulhi((uint32_t)y_first, G.t_magic32), ty1 = (int)__umulhi((uint32_t)y_last, G.t_magic32);
+    // tile rows: umulhi is exact for y * tile < N < 2^30, but one-pixel tiles (PIXEL only) have no 32-bit magic
+    const int ty0 = (COLS == PrepCols::PIXEL) ? (int)div_magic((uint32_t)y_first, G.t_magic) : (int)__umulhi((uint32_t)y_first, G.t_magic32);
+    const int ty1 = (COLS == PrepCols::PIXEL) ? (int)div_magic((uint32_t)y_last, G.t_magic) : (int)__umulhi((uint32_t)y_last, G.t_magic32);
     const int nlb = (ty1 - ty0 + 1) * G.nbx;
     unsigned long long* lb = reinterpret_cast<unsigned long long*>(smem_raw);            // [nlb] (p bits << 32) | ~index
     for (int i = tid; i < nlb; i += KS_THREADS) lb[i] = 0ull;
@@ -544,7 +414,7 @@ ldp_prep_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const
     int lpos = 0;
     uint32_t lmin1 = 0xFFFFFFFFu;                      // (bit pattern - 1) of the smallest positive p; zeros wrap to the top
     int y = (int)div_magic((uint32_t)px, G.w_magic), x = px - y * W;
-    // tile geometry of the quad: pixels [0, nsplit) lie in tile column tx0, the rest in tx0 + 1 (a quad lies in one row)
+    // tile geometry of a CONST / QUAD quad: pixels [0, nsplit) lie in tile column tx0, the rest in tx0 + 1
     int tx0 = (int)__umulhi((uint32_t)x, G.t_magic32);
     int nsplit = (tx0 + 1) * G.tile - x;               // >= 4: no straddle
 #pragma unroll
@@ -571,24 +441,38 @@ ldp_prep_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const
             *reinterpret_cast<float4*>(w + px) = make_float4(p0, p1, p2, p3);
             a = ((double)p0 + (double)p1) + ((double)p2 + (double)p3);
             // ---- per-tile arg-max of p, lowest index on ties: 64-bit key, exact pre-filter, rare CAS
-            if (!XCONST) {
-                tx0 = (int)__umulhi((uint32_t)x, G.t_magic32);
-                nsplit = (tx0 + 1) * G.tile - x;
-            }
-            const int b0 = ((int)__umulhi((uint32_t)y, G.t_magic32) - ty0) * G.nbx + tx0;
-            const bool s1 = nsplit > 1, s2 = nsplit > 2, s3 = nsplit > 3;               // pixel j belongs to the first tile
-            const float m0 = fmaxf(fmaxf(p0, s1 ? p1 : 0.f), fmaxf(s2 ? p2 : 0.f, s3 ? p3 : 0.f));
-            const unsigned long long k0 = ((unsigned long long)__float_as_uint(m0) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)px);
-            if (k0 > lb[b0]) {                         // could improve the tile (k0 bounds the exact key from above)
-                const int j0 = (p0 == m0) ? 0 : (s1 && p1 == m0) ? 1 : (s2 && p2 == m0) ? 2 : 3;
-                if (m0 > 0.f) atomicMax(&lb[b0], k0 - (unsigned long long)j0);
-            }
-            if (!s3) {                                 // the quad straddles a tile edge
-                const float m1 = fmaxf(fmaxf(s1 ? 0.f : p1, s2 ? 0.f : p2), p3);
-                const unsigned long long k1 = ((unsigned long long)__float_as_uint(m1) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)px);
-                if (k1 > lb[b0 + 1]) {
-                    const int j1 = (!s1 && p1 == m1) ? 1 : (!s2 && p2 == m1) ? 2 : 3;
-                    if (m1 > 0.f) atomicMax(&lb[b0 + 1], k1 - (unsigned long long)j1);
+            if (COLS == PrepCols::PIXEL) {                 // the quad may wrap a row end or cover several tiles
+                const float pv[4] = {p0, p1, p2, p3};
+                int xx = x, yy = y;
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    if (pv[j] > 0.f && px + j < N) {
+                        const int b = ((int)div_magic((uint32_t)yy, G.t_magic) - ty0) * G.nbx + (int)div_magic((uint32_t)xx, G.t_magic);
+                        const unsigned long long key = cov_key(pv[j], px + j);
+                        if (lb[b] < key) atomicMax(&lb[b], key);
+                    }
+                    if (++xx == W) { xx = 0; ++yy; }
+                }
+            } else {
+                if (COLS == PrepCols::QUAD) {
+                    tx0 = (int)__umulhi((uint32_t)x, G.t_magic32);
+                    nsplit = (tx0 + 1) * G.tile - x;
+                }
+                const int b0 = ((int)__umulhi((uint32_t)y, G.t_magic32) - ty0) * G.nbx + tx0;
+                const bool s1 = nsplit > 1, s2 = nsplit > 2, s3 = nsplit > 3;               // pixel j belongs to the first tile
+                const float m0 = fmaxf(fmaxf(p0, s1 ? p1 : 0.f), fmaxf(s2 ? p2 : 0.f, s3 ? p3 : 0.f));
+                const unsigned long long k0 = ((unsigned long long)__float_as_uint(m0) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)px);
+                if (k0 > lb[b0]) {                         // could improve the tile (k0 bounds the exact key from above)
+                    const int j0 = (p0 == m0) ? 0 : (s1 && p1 == m0) ? 1 : (s2 && p2 == m0) ? 2 : 3;
+                    if (m0 > 0.f) atomicMax(&lb[b0], k0 - (unsigned long long)j0);
+                }
+                if (!s3) {                                 // the quad straddles a tile edge
+                    const float m1 = fmaxf(fmaxf(s1 ? 0.f : p1, s2 ? 0.f : p2), p3);
+                    const unsigned long long k1 = ((unsigned long long)__float_as_uint(m1) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)px);
+                    if (k1 > lb[b0 + 1]) {
+                        const int j1 = (!s1 && p1 == m1) ? 1 : (!s2 && p2 == m1) ? 2 : 3;
+                        if (m1 > 0.f) atomicMax(&lb[b0 + 1], k1 - (unsigned long long)j1);
+                    }
                 }
             }
         }
@@ -605,7 +489,7 @@ ldp_prep_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const
             if (px < N && lane == 0) { atomicAdd(&csum[px >> cs], a); atomicAdd(&csum0[px >> cs], a); }
         }
         px += STEP;
-        if (XCONST) {
+        if (COLS == PrepCols::CONST) {
             y += G.step_dy;
         } else {
             x += G.step_dx; y += G.step_dy;

@@ -210,7 +210,7 @@ def test_config5_base_640_sharding_invariance(engine):
 
 @pytest.mark.parametrize("case", list(range(24)) + [34, 38, 44])      # 34 / 38 / 44: maps 36 px wide, coverage tiles of ONE pixel
 def test_randomised_shapes(engine, case):
-    """Seeded random shapes through every kernel variant (vector / scalar rows, column-constant or not, generic prep,
+    """Seeded random shapes through every kernel variant (vector / scalar rows, every column mode of the prep kernel,
     ragged neighbour counts, map != match resolution, small and binding coverage budgets) against the oracle."""
     from lichtfeld_densification_plugin_b200 import synth
     rs = np.random.RandomState(1000 + case)

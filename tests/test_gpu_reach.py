@@ -2,8 +2,8 @@
 
 A. Neighbour counts 5-16: ldp_stream_kernel<0, *> (the generic neighbour count, and raw planes at nn >= 5), the 16-slot
    group tables of the geometry, fix and pack kernels, multiview masks above bit 7, the last lens-table entries.
-B. Maps above 2^21 pixels: chunk_shift >= 8 (ldp_prep_kernel<0, *>, chunk sums accumulated with f64 atomics) and maps
-   wider than 8192 pixels (generic prep kernel on the vector path).
+B. Maps above 2^19 pixels: chunk_shift 6 and 7, chunk_shift >= 8 (ldp_prep_kernel<0, *>, chunk sums accumulated with f64
+   atomics), each in every column mode of the prep kernel.
 
 Every test holds the kernels to the oracle with the bars of tests/gpu_harness.py: samples, uniforms consumed and rounds
 exact; keep masks exact up to the solver-noise flips compare_ref admits; xyz / rgb within the harness tolerances; group
@@ -54,9 +54,13 @@ def chunk_shift(H: int, W: int, tiles: int = 24) -> int:
         cs += 1
 
 
-def prep_lean(H: int, W: int, tiles: int = 24) -> bool:
-    """make_plan's g.prep_lean (ldp_api.cu:180): the specialised prep kernels serve maps up to 8192 on a side."""
-    return W <= 8192 and H <= 8192 and max(1, W // tiles) > 1
+def prep_cols(H: int, W: int, tiles: int = 24) -> str:
+    """launch_sample's column mode of ldp_prep_kernel: QUAD when every quad lies in one row and in at most two tiles whose
+    columns umulhi(x, t_magic32) finds exactly; CONST when W also divides the 1024-pixel pass stride; PIXEL otherwise."""
+    tile = max(1, W // tiles)
+    if W % 4 or tile == 1 or (W - 1) * tile >= 1 << 32:
+        return "PIXEL"
+    return "CONST" if 1024 % W == 0 else "QUAD"
 
 
 def topm_generic(H: int, W: int, M: int) -> bool:
@@ -73,7 +77,10 @@ def topm_generic(H: int, W: int, M: int) -> bool:
 def test_host_rules_restated():
     assert chunk_shift(1280, 1280) == 7 and chunk_shift(512, 512) == 5       # the largest / the bench map of the other suites
     assert chunk_shift(1536, 1536) == 8 and chunk_shift(2048, 2048) == 8 and chunk_shift(2560, 2560) == 9
-    assert not prep_lean(64, 8448) and prep_lean(64, 8192)
+    assert prep_cols(512, 512) == "CONST"
+    assert prep_cols(640, 640) == "QUAD" and prep_cols(64, 8448) == "QUAD"
+    assert all(prep_cols(H, W) == "PIXEL" for H, W in ((50, 61), (40, 36), (1001, 1001), (1281, 1279), (8, 327680)))
+    assert prep_cols(64, 2, tiles=1) == "PIXEL"           # W divides the stride, but a quad spans two rows
 
 
 # ---- comparison against the oracle --------------------------------------------------------------------------------------------
@@ -288,15 +295,17 @@ def test_lens_cameras_at_16_neighbours(engine):
 
 
 # ---- B. large maps ----------------------------------------------------------------------------------------------------------
-LARGE = [(1536, 1536, 8), (2048, 2048, 8), (2560, 2560, 9), (64, 8448, 6)]
+LARGE = [(1536, 1536, 8, "QUAD"), (2048, 2048, 8, "QUAD"), (2560, 2560, 9, "QUAD"), (64, 8448, 6, "QUAD"),
+         (1024, 1024, 6, "CONST"), (1536, 1024, 7, "CONST"), (2304, 1024, 8, "CONST"),
+         (1001, 1001, 6, "PIXEL"), (1281, 1279, 7, "PIXEL"), (8, 327680, 8, "PIXEL")]
 
 
-@pytest.mark.parametrize("H,W,cs", LARGE, ids=[f"{h}x{w}" for h, w, _ in LARGE])
-def test_large_maps_vs_oracle(engine, H, W, cs):
-    """chunk_shift >= 8 (ldp_prep_kernel<0, *>, atomic chunk sums, wide in-chunk scans) and a map wider than 8192
-    (the generic prep kernel on the vector path)."""
-    assert chunk_shift(H, W) == cs
-    assert (cs > 7) or not prep_lean(H, W)                # every case leaves the branches the other suites cover
+@pytest.mark.parametrize("H,W,cs,cols", LARGE, ids=[f"{h}x{w}" for h, w, _, _ in LARGE])
+def test_large_maps_vs_oracle(engine, H, W, cs, cols):
+    """chunk_shift >= 8 (ldp_prep_kernel<0, *>, atomic chunk sums, wide in-chunk scans), and every column mode of
+    ldp_prep_kernel at chunk_shift 6, 7 and >= 8, which the maps of the other suites do not reach.  64x8448 is QUAD above
+    8192 columns; 8x327680 is PIXEL because (W - 1) * tile passes 2^32 there."""
+    assert chunk_shift(H, W) == cs and prep_cols(H, W) == cols
     scene = _scene(4, n_views=10)
     scene.H, scene.W = H, W
     c = dict(M=10000, no_filter=False, wm=scene.w_match, hm=scene.h_match)
