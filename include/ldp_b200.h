@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define LDP_ABI_VERSION 17
+#define LDP_ABI_VERSION 18
 #define LDP_MAX_NN 16          /* neighbours per reference view (the panel clamps to 10) */
 #define LDP_MAX_BINS 4096      /* coverage tiles per map: ceil(W/tile)*ceil(H/tile), tile = max(1, W/24) */
 
@@ -381,6 +381,41 @@ int ldp_normals_workspace_bytes(int64_t n, int32_t k, size_t* bytes_out);
 int ldp_estimate_normals(const float* xyz, int64_t n, int32_t k, const float* centers, int32_t n_centers, const int32_t* center_idx,
                          float* normals_out, float* curvature_out, int32_t* knn_idx_out, int32_t* status_out, void* workspace,
                          size_t workspace_bytes, void* stream);
+
+/* ---- 3DGS initialisation (not in the reference) ---------------------------------------------------------------------
+ * graphdeco 3DGS's GaussianModel.create_from_pcd on the device, optionally flattened into discs along oriented normals.
+ * Inputs: xyz [n,3] f32 device, rgb [n,3] f32 device in [0, 1], normals [n,3] f32 device or NULL; k in [1, 63] (3DGS: 3);
+ * opacity alpha in (0, 1) (3DGS: 0.1); flatten in (0, 1] (1: isotropic; < 1 needs normals).  For every point i:
+ *   1. dist2: k_eff = min(k, n - 1).  With the outlier rule's d^2 = (dx*dx + dy*dy) + dz*dz in f64 without FMA over the
+ *      points j != i (exact duplicates count, at 0), m_i = (sequential f64 sum of the k_eff smallest d^2, ascending) /
+ *      k_eff; m_i = 0 when n = 1.  dist2_i = max(f32(m_i), f32(1e-7)) (3DGS: clamp_min(distCUDA2, 0.0000001)).
+ *   2. scales: s_i = f32(log(sqrt(f64(dist2_i)))), log and sqrt in f64; (s, s, s).  A point with a defined normal (step 4)
+ *      has the third scale f32(log(sqrt(f64(dist2_i))) + log(f64(flatten))) instead: its flat axis lies along the normal.
+ *   3. sh_dc per channel: __fdiv_rn(__fsub_rn(rgb_c, 0.5f), 0.28209479177387814f) (3DGS's RGB2SH in f32, bit-exact);
+ *      opacity: f32(log(alpha / (1 - alpha))) in f64, the same for every point (3DGS's inverse_sigmoid).
+ *   4. rotation (w, x, y, z), 3DGS's rot_0..rot_3.  Without normals, or when the normal's f64 length is 0 or not finite,
+ *      the point is undefined: (1, 0, 0, 0) and isotropic scales, counted.  Otherwise, with u the normal renormalised in
+ *      f64: q = (1 + u_z, -u_y, u_x, 0) / |.| (the shortest arc taking e_z to u) when 1 + u_z > 1e-12, else (0, 1, 0, 0);
+ *      each component rounded to f32 once.  3DGS's build_rotation(q) e_z is then u.
+ *   5. The search is ldp_statistical_outliers' values-only k-NN with k_eff + 1 entries, the point itself included: its own
+ *      d^2 = 0 is never larger than another, so entries 1..k_eff of the ascending list are the k_eff smallest d^2 over
+ *      j != i.  It stops only on the conservative bound of DESIGN.md §4.5, so dist2 is bit-exact.
+ * Parity with simple-knn's distCUDA2 is unpinned: it sums f32 squared distances; here each is exact in f64, rounded once.
+ * Outputs (device, f32): sh_dc_out [n,3], opacity_out [n], scales_out [n,3] (log scales), rotations_out [n,4], dist2_out
+ * [n] or NULL.  status_out: int32 [3] device = {1 if a coordinate is not finite (then nothing else is written), undefined
+ * normals, points whose search left the finest grid}.  n = 0 zeroes status_out and writes nothing else.  Synchronises the
+ * stream once (the trial grid, as ldp_statistical_outliers); ldp_debug_outlier_max_shells applies.  Results do not depend
+ * on the grid, the launch or the stream.
+ * ldp_pack_gaussian_ply_records: the vertices of 3DGS's save_ply, x y z nx ny nz f_dc_0..2 f_rest_0..(3((d+1)^2-1)-1)
+ * opacity scale_0..2 rot_0..3, all <f4: 68, 104, 164 or 248 bytes for sh_degree d = 0..3.  f_rest is zeros; the normals
+ * are zeros when normals is NULL.  n_dev as for ldp_pack_ply_records; records_out: device, 4-byte aligned. */
+int ldp_gaussian_workspace_bytes(int64_t n, int32_t k, size_t* bytes_out);
+int ldp_gaussian_init(const float* xyz, const float* rgb, const float* normals, int64_t n, int32_t k, double opacity, double flatten,
+                      float* sh_dc_out, float* opacity_out, float* scales_out, float* rotations_out, float* dist2_out,
+                      int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream);
+int ldp_pack_gaussian_ply_records(const float* xyz, const float* normals, const float* sh_dc, const float* opacity, const float* scales,
+                                  const float* rotations, int64_t n, const int64_t* n_dev, int32_t sh_degree, uint8_t* records_out,
+                                  void* stream);
 
 /* SMs the one-CTA-per-SM first draw kernel leaves free when ldp_params.sm_reserve is -1 (process-wide default, initially 0).
  * With several launches in flight on different streams (engine.DensifyRing) or a collective running beside the path, the

@@ -62,6 +62,10 @@ class DensePipelineConfig:
     outlier_std_ratio: float = 2.0
     normal_neighbors: int = 0        # > 0: PipelineResult.normals, PCA over this many nearest points, each normal facing
                                      # the camera that triangulated its point; 0 = off
+    gaussian_neighbors: int = 0      # > 0: PipelineResult.gaussians, 3DGS's initial splats (create_from_pcd), scales from
+                                     # this many nearest other points (3DGS: 3); 0 = off
+    gaussian_opacity: float = 0.1    # initial opacity of every splat (3DGS: 0.1)
+    gaussian_flatten: float = 1.0    # < 1: splats become discs along the normals (needs normal_neighbors); 1 = isotropic
 
     def validate(self) -> "DensePipelineConfig":
         if self.matches_per_ref < 0:
@@ -76,6 +80,14 @@ class DensePipelineConfig:
             raise ValueError("outlier_std_ratio must be positive")
         if not (int(self.normal_neighbors) == 0 or 3 <= int(self.normal_neighbors) <= 64):
             raise ValueError("normal_neighbors must be 0 (off) or lie in [3, 64]")
+        if not 0 <= int(self.gaussian_neighbors) <= 63:
+            raise ValueError("gaussian_neighbors must lie in [0, 63] (0 = off)")
+        if not 0.0 < float(self.gaussian_opacity) < 1.0:
+            raise ValueError("gaussian_opacity must lie in (0, 1)")
+        if not 0.0 < float(self.gaussian_flatten) <= 1.0:
+            raise ValueError("gaussian_flatten must lie in (0, 1]")
+        if float(self.gaussian_flatten) < 1.0 and int(self.normal_neighbors) == 0:
+            raise ValueError("gaussian_flatten < 1 needs normal_neighbors")
         if self.rng_mode not in (RNG_PHILOX, RNG_NUMPY_GLOBAL, RNG_EXPLICIT):
             raise ValueError(f"unknown rng_mode {self.rng_mode!r}")
         return self

@@ -41,6 +41,8 @@ class PipelineResult:
     n_views: Optional[np.ndarray] = None          # extra, config.multiview: uint8 cameras per point, the reference view included
     normals: Optional[np.ndarray] = None          # extra, config.normal_neighbors: f32 [n,3] unit normals facing each point's
                                                   # reference camera; (0, 0, 0) where undefined
+    gaussians: Optional[Dict[str, np.ndarray]] = None   # extra, config.gaussian_neighbors: 3DGS's initial splats, f32
+                                                  # sh_dc [n,3], opacity [n], scales [n,3] (log), rotations [n,4] (w, x, y, z)
 
 
 class PipelineCancelled(RuntimeError):
@@ -699,8 +701,9 @@ def run_dense_pipeline(
     ref_uid = np.concatenate(parts_ref, axis=0)
     k_out = int(getattr(config, "outlier_neighbors", 0))
     k_nrm = int(getattr(config, "normal_neighbors", 0))
-    normals = None
-    if k_out > 0 or k_nrm > 0:
+    k_gs = int(getattr(config, "gaussian_neighbors", 0))
+    normals = gaussians = None
+    if k_out > 0 or k_nrm > 0 or k_gs > 0:
         dev = torch.device("cuda", torch.cuda.current_device())
         xyz_dev = torch.from_numpy(np.ascontiguousarray(xyz, dtype=np.float32)).to(dev)
     if k_out > 0:
@@ -725,5 +728,14 @@ def run_dense_pipeline(
         nres = estimate_normals(xyz_dev, nb_neighbors=k_nrm, centers=torch.from_numpy(centers).to(dev),
                                 center_idx=torch.from_numpy(center_idx.astype(np.int32)).to(dev))
         normals = nres.normals.cpu().numpy()
+    if k_gs > 0:
+        # the final cloud, after the outlier filter; discs along the normals above when there are any
+        if progress_callback:
+            progress_callback(98.0, "Initialising Gaussians...")
+        from ..output import init_gaussians
+        rgb_dev = torch.from_numpy(np.ascontiguousarray(rgb, dtype=np.float32)).to(dev)
+        g = init_gaussians(xyz_dev, rgb_dev, normals=nres.normals if k_nrm > 0 else None, nb_neighbors=k_gs,
+                           opacity=float(config.gaussian_opacity), flatten=float(config.gaussian_flatten))
+        gaussians = {name: getattr(g, name).cpu().numpy() for name in ("sh_dc", "opacity", "scales", "rotations")}
     return PipelineResult(xyz=xyz, rgb=rgb, err=err, elapsed_seconds=time.time() - t0, pairs_processed=pairs, n_views=n_views,
-                          normals=normals)
+                          normals=normals, gaussians=gaussians)

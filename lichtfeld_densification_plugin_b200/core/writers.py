@@ -7,6 +7,8 @@ written here as one structured-array ``tofile``:
                            with ``normals`` (not in the reference) ``nx ny nz`` floats between ``z`` and ``red``, 27 bytes
 * ``write_points3D_bin``   ``<Q n`` then per point ``<Q id=i+1``, ``<ddd xyz``, ``<BBB rgb``, ``<d err`` (no track list)
 * ``to_uint8_rgb``         ``clip(round(x * 255), 0, 255)`` with round-half-to-even (core/image_utils.py:24-26)
+* ``write_gaussian_ply``   not in the reference: the 3DGS PLY of initialised splats (graphdeco 3DGS ``save_ply``), the
+                           byte reference for ``output.write_gaussian_ply``
 """
 from __future__ import annotations
 
@@ -65,3 +67,39 @@ def write_points3D_bin(path_out: str, xyz: np.ndarray, rgb_uint8: np.ndarray,
     with open(path_out, "wb") as f:
         f.write(np.uint64(n).tobytes())
         rec.tofile(f)
+
+
+def gaussian_ply_attributes(sh_degree: int) -> list:
+    """Vertex property names of graphdeco 3DGS's ``construct_list_of_attributes`` for SH degree ``sh_degree``, in order."""
+    if not 0 <= int(sh_degree) <= 3:
+        raise ValueError("sh_degree must lie in [0, 3]")
+    n_rest = 3 * ((int(sh_degree) + 1) ** 2 - 1)
+    return (["x", "y", "z", "nx", "ny", "nz"] + [f"f_dc_{i}" for i in range(3)] + [f"f_rest_{i}" for i in range(n_rest)]
+            + ["opacity"] + [f"scale_{i}" for i in range(3)] + [f"rot_{i}" for i in range(4)])
+
+
+def gaussian_ply_header(n: int, sh_degree: int = 3) -> bytes:
+    return (f"ply\nformat binary_little_endian 1.0\nelement vertex {n}\n"
+            + "".join(f"property float {a}\n" for a in gaussian_ply_attributes(sh_degree)) + "end_header\n").encode("ascii")
+
+
+def gaussian_ply_vertices(xyz: np.ndarray, sh_dc: np.ndarray, opacity: np.ndarray, scales: np.ndarray,
+                          rotations: np.ndarray, normals: Optional[np.ndarray] = None, sh_degree: int = 3) -> np.ndarray:
+    """f32 [n, 17 + 3((d+1)^2 - 1)]: one row per vertex in ``gaussian_ply_attributes`` order (f_rest zeros, normals zeros
+    when None)."""
+    n = int(xyz.shape[0])
+    n_rest = 3 * ((int(sh_degree) + 1) ** 2 - 1)
+    f32 = lambda a, c: np.asarray(a, np.float32).reshape(n, c)          # noqa: E731
+    nrm = np.zeros((n, 3), np.float32) if normals is None else f32(normals, 3)
+    return np.concatenate([f32(xyz, 3), nrm, f32(sh_dc, 3), np.zeros((n, n_rest), np.float32), f32(opacity, 1),
+                           f32(scales, 3), f32(rotations, 4)], axis=1)
+
+
+def write_gaussian_ply(path_out: str, xyz: np.ndarray, sh_dc: np.ndarray, opacity: np.ndarray, scales: np.ndarray,
+                       rotations: np.ndarray, normals: Optional[np.ndarray] = None, sh_degree: int = 3) -> None:
+    """The 3DGS PLY (``save_ply``) of initialised splats: sh_dc [n,3], opacity [n] (logit), scales [n,3] (log),
+    rotations [n,4] (w, x, y, z), e.g. from ``output.init_gaussians``; every property ``<f4``."""
+    rec = gaussian_ply_vertices(xyz, sh_dc, opacity, scales, rotations, normals, sh_degree)
+    with open(path_out, "wb") as f:
+        f.write(gaussian_ply_header(int(xyz.shape[0]), sh_degree))
+        rec.astype("<f4").tofile(f)

@@ -934,7 +934,7 @@ static int outlier_insert(const float* xyz, int64_t n, double h, const double* h
     return scan_exclusive(ws.flag, ws.rank, n, ws.block_tot, cells_out, st);
 }
 
-// Steps 1 and 2 of the k-NN search, shared by ldp_statistical_outliers and ldp_estimate_normals: bounds and a trial grid,
+// Steps 1 and 2 of the k-NN search, shared by ldp_statistical_outliers, ldp_estimate_normals and ldp_gaussian_init: bounds and a trial grid,
 // whose cell count sets the level-0 cell size (the one host synchronisation), then the pyramid and its level descriptors
 // in pl.levels.  A coordinate that is not finite sets status_out[0] = 1 and leaves *n_levels_out = 0 (and returns LDP_OK);
 // any CUDA failure returns LDP_ERR_CUDA.
@@ -1052,7 +1052,7 @@ int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, 
     {
         KernelTimer kt(st, "ldp_outlier_knn_kernel");
         const unsigned kgrid = (unsigned)((n + ldp::OL_THREADS - 1) / ldp::OL_THREADS);
-        rc = launch("ldp_outlier_knn_kernel", ldp::ldp_outlier_knn_kernel<false>, dim3(kgrid), dim3(ldp::OL_THREADS),
+        rc = launch("ldp_outlier_knn_kernel", ldp::ldp_outlier_knn_kernel<ldp::KNN_MEAN>, dim3(kgrid), dim3(ldp::OL_THREADS),
                     (size_t)k * ldp::OL_THREADS * sizeof(double), st, (const ldp::OutlierLevel*)pl.levels, n_levels, (long long)n, k,
                     g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, m, (int*)status_out, ldp::NormalArgs{});
         if (rc != LDP_OK) return rc;
@@ -1078,7 +1078,7 @@ int ldp_statistical_outliers(const float* xyz, int64_t n, int32_t nb_neighbors, 
                   (const int*)ws.rank, (long long)n, reinterpret_cast<long long*>(kept_idx_out));
 }
 
-// ---- oriented normals (ldp_outlier.cu: ldp_outlier_knn_kernel<true> and its epilogue)
+// ---- oriented normals (ldp_outlier.cu: ldp_outlier_knn_kernel<KNN_NORMALS> and its epilogue)
 int ldp_normals_workspace_bytes(int64_t n, int32_t k, size_t* bytes_out) {
     if (!bytes_out) return fail(LDP_ERR_INVALID, "null bytes_out");
     if (k < 3 || k > ldp::OL_MAX_K) return fail(LDP_ERR_INVALID, "k must lie in [3, 64]");
@@ -1108,10 +1108,68 @@ int ldp_estimate_normals(const float* xyz, int64_t n, int32_t k, const float* ce
     KernelTimer kt(st, "ldp_normals_knn_kernel");
     const ldp::NormalArgs na{xyz, centers, center_idx, normals_out, curvature_out, knn_idx_out, centers ? n_centers : 0, 0};
     const unsigned kgrid = (unsigned)((n + ldp::OL_THREADS - 1) / ldp::OL_THREADS);
-    return launch("ldp_outlier_knn_kernel", ldp::ldp_outlier_knn_kernel<true>, dim3(kgrid), dim3(ldp::OL_THREADS),
+    return launch("ldp_outlier_knn_kernel", ldp::ldp_outlier_knn_kernel<ldp::KNN_NORMALS>, dim3(kgrid), dim3(ldp::OL_THREADS),
                   (size_t)k_eff * ldp::OL_THREADS * (sizeof(double) + sizeof(int)), st, (const ldp::OutlierLevel*)pl.levels, n_levels,
                   (long long)n, k_eff, g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, (double*)nullptr,
                   (int*)status_out, na);
+}
+
+// ---- 3DGS initialisation (ldp_outlier.cu: ldp_outlier_knn_kernel<KNN_GAUSSIANS> and its epilogue; ldp_output.cu)
+int ldp_gaussian_workspace_bytes(int64_t n, int32_t k, size_t* bytes_out) {
+    if (!bytes_out) return fail(LDP_ERR_INVALID, "null bytes_out");
+    if (k < 1 || k > ldp::OL_MAX_K - 1) return fail(LDP_ERR_INVALID, "k must lie in [1, 63]");
+    OutlierPlan pl;
+    return outlier_plan(n, nullptr, &pl, bytes_out, false);
+}
+
+int ldp_gaussian_init(const float* xyz, const float* rgb, const float* normals, int64_t n, int32_t k, double opacity, double flatten,
+                      float* sh_dc_out, float* opacity_out, float* scales_out, float* rotations_out, float* dist2_out,
+                      int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream) {
+    begin_call();
+    if (k < 1 || k > ldp::OL_MAX_K - 1) return fail(LDP_ERR_INVALID, "k must lie in [1, 63]");
+    if (!(opacity > 0.0 && opacity < 1.0)) return fail(LDP_ERR_INVALID, "opacity must lie in (0, 1)");
+    if (!(flatten > 0.0 && flatten <= 1.0)) return fail(LDP_ERR_INVALID, "flatten must lie in (0, 1]");
+    if (flatten < 1.0 && !normals) return fail(LDP_ERR_INVALID, "flatten < 1 needs normals");
+    if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    int rc = check(cudaMemsetAsync(status_out, 0, 3 * sizeof(int32_t), st), "cudaMemsetAsync(status)");
+    if (rc != LDP_OK || n == 0) return rc;
+    if (!xyz || !rgb || !sh_dc_out || !opacity_out || !scales_out || !rotations_out || !workspace)
+        return fail(LDP_ERR_INVALID, "null pointer");
+    OutlierPlan pl;
+    size_t need = 0;
+    if ((rc = outlier_plan(n, workspace, &pl, &need, false)) != LDP_OK) return rc;
+    if (workspace_bytes < need) return fail(LDP_ERR_WORKSPACE, "gaussian workspace too small");
+    const int kk = (int)std::min<int64_t>((int64_t)k + 1, n);          // k_eff + 1: the point itself and its k_eff nearest
+    int n_levels = 0;
+    if ((rc = knn_pyramid(xyz, n, kk, pl, st, status_out, &n_levels)) != LDP_OK || n_levels == 0) return rc;
+    KernelTimer kt(st, "ldp_gaussian_knn_kernel");
+    const ldp::GaussianArgs ga{rgb, normals, sh_dc_out, opacity_out, scales_out, rotations_out, dist2_out, std::log(flatten),
+                               (float)std::log(opacity / (1.0 - opacity)), 0};
+    const unsigned kgrid = (unsigned)((n + ldp::OL_THREADS - 1) / ldp::OL_THREADS);
+    return launch("ldp_outlier_knn_kernel", ldp::ldp_outlier_knn_kernel<ldp::KNN_GAUSSIANS>, dim3(kgrid), dim3(ldp::OL_THREADS),
+                  (size_t)kk * ldp::OL_THREADS * sizeof(double), st, (const ldp::OutlierLevel*)pl.levels, n_levels, (long long)n, kk,
+                  g_outlier_shells > 0 ? g_outlier_shells : ldp::OL_DEFAULT_SHELLS, (double*)nullptr, (int*)status_out, ga);
+}
+
+int ldp_pack_gaussian_ply_records(const float* xyz, const float* normals, const float* sh_dc, const float* opacity, const float* scales,
+                                  const float* rotations, int64_t n, const int64_t* n_dev, int32_t sh_degree, uint8_t* records_out,
+                                  void* stream) {
+    begin_call();
+    if (n < 0) return fail(LDP_ERR_INVALID, "negative point count");
+    if (sh_degree < 0 || sh_degree > 3) return fail(LDP_ERR_INVALID, "sh_degree must lie in [0, 3]");
+    if (n == 0) return LDP_OK;
+    if (!xyz || !sh_dc || !opacity || !scales || !rotations || !records_out) return fail(LDP_ERR_INVALID, "null pointer");
+    if (reinterpret_cast<uintptr_t>(records_out) & 3u) return fail(LDP_ERR_INVALID, "records_out must be 4-byte aligned");
+    static const decltype(&ldp::ldp_gaussian_records_kernel<0>) k_records[4] = {
+        ldp::ldp_gaussian_records_kernel<0>, ldp::ldp_gaussian_records_kernel<1>, ldp::ldp_gaussian_records_kernel<2>,
+        ldp::ldp_gaussian_records_kernel<3>};
+    const long long floats = (long long)n * (17 + 3 * ((sh_degree + 1) * (sh_degree + 1) - 1));
+    const unsigned grid = (unsigned)((floats + ldp::KO_THREADS - 1) / ldp::KO_THREADS);
+    KernelTimer kt(reinterpret_cast<cudaStream_t>(stream), "ldp_gaussian_records_kernel");
+    return launch("ldp_gaussian_records_kernel", k_records[sh_degree], dim3(grid), dim3(ldp::KO_THREADS), 0,
+                  reinterpret_cast<cudaStream_t>(stream), xyz, normals, sh_dc, opacity, scales, rotations, (long long)n,
+                  reinterpret_cast<const long long*>(n_dev), reinterpret_cast<float*>(records_out));
 }
 
 int ldp_set_sm_reserve(int n_sms) {

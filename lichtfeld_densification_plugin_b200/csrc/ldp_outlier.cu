@@ -9,8 +9,9 @@
 // than a lower bound on the distance to every cell not yet visited; that bound carries a margin far above the rounding of
 // the cell-index computation, so the list holds exactly the k smallest distances.  After R shells without stopping the
 // point starts again one level coarser; the coarsest level has at most 3 cells per axis and is searched to the end.
-// The same search with neighbour identities (NBR = true: (d^2, index) pairs, ties by index) ends in a PCA epilogue that
-// gives oriented normals (ldp_estimate_normals, DESIGN.md §4.6).  Included by ldp_api.cu (unity build).
+// The same search with neighbour identities ((d^2, index) pairs, ties by index) ends in a PCA epilogue that gives oriented
+// normals (ldp_estimate_normals, DESIGN.md §4.6); the values-only search ends in the 3DGS initialisation epilogue
+// (ldp_gaussian_init, DESIGN.md §4.7).  Included by ldp_api.cu (unity build).
 #include "ldp_device.cuh"
 
 namespace ldp {
@@ -104,7 +105,7 @@ __device__ __forceinline__ double outlier_gap(int d, double f) {
     return fmax(g - OL_CELL_EPS, 0.0);
 }
 
-// ---- oriented normals (ldp_estimate_normals; rule in include/ldp_b200.h, DESIGN.md §4.6): the k-NN kernel's NBR = true
+// ---- oriented normals (ldp_estimate_normals; rule in include/ldp_b200.h, DESIGN.md §4.6): the k-NN kernel's KNN_NORMALS
 // instantiation keeps (d^2, index) pairs and ends in this epilogue, in the same thread
 struct NormalArgs {
     const float* xyz;                   // [n,3] the input: the neighbours' coordinates, gathered by index
@@ -264,11 +265,74 @@ __device__ __forceinline__ void normal_epilogue(const NormalArgs& na, int i, con
     if (na.curvature) na.curvature[i] = (float)curv;
 }
 
-template <bool NBR>
+// ---- 3DGS initialisation (ldp_gaussian_init; rule in include/ldp_b200.h, DESIGN.md §4.7): the values-only search over
+// k_eff + 1 entries, the point itself first at d^2 = 0, ends in this epilogue
+struct GaussianArgs {
+    const float* rgb;                   // [n,3]
+    const float* normals;               // [n,3] or NULL (every point undefined: identity rotation, isotropic scales)
+    float* sh_dc;                       // [n,3]
+    float* opacity;                     // [n]
+    float* scales;                      // [n,3]
+    float* rotations;                   // [n,4] (w, x, y, z)
+    float* dist2;                       // [n] or NULL
+    double log_flatten;                 // log(flatten), added to the third scale of a point with a defined normal
+    float opacity_logit;                // f32(log(alpha / (1 - alpha))), the same for every point
+    int pad;
+};
+
+__device__ __forceinline__ void gaussian_epilogue(const GaussianArgs& ga, int i, int kk, const double* L, int* status)
+{
+    const int ke = kk - 1;                               // entry 0 is the point itself (or a duplicate: also 0)
+    double m = 0.0;
+    for (int j = 1; j <= ke; ++j) m = __dadd_rn(m, L[j * OL_THREADS]);
+    if (ke > 0) m = __ddiv_rn(m, (double)ke);
+    const float d2 = fmaxf(__double2float_rn(m), 1e-7f);
+    const double ls = log(__dsqrt_rn((double)d2));
+    const float s = __double2float_rn(ls);
+    float s2 = s, q[4] = {1.0f, 0.0f, 0.0f, 0.0f};
+    bool defined = false;
+    if (ga.normals) {
+        const double nx = ga.normals[3 * (size_t)i], ny = ga.normals[3 * (size_t)i + 1], nz = ga.normals[3 * (size_t)i + 2];
+        const double len = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(nx, nx), __dmul_rn(ny, ny)), __dmul_rn(nz, nz)));
+        if (len > 0.0 && isfinite(len)) {
+            defined = true;
+            const double ux = __ddiv_rn(nx, len), uy = __ddiv_rn(ny, len), uz = __ddiv_rn(nz, len);
+            const double w = __dadd_rn(1.0, uz);
+            if (w > 1e-12) {                              // shortest arc e_z -> u: (1 + u_z, e_z x u) / |.|
+                const double qn = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(w, w), __dmul_rn(uy, uy)), __dmul_rn(ux, ux)));
+                q[0] = __double2float_rn(__ddiv_rn(w, qn));
+                q[1] = __double2float_rn(__ddiv_rn(-uy, qn));
+                q[2] = __double2float_rn(__ddiv_rn(ux, qn));
+                q[3] = 0.0f;
+            } else {                                      // u = -e_z: half a turn about x
+                q[0] = 0.0f; q[1] = 1.0f;
+            }
+            s2 = __double2float_rn(__dadd_rn(ls, ga.log_flatten));
+        }
+    }
+    if (!defined) atomicAdd(&status[1], 1);
+    const size_t i3 = 3 * (size_t)i;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) ga.sh_dc[i3 + c] = __fdiv_rn(__fsub_rn(ga.rgb[i3 + c], 0.5f), 0.28209479177387814f);
+    ga.opacity[i] = ga.opacity_logit;
+    ga.scales[i3] = s; ga.scales[i3 + 1] = s; ga.scales[i3 + 2] = s2;
+#pragma unroll
+    for (int c = 0; c < 4; ++c) ga.rotations[4 * (size_t)i + c] = q[c];
+    if (ga.dist2) ga.dist2[i] = d2;
+}
+
+// The k-NN kernel's epilogues: the outlier filter's mean distance, the normals' PCA (the only one that keeps the neighbours'
+// identities), the 3DGS initialisation
+enum KnnMode { KNN_MEAN = 0, KNN_NORMALS = 1, KNN_GAUSSIANS = 2 };
+template <int MODE> struct KnnEpilogueArgs { using type = NormalArgs; };
+template <> struct KnnEpilogueArgs<KNN_GAUSSIANS> { using type = GaussianArgs; };
+
+template <int MODE>
 __global__ void __launch_bounds__(OL_THREADS)
 ldp_outlier_knn_kernel(const OutlierLevel* __restrict__ levels, int n_levels, long long n, int k, int max_shells,
-                       double* __restrict__ mean_dist, int* __restrict__ status, NormalArgs na)
+                       double* __restrict__ mean_dist, int* __restrict__ status, typename KnnEpilogueArgs<MODE>::type na)
 {
+    constexpr bool NBR = (MODE == KNN_NORMALS);
     extern __shared__ double s_list[];                   // [k][OL_THREADS]: entry j of this thread at s_list[j * OL_THREADS + tid]
     grid_dependency_sync();
     const long long p = (long long)blockIdx.x * OL_THREADS + threadIdx.x;
@@ -369,12 +433,14 @@ ldp_outlier_knn_kernel(const OutlierLevel* __restrict__ levels, int n_levels, lo
         }
         if (!done && l == 0) atomicAdd(&status[2], 1);
     }
-    if constexpr (!NBR) {
+    if constexpr (MODE == KNN_MEAN) {
         double s = 0.0;
         for (int j = 0; j < k; ++j) s = __dadd_rn(s, __dsqrt_rn(L[j * OL_THREADS]));
         mean_dist[__float_as_int(q4.w)] = __ddiv_rn(s, (double)k);
-    } else {
+    } else if constexpr (MODE == KNN_NORMALS) {
         normal_epilogue(na, __float_as_int(q4.w), q, k, I, status);
+    } else {
+        gaussian_epilogue(na, __float_as_int(q4.w), k, L, status);
     }
 }
 

@@ -78,6 +78,34 @@ ldp_records_kernel(const float* __restrict__ xyz, const float* __restrict__ rgb,
     flush_records(rec, out + p0 * REC, cnt * REC, aligned != 0);
 }
 
+// 3DGS PLY vertex (graphdeco 3DGS GaussianModel.save_ply): x y z nx ny nz f_dc_0..2 f_rest_0..(3((D+1)^2-1)-1) opacity
+// scale_0..2 rot_0..3, all <f4, f_rest zeros, the normals zeros without nrm.  Every field is a whole float, so one thread
+// per output float stores coalesced without staging.  out: 4-byte aligned.
+template <int D>
+__global__ void __launch_bounds__(KO_THREADS)
+ldp_gaussian_records_kernel(const float* __restrict__ xyz, const float* __restrict__ nrm, const float* __restrict__ dc,
+                            const float* __restrict__ opacity, const float* __restrict__ scales, const float* __restrict__ rot,
+                            long long n_max, const long long* __restrict__ n_dev, float* __restrict__ out)
+{
+    constexpr int REST = 3 * ((D + 1) * (D + 1) - 1), V = 17 + REST;
+    grid_dependency_sync();
+    long long n = n_max;
+    if (n_dev) { const long long nd = *n_dev; n = nd < n ? nd : n; }
+    const long long e = (long long)blockIdx.x * KO_THREADS + threadIdx.x;
+    if (e >= n * V) return;
+    const long long i = e / V;
+    const int f = (int)(e - i * V);
+    float v = 0.0f;
+    if (f < 3) v = xyz[3 * i + f];
+    else if (f < 6) v = nrm ? nrm[3 * i + f - 3] : 0.0f;
+    else if (f < 9) v = dc[3 * i + f - 6];
+    else if (f < 9 + REST) v = 0.0f;
+    else if (f == 9 + REST) v = opacity[i];
+    else if (f < 13 + REST) v = scales[3 * i + f - 10 - REST];
+    else v = rot[4 * i + f - 13 - REST];
+    out[e] = v;
+}
+
 __global__ void __launch_bounds__(KO_THREADS)
 ldp_rgb_u8_kernel(const float* __restrict__ rgb, long long n_values, uint8_t* __restrict__ out)
 {

@@ -8,6 +8,8 @@ Mirrors, on tensors that stay on the GPU (SURVEY.md 8a row a15, 8f rows 2 and 4)
 * ``voxel_downsample``                 reference densify.py:29-50 (Open3D voxel grid mean; parity unpinned, see the function)
 * ``remove_statistical_outliers``      not in the reference: Open3D's ``remove_statistical_outlier`` (parity unpinned)
 * ``estimate_normals``                 not in the reference: oriented normals by PCA over the exact k nearest neighbours
+* ``init_gaussians`` / ``write_gaussian_ply``   not in the reference: 3DGS's ``create_from_pcd`` initialisation (scales from
+  the exact nearest neighbours, optionally flattened along the normals) and its ``save_ply`` layout
 * ``apply_point_cap``                  reference densify.py:110-120 (the indices are numpy's own
   ``default_rng(seed).choice`` on the host - PCG64 + a sequential shuffle, microseconds; only the gather is device work)
 * ``subsample_preview_matches``        reference core/pipeline.py:573-582 (debug preview subsample of the kept matches)
@@ -27,7 +29,7 @@ import numpy as np
 import torch
 
 from . import _native as N
-from .core.writers import ply_header
+from .core.writers import gaussian_ply_header, ply_header
 
 PLY_RECORD_BYTES = 15
 PLY_NORMAL_RECORD_BYTES = 27
@@ -367,6 +369,97 @@ def estimate_normals(xyz: torch.Tensor, *, nb_neighbors: int, centers: Optional[
     if bad & 2:
         raise ValueError("a centre index is out of range")
     return NormalResult(normals=normals, curvature=curvature, neighbors=nbrs, undefined=undefined)
+
+
+@dataclass
+class GaussianInit:
+    """What ``init_gaussians`` returns: 3DGS's initial parameters (device tensors, rows in input order, all f32)."""
+    sh_dc: torch.Tensor                 # [n, 3] (rgb - 0.5) / C0, 3DGS's RGB2SH
+    opacity: torch.Tensor               # [n] logit of the initial opacity
+    scales: torch.Tensor                # [n, 3] log scales; the third lies along the normal
+    rotations: torch.Tensor             # [n, 4] unit quaternions (w, x, y, z)
+    dist2: torch.Tensor                 # [n] mean squared distance to the k nearest other points, clamped to 1e-7
+    undefined: int                      # points without a usable normal: identity rotation, isotropic scales
+
+
+def init_gaussians(xyz: torch.Tensor, rgb: torch.Tensor, *, normals: Optional[torch.Tensor] = None, nb_neighbors: int = 3,
+                   opacity: float = 0.1, flatten: float = 1.0) -> GaussianInit:
+    """graphdeco 3DGS's ``create_from_pcd`` on a device cloud: scale from the mean squared distance to the ``nb_neighbors``
+    nearest other points (exact; 3DGS uses simple-knn's ``distCUDA2`` with 3), SH DC from ``rgb`` in [0, 1], opacity
+    ``inverse_sigmoid(opacity)``.  With ``normals`` (e.g. ``estimate_normals``) each splat is rotated so that its third axis
+    lies along its normal, and ``flatten`` < 1 shrinks that axis by that factor: discs in the surface.  The rule is in
+    include/ldp_b200.h.  Synchronises twice: once inside the call (the grid's cell size) and once to read the status."""
+    if not 1 <= int(nb_neighbors) <= 63:
+        raise ValueError("nb_neighbors must lie in [1, 63]")
+    if not 0.0 < float(opacity) < 1.0:
+        raise ValueError("opacity must lie in (0, 1)")
+    if not 0.0 < float(flatten) <= 1.0:
+        raise ValueError("flatten must lie in (0, 1]")
+    if float(flatten) < 1.0 and normals is None:
+        raise ValueError("flatten < 1 needs normals")
+    xyz, rgb = _f32c(xyz, "xyz"), _f32c(rgb, "rgb")
+    if tuple(rgb.shape) != tuple(xyz.shape):
+        raise ValueError("rgb must have the shape of xyz")
+    if normals is not None:
+        normals = _f32c(normals, "normals")
+        if tuple(normals.shape) != tuple(xyz.shape):
+            raise ValueError("normals must have the shape of xyz")
+    lib, stream = _lib_and_stream(xyz)
+    dev, n = xyz.device, int(xyz.shape[0])
+    need = C.c_size_t(0)
+    N.check(lib.ldp_gaussian_workspace_bytes(n, int(nb_neighbors), C.byref(need)), "ldp_gaussian_workspace_bytes")
+    ws = torch.empty((max(1, need.value),), dtype=torch.uint8, device=dev)
+    f32 = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)      # noqa: E731
+    g = GaussianInit(sh_dc=f32(n, 3), opacity=f32(n), scales=f32(n, 3), rotations=f32(n, 4), dist2=f32(n), undefined=0)
+    status = torch.zeros((3,), dtype=torch.int32, device=dev)
+    ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)          # noqa: E731
+    N.check(lib.ldp_gaussian_init(ptr(xyz), ptr(rgb), ptr(normals), n, int(nb_neighbors), float(opacity), float(flatten),
+                                  ptr(g.sh_dc), ptr(g.opacity), ptr(g.scales), ptr(g.rotations), ptr(g.dist2), ptr(status),
+                                  ptr(ws), C.c_size_t(need.value), C.c_void_p(stream)), "ldp_gaussian_init")
+    bad, undefined, _ = (int(v) for v in status.cpu().tolist())
+    if bad & 1:
+        raise ValueError("a coordinate is not finite")
+    g.undefined = undefined
+    return g
+
+
+def gaussian_record_bytes(sh_degree: int) -> int:
+    """68, 104, 164 or 248 bytes per vertex of the 3DGS PLY for SH degree 0..3."""
+    return 4 * (17 + 3 * ((int(sh_degree) + 1) ** 2 - 1))
+
+
+def gaussian_ply_records(xyz: torch.Tensor, g: GaussianInit, normals: Optional[torch.Tensor] = None, sh_degree: int = 3,
+                         n: Optional[int] = None, n_dev: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """uint8 [n * gaussian_record_bytes(sh_degree)] device tensor of 3DGS PLY vertices (``core.writers.gaussian_ply_vertices``
+    order: x y z nx ny nz f_dc f_rest opacity scale rot, all ``<f4``; f_rest zeros, normals zeros when None).  ``n`` and
+    ``n_dev`` as for ``ply_records``."""
+    if not 0 <= int(sh_degree) <= 3:
+        raise ValueError("sh_degree must lie in [0, 3]")
+    xyz = _f32c(xyz, "xyz")
+    arrs = [_f32c(t, name) for t, name in ((g.sh_dc, "sh_dc"), (g.opacity, "opacity"), (g.scales, "scales"),
+                                           (g.rotations, "rotations"))]
+    if normals is not None:
+        normals = _f32c(normals, "normals")
+        if tuple(normals.shape) != tuple(xyz.shape):
+            raise ValueError("normals must have the shape of xyz")
+    lib, stream = _lib_and_stream(xyz)
+    n = int(xyz.shape[0]) if n is None else int(n)
+    out = torch.empty((n * gaussian_record_bytes(sh_degree),), dtype=torch.uint8, device=xyz.device)
+    ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)          # noqa: E731
+    N.check(lib.ldp_pack_gaussian_ply_records(ptr(xyz), ptr(normals), *(ptr(t) for t in arrs), n, ptr(n_dev), int(sh_degree),
+                                              ptr(out), C.c_void_p(stream)), "ldp_pack_gaussian_ply_records")
+    return out
+
+
+def write_gaussian_ply(path_out: str, xyz: torch.Tensor, g: GaussianInit, normals: Optional[torch.Tensor] = None,
+                       sh_degree: int = 3) -> None:
+    """The 3DGS PLY of ``init_gaussians``' splats, loadable by 3DGS-style trainers and viewers: the bytes of
+    ``core.writers.write_gaussian_ply`` on the same arrays."""
+    n = int(xyz.shape[0])
+    rec = gaussian_ply_records(xyz, g, normals, sh_degree).cpu().numpy() if n else np.zeros((0,), np.uint8)
+    with open(path_out, "wb") as f:
+        f.write(gaussian_ply_header(n, sh_degree))
+        rec.tofile(f)
 
 
 PREVIEW_MAX_MATCHES = 10000       # reference core/pipeline.py:50 _PREVIEW_MAX_MATCHES
