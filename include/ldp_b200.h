@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define LDP_ABI_VERSION 18
+#define LDP_ABI_VERSION 19
 #define LDP_MAX_NN 16          /* neighbours per reference view (the panel clamps to 10) */
 #define LDP_MAX_BINS 4096      /* coverage tiles per map: ceil(W/tile)*ceil(H/tile), tile = max(1, W/24) */
 
@@ -240,6 +240,37 @@ int ldp_undistort_points(const ldp_lens* lens, int64_t n, const float* uv_in, fl
 int ldp_postprocess_certainty(const ldp_params* params, const ldp_ref_desc* refs, float* out,
                               size_t ref_stride, size_t plane_stride, void* stream);
 
+/* ---- dense depth maps of the reference views (not in the reference) -----------------------------------------------------
+ * The reference triangulates the M sampled pixels of a view and drops the rest of the matcher's output.  ldp_depth_maps
+ * evaluates EVERY confident pixel of the map the same way.  For reference view r and map pixel i (indexed like the
+ * certainty planes):
+ *   1. c, k = the best certainty over the view's neighbours at i and its slot, first index on ties (NaN wins): the arg-max of
+ *      core/pipeline.py:634-635 and of ldp_densify_refs.  With params->prologue the floor and the masks apply, as for the
+ *      sampler.  A view with nn = 0 has no candidate.
+ *   2. i is a CANDIDATE iff c >= f32(min_certainty), min_certainty in (0, 1].  With raw planes every pixel has c >=
+ *      certainty_floor, so min_certainty is what selects pixels.  The sampler's cap and border do not apply.
+ *   3. A candidate is evaluated exactly as a sampled pixel with winner k: decode of the warp row, lens undistortion, the
+ *      Sampson gate, the DLT (Jacobi in the fix-up when inverse iteration does not converge), reprojection, cheirality and
+ *      parallax or no_filter's finiteness test, and with params->multiview the multi-view refinement (same device code).
+ *   4. Outputs, DEVICE arrays of n_refs * H * W entries (xyz: * 3), NaN where not written as stated:
+ *        depth  the reference camera's z of the final point, row 3 of P1 applied to (X, Y, Z, W) as the reprojection test
+ *               forms it (core/geometry.py:91-110), where the pixel is kept; NaN elsewhere.  Required.
+ *        err    the point's reprojection error wherever it was triangulated (candidate through the Sampson gate; with
+ *               multiview, a refined point's error), NaN elsewhere.  Optional.
+ *        xyz    the world point where kept, NaN elsewhere.  Optional.
+ *        flags  u8: bit 0 candidate, bit 1 Sampson pass, bit 2 kept, bits 4-7 the winning slot k.  Optional.
+ *        kept   int64 [n_refs]: kept pixels per view.  Required.
+ * Consequence: at every pixel ldp_densify_refs samples (and that is a candidate), the verdict, depth, err and xyz are
+ * bit-identical to that launch's own values (sample_flags, sample_xyzerr, and xyz / err of the packed cloud with multiview).
+ * Every params field that ldp_densify_refs reads for the geometry is read here; matches_per_ref, border, tiles,
+ * sample_cap, collect_debug and the RNG fields are not.  Images are not read.
+ * Workspace: ldp_depth_workspace_bytes (4 bytes per pixel of the launch: the fix-up's worklist cannot overflow).  Its first
+ * n_refs int32 from its first 256-byte boundary count each view's fix-up entries of the last call.  ldp_debug_force_fixup
+ * applies here in every launch (multiview or not), by pixel index i instead of sample position.  Enqueues on `stream`. */
+int ldp_depth_workspace_bytes(const ldp_params* params, size_t* bytes_out);
+int ldp_depth_maps(const ldp_params* params, const ldp_ref_desc* refs, double min_certainty, float* depth, float* err, float* xyz,
+                   uint8_t* flags, int64_t* kept, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- output contract on the device (SURVEY 8a row a15, 8f row 2) ---------------------------------
  * The reference converts colours with to_uint8_rgb (core/image_utils.py:24-26: clip(round(rgb * 255), 0, 255), half to
  * even) and writes one struct.pack per point (core/writers.py:15-46).  These build the same bytes where the points are:
@@ -444,8 +475,8 @@ int ldp_debug_read_clocks(const ldp_params* params, void* workspace, long long* 
  * thread (0, 0 restores the default), every sample i (position in its view's sample list) with i % two_view_every == 0 is sent
  * to the fix-up as if its two-view null-vector iteration had not converged, and every kept sample with i % multiview_every == 0
  * as if its multi-view solve had not converged (0 = never); the fix-up solves them with Jacobi.  The plain path's kernels do not
- * read it.  ldp_debug_read_fixups: after a launch (synchronises), host_out[0] = entries of the worklist, host_out[1] = those
- * that redo only a multi-view solve; params and workspace as given to that launch. */
+ * read it; the depth-map kernels do (see ldp_depth_maps).  ldp_debug_read_fixups: after a launch (synchronises), host_out[0] =
+ * entries of the worklist, host_out[1] = those that redo only a multi-view solve; params and workspace as given to that launch. */
 int ldp_debug_force_fixup(int two_view_every, int multiview_every);
 int ldp_debug_read_fixups(const ldp_params* params, void* workspace, int32_t* host_out);
 

@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-LDP_ABI_VERSION = 18
+LDP_ABI_VERSION = 19
 LDP_MAX_NN = 16
 LDP_MAX_BINS = 4096
 
@@ -121,6 +121,8 @@ SIGNATURES = {
     "ldp_triangulate_samples": (C.c_int, [_PARAMS, _P, _OUTPUTS, _P, _SZ, _P]),
     "ldp_undistort_points": (C.c_int, [C.POINTER(LdpLens), _I64, _P, _P, _P]),
     "ldp_postprocess_certainty": (C.c_int, [_PARAMS, _P, _P, _SZ, _SZ, _P]),
+    "ldp_depth_workspace_bytes": (C.c_int, [_PARAMS, _SZ_OUT]),
+    "ldp_depth_maps": (C.c_int, [_PARAMS, _P, C.c_double, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "ldp_pack_ply_records": (C.c_int, [_P, _P, _I64, _P, _P, _P]),
     "ldp_pack_ply_normal_records": (C.c_int, [_P, _P, _P, _I64, _P, _P, _P]),
     "ldp_pack_points3d_records": (C.c_int, [_P, _P, _P, _I64, _P, C.c_uint64, _P, _P]),

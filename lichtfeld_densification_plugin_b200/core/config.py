@@ -66,6 +66,10 @@ class DensePipelineConfig:
                                      # this many nearest other points (3DGS: 3); 0 = off
     gaussian_opacity: float = 0.1    # initial opacity of every splat (3DGS: 0.1)
     gaussian_flatten: float = 1.0    # < 1: splats become discs along the normals (needs normal_neighbors); 1 = isotropic
+    depth_dir: str = ""              # non-empty: one float32 depth map <depth_dir>/<image stem>.npy per reference view (every
+                                     # pixel whose best certainty is >= depth_min_certainty, triangulated and filtered like a
+                                     # sample) plus depth_maps.json; "" = off
+    depth_min_certainty: float = 0.5 # depth maps: certainty a pixel's best match needs to be evaluated, in (0, 1]
 
     def validate(self) -> "DensePipelineConfig":
         if self.matches_per_ref < 0:
@@ -88,6 +92,10 @@ class DensePipelineConfig:
             raise ValueError("gaussian_flatten must lie in (0, 1]")
         if float(self.gaussian_flatten) < 1.0 and int(self.normal_neighbors) == 0:
             raise ValueError("gaussian_flatten < 1 needs normal_neighbors")
+        if not isinstance(self.depth_dir, str):
+            raise ValueError("depth_dir must be a string (\"\" = off)")
+        if not 0.0 < float(self.depth_min_certainty) <= 1.0:
+            raise ValueError("depth_min_certainty must lie in (0, 1]")
         if self.rng_mode not in (RNG_PHILOX, RNG_NUMPY_GLOBAL, RNG_EXPLICIT):
             raise ValueError(f"unknown rng_mode {self.rng_mode!r}")
         return self

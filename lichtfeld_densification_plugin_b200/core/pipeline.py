@@ -17,6 +17,7 @@ raise (no CPU fallback).
 """
 from __future__ import annotations
 
+import json
 import os
 import time
 from dataclasses import dataclass, field
@@ -26,7 +27,7 @@ import numpy as np
 import torch
 
 from .. import _native as N
-from ..engine import DensifyEngine, DensifyOutputs, PathConfig, RefBatch
+from ..engine import DensifyEngine, DensifyOutputs, DepthMaps, PathConfig, RefBatch
 from .camera_models import CameraRecord
 from .config import RNG_EXPLICIT, RNG_NUMPY_GLOBAL, RNG_PHILOX, DensePipelineConfig
 
@@ -43,6 +44,7 @@ class PipelineResult:
                                                   # reference camera; (0, 0, 0) where undefined
     gaussians: Optional[Dict[str, np.ndarray]] = None   # extra, config.gaussian_neighbors: 3DGS's initial splats, f32
                                                   # sh_dc [n,3], opacity [n], scales [n,3] (log), rotations [n,4] (w, x, y, z)
+    depth_paths: Optional[Dict[int, str]] = None  # extra, config.depth_dir: reference camera uid -> its depth map file
 
 
 class PipelineCancelled(RuntimeError):
@@ -304,6 +306,7 @@ class _PendingLaunch:
     n: int
     collect_debug: bool
     ply_records: bool
+    depth: Optional[DepthMaps] = None            # config.depth_dir: the launch's depth maps, written when it is collected
 
 
 def submit_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _TriangulationContext,
@@ -344,15 +347,48 @@ def submit_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triangulati
     if uniforms is not None:
         u_dev = torch.from_numpy(np.ascontiguousarray(uniforms, dtype=np.float64)).to(dev)
         batch._keep_alive.append(u_dev)      # read by kernels on a ring stream: alive until the launch is collected, like the planes
+    depth = None
     if ring is None:
         out = eng.densify(batch, pcfg, uniforms=u_dev, collect_debug=collect_debug_matches)
+        if getattr(cfg, "depth_dir", ""):
+            depth = eng.depth_maps(batch, pcfg, float(cfg.depth_min_certainty))
     else:
         out = ring.submit(batch, pcfg, uniforms=u_dev, collect_debug=collect_debug_matches)
-    return _PendingLaunch(out=out, batch=batch, n=n, collect_debug=collect_debug_matches, ply_records=ply_records)
+        if getattr(cfg, "depth_dir", ""):
+            depth = ring.submit_depth_maps(batch, pcfg, float(cfg.depth_min_certainty))
+    return _PendingLaunch(out=out, batch=batch, n=n, collect_debug=collect_debug_matches, ply_records=ply_records, depth=depth)
 
 
-def collect_refs(pending: _PendingLaunch, errors: Optional[list] = None, ring=None) -> List[Optional[_TriangulatedReference]]:
-    """Second half: one synchronising read of the launch's results, split per view."""
+def depth_map_name(cameras, uid: int) -> str:
+    """File name of reference view ``uid``'s depth map: the stem of its image path (its uid when it has none) + ``.npy``."""
+    path = cameras.path_by.get(int(uid), "") if hasattr(cameras, "path_by") else ""
+    stem = os.path.splitext(os.path.basename(path))[0] if path else ""
+    return (stem or str(int(uid))) + ".npy"
+
+
+def _write_depth_maps(pending: _PendingLaunch, tri_ctx: _TriangulationContext, ok: List[bool], ring,
+                      depth_paths: Optional[Dict[int, str]]) -> None:
+    """The launch's depth maps, one file per view whose sampling succeeded (the views the cloud has too)."""
+    from ..output import write_depth_map
+    if ring is not None:
+        ring.wait(pending.depth)
+    maps = pending.depth.depth.cpu().numpy()              # only these maps travel to the host, one launch at a time
+    out_dir = tri_ctx.config.depth_dir
+    os.makedirs(out_dir, exist_ok=True)
+    for r in range(pending.n):
+        if not ok[r]:
+            continue
+        uid = int(pending.batch.ref_uids[r])
+        path = os.path.join(out_dir, depth_map_name(tri_ctx.cameras, uid))
+        write_depth_map(path, maps[r])
+        if depth_paths is not None:
+            depth_paths[uid] = path
+
+
+def collect_refs(pending: _PendingLaunch, errors: Optional[list] = None, ring=None, tri_ctx: Optional[_TriangulationContext] = None,
+                 depth_paths: Optional[Dict[int, str]] = None) -> List[Optional[_TriangulatedReference]]:
+    """Second half: one synchronising read of the launch's results, split per view.  A launch with depth maps writes them
+    under ``tri_ctx.config.depth_dir`` and records each file in ``depth_paths`` (reference camera uid -> path)."""
     out, batch = pending.out, pending.batch
     if ring is not None:
         ring.wait(out)                                 # the current stream (which does the read-back) follows the ring stream
@@ -360,14 +396,21 @@ def collect_refs(pending: _PendingLaunch, errors: Optional[list] = None, ring=No
     triangulate_refs.last_uniforms_used = host["uniforms_used"].copy()
     # the per-view results are slices of the launch's own host block (see _download): nothing is copied again
     results: List[Optional[_TriangulatedReference]] = []
+    ok: List[bool] = []
     for r in range(pending.n):
         try:
             _raise_for_status(int(host["status"][r]))
+            ok.append(True)
             results.append(_split_reference(out, host, r, batch.nbr_uids[r], pending.collect_debug))
         except Exception as exc:      # the reference's caller logs and skips (core/pipeline.py:874-879)
             if errors is not None:
                 errors.append((r, exc))
+            ok.append(False)
             results.append(None)
+    if pending.depth is not None:
+        if tri_ctx is None:
+            raise ValueError("a launch with depth maps is collected with its tri_ctx")
+        _write_depth_maps(pending, tri_ctx, ok, ring, depth_paths)
     triangulate_refs.last_launches = out.launches
     return results
 
@@ -376,23 +419,26 @@ def triangulate_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triang
                      collect_debug_matches: bool = False, *, rng_streams: Optional[Sequence[int]] = None,
                      uniforms: Optional[np.ndarray] = None,
                      weight_sums: Optional[Sequence[float]] = None,
-                     errors: Optional[list] = None, ply_records: bool = False) -> List[Optional[_TriangulatedReference]]:
+                     errors: Optional[list] = None, ply_records: bool = False,
+                     depth_paths: Optional[Dict[int, str]] = None) -> List[Optional[_TriangulatedReference]]:
     """Batched ``_triangulate_ref``: every view of ``matched_refs`` in one launch sequence.
 
     RNG: ``uniforms`` (f64 [n, U], explicit parity stream per view) or Philox keyed by
     (config.seed, rng_streams[i]).  Views the reference would skip (None return / exception) come back as
     None; the exception a per-view call would raise is appended to ``errors`` as (index, exc).
     ``ply_records``: also return every view's PLY vertex records (built on the device, 15 bytes per point).
+    ``config.depth_dir``: also write every view's depth map there (``depth_paths``: see ``collect_refs``).
     """
     if len(matched_refs) == 0:
         return []
     pending = submit_refs(matched_refs, tri_ctx, collect_debug_matches, rng_streams=rng_streams, uniforms=uniforms,
                           weight_sums=weight_sums, ply_records=ply_records)
-    return collect_refs(pending, errors)
+    return collect_refs(pending, errors, tri_ctx=tri_ctx, depth_paths=depth_paths)
 
 
 def _triangulate_ref(matched_ref: _MatchedReference, tri_ctx: _TriangulationContext,
-                     collect_debug_matches: bool = False) -> Optional[_TriangulatedReference]:
+                     collect_debug_matches: bool = False, *,
+                     depth_paths: Optional[Dict[int, str]] = None) -> Optional[_TriangulatedReference]:
     """Triangulate matches for a single reference view (reference core/pipeline.py:602-780).
 
     ``config.rng_mode``: "numpy" consumes the process-global MT19937 stream like the reference's ``np.random.choice``:
@@ -414,7 +460,8 @@ def _triangulate_ref(matched_ref: _MatchedReference, tri_ctx: _TriangulationCont
         n_uni = 2 * size + 64
         while True:
             U = _mt_stream_from_global(n_uni)
-            res = triangulate_refs([matched_ref], tri_ctx, collect_debug_matches, uniforms=U[None, :], errors=errs)
+            res = triangulate_refs([matched_ref], tri_ctx, collect_debug_matches, uniforms=U[None, :], errors=errs,
+                                   depth_paths=depth_paths)
             if errs and "exhausted" in str(errs[0][1]):
                 errs.clear()
                 n_uni *= 2
@@ -425,7 +472,7 @@ def _triangulate_ref(matched_ref: _MatchedReference, tri_ctx: _TriangulationCont
             np.random.random_sample(used)          # advance the global stream like np.random.choice did
     else:
         res = triangulate_refs([matched_ref], tri_ctx, collect_debug_matches,
-                               rng_streams=[int(matched_ref.packed.ref_id)], errors=errs)
+                               rng_streams=[int(matched_ref.packed.ref_id)], errors=errs, depth_paths=depth_paths)
     if errs:
         raise errs[0][1]
     return res[0]
@@ -620,6 +667,7 @@ def run_dense_pipeline(
     n_chunks = (total + step - 1) // step
     ring = get_ring() if (n_chunks > 1 and getattr(config, "rng_mode", RNG_PHILOX) != RNG_NUMPY_GLOBAL) else None
     in_flight: List[tuple] = []      # (views done when this launch is collected, launch, its matched references)
+    depth_paths: Optional[Dict[int, str]] = {} if getattr(config, "depth_dir", "") else None
 
     def consume(outs, done: int, matched_refs) -> None:
         nonlocal pairs, ply_points, pair_counter
@@ -669,24 +717,24 @@ def run_dense_pipeline(
                 outs = []
                 for m in mrs:
                     try:
-                        outs.append(_triangulate_ref(m, tri_ctx, collect_debug))
+                        outs.append(_triangulate_ref(m, tri_ctx, collect_debug, depth_paths=depth_paths))
                     except Exception:
                         outs.append(None)
                 consume(outs, done, mrs)
             elif ring is None:
                 consume(triangulate_refs(mrs, tri_ctx, collect_debug, rng_streams=[int(r) for r, _ in matched],
-                                         ply_records=ply_base is not None), done, mrs)
+                                         ply_records=ply_base is not None, depth_paths=depth_paths), done, mrs)
             else:
                 # several launches in flight: the next chunk is uploaded and enqueued before the oldest one is read back
                 in_flight.append((done, submit_refs(mrs, tri_ctx, collect_debug, rng_streams=[int(r) for r, _ in matched],
                                                     ply_records=ply_base is not None, ring=ring), mrs))
                 if len(in_flight) >= ring.depth:
                     d, pend, pm = in_flight.pop(0)
-                    consume(collect_refs(pend, ring=ring), d, pm)
+                    consume(collect_refs(pend, ring=ring, tri_ctx=tri_ctx, depth_paths=depth_paths), d, pm)
         for d, pend, pm in in_flight:
             if _is_cancelled(cancel_requested):
                 raise PipelineCancelled("Cancelled")
-            consume(collect_refs(pend, ring=ring), d, pm)
+            consume(collect_refs(pend, ring=ring, tri_ctx=tri_ctx, depth_paths=depth_paths), d, pm)
     finally:
         if debug_state is not None and hasattr(debug_state, "release_waiters"):
             debug_state.release_waiters()                              # core/pipeline.py:547-548
@@ -694,6 +742,8 @@ def run_dense_pipeline(
         raise PipelineCancelled("Cancelled")
     if progress_callback:
         progress_callback(90.0, "Finalizing triangulation...")
+    if depth_paths is not None:
+        _write_depth_index(config, tri_ctx, depth_paths)
     if not parts_xyz:
         raise RuntimeError("No points triangulated. Try adjusting parameters.")
     xyz, rgb, err = np.concatenate(parts_xyz, axis=0), np.concatenate(parts_rgb, axis=0), np.concatenate(parts_err, axis=0)
@@ -738,4 +788,18 @@ def run_dense_pipeline(
                            opacity=float(config.gaussian_opacity), flatten=float(config.gaussian_flatten))
         gaussians = {name: getattr(g, name).cpu().numpy() for name in ("sh_dc", "opacity", "scales", "rotations")}
     return PipelineResult(xyz=xyz, rgb=rgb, err=err, elapsed_seconds=time.time() - t0, pairs_processed=pairs, n_views=n_views,
-                          normals=normals, gaussians=gaussians)
+                          normals=normals, gaussians=gaussians, depth_paths=depth_paths)
+
+
+def _write_depth_index(config: DensePipelineConfig, tri_ctx: _TriangulationContext, depth_paths: Dict[int, str]) -> None:
+    """``<depth_dir>/depth_maps.json``: what a reader needs to place each map (see output.write_depth_map)."""
+    os.makedirs(config.depth_dir, exist_ok=True)
+    maps = []
+    for uid, path in depth_paths.items():
+        H, W = np.load(path, mmap_mode="r").shape
+        width, height = tri_ctx.cameras.size_by[uid]
+        maps.append(dict(file=os.path.basename(path), camera_uid=int(uid), H=int(H), W=int(W), w_match=int(tri_ctx.w_match),
+                         h_match=int(tri_ctx.h_match), width=int(width), height=int(height)))
+    index = dict(min_certainty=float(config.depth_min_certainty), nan="no depth", maps=maps)
+    with open(os.path.join(config.depth_dir, "depth_maps.json"), "w") as f:
+        json.dump(index, f, indent=1)

@@ -506,13 +506,13 @@ float parallax_cos_threshold(float min_deg) {
     return unord(lo);
 }
 
-ldp::GeomArgs make_geom_args(const ldp_params* p, const Plan& plan, int have_bestk) {
+ldp::GeomArgs make_geom_args(const ldp_params* p, int nb2, int have_bestk) {
     thread_local float cached_deg = -1.f, cached_cos = 1.f;
     if (p->min_parallax_deg != cached_deg) { cached_cos = parallax_cos_threshold(p->min_parallax_deg); cached_deg = p->min_parallax_deg; }
     ldp::GeomArgs ga;
     ga.par_cos_max = cached_cos;
     ga.have_bestk = have_bestk;
-    ga.nb2 = plan.nb2;
+    ga.nb2 = nb2;
     ga.force_fix_two = g_force_fix_two;
     ga.force_fix_mv = g_force_fix_mv;
     return ga;
@@ -521,7 +521,7 @@ ldp::GeomArgs make_geom_args(const ldp_params* p, const Plan& plan, int have_bes
 // gather + compute -> fix + plan, then the ordered scatter of all views of the launch (needs every view's kept count)
 int launch_triangulate(const ldp_params* p, const ldp_ref_desc* refs, const ldp_outputs* out, const Plan& plan,
                        int have_bestk, cudaStream_t st) {
-    ldp::GeomArgs ga = make_geom_args(p, plan, have_bestk);
+    ldp::GeomArgs ga = make_geom_args(p, plan.nb2, have_bestk);
     const dim3 grid((unsigned)plan.nb2, (unsigned)p->n_refs);
     int rc;
     // The order in which these instantiations are first named here steers the device compiler's inlining: as a [lens][mv]
@@ -537,6 +537,26 @@ int launch_triangulate(const ldp_params* p, const ldp_ref_desc* refs, const ldp_
     ga.have_bestk = 1;
     KernelTimer kt(st, "ldp_pack_kernel");
     return launch("ldp_pack_kernel", ldp::ldp_pack_kernel, grid, dim3(ldp::K3_THREADS), 0, st, *p, refs, plan.ws, *out, ga);
+}
+
+// ---- depth maps: the worklist of the fix-up (one slot per pixel of every view) and its counters
+struct DepthPlan {
+    int32_t* fix_count;
+    uint32_t* fix_list;
+    size_t bytes;
+};
+
+int make_depth_plan(const ldp_params* p, void* base, DepthPlan* dp) {
+    if (!p || p->n_refs < 0 || p->n_refs > 65535 || p->H <= 0 || p->W <= 0 || p->w_match <= 0 || p->h_match <= 0)
+        return fail(LDP_ERR_INVALID, "bad ldp_params");
+    const long long N = (long long)p->H * (long long)p->W;
+    if (N > 0x3fffffffLL) return fail(LDP_ERR_INVALID, "map too large");
+    const size_t R = (size_t)p->n_refs;
+    Carver c{static_cast<char*>(base)};
+    dp->fix_count = c.take<int32_t>(R);
+    dp->fix_list = c.take<uint32_t>(R * (size_t)N);
+    dp->bytes = align_up(c.off, 256);
+    return LDP_OK;
 }
 
 }  // namespace
@@ -1243,6 +1263,54 @@ int ldp_triangulate_samples(const ldp_params* params, const ldp_ref_desc* refs, 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if ((rc = clear_launch_state(plan, st)) != LDP_OK) return rc;
     return launch_triangulate(params, refs, out, plan, 0, st);
+}
+
+int ldp_depth_workspace_bytes(const ldp_params* params, size_t* bytes_out) {
+    if (!bytes_out) return fail(LDP_ERR_INVALID, "null bytes_out");
+    DepthPlan dp;
+    const int rc = make_depth_plan(params, nullptr, &dp);
+    if (rc != LDP_OK) return rc;
+    *bytes_out = dp.bytes + 256;
+    return LDP_OK;
+}
+
+int ldp_depth_maps(const ldp_params* params, const ldp_ref_desc* refs, double min_certainty, float* depth, float* err, float* xyz,
+                   uint8_t* flags, int64_t* kept, void* workspace, size_t workspace_bytes, void* stream) {
+    begin_call();
+    if (!params) return fail(LDP_ERR_INVALID, "null params");
+    if (!(min_certainty > 0.0 && min_certainty <= 1.0)) return fail(LDP_ERR_INVALID, "min_certainty must lie in (0, 1]");
+    if (params->multiview && params->no_filter) return fail(LDP_ERR_INVALID, "multiview needs the filters (no_filter = 0)");
+    if (params->multiview && !(params->multiview_min_cert > 0.0f && params->multiview_min_cert <= 1.0f))
+        return fail(LDP_ERR_INVALID, "multiview_min_cert must lie in (0, 1]");
+    DepthPlan dp;
+    int rc = make_depth_plan(params, nullptr, &dp);
+    if (rc != LDP_OK) return rc;
+    if (params->n_refs == 0) return LDP_OK;
+    if (!refs || !depth || !kept || !workspace) return fail(LDP_ERR_INVALID, "null refs / depth / kept / workspace");
+    char* base = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace), 256));
+    if ((rc = make_depth_plan(params, base, &dp)) != LDP_OK) return rc;
+    if (dp.bytes + (size_t)(base - static_cast<char*>(workspace)) > workspace_bytes) return fail(LDP_ERR_WORKSPACE, "workspace too small");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int R = params->n_refs, N = params->H * params->W;
+    if ((rc = check(cudaMemsetAsync(kept, 0, (size_t)R * sizeof(int64_t), st), "cudaMemsetAsync(kept)")) != LDP_OK) return rc;
+    if ((rc = check(cudaMemsetAsync(dp.fix_count, 0, (size_t)R * sizeof(int32_t), st), "cudaMemsetAsync(fix_count)")) != LDP_OK)
+        return rc;
+    const ldp::GeomArgs ga = make_geom_args(params, 0, 0);
+    const ldp::DepthArgs d{depth, err, xyz, flags, reinterpret_cast<unsigned long long*>(kept), dp.fix_list, dp.fix_count,
+                           (float)min_certainty, N};
+    // enough CTAs per view for about 16 resident per SM over the launch; each strides over its share of the view's map
+    const int tiles = (N + ldp::K2_THREADS - 1) / ldp::K2_THREADS;
+    const int per_view = std::max(1, std::min(tiles, (sm_count() * 16 + R - 1) / R));
+    { KernelTimer kt(st, "ldp_depth_kernel");
+      auto* kd = params->multiview ? (params->lens ? ldp::ldp_depth_kernel<true, true> : ldp::ldp_depth_kernel<false, true>)
+                                   : (params->lens ? ldp::ldp_depth_kernel<true, false> : ldp::ldp_depth_kernel<false, false>);
+      if ((rc = launch("ldp_depth_kernel", kd, dim3((unsigned)per_view, (unsigned)R), dim3(ldp::K2_THREADS), 0, st, *params, refs, ga, d))
+          != LDP_OK)
+          return rc; }
+    KernelTimer kt(st, "ldp_depth_fix_kernel");
+    auto* kf = params->multiview ? (params->lens ? ldp::ldp_depth_fix_kernel<true, true> : ldp::ldp_depth_fix_kernel<false, true>)
+                                 : (params->lens ? ldp::ldp_depth_fix_kernel<true, false> : ldp::ldp_depth_fix_kernel<false, false>);
+    return launch("ldp_depth_fix_kernel", kf, dim3(ldp::KDF_BLOCKS, (unsigned)R), dim3(ldp::K2_THREADS), 0, st, *params, refs, ga, d);
 }
 
 int ldp_postprocess_certainty(const ldp_params* params, const ldp_ref_desc* refs, float* outp,

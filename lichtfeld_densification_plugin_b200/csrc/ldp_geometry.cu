@@ -480,6 +480,7 @@ __device__ __forceinline__ bool parallax_pass(float X0, float X1, float X2, cons
 
 struct SampleResult {
     float X0, X1, X2, err;
+    float z1;               // the reference camera's depth of the point (reproj_err's z), NaN where not triangulated
     float cr, cg, cb, dcert;
     float4 dbg;
     int keep, good, grp;
@@ -641,7 +642,7 @@ __device__ __forceinline__ void eval_sample(const ldp_params& P, const RefConst&
 
     GCLK_USE(o.cr); GCLK_USE(o.cg); GCLK_USE(o.cb); GCLK_USE(o.good); GCLK(3);
     o.X0 = o.X1 = o.X2 = 0.f;
-    o.err = __int_as_float(0x7fc00000);
+    o.err = o.z1 = __int_as_float(0x7fc00000);
     o.keep = 0;
     o.converged = true;
     if (o.good) {          // the reference triangulates only the Sampson survivors (core/pipeline.py:721-733)
@@ -702,7 +703,7 @@ __device__ __forceinline__ void eval_sample(const ldp_params& P, const RefConst&
                 keep = (!dnan && d <= ga.par_cos_max) ? 1 : 0;
             }
         }
-        o.X0 = X0; o.X1 = X1; o.X2 = X2; o.err = err; o.keep = keep;
+        o.X0 = X0; o.X1 = X1; o.X2 = X2; o.err = err; o.z1 = z1; o.keep = keep;
         GCLK_USE(o.X0); GCLK_USE(o.err); GCLK_USE(o.keep); GCLK(6);
     }
     o.dcert = 0.f;
@@ -774,10 +775,12 @@ __device__ __forceinline__ float mv_view_err(const ldp_lens* L, const float* Pm,
 
 // Refines the kept two-view point (X, err) of the sample at map pixel idx, winner k, winner warp row wv.  On return X / err
 // hold the point to emit and mask its view mask.  ROBUST = false: returns false if a solve did not converge (nothing is
-// changed; the fix-up repeats the refinement with ROBUST = true, which always converges).
+// changed; the fix-up repeats the refinement with ROBUST = true, which always converges).  z_ref: when not null, receives the
+// reference camera's depth of an accepted refined point (left alone otherwise).
 template <bool ROBUST, bool LENS>
 __device__ bool mv_refine(const ldp_params& P, const RefConst& rc, const PairTable& pc, const ProView& pv, const GeomArgs& ga,
-                          const ldp_lens* lt, int idx, int k, float4 wv, float& X0, float& X1, float& X2, float& err, int& mask) {
+                          const ldp_lens* lt, int idx, int k, float4 wv, float& X0, float& X1, float& X2, float& err, int& mask,
+                          float* z_ref = nullptr) {
     mask = 1 << k;
     const float wm1 = (float)(P.w_match - 1), hm1 = (float)(P.h_match - 1);
     MvPix a, bk;
@@ -847,7 +850,7 @@ __device__ bool mv_refine(const ldp_params& P, const RefConst& rc, const PairTab
         emax = fmaxf(emax, e);
     }
     if (ok && P.min_parallax_deg > 0.0f) ok = parallax_pass(Y0, Y1, Y2, rc.C1, pc.C2[k], ga.par_cos_max);
-    if (ok) { X0 = Y0; X1 = Y1; X2 = Y2; err = emax; mask |= (int)used; }
+    if (ok) { X0 = Y0; X1 = Y1; X2 = Y2; err = emax; mask |= (int)used; if (z_ref) *z_ref = zA; }
     return true;
 }
 
@@ -1250,6 +1253,175 @@ ldp_undistort_kernel(const ldp_lens L, long long n, const float2* __restrict__ i
         if (L.model != LDP_LENS_PINHOLE) lens_undistort_px(L, p.x, p.y, q.x, q.y);
         out[i] = q;
     }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Depth maps (ldp_depth_maps; the rule is stated in include/ldp_b200.h).  Not in the reference.
+// KD1: one thread per map pixel, grid (CTAs per view, views); a CTA strides over its view's map, so the camera constants are
+//      staged once per CTA and not once per 128 pixels.  The arg-max reads the neighbours' certainty words and a candidate
+//      the winner's 16-byte warp row, both coalesced over the map.  A candidate is evaluated by eval_sample (and mv_refine)
+//      like a sampled pixel; its texels are not gathered (zero records: the colour eval_sample computes from them is dead
+//      code here).  A solve that does not converge puts the pixel on its view's worklist instead of writing it.
+// KD2: the fix-up.  Redoes every worklist entry with Jacobi (ROBUST = true) and writes it.
+// ---------------------------------------------------------------------------------------------
+struct DepthArgs {
+    float* depth;                    // [R][N]
+    float* err;                      // [R][N] or null
+    float* xyz;                      // [R][N][3] or null
+    uint8_t* flags;                  // [R][N] or null
+    unsigned long long* kept;        // [R], zeroed by the host
+    uint32_t* fix_list;              // [R][N] worklist, pixel | MV_FIX (one entry per pixel at most: it cannot overflow)
+    int32_t* fix_count;              // [R], zeroed by the host
+    float min_cert;                  // f32(min_certainty)
+    int N;                           // H * W
+};
+constexpr int KDF_BLOCKS = 16;       // fix-up CTAs per view
+
+// best post-processed certainty over the view's nn >= 1 neighbours at pixel idx and its slot: first index on ties, NaN wins
+// (the stream kernel's arg-max, core/pipeline.py:634-635)
+__device__ __forceinline__ float depth_argmax(const ldp_params& P, const PairTable& pc, const ProView& pv, int nn, int idx, int& k) {
+    k = 0;
+    float best = cert_at(P, pc, pv, 0, idx);
+    for (int q = 1; q < nn; ++q) {
+        const float c = cert_at(P, pc, pv, q, idx);
+        if (c > best || c != c) { best = c; k = q; }
+    }
+    return best;
+}
+
+__device__ __forceinline__ void depth_store(const DepthArgs& d, size_t o, int flags, float z, float err, float X0, float X1, float X2) {
+    d.depth[o] = z;
+    if (d.err) d.err[o] = err;
+    if (d.xyz) { d.xyz[3 * o] = X0; d.xyz[3 * o + 1] = X1; d.xyz[3 * o + 2] = X2; }
+    if (d.flags) d.flags[o] = (uint8_t)flags;
+}
+
+__device__ __forceinline__ void depth_push(const DepthArgs& d, int r, uint32_t entry) {
+    const int slot = atomicAdd(d.fix_count + r, 1);
+    d.fix_list[(size_t)r * d.N + slot] = entry;
+}
+
+__device__ __forceinline__ void depth_count_kept(const DepthArgs& d, int r, unsigned kept) {
+    kept = __reduce_add_sync(0xffffffffu, kept);
+    if ((threadIdx.x & 31) == 0 && kept) atomicAdd(d.kept + r, (unsigned long long)kept);
+}
+
+// the view's constants (and lens table, post-processing view) in shared memory
+template <bool LENS>
+__device__ __forceinline__ const ldp_lens* depth_stage(const ldp_params& P, const ldp_ref_desc* rd, RefConst& rc, PairTable& pc,
+                                                       ProView& pv, ldp_lens* s_lens) {
+    stage_constants(rd, rc, pc, threadIdx.x, K2_THREADS);
+    if (P.prologue) stage_proview(rd, pv, threadIdx.x);
+    if constexpr (LENS) {
+        StagedLens sl;
+        lens_load(rd, threadIdx.x, sl);
+        lens_store(sl, s_lens, threadIdx.x);
+        return s_lens;
+    }
+    return nullptr;
+}
+
+__device__ __forceinline__ SampleRec depth_record(const PairTable& pc, int k, int idx) {
+    SampleRec rec;
+    rec.wv = __ldg(reinterpret_cast<const float4*>(pc.warp[k]) + idx);
+    rec.tex[0] = rec.tex[1] = rec.tex[2] = 0u;
+    rec.k_cert = (uint32_t)k;
+    return rec;
+}
+
+template <bool LENS, bool MV>
+__global__ void __launch_bounds__(K2_THREADS, K2_MIN_BLOCKS)
+ldp_depth_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const GeomArgs ga, const DepthArgs d)
+{
+    __shared__ RefConst rc;
+    __shared__ PairTable pc;
+    __shared__ ProView pv;
+    __shared__ __align__(8) ldp_lens s_lens[LENS ? LDP_MAX_NN + 1 : 1];
+    const int r = blockIdx.y;
+    grid_dependency_sync();
+    const ldp_lens* lt = depth_stage<LENS>(P, refs + r, rc, pc, pv, s_lens);
+    __syncthreads();
+    const int nn = rc.nn, N = d.N;
+    const float nan = __int_as_float(0x7fc00000);
+    unsigned kept = 0;
+    for (int base = blockIdx.x * K2_THREADS; base < N; base += gridDim.x * K2_THREADS) {
+        const int idx = base + threadIdx.x;
+        if (idx >= N) break;
+        int k = 0;
+        const float c = (nn > 0) ? depth_argmax(P, pc, pv, nn, idx, k) : nan;
+        const int cand = (c >= d.min_cert) ? 1 : 0;
+        int f = cand | (k << 4);
+        float z = nan, err = nan, X0 = nan, X1 = nan, X2 = nan;
+        if (cand) {
+            const SampleRec rec = depth_record(pc, k, idx);
+            SampleResult s;
+            GCLK_DECL
+            eval_sample<false, LENS>(P, rc, pc, ga, lt, rec, 0.f, s GCLK_PASS);
+            if (!s.converged || (ga.force_fix_two > 0 && idx % ga.force_fix_two == 0)) {
+                depth_push(d, r, (uint32_t)idx);
+                continue;
+            }
+            f |= (s.good << 1) | (s.keep << 2);
+            err = s.err;
+            if (s.keep) { X0 = s.X0; X1 = s.X1; X2 = s.X2; z = s.z1; }
+            if constexpr (MV) {
+                if (s.keep) {
+                    int mask;
+                    if (!mv_refine<false, LENS>(P, rc, pc, pv, ga, lt, idx, k, rec.wv, X0, X1, X2, err, mask, &z) ||
+                        (ga.force_fix_mv > 0 && idx % ga.force_fix_mv == 0)) {
+                        depth_push(d, r, (uint32_t)idx | MV_FIX);
+                        continue;
+                    }
+                }
+            }
+            kept += s.keep;
+        }
+        depth_store(d, (size_t)r * N + idx, f, z, err, X0, X1, X2);
+    }
+    depth_count_kept(d, r, kept);
+}
+
+template <bool LENS, bool MV>
+__global__ void __launch_bounds__(K2_THREADS)
+ldp_depth_fix_kernel(const ldp_params P, const ldp_ref_desc* __restrict__ refs, const GeomArgs ga, const DepthArgs d)
+{
+    __shared__ RefConst rc;
+    __shared__ PairTable pc;
+    __shared__ ProView pv;
+    __shared__ __align__(8) ldp_lens s_lens[LENS ? LDP_MAX_NN + 1 : 1];
+    const int r = blockIdx.y;
+    grid_dependency_sync();
+    const int n = d.fix_count[r];
+    if ((int)blockIdx.x * K2_THREADS >= n) return;
+    const ldp_lens* lt = depth_stage<LENS>(P, refs + r, rc, pc, pv, s_lens);
+    __syncthreads();
+    const float nan = __int_as_float(0x7fc00000);
+    unsigned kept = 0;
+    for (int base = blockIdx.x * K2_THREADS; base < n; base += gridDim.x * K2_THREADS) {
+        const int e = base + threadIdx.x;
+        if (e < n) {
+            const uint32_t it = d.fix_list[(size_t)r * d.N + e];
+            const int idx = (int)(it & ~(uint32_t)MV_FIX);
+            int k;
+            depth_argmax(P, pc, pv, rc.nn, idx, k);
+            const SampleRec rec = depth_record(pc, k, idx);
+            SampleResult s;
+            GCLK_DECL
+            if (MV && (it & MV_FIX)) eval_sample<false, LENS>(P, rc, pc, ga, lt, rec, 0.f, s GCLK_PASS);   // converged: as before
+            else eval_sample<true, LENS>(P, rc, pc, ga, lt, rec, 0.f, s GCLK_PASS);
+            float z = nan, err = s.err, X0 = nan, X1 = nan, X2 = nan;
+            if (s.keep) { X0 = s.X0; X1 = s.X1; X2 = s.X2; z = s.z1; }
+            if constexpr (MV) {
+                if (s.keep) {
+                    int mask;
+                    mv_refine<true, LENS>(P, rc, pc, pv, ga, lt, idx, k, rec.wv, X0, X1, X2, err, mask, &z);
+                }
+            }
+            depth_store(d, (size_t)r * d.N + idx, 1 | (s.good << 1) | (s.keep << 2) | (k << 4), z, err, X0, X1, X2);
+            kept += s.keep;
+        }
+    }
+    depth_count_kept(d, r, kept);
 }
 
 }  // namespace ldp

@@ -324,6 +324,18 @@ class DensifyOutputs:
         return int(self.ref_offset[-1].item()) if self.n_refs else 0
 
 
+@dataclass
+class DepthMaps:
+    """Device tensors of one ``DensifyEngine.depth_maps`` call (include/ldp_b200.h: ldp_depth_maps).  Map pixel i of view r is
+    ``[r].view(-1)[i]``, indexed like the certainty planes."""
+    depth: torch.Tensor                       # f32 [R, H, W]: the reference camera's z of the kept point, NaN elsewhere
+    kept: torch.Tensor                        # int64 [R]: kept pixels per view
+    err: Optional[torch.Tensor] = None        # f32 [R, H, W]: reprojection error where triangulated, NaN elsewhere
+    xyz: Optional[torch.Tensor] = None        # f32 [R, H, W, 3]: world point where kept, NaN elsewhere
+    flags: Optional[torch.Tensor] = None      # u8 [R, H, W]: bit 0 candidate, 1 Sampson pass, 2 kept, bits 4-7 winning slot
+    ready: Optional[torch.cuda.Event] = None  # DensifyRing.submit_depth_maps: recorded on the ring stream after the launch
+
+
 class DensifyEngine:
     """Owns the scratch workspace and enqueues launches on the current torch CUDA stream."""
 
@@ -333,6 +345,7 @@ class DensifyEngine:
         self.lib = N.load()
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
         self._workspace: Optional[torch.Tensor] = None
+        self._depth_workspace: Optional[torch.Tensor] = None
         self.sm_reserve = -1         # SMs the first draw kernel leaves to other launches in flight (-1: process default, 0: none)
         self.pairs = PairConstantCache()
 
@@ -430,6 +443,46 @@ class DensifyEngine:
         """Run the whole path for ``batch``.  ``uniforms``: f64 [n_refs, U] device tensor selects the
         explicit (parity) RNG mode; otherwise Philox keyed by (cfg.seed, rng_stream)."""
         return self.prepare(batch, cfg, uniforms, collect_debug, taps, descs_dev, outputs).launch()
+
+    def depth_maps(self, batch: RefBatch, cfg: PathConfig, min_certainty: float, want_err: bool = False,
+                   want_xyz: bool = False, want_flags: bool = False) -> DepthMaps:
+        """``ldp_depth_maps``: every pixel of every view of ``batch`` whose best certainty is >= ``min_certainty`` (in (0, 1])
+        triangulated and filtered as a sampled pixel with the same winner is by ``densify(batch, cfg)``.  Enqueued on the
+        current torch stream."""
+        if not 0.0 < float(min_certainty) <= 1.0:
+            raise ValueError("min_certainty must lie in (0, 1]")
+        R, H, W = len(batch), batch.H, batch.W
+        params = self._params(batch, cfg, False, N.LDP_RNG_PHILOX, 0)
+        dev = self.device
+        f32 = dict(dtype=torch.float32, device=dev)
+        out = DepthMaps(depth=torch.empty((R, H, W), **f32), kept=torch.zeros((R,), dtype=torch.int64, device=dev),
+                        err=torch.empty((R, H, W), **f32) if want_err else None,
+                        xyz=torch.empty((R, H, W, 3), **f32) if want_xyz else None,
+                        flags=torch.empty((R, H, W), dtype=torch.uint8, device=dev) if want_flags else None)
+        if R == 0:
+            return out
+        need = C.c_size_t(0)
+        N.check(self.lib.ldp_depth_workspace_bytes(C.byref(params), C.byref(need)), "ldp_depth_workspace_bytes")
+        if self._depth_workspace is None or self._depth_workspace.numel() < need.value:
+            self._depth_workspace = None
+            self._depth_workspace = torch.empty(int(need.value), dtype=torch.uint8, device=dev)
+        ws = self._depth_workspace
+        descs = self.upload_descs(batch)
+        ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = self.lib.ldp_depth_maps(C.byref(params), ptr(descs), float(min_certainty), ptr(out.depth), ptr(out.err), ptr(out.xyz),
+                                     ptr(out.flags), ptr(out.kept), ptr(ws), C.c_size_t(ws.numel()), C.c_void_p(stream))
+        N.check(rc, "ldp_depth_maps")
+        out._keep = (descs, batch)          # read by the kernels: alive until the stream is done with them
+        return out
+
+    def depth_fixups(self, n_refs: int) -> np.ndarray:
+        """Entries of the last ``depth_maps`` call's fix-up worklist per view (synchronises)."""
+        ws = self._depth_workspace
+        if ws is None:
+            return np.zeros((n_refs,), dtype=np.int32)
+        a = (-ws.data_ptr()) % 256
+        return ws[a:a + 4 * n_refs].view(torch.int32).cpu().numpy()
 
     def postprocess_certainty(self, batch: RefBatch, certainty_floor: float) -> torch.Tensor:
         """``ldp_postprocess_certainty``: the reference's certainty post-processing alone (core/pipeline.py:405-430).
@@ -602,8 +655,20 @@ class DensifyRing:
             out.ready.record(st)
         return out
 
-    def wait(self, out: DensifyOutputs) -> None:
-        """Order the caller's current stream after ``out``."""
+    def submit_depth_maps(self, batch: RefBatch, cfg: PathConfig, min_certainty: float, **kw) -> DepthMaps:
+        """``DensifyEngine.depth_maps`` on the next ring stream, ordered like ``submit``; ``ready`` is recorded behind it."""
+        j = self._n % self.depth
+        self._n += 1
+        st = self.streams[j]
+        st.wait_stream(torch.cuda.current_stream(self.device))
+        with torch.cuda.stream(st):
+            out = self.engines[j].depth_maps(batch, cfg, min_certainty, **kw)
+            out.ready = torch.cuda.Event()
+            out.ready.record(st)
+        return out
+
+    def wait(self, out) -> None:
+        """Order the caller's current stream after ``out`` (``DensifyOutputs`` or ``DepthMaps``)."""
         if out.ready is not None:
             torch.cuda.current_stream(self.device).wait_event(out.ready)
 

@@ -505,3 +505,20 @@ class IncrementalPly:
             f.write(ply_header(self.n_points))
             for p in self._parts:
                 p.tofile(f)
+
+
+def write_depth_map(path_out: str, depth) -> None:
+    """One reference view's depth map (``DensifyEngine.depth_maps(...).depth[r]``, a tensor or array [H, W]) as a float32
+    ``.npy`` [H, W]; NaN = no depth.  Pixel (y, x) of the map is map pixel i = y * W + x, indexed like the certainty planes;
+    its camera pixel is the decoded ``(uA_obs, vA_obs)`` of its own warp row: ((xA + 1) / 2 * (w_match - 1) * sxA,
+    (yA + 1) / 2 * (h_match - 1) * syA) with sxA = width / w_match, syA = height / h_match (the reference camera's full
+    resolution over the matcher's), in float32 as the kernels decode it.  The value is that camera's z of the kept point
+    (the distance along its optical axis), not a distance along the ray.  For the synthetic grid of ``synth``, whose warp rows
+    hold each map pixel's own grid coordinates (gx, gy) in [-1, 1] as (xA, yA), that is
+    ((gx + 1) / 2 * (w_match - 1) * sxA, (gy + 1) / 2 * (h_match - 1) * syA)."""
+    if isinstance(depth, torch.Tensor):
+        depth = depth.detach().cpu().numpy()
+    a = np.asarray(depth)
+    if a.ndim != 2:
+        raise ValueError(f"a depth map is [H, W], got shape {a.shape}")
+    np.save(path_out, np.ascontiguousarray(a, dtype=np.float32), allow_pickle=False)
