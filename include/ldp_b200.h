@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define LDP_ABI_VERSION 19
+#define LDP_ABI_VERSION 20
 #define LDP_MAX_NN 16          /* neighbours per reference view (the panel clamps to 10) */
 #define LDP_MAX_BINS 4096      /* coverage tiles per map: ceil(W/tile)*ceil(H/tile), tile = max(1, W/24) */
 
@@ -447,6 +447,34 @@ int ldp_gaussian_init(const float* xyz, const float* rgb, const float* normals, 
 int ldp_pack_gaussian_ply_records(const float* xyz, const float* normals, const float* sh_dc, const float* opacity, const float* scales,
                                   const float* rotations, int64_t n, const int64_t* n_dev, int32_t sh_degree, uint8_t* records_out,
                                   void* stream);
+
+/* ---- cross-view depth consistency (not in the reference) -------------------------------------------------------------
+ * The visibility test of MVS fusion: every point is projected into the other views' depth maps (ldp_depth_maps) and compared
+ * with the depth each view sees there.  Inputs: xyz [n,3] f32 device; owner [n] int32 device or NULL: the view each point
+ * came from, or -1 (a point is never checked against its own view, whose map contains the point itself); V = n_views maps
+ * of one shape H x W.  Per view v, all DEVICE arrays: depth_ptrs[v] the map ([H*W] f32, indexed like the certainty
+ * planes); P[v] f32 [12], the P1 the map was made with, row-major; scales[v] f64 [2] = (ax, ay), camera pixel -> map pixel;
+ * lens[v] (ldp_lens [V]), or lens = NULL when every view is pinhole.  rel_tol in (0, 1), min_views >= 0, max_violations >= 0.
+ * For every point i and every view v != owner[i]:
+ *   1. Projection in f64 without FMA contraction: q_r = ((P[r,0] X + P[r,1] Y) + P[r,2] Z) + P[r,3] (each product of two
+ *      f32 values is exact in f64, so only the additions round), z = q_2.  The view does not see the point unless z > 0.
+ *      Pinhole: u = q_0 / z, v = q_1 / z.  Lens: the forward model of the reprojection test (see ldp_lens) applied to
+ *      ((u - cx) / fx, (v - cy) / fy), then back to pixels, in f64 (contraction allowed there).
+ *   2. Map pixel (nearest): x = floor(u * ax), y = floor(v * ay), in f64; ax = W / ((w_match - 1) * f64(sxA)), ay = H /
+ *      ((h_match - 1) * f64(syA)), sxA and syA the view's f32 ldp_ref_desc scales.  This inverts the decode of the matcher's
+ *      grid, linspace(-1 + 1/W, 1 - 1/W, W): map pixel x is centred at u * ax = x + 1/2.  The view does not see the point
+ *      unless 0 <= x < W and 0 <= y < H.
+ *   3. D = the map at (y, x).  NaN or D <= 0: no evidence.  Otherwise, in f64, d = z - D, t = rel_tol * D:
+ *      |d| <= t consistent; d < -t a VIOLATION (the point lies in front of the surface the view sees: the view looks
+ *      through it); otherwise occluded, which counts for nothing.
+ *   4. Point i is kept iff n_consistent >= min_views && n_violations <= max_violations.
+ * Outputs (device): n_consistent_out, n_violations_out int32 [n] or NULL; kept_idx_out int64 [n], the first status_out[1]
+ * entries written, the kept points in ascending index (the emission order stays); status_out int32 [2] = {bit mask: 1 a
+ * coordinate is not finite (then nothing else is written), 2 an owner outside [-1, V) (that point is checked against every
+ * view); kept count}.  n = 0 zeroes status_out and writes nothing else.  No host synchronisation.  Results do not depend on
+ * the launch configuration.  Workspace: ldp_consistency_workspace_bytes(n). */
+int ldp_consistency_workspace_bytes(int64_t n, size_t* bytes_out);
+int ldp_depth_consistency(const float* xyz, int64_t n, const int32_t* owner, const float* const* depth_ptrs, int32_t H, int32_t W, const float* P, const double* scales, const ldp_lens* lens, int32_t n_views, double rel_tol, int32_t min_views, int32_t max_violations, int32_t* n_consistent_out, int32_t* n_violations_out, int64_t* kept_idx_out, int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream);
 
 /* SMs the one-CTA-per-SM first draw kernel leaves free when ldp_params.sm_reserve is -1 (process-wide default, initially 0).
  * With several launches in flight on different streams (engine.DensifyRing) or a collective running beside the path, the

@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-LDP_ABI_VERSION = 19
+LDP_ABI_VERSION = 20
 LDP_MAX_NN = 16
 LDP_MAX_BINS = 4096
 
@@ -143,6 +143,8 @@ SIGNATURES = {
     "ldp_gaussian_workspace_bytes": (C.c_int, [_I64, _I32, _SZ_OUT]),
     "ldp_gaussian_init": (C.c_int, [_P, _P, _P, _I64, _I32, C.c_double, C.c_double, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "ldp_pack_gaussian_ply_records": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, _P, _I32, _P, _P]),
+    "ldp_consistency_workspace_bytes": (C.c_int, [_I64, _SZ_OUT]),
+    "ldp_depth_consistency": (C.c_int, [_P, _I64, _P, _P, _I32, _I32, _P, _P, _P, _I32, C.c_double, _I32, _I32, _P, _P, _P, _P, _P, _SZ, _P]),
     "ldp_set_sm_reserve": (C.c_int, [C.c_int]),
     "ldp_last_launch_count": (C.c_int, []),
     "ldp_profile_enable": (C.c_int, [C.c_int]),

@@ -70,6 +70,13 @@ class DensePipelineConfig:
                                      # pixel whose best certainty is >= depth_min_certainty, triangulated and filtered like a
                                      # sample) plus depth_maps.json; "" = off
     depth_min_certainty: float = 0.5 # depth maps: certainty a pixel's best match needs to be evaluated, in (0, 1]
+    depth_consistency: bool = False  # keep a point only where the other reference views' depth maps agree with it (MVS
+                                     # fusion's visibility test, include/ldp_b200.h: ldp_depth_consistency); the maps of every
+                                     # view stay on the device until the end: R * H * W * 4 bytes (46 views at 512^2: 48 MB,
+                                     # 250 views at 640^2: 410 MB)
+    consistency_rel_tol: float = 0.01    # relative depth difference that still agrees (COLMAP fusion's default), in (0, 1)
+    consistency_min_views: int = 1   # other views that must agree with a point
+    consistency_max_violations: int = 0  # other views that may look through a point (see it in front of their surface)
 
     def validate(self) -> "DensePipelineConfig":
         if self.matches_per_ref < 0:
@@ -96,6 +103,12 @@ class DensePipelineConfig:
             raise ValueError("depth_dir must be a string (\"\" = off)")
         if not 0.0 < float(self.depth_min_certainty) <= 1.0:
             raise ValueError("depth_min_certainty must lie in (0, 1]")
+        if not 0.0 < float(self.consistency_rel_tol) < 1.0:
+            raise ValueError("consistency_rel_tol must lie in (0, 1)")
+        if int(self.consistency_min_views) < 0:
+            raise ValueError("consistency_min_views must be >= 0")
+        if int(self.consistency_max_violations) < 0:
+            raise ValueError("consistency_max_violations must be >= 0")
         if self.rng_mode not in (RNG_PHILOX, RNG_NUMPY_GLOBAL, RNG_EXPLICIT):
             raise ValueError(f"unknown rng_mode {self.rng_mode!r}")
         return self

@@ -45,6 +45,8 @@ class PipelineResult:
     gaussians: Optional[Dict[str, np.ndarray]] = None   # extra, config.gaussian_neighbors: 3DGS's initial splats, f32
                                                   # sh_dc [n,3], opacity [n], scales [n,3] (log), rotations [n,4] (w, x, y, z)
     depth_paths: Optional[Dict[int, str]] = None  # extra, config.depth_dir: reference camera uid -> its depth map file
+    consistent_views: Optional[np.ndarray] = None  # extra, config.depth_consistency: int32 per point, the other reference
+                                                  # views whose depth maps agree with it
 
 
 class PipelineCancelled(RuntimeError):
@@ -306,7 +308,9 @@ class _PendingLaunch:
     n: int
     collect_debug: bool
     ply_records: bool
-    depth: Optional[DepthMaps] = None            # config.depth_dir: the launch's depth maps, written when it is collected
+    depth: Optional[DepthMaps] = None            # config.depth_dir / depth_consistency: the launch's depth maps, written
+                                                 # or kept when it is collected
+    ref_cams: Optional[List[CameraRecord]] = None   # the reference camera of every view, as the launch used it
 
 
 def submit_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _TriangulationContext,
@@ -328,6 +332,7 @@ def submit_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triangulati
     first = matched_refs[0].cert_list_cpu[0]
     H, W = int(first.shape[0]), int(first.shape[1])
     batch = eng.new_batch(H, W, tri_ctx.w_match, tri_ctx.h_match)
+    ref_cams: List[CameraRecord] = []
     for i, mr in enumerate(matched_refs):
         packed = mr.packed
         certs = [_to_device(c, dev, torch.float32) for c in mr.cert_list_cpu]
@@ -335,6 +340,7 @@ def submit_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triangulati
         image = _to_device(packed.imA_np, dev, torch.uint8)
         ref_cam = _record_for(tri_ctx.cameras, packed.ref_id, size=(packed.wA_cam, packed.hA_cam))
         nbrs = [_record_for(tri_ctx.cameras, uid) for uid in packed.nn_ids]
+        ref_cams.append(ref_cam)
         mask_a = masks_b = None
         if raw[i]:
             mask_a = None if packed.maskA_np is None else _to_device(packed.maskA_np, dev, torch.uint8)
@@ -348,15 +354,17 @@ def submit_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triangulati
         u_dev = torch.from_numpy(np.ascontiguousarray(uniforms, dtype=np.float64)).to(dev)
         batch._keep_alive.append(u_dev)      # read by kernels on a ring stream: alive until the launch is collected, like the planes
     depth = None
+    want_depth = bool(getattr(cfg, "depth_dir", "")) or bool(getattr(cfg, "depth_consistency", False))
     if ring is None:
         out = eng.densify(batch, pcfg, uniforms=u_dev, collect_debug=collect_debug_matches)
-        if getattr(cfg, "depth_dir", ""):
+        if want_depth:
             depth = eng.depth_maps(batch, pcfg, float(cfg.depth_min_certainty))
     else:
         out = ring.submit(batch, pcfg, uniforms=u_dev, collect_debug=collect_debug_matches)
-        if getattr(cfg, "depth_dir", ""):
+        if want_depth:
             depth = ring.submit_depth_maps(batch, pcfg, float(cfg.depth_min_certainty))
-    return _PendingLaunch(out=out, batch=batch, n=n, collect_debug=collect_debug_matches, ply_records=ply_records, depth=depth)
+    return _PendingLaunch(out=out, batch=batch, n=n, collect_debug=collect_debug_matches, ply_records=ply_records, depth=depth,
+                          ref_cams=ref_cams)
 
 
 def depth_map_name(cameras, uid: int) -> str:
@@ -386,9 +394,10 @@ def _write_depth_maps(pending: _PendingLaunch, tri_ctx: _TriangulationContext, o
 
 
 def collect_refs(pending: _PendingLaunch, errors: Optional[list] = None, ring=None, tri_ctx: Optional[_TriangulationContext] = None,
-                 depth_paths: Optional[Dict[int, str]] = None) -> List[Optional[_TriangulatedReference]]:
+                 depth_paths: Optional[Dict[int, str]] = None, depth_kept: Optional[list] = None) -> List[Optional[_TriangulatedReference]]:
     """Second half: one synchronising read of the launch's results, split per view.  A launch with depth maps writes them
-    under ``tri_ctx.config.depth_dir`` and records each file in ``depth_paths`` (reference camera uid -> path)."""
+    under ``tri_ctx.config.depth_dir`` and records each file in ``depth_paths`` (reference camera uid -> path); with
+    ``depth_kept`` it appends (uid, device map [H, W], reference camera) for every view whose sampling succeeded."""
     out, batch = pending.out, pending.batch
     if ring is not None:
         ring.wait(out)                                 # the current stream (which does the read-back) follows the ring stream
@@ -410,7 +419,14 @@ def collect_refs(pending: _PendingLaunch, errors: Optional[list] = None, ring=No
     if pending.depth is not None:
         if tri_ctx is None:
             raise ValueError("a launch with depth maps is collected with its tri_ctx")
-        _write_depth_maps(pending, tri_ctx, ok, ring, depth_paths)
+        if getattr(tri_ctx.config, "depth_dir", ""):
+            _write_depth_maps(pending, tri_ctx, ok, ring, depth_paths)
+        if depth_kept is not None:
+            if ring is not None:
+                ring.wait(pending.depth)           # the maps are read later on the current stream
+            for r in range(pending.n):
+                if ok[r]:
+                    depth_kept.append((int(pending.batch.ref_uids[r]), pending.depth.depth[r], pending.ref_cams[r]))
     triangulate_refs.last_launches = out.launches
     return results
 
@@ -420,25 +436,28 @@ def triangulate_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triang
                      uniforms: Optional[np.ndarray] = None,
                      weight_sums: Optional[Sequence[float]] = None,
                      errors: Optional[list] = None, ply_records: bool = False,
-                     depth_paths: Optional[Dict[int, str]] = None) -> List[Optional[_TriangulatedReference]]:
+                     depth_paths: Optional[Dict[int, str]] = None,
+                     depth_kept: Optional[list] = None) -> List[Optional[_TriangulatedReference]]:
     """Batched ``_triangulate_ref``: every view of ``matched_refs`` in one launch sequence.
 
     RNG: ``uniforms`` (f64 [n, U], explicit parity stream per view) or Philox keyed by
     (config.seed, rng_streams[i]).  Views the reference would skip (None return / exception) come back as
     None; the exception a per-view call would raise is appended to ``errors`` as (index, exc).
     ``ply_records``: also return every view's PLY vertex records (built on the device, 15 bytes per point).
-    ``config.depth_dir``: also write every view's depth map there (``depth_paths``: see ``collect_refs``).
+    ``config.depth_dir``: also write every view's depth map there (``depth_paths``: see ``collect_refs``);
+    ``depth_kept``: keep the maps on the device (see ``collect_refs``).
     """
     if len(matched_refs) == 0:
         return []
     pending = submit_refs(matched_refs, tri_ctx, collect_debug_matches, rng_streams=rng_streams, uniforms=uniforms,
                           weight_sums=weight_sums, ply_records=ply_records)
-    return collect_refs(pending, errors, tri_ctx=tri_ctx, depth_paths=depth_paths)
+    return collect_refs(pending, errors, tri_ctx=tri_ctx, depth_paths=depth_paths, depth_kept=depth_kept)
 
 
 def _triangulate_ref(matched_ref: _MatchedReference, tri_ctx: _TriangulationContext,
                      collect_debug_matches: bool = False, *,
-                     depth_paths: Optional[Dict[int, str]] = None) -> Optional[_TriangulatedReference]:
+                     depth_paths: Optional[Dict[int, str]] = None,
+                     depth_kept: Optional[list] = None) -> Optional[_TriangulatedReference]:
     """Triangulate matches for a single reference view (reference core/pipeline.py:602-780).
 
     ``config.rng_mode``: "numpy" consumes the process-global MT19937 stream like the reference's ``np.random.choice``:
@@ -460,19 +479,23 @@ def _triangulate_ref(matched_ref: _MatchedReference, tri_ctx: _TriangulationCont
         n_uni = 2 * size + 64
         while True:
             U = _mt_stream_from_global(n_uni)
+            kept_here: Optional[list] = [] if depth_kept is not None else None
             res = triangulate_refs([matched_ref], tri_ctx, collect_debug_matches, uniforms=U[None, :], errors=errs,
-                                   depth_paths=depth_paths)
+                                   depth_paths=depth_paths, depth_kept=kept_here)
             if errs and "exhausted" in str(errs[0][1]):
                 errs.clear()
                 n_uni *= 2
                 continue
+            if depth_kept is not None:
+                depth_kept += kept_here
             break
         used = int(triangulate_refs.last_uniforms_used[0])
         if used > 0:
             np.random.random_sample(used)          # advance the global stream like np.random.choice did
     else:
         res = triangulate_refs([matched_ref], tri_ctx, collect_debug_matches,
-                               rng_streams=[int(matched_ref.packed.ref_id)], errors=errs, depth_paths=depth_paths)
+                               rng_streams=[int(matched_ref.packed.ref_id)], errors=errs, depth_paths=depth_paths,
+                               depth_kept=depth_kept)
     if errs:
         raise errs[0][1]
     return res[0]
@@ -668,6 +691,7 @@ def run_dense_pipeline(
     ring = get_ring() if (n_chunks > 1 and getattr(config, "rng_mode", RNG_PHILOX) != RNG_NUMPY_GLOBAL) else None
     in_flight: List[tuple] = []      # (views done when this launch is collected, launch, its matched references)
     depth_paths: Optional[Dict[int, str]] = {} if getattr(config, "depth_dir", "") else None
+    depth_kept: Optional[list] = [] if getattr(config, "depth_consistency", False) else None
 
     def consume(outs, done: int, matched_refs) -> None:
         nonlocal pairs, ply_points, pair_counter
@@ -717,24 +741,25 @@ def run_dense_pipeline(
                 outs = []
                 for m in mrs:
                     try:
-                        outs.append(_triangulate_ref(m, tri_ctx, collect_debug, depth_paths=depth_paths))
+                        outs.append(_triangulate_ref(m, tri_ctx, collect_debug, depth_paths=depth_paths, depth_kept=depth_kept))
                     except Exception:
                         outs.append(None)
                 consume(outs, done, mrs)
             elif ring is None:
                 consume(triangulate_refs(mrs, tri_ctx, collect_debug, rng_streams=[int(r) for r, _ in matched],
-                                         ply_records=ply_base is not None, depth_paths=depth_paths), done, mrs)
+                                         ply_records=ply_base is not None, depth_paths=depth_paths, depth_kept=depth_kept),
+                        done, mrs)
             else:
                 # several launches in flight: the next chunk is uploaded and enqueued before the oldest one is read back
                 in_flight.append((done, submit_refs(mrs, tri_ctx, collect_debug, rng_streams=[int(r) for r, _ in matched],
                                                     ply_records=ply_base is not None, ring=ring), mrs))
                 if len(in_flight) >= ring.depth:
                     d, pend, pm = in_flight.pop(0)
-                    consume(collect_refs(pend, ring=ring, tri_ctx=tri_ctx, depth_paths=depth_paths), d, pm)
+                    consume(collect_refs(pend, ring=ring, tri_ctx=tri_ctx, depth_paths=depth_paths, depth_kept=depth_kept), d, pm)
         for d, pend, pm in in_flight:
             if _is_cancelled(cancel_requested):
                 raise PipelineCancelled("Cancelled")
-            consume(collect_refs(pend, ring=ring, tri_ctx=tri_ctx, depth_paths=depth_paths), d, pm)
+            consume(collect_refs(pend, ring=ring, tri_ctx=tri_ctx, depth_paths=depth_paths, depth_kept=depth_kept), d, pm)
     finally:
         if debug_state is not None and hasattr(debug_state, "release_waiters"):
             debug_state.release_waiters()                              # core/pipeline.py:547-548
@@ -749,6 +774,17 @@ def run_dense_pipeline(
     xyz, rgb, err = np.concatenate(parts_xyz, axis=0), np.concatenate(parts_rgb, axis=0), np.concatenate(parts_err, axis=0)
     n_views = np.concatenate(parts_nv, axis=0) if getattr(config, "multiview", False) else None
     ref_uid = np.concatenate(parts_ref, axis=0)
+    consistent = None
+    if depth_kept is not None:
+        # visibility test against the other reference views' maps, before the outlier filter, normals and Gaussians; the
+        # intermediate PLYs above stay unfiltered
+        if progress_callback:
+            progress_callback(93.0, "Checking depth consistency...")
+        consistent, keep = _check_consistency(xyz, ref_uid, depth_kept, tri_ctx)
+        depth_kept = None                      # the maps are not needed any more
+        xyz, rgb, err, ref_uid = xyz[keep], rgb[keep], err[keep], ref_uid[keep]
+        if n_views is not None:
+            n_views = n_views[keep]
     k_out = int(getattr(config, "outlier_neighbors", 0))
     k_nrm = int(getattr(config, "normal_neighbors", 0))
     k_gs = int(getattr(config, "gaussian_neighbors", 0))
@@ -768,6 +804,8 @@ def run_dense_pipeline(
         xyz_dev = res.xyz
         if n_views is not None:
             n_views = n_views[keep]
+        if consistent is not None:
+            consistent = consistent[keep]
     if k_nrm > 0:
         # every point faces the camera it was triangulated from (its reference view, a contributing view in every mode)
         if progress_callback:
@@ -788,7 +826,27 @@ def run_dense_pipeline(
                            opacity=float(config.gaussian_opacity), flatten=float(config.gaussian_flatten))
         gaussians = {name: getattr(g, name).cpu().numpy() for name in ("sh_dc", "opacity", "scales", "rotations")}
     return PipelineResult(xyz=xyz, rgb=rgb, err=err, elapsed_seconds=time.time() - t0, pairs_processed=pairs, n_views=n_views,
-                          normals=normals, gaussians=gaussians, depth_paths=depth_paths)
+                          normals=normals, gaussians=gaussians, depth_paths=depth_paths, consistent_views=consistent)
+
+
+def _check_consistency(xyz: np.ndarray, ref_uid: np.ndarray, depth_kept: list, tri_ctx: _TriangulationContext):
+    """``output.check_depth_consistency`` of the cloud against the kept maps (``collect_refs``), each point owned by the map of
+    its reference view.  Returns (n_consistent of the kept points, kept indices), host arrays."""
+    from ..engine import DepthViews
+    from ..output import check_depth_consistency
+    cfg = tri_ctx.config
+    m0 = depth_kept[0][1]
+    views = DepthViews(int(m0.shape[0]), int(m0.shape[1]), tri_ctx.w_match, tri_ctx.h_match, m0.device)
+    index: Dict[int, int] = {}
+    for uid, depth, cam in depth_kept:
+        index[uid] = views.add(depth, cam)
+    uids, inv = np.unique(ref_uid, return_inverse=True)
+    owner = np.array([index.get(int(u), -1) for u in uids], dtype=np.int32)[inv.reshape(-1)]
+    xyz_dev = torch.from_numpy(np.ascontiguousarray(xyz, dtype=np.float32)).to(m0.device)
+    res = check_depth_consistency(xyz_dev, views, owner=torch.from_numpy(owner), rel_tol=float(cfg.consistency_rel_tol),
+                                  min_views=int(cfg.consistency_min_views), max_violations=int(cfg.consistency_max_violations))
+    keep = res.kept_idx.cpu().numpy()
+    return res.n_consistent.cpu().numpy()[keep], keep
 
 
 def _write_depth_index(config: DensePipelineConfig, tri_ctx: _TriangulationContext, depth_paths: Dict[int, str]) -> None:

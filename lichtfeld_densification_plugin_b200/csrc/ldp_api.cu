@@ -14,6 +14,7 @@
 #include "ldp_select.cu"
 #include "ldp_voxel.cu"
 #include "ldp_outlier.cu"
+#include "ldp_consistency.cu"
 
 namespace {
 
@@ -1327,6 +1328,72 @@ int ldp_postprocess_certainty(const ldp_params* params, const ldp_ref_desc* refs
     KernelTimer kt(st, "ldp_prologue_kernel");
     return launch("ldp_prologue_kernel", ldp::ldp_prologue_kernel, grid, dim3(ldp::KP_THREADS), 0, st, *params, refs, outp, ref_stride,
                   plane_stride);
+}
+
+
+// ---- cross-view depth consistency (ldp_consistency.cu; the compaction is the outlier filter's scan + ldp_outlier_kept_kernel).
+// Last in the file: the device compiler places kernel instantiations in reverse order of first use, so the new kernels go
+// ahead of all others and the layout of the existing kernels relative to one another does not change.
+struct ConsistencyPlan {
+    int* flag;                             // [n] keep flags
+    int* rank;                             // [n] their exclusive prefix
+    int* block_tot;                        // the scan's per-block totals
+};
+
+static int consistency_plan(int64_t n, void* base, ConsistencyPlan* pl, size_t* bytes) {
+    if (n < 0 || n > 500000000ll) return fail(LDP_ERR_INVALID, "depth consistency: bad point count");
+    const size_t N = (size_t)std::max<int64_t>(n, 1);
+    Carver c{static_cast<char*>(base)};
+    pl->flag = c.take<int>(N);
+    pl->rank = c.take<int>(N);
+    pl->block_tot = c.take<int>(N / ldp::SC_THREADS + 2);
+    *bytes = c.off;
+    return LDP_OK;
+}
+
+int ldp_consistency_workspace_bytes(int64_t n, size_t* bytes_out) {
+    if (!bytes_out) return fail(LDP_ERR_INVALID, "null bytes_out");
+    ConsistencyPlan pl;
+    return consistency_plan(n, nullptr, &pl, bytes_out);
+}
+
+int ldp_depth_consistency(const float* xyz, int64_t n, const int32_t* owner, const float* const* depth_ptrs, int32_t H, int32_t W,
+                          const float* P, const double* scales, const ldp_lens* lens, int32_t n_views, double rel_tol,
+                          int32_t min_views, int32_t max_violations, int32_t* n_consistent_out, int32_t* n_violations_out,
+                          int64_t* kept_idx_out, int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream) {
+    begin_call();
+    if (!(rel_tol > 0.0 && rel_tol < 1.0)) return fail(LDP_ERR_INVALID, "rel_tol must lie in (0, 1)");
+    if (min_views < 0 || max_violations < 0) return fail(LDP_ERR_INVALID, "min_views and max_violations must be >= 0");
+    if (n_views < 0 || H <= 0 || W <= 0 || (long long)H * W > 0x3fffffffLL) return fail(LDP_ERR_INVALID, "bad view count or map shape");
+    if (n_views > 0 && (!depth_ptrs || !P || !scales)) return fail(LDP_ERR_INVALID, "null depth_ptrs / P / scales");
+    if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    int rc = check(cudaMemsetAsync(status_out, 0, 2 * sizeof(int32_t), st), "cudaMemsetAsync(status)");
+    if (rc != LDP_OK || n == 0) return rc;
+    if (!xyz || !kept_idx_out || !workspace) return fail(LDP_ERR_INVALID, "null pointer");
+    ConsistencyPlan pl;
+    size_t need = 0;
+    if ((rc = consistency_plan(n, workspace, &pl, &need)) != LDP_OK) return rc;
+    if (workspace_bytes < need) return fail(LDP_ERR_WORKSPACE, "consistency workspace too small");
+    const unsigned grid = (unsigned)((n + ldp::CS_THREADS - 1) / ldp::CS_THREADS);
+    rc = launch("ldp_consistency_check_kernel", owner ? ldp::ldp_consistency_check_kernel<true> : ldp::ldp_consistency_check_kernel<false>,
+                dim3(grid), dim3(ldp::CS_THREADS), 0, st, xyz, (const int*)owner, (long long)n, (int)n_views, (int*)status_out);
+    if (rc != LDP_OK) return rc;
+    const ldp::ConsistencyArgs a{xyz, (const int*)owner, depth_ptrs, P, scales, lens, (int*)n_consistent_out, (int*)n_violations_out,
+                                 pl.flag, (int*)status_out, (long long)n, rel_tol, (int)n_views, (int)H, (int)W, (int)min_views,
+                                 (int)max_violations};
+    // a few resident CTAs per SM; each strides over the cloud, so a table of one chunk is staged once per CTA
+    const unsigned cgrid = (unsigned)std::min<long long>(grid, (long long)sm_count() * 8);
+    {
+        KernelTimer kt(st, "ldp_consistency_kernel");
+        rc = launch("ldp_consistency_kernel", lens ? ldp::ldp_consistency_kernel<true> : ldp::ldp_consistency_kernel<false>,
+                    dim3(cgrid), dim3(ldp::CS_THREADS), 0, st, a);
+        if (rc != LDP_OK) return rc;
+    }
+    if ((rc = scan_exclusive(pl.flag, pl.rank, n, pl.block_tot, (int*)status_out + 1, st)) != LDP_OK) return rc;
+    const unsigned kgrid = (unsigned)((n + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
+    return launch("ldp_outlier_kept_kernel", ldp::ldp_outlier_kept_kernel, dim3(kgrid), dim3(ldp::KV_THREADS), 0, st, (const int*)pl.flag,
+                  (const int*)pl.rank, (long long)n, reinterpret_cast<long long*>(kept_idx_out));
 }
 
 }  // extern "C"

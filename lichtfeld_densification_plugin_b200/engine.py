@@ -336,6 +336,102 @@ class DepthMaps:
     ready: Optional[torch.cuda.Event] = None  # DensifyRing.submit_depth_maps: recorded on the ring stream after the launch
 
 
+def depth_map_scales(width: int, height: int, H: int, W: int, w_match: int, h_match: int) -> Tuple[float, float]:
+    """(ax, ay): camera pixel -> map pixel of an H x W depth map of a camera of ``width`` x ``height`` pixels, the inverse of
+    the decode of the matcher's grid (include/ldp_b200.h: ldp_depth_consistency, step 2): W / ((w_match - 1) * f64(sxA)) with
+    sxA = f32(width / w_match) as ``RefBatch.add`` computes it, and likewise for y.  Map pixel x is centred at u * ax = x + 1/2."""
+    if min(int(w_match), int(h_match)) < 2:
+        raise ValueError("w_match and h_match must be >= 2")
+    sxA, syA = np.float32(width / float(w_match)), np.float32(height / float(h_match))
+    return float(W) / (float(int(w_match) - 1) * float(sxA)), float(H) / (float(int(h_match) - 1) * float(syA))
+
+
+class DepthViews:
+    """Depth maps of one shape, each with the reference camera it was made with: what ``output.check_depth_consistency``
+    tests a cloud against.  Device maps are referenced, not copied (a slice of ``DepthMaps.depth`` works), and kept alive
+    here; host arrays, e.g. the ``.npy`` files of ``DensePipelineConfig.depth_dir``, are uploaded."""
+
+    def __init__(self, H: int, W: int, w_match: int, h_match: int, device=None) -> None:
+        if not torch.cuda.is_available():
+            raise N.NativeLibraryError("DepthViews needs a CUDA device (there is no CPU fallback)")
+        dev = torch.device(device if device is not None else "cuda")
+        if dev.type != "cuda":
+            raise N.NativeLibraryError("DepthViews lives on a CUDA device (there is no CPU fallback)")
+        self.device = dev if dev.index is not None else torch.device("cuda", torch.cuda.current_device())
+        self.H, self.W, self.w_match, self.h_match = int(H), int(W), int(w_match), int(h_match)
+        if self.H <= 0 or self.W <= 0:
+            raise ValueError("H and W must be positive")
+        depth_map_scales(1, 1, self.H, self.W, self.w_match, self.h_match)         # validates the matcher size
+        self.maps: List[torch.Tensor] = []
+        self.cameras: List[CameraRecord] = []
+        self._tables = None
+
+    def __len__(self) -> int:
+        return len(self.maps)
+
+    def add(self, depth, camera: CameraRecord) -> int:
+        """Append one view: its f32 [H, W] map (a device tensor or a host array; NaN = no depth) and the ``CameraRecord`` its
+        map was made with (the P1 and lens of the launch, its full-resolution width and height).  Returns the view index,
+        the value ``owner`` takes for the points of this view."""
+        if isinstance(depth, np.ndarray):
+            depth = torch.from_numpy(np.ascontiguousarray(depth, dtype=np.float32)).to(self.device)
+        if not isinstance(depth, torch.Tensor) or depth.device != self.device or depth.dtype != torch.float32 \
+                or tuple(depth.shape) != (self.H, self.W):
+            raise ValueError(f"a depth map must be a float32 ({self.H}, {self.W}) tensor on {self.device} or a host array")
+        check_lens(camera)
+        self.maps.append(depth.contiguous())
+        self.cameras.append(camera)
+        self._tables = None
+        return len(self.maps) - 1
+
+    @classmethod
+    def from_depth_dir(cls, depth_dir: str, cameras: Sequence[CameraRecord], device=None) -> "DepthViews":
+        """The maps ``run_dense_pipeline`` wrote under ``depth_dir`` (``depth_maps.json`` and its ``.npy`` files), each with the
+        record of its camera uid from ``cameras``, sized as the index says.  View order = the index's order."""
+        import json
+        import os
+        with open(os.path.join(depth_dir, "depth_maps.json")) as f:
+            index = json.load(f)
+        maps = index["maps"]
+        if not maps:
+            raise ValueError("the depth index lists no map")
+        m0 = maps[0]
+        views = cls(m0["H"], m0["W"], m0["w_match"], m0["h_match"], device)
+        by_uid = {int(c.uid): c for c in cameras}
+        for m in maps:
+            if (m["H"], m["W"], m["w_match"], m["h_match"]) != (m0["H"], m0["W"], m0["w_match"], m0["h_match"]):
+                raise ValueError("the maps of a depth index must share one shape and matcher size")
+            cam = by_uid[int(m["camera_uid"])]
+            if (int(cam.width), int(cam.height)) != (int(m["width"]), int(m["height"])):
+                cam = CameraRecord(uid=cam.uid, image_path=cam.image_path, width=int(m["width"]), height=int(m["height"]),
+                                   K=cam.K, R=cam.R, t=cam.t, P=cam.P, C=cam.C, lens_model=getattr(cam, "lens_model", None),
+                                   lens_coeffs=getattr(cam, "lens_coeffs", None))
+            views.add(np.load(os.path.join(depth_dir, m["file"])), cam)
+        return views
+
+    @property
+    def has_lens(self) -> bool:
+        return any(getattr(c, "lens_model", None) is not None for c in self.cameras)
+
+    def tables(self):
+        """Device tables of ``ldp_depth_consistency``: (map pointers int64 [V], P f32 [V, 12], scales f64 [V, 2], lens as the
+        bytes of ldp_lens [V] or None when every view is pinhole); built once per set of views."""
+        if self._tables is None:
+            V, dev = len(self.maps), self.device
+            ptrs = torch.tensor([m.data_ptr() for m in self.maps] or [0], dtype=torch.int64).to(dev)
+            P = np.zeros((max(V, 1), 12), np.float32)
+            S = np.zeros((max(V, 1), 2), np.float64)
+            for v, cam in enumerate(self.cameras):
+                P[v] = np.asarray(cam.P, dtype=np.float32).reshape(12)
+                S[v] = depth_map_scales(cam.width, cam.height, self.H, self.W, self.w_match, self.h_match)
+            lens = None
+            if self.has_lens:
+                arr = (N.LdpLens * V)(*[lens_of(c) for c in self.cameras])
+                lens = torch.frombuffer(bytearray(bytes(arr)), dtype=torch.uint8).to(dev)
+            self._tables = (ptrs, torch.from_numpy(P).to(dev), torch.from_numpy(S).to(dev), lens)
+        return self._tables
+
+
 class DensifyEngine:
     """Owns the scratch workspace and enqueues launches on the current torch CUDA stream."""
 

@@ -10,6 +10,8 @@ Mirrors, on tensors that stay on the GPU (SURVEY.md 8a row a15, 8f rows 2 and 4)
 * ``estimate_normals``                 not in the reference: oriented normals by PCA over the exact k nearest neighbours
 * ``init_gaussians`` / ``write_gaussian_ply``   not in the reference: 3DGS's ``create_from_pcd`` initialisation (scales from
   the exact nearest neighbours, optionally flattened along the normals) and its ``save_ply`` layout
+* ``check_depth_consistency``          not in the reference: MVS fusion's visibility test of a cloud against the reference
+  views' depth maps (``engine.DepthViews``)
 * ``apply_point_cap``                  reference densify.py:110-120 (the indices are numpy's own
   ``default_rng(seed).choice`` on the host - PCG64 + a sequential shuffle, microseconds; only the gather is device work)
 * ``subsample_preview_matches``        reference core/pipeline.py:573-582 (debug preview subsample of the kept matches)
@@ -421,6 +423,58 @@ def init_gaussians(xyz: torch.Tensor, rgb: torch.Tensor, *, normals: Optional[to
         raise ValueError("a coordinate is not finite")
     g.undefined = undefined
     return g
+
+
+@dataclass
+class DepthConsistency:
+    """What ``check_depth_consistency`` returns (device tensors)."""
+    kept_idx: torch.Tensor              # [m] int64, the kept points in ascending index (apply to every per-point array)
+    n_consistent: torch.Tensor          # [n] int32: other views whose depth agrees with the point
+    n_violations: torch.Tensor          # [n] int32: other views that see their surface behind the point (look through it)
+
+
+def check_depth_consistency(xyz: torch.Tensor, views, *, owner=None, rel_tol: float = 0.01, min_views: int = 1,
+                            max_violations: int = 0) -> DepthConsistency:
+    """MVS fusion's visibility test on a device cloud: every point is projected into every view of ``views``
+    (``engine.DepthViews``) but its own (``owner[i]``, the view index it came from, or -1; None = no owner) and compared
+    with the depth that view's map holds at the pixel.  A view whose depth agrees within ``rel_tol`` of it supports the
+    point; a view whose surface lies clearly behind the point looks through it (a violation).  The point is kept iff at
+    least ``min_views`` views support it and at most ``max_violations`` look through it.  The rule (f64 projection without
+    FMA, nearest map pixel) is in include/ldp_b200.h.  Raises on a non-finite coordinate or an owner outside [-1, V).
+    Synchronises once, to read the kept count."""
+    if not 0.0 < float(rel_tol) < 1.0:
+        raise ValueError("rel_tol must lie in (0, 1)")
+    if int(min_views) < 0 or int(max_violations) < 0:
+        raise ValueError("min_views and max_violations must be >= 0")
+    xyz = _f32c(xyz, "xyz")
+    lib, stream = _lib_and_stream(xyz)
+    if xyz.dim() != 2 or xyz.shape[1] != 3:
+        raise ValueError("xyz must be [n, 3]")
+    dev, n = xyz.device, int(xyz.shape[0])
+    if views.device != dev:
+        raise ValueError("the cloud and the depth maps must be on one device")
+    if owner is not None:
+        owner = torch.as_tensor(owner).to(device=dev, dtype=torch.int32).contiguous()
+        if tuple(owner.shape) != (n,):
+            raise ValueError("owner must hold one view index per point")
+    need = C.c_size_t(0)
+    N.check(lib.ldp_consistency_workspace_bytes(n, C.byref(need)), "ldp_consistency_workspace_bytes")
+    ws = torch.empty((max(1, need.value),), dtype=torch.uint8, device=dev)
+    kept = torch.empty((n,), dtype=torch.int64, device=dev)
+    nc = torch.empty((n,), dtype=torch.int32, device=dev)
+    nv = torch.empty((n,), dtype=torch.int32, device=dev)
+    status = torch.zeros((2,), dtype=torch.int32, device=dev)
+    ptrs, P, S, lens = views.tables()
+    ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)          # noqa: E731
+    N.check(lib.ldp_depth_consistency(ptr(xyz), n, ptr(owner), ptr(ptrs), views.H, views.W, ptr(P), ptr(S), ptr(lens), len(views),
+                                      float(rel_tol), int(min_views), int(max_violations), ptr(nc), ptr(nv), ptr(kept), ptr(status),
+                                      ptr(ws), C.c_size_t(need.value), C.c_void_p(stream)), "ldp_depth_consistency")
+    bad, m = (int(v) for v in status.cpu().tolist())
+    if bad & 1:
+        raise ValueError("a coordinate is not finite")
+    if bad & 2:
+        raise ValueError("an owner index is out of range")
+    return DepthConsistency(kept_idx=kept[:m], n_consistent=nc, n_violations=nv)
 
 
 def gaussian_record_bytes(sh_degree: int) -> int:

@@ -15,6 +15,9 @@ observed (distorted) pixel, through the inverse lens to its ray, through the dep
 neighbour's pinhole projection and through the neighbour's forward lens.  The lens arithmetic here is a torch f64
 statement of its own (fixed-point inversion for OpenCV, Newton on theta for the fisheye); without a lens nothing of it runs.
 
+``surface="sphere"`` replaces the per-view depth field by one world surface, a sphere about the orbit centre that fills
+every view: the reference views then see the same world, so their depth maps can be checked against each other.
+
 Everything is generated with torch on the requested device (CPU for tests, GPU for the bench).
 """
 from __future__ import annotations
@@ -108,6 +111,22 @@ def make_scene(n_views: int, setting: str = "fast", ref_fraction: float = 0.25, 
                       h_match=h_lr, w_match=h_lr, nn=nn_table.shape[1])
 
 
+SPHERE_RADIUS = 2.6        # surface="sphere": centred at the origin; from the orbit radius 4 it covers the whole field of view
+
+
+def sphere_depth(cam: CameraRecord, ray: torch.Tensor, radius: float = SPHERE_RADIUS) -> torch.Tensor:
+    """Camera z of the first hit of the rays ``ray`` [..., 3] (camera coordinates, z = 1) with the world sphere of ``radius``
+    about the origin, f64; NaN where a ray misses it."""
+    R = torch.from_numpy(cam.R.astype(np.float64)).to(ray.device)
+    C = torch.from_numpy(np.asarray(cam.C, dtype=np.float64).reshape(3)).to(ray.device)
+    d = ray.double() @ R                                          # R^T ray: the world direction per unit camera z
+    a = (d * d).sum(-1)
+    b = d @ C
+    c = float(C @ C) - radius * radius
+    disc = b * b - a * c
+    return torch.where(disc >= 0, (-b - torch.sqrt(disc.clamp(min=0.0))) / a, torch.full_like(a, float("nan")))
+
+
 def _gen(device, seed: int) -> torch.Generator:
     g = torch.Generator(device=device)
     g.manual_seed(int(seed))
@@ -165,8 +184,11 @@ def _undistort_t(lens, xd: torch.Tensor, yd: torch.Tensor):
 
 def synth_ref_inputs(scene: SynthScene, ref_pos: int, device="cpu", cert_family: str = "R",
                      seed: int = 0, noise_sigma: float = 1e-3, outlier_frac: float = 0.10,
-                     certainty_thresh: float = 0.20, return_points: bool = False) -> Dict[str, object]:
+                     certainty_thresh: float = 0.20, return_points: bool = False, surface: str = "field") -> Dict[str, object]:
     """Matcher-shaped inputs for the ``ref_pos``-th reference view of ``scene``.
+
+    ``surface``: "field" (default) gives every reference view an analytic depth field of its own; "sphere" ray-casts every
+    map pixel against the one world sphere of ``sphere_depth`` (a pixel whose ray misses it gets an outlier match).
 
     Returns dict(cert f32 [nn,H,W], warp f32 [nn,H,W,4], image u8 [h_match,w_match,3],
     ref_index, nbr_indices); with ``return_points`` also ``points`` f64 [H,W,3], the world point of every map pixel.
@@ -186,6 +208,8 @@ def synth_ref_inputs(scene: SynthScene, ref_pos: int, device="cpu", cert_family:
     # pixel coords the path will decode (reference core/pipeline.py:655-656,681-683), in f64
     xA = (gx.double() + 1.0) * 0.5 * (wm - 1) * (camA.width / float(wm))
     yA = (gy.double() + 1.0) * 0.5 * (hm - 1) * (camA.height / float(hm))
+    if surface not in ("field", "sphere"):
+        raise ValueError("surface must be 'field' or 'sphere'")
     depth = 3.6 + 0.5 * torch.sin(2.1 * gx.double() + 0.3 * ref_i) * torch.cos(1.7 * gy.double())
     Kinv = torch.from_numpy(np.linalg.inv(camA.K.astype(np.float64))).to(dev)
     RA = torch.from_numpy(camA.R.astype(np.float64)).to(dev)
@@ -193,11 +217,14 @@ def synth_ref_inputs(scene: SynthScene, ref_pos: int, device="cpu", cert_family:
     lensA = _lens_t(camA)
     if lensA is None:
         pix = torch.stack([xA, yA, torch.ones_like(xA)], dim=-1)                # [H,W,3]
-        Xc = (pix @ Kinv.T) * depth.unsqueeze(-1)
+        ray = pix @ Kinv.T
     else:                  # the matcher pixel is an observed (distorted) pixel: its ray is that of the undistorted one
         K64 = camA.K.astype(np.float64)
         xu, yu = _undistort_t(lensA, (xA - K64[0, 2]) / K64[0, 0], (yA - K64[1, 2]) / K64[1, 1])
-        Xc = torch.stack([xu, yu, torch.ones_like(xu)], dim=-1) * depth.unsqueeze(-1)
+        ray = torch.stack([xu, yu, torch.ones_like(xu)], dim=-1)
+    if surface == "sphere":
+        depth = sphere_depth(camA, ray)
+    Xc = ray * depth.unsqueeze(-1)
     Xw = (Xc - tA) @ RA                                                       # R^T (Xc - t)
 
     warp = torch.empty((len(nbrs), H, W, 4), dtype=torch.float32, device=dev)
@@ -221,7 +248,7 @@ def synth_ref_inputs(scene: SynthScene, ref_pos: int, device="cpu", cert_family:
         bad = torch.rand((H, W), generator=g, device=dev) < outlier_frac
         rx = torch.rand((H, W), generator=g, device=dev, dtype=torch.float64) * 2 - 1
         ry = torch.rand((H, W), generator=g, device=dev, dtype=torch.float64) * 2 - 1
-        if lensA is not None or lensB is not None:      # no valid inverse at this pixel: an outlier like the others
+        if lensA is not None or lensB is not None or surface == "sphere":   # no valid inverse / no surface: an outlier
             bad = bad | ~torch.isfinite(xBn) | ~torch.isfinite(yBn)
         xBn = torch.where(bad, rx, xBn)
         yBn = torch.where(bad, ry, yBn)
