@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define LDP_ABI_VERSION 20
+#define LDP_ABI_VERSION 21
 #define LDP_MAX_NN 16          /* neighbours per reference view (the panel clamps to 10) */
 #define LDP_MAX_BINS 4096      /* coverage tiles per map: ceil(W/tile)*ceil(H/tile), tile = max(1, W/24) */
 
@@ -475,6 +475,39 @@ int ldp_pack_gaussian_ply_records(const float* xyz, const float* normals, const 
  * the launch configuration.  Workspace: ldp_consistency_workspace_bytes(n). */
 int ldp_consistency_workspace_bytes(int64_t n, size_t* bytes_out);
 int ldp_depth_consistency(const float* xyz, int64_t n, const int32_t* owner, const float* const* depth_ptrs, int32_t H, int32_t W, const float* P, const double* scales, const ldp_lens* lens, int32_t n_views, double rel_tol, int32_t min_views, int32_t max_violations, int32_t* n_consistent_out, int32_t* n_violations_out, int64_t* kept_idx_out, int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- depth-map fusion (not in the reference) ----------------------------------------------------------------------------
+ * ldp_depth_colors: the colour maps of an ldp_depth_maps call.  params and refs as given to that call (the images are read),
+ * flags its flags output ([n_refs * H * W] u8, DEVICE).  For every pixel with flag bit 2 (kept): k = flag bits 4-7 (the winner
+ * slot; k >= the view's nn writes NaN), xA, yA decoded from neighbour k's warp row at the pixel, and the colour is the bilinear
+ * blend of the view's image at (xA * sx_img, yA * sy_img) that ldp_densify_refs computes for a sampled pixel (f64 weights,
+ * clipped corners, /255 correctly rounded, rounded to f32).  NaN elsewhere.  rgb_out: f32 [n_refs * H * W * 3] DEVICE.
+ * Consequence: at every sampled pixel that is kept, the colour is bit-identical to that launch's rgb.  Enqueues on `stream`.
+ *
+ * ldp_fuse_depth_maps: MVS fusion of V = n_views maps of one shape H x W, in the given order, into one cloud in which each
+ * surface point appears once.  Per view v, all DEVICE: depth_ptrs[v] (f32 [H*W], NaN = no depth), xyz_ptrs[v] (f32 [H*W*3]),
+ * rgb_ptrs[v] (f32 [H*W*3]) and err_ptrs[v] (f32 [H*W]), as ldp_depth_maps and ldp_depth_colors write them; P, scales and
+ * lens exactly as ldp_depth_consistency takes them (lens = NULL when every view is pinhole).  rel_tol in (0, 1),
+ * min_views >= 0, max_violations >= 0.  n_views * H * W < 2^31.
+ *   1. Verdict (pass 1).  Every pixel (r, i) with a finite depth is the point X = xyz[r, i] of view r.  It gets steps 1-3 of
+ *      ldp_depth_consistency against every view v != r (same f64 projection, same nearest map pixel j, same consistent /
+ *      violation / occluded verdicts).  kept(r, i) iff n_consistent >= min_views && n_violations <= max_violations.
+ *   2. Members.  For a kept (r, i), view v != r is a MEMBER iff its verdict in step 1 is consistent at map pixel j and
+ *      kept(v, j).
+ *   3. (r, i) is EMITTED iff it is kept and no member has v < r: each surface point comes out of the lowest view that holds a
+ *      kept pixel of it.
+ *   4. Fused values of an emitted (r, i): xyz and rgb are the f64 sums over (r, i) and its members, added one by one in
+ *      ascending view order, divided by members + 1 (correctly rounded) and rounded to f32 once; err = err[r, i];
+ *      n_views = members + 1; n_consistent = the count of step 1; source = r * H * W + i.
+ *   5. Output order: ascending source (view order, then pixel order).
+ * Outputs (DEVICE, capacity n_views * H * W entries, the first status_out[1] written): xyz_out f32 [.,3], rgb_out f32 [.,3],
+ * err_out f32, n_views_out int32, n_consistent_out int32, source_out int64.  status_out int32 [2] = {bit mask: 1 a non-finite
+ * xyz where the depth is finite, 2 a view whose depth, xyz, rgb or err pointer is NULL (with either bit nothing is emitted);
+ * emitted count}.  n_views = 0 zeroes status_out and writes nothing else.  No host synchronisation.  Results do not depend on
+ * the launch configuration.  Workspace: ldp_fuse_workspace_bytes (13 bytes per pixel). */
+int ldp_depth_colors(const ldp_params* params, const ldp_ref_desc* refs, const uint8_t* flags, float* rgb_out, void* stream);
+int ldp_fuse_workspace_bytes(int32_t n_views, int32_t H, int32_t W, size_t* bytes_out);
+int ldp_fuse_depth_maps(const float* const* depth_ptrs, const float* const* xyz_ptrs, const float* const* rgb_ptrs, const float* const* err_ptrs, int32_t n_views, int32_t H, int32_t W, const float* P, const double* scales, const ldp_lens* lens, double rel_tol, int32_t min_views, int32_t max_violations, float* xyz_out, float* rgb_out, float* err_out, int32_t* n_views_out, int32_t* n_consistent_out, int64_t* source_out, int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream);
 
 /* SMs the one-CTA-per-SM first draw kernel leaves free when ldp_params.sm_reserve is -1 (process-wide default, initially 0).
  * With several launches in flight on different streams (engine.DensifyRing) or a collective running beside the path, the

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(CSRC, "libldp_b200.so")
 SOURCES = ["ldp_api.cu"]                      # unity build: includes ldp_sample.cu / ldp_geometry.cu
-DEPS = ["ldp_api.cu", "ldp_sample.cu", "ldp_geometry.cu", "ldp_output.cu", "ldp_select.cu", "ldp_voxel.cu", "ldp_outlier.cu", "ldp_consistency.cu", "ldp_device.cuh", os.path.join("..", "..", "include", "ldp_b200.h")]
+DEPS = ["ldp_api.cu", "ldp_sample.cu", "ldp_geometry.cu", "ldp_output.cu", "ldp_select.cu", "ldp_voxel.cu", "ldp_outlier.cu", "ldp_consistency.cu", "ldp_fusion.cu", "ldp_device.cuh", os.path.join("..", "..", "include", "ldp_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
 

@@ -45,8 +45,9 @@ class PipelineResult:
     gaussians: Optional[Dict[str, np.ndarray]] = None   # extra, config.gaussian_neighbors: 3DGS's initial splats, f32
                                                   # sh_dc [n,3], opacity [n], scales [n,3] (log), rotations [n,4] (w, x, y, z)
     depth_paths: Optional[Dict[int, str]] = None  # extra, config.depth_dir: reference camera uid -> its depth map file
-    consistent_views: Optional[np.ndarray] = None  # extra, config.depth_consistency: int32 per point, the other reference
-                                                  # views whose depth maps agree with it
+    consistent_views: Optional[np.ndarray] = None  # extra, config.depth_consistency / depth_fusion: int32 per point, the other
+                                                  # reference views whose depth maps agree with it
+    fused_views: Optional[np.ndarray] = None      # extra, config.depth_fusion: int32 per point, the views averaged into it
 
 
 class PipelineCancelled(RuntimeError):
@@ -354,15 +355,17 @@ def submit_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triangulati
         u_dev = torch.from_numpy(np.ascontiguousarray(uniforms, dtype=np.float64)).to(dev)
         batch._keep_alive.append(u_dev)      # read by kernels on a ring stream: alive until the launch is collected, like the planes
     depth = None
-    want_depth = bool(getattr(cfg, "depth_dir", "")) or bool(getattr(cfg, "depth_consistency", False))
+    fusion = bool(getattr(cfg, "depth_fusion", False))
+    want_depth = bool(getattr(cfg, "depth_dir", "")) or bool(getattr(cfg, "depth_consistency", False)) or fusion
+    maps = dict(want_err=True, want_xyz=True, want_rgb=True) if fusion else {}
     if ring is None:
         out = eng.densify(batch, pcfg, uniforms=u_dev, collect_debug=collect_debug_matches)
         if want_depth:
-            depth = eng.depth_maps(batch, pcfg, float(cfg.depth_min_certainty))
+            depth = eng.depth_maps(batch, pcfg, float(cfg.depth_min_certainty), **maps)
     else:
         out = ring.submit(batch, pcfg, uniforms=u_dev, collect_debug=collect_debug_matches)
         if want_depth:
-            depth = ring.submit_depth_maps(batch, pcfg, float(cfg.depth_min_certainty))
+            depth = ring.submit_depth_maps(batch, pcfg, float(cfg.depth_min_certainty), **maps)
     return _PendingLaunch(out=out, batch=batch, n=n, collect_debug=collect_debug_matches, ply_records=ply_records, depth=depth,
                           ref_cams=ref_cams)
 
@@ -397,7 +400,8 @@ def collect_refs(pending: _PendingLaunch, errors: Optional[list] = None, ring=No
                  depth_paths: Optional[Dict[int, str]] = None, depth_kept: Optional[list] = None) -> List[Optional[_TriangulatedReference]]:
     """Second half: one synchronising read of the launch's results, split per view.  A launch with depth maps writes them
     under ``tri_ctx.config.depth_dir`` and records each file in ``depth_paths`` (reference camera uid -> path); with
-    ``depth_kept`` it appends (uid, device map [H, W], reference camera) for every view whose sampling succeeded."""
+    ``depth_kept`` it appends (uid, device map [H, W], reference camera, xyz, rgb, err maps or None) for every view whose
+    sampling succeeded."""
     out, batch = pending.out, pending.batch
     if ring is not None:
         ring.wait(out)                                 # the current stream (which does the read-back) follows the ring stream
@@ -426,7 +430,9 @@ def collect_refs(pending: _PendingLaunch, errors: Optional[list] = None, ring=No
                 ring.wait(pending.depth)           # the maps are read later on the current stream
             for r in range(pending.n):
                 if ok[r]:
-                    depth_kept.append((int(pending.batch.ref_uids[r]), pending.depth.depth[r], pending.ref_cams[r]))
+                    dm = pending.depth
+                    depth_kept.append((int(pending.batch.ref_uids[r]), dm.depth[r], pending.ref_cams[r],
+                                       *(None if t is None else t[r] for t in (dm.xyz, dm.rgb, dm.err))))
     triangulate_refs.last_launches = out.launches
     return results
 
@@ -691,7 +697,8 @@ def run_dense_pipeline(
     ring = get_ring() if (n_chunks > 1 and getattr(config, "rng_mode", RNG_PHILOX) != RNG_NUMPY_GLOBAL) else None
     in_flight: List[tuple] = []      # (views done when this launch is collected, launch, its matched references)
     depth_paths: Optional[Dict[int, str]] = {} if getattr(config, "depth_dir", "") else None
-    depth_kept: Optional[list] = [] if getattr(config, "depth_consistency", False) else None
+    fusion = bool(getattr(config, "depth_fusion", False))
+    depth_kept: Optional[list] = [] if (getattr(config, "depth_consistency", False) or fusion) else None
 
     def consume(outs, done: int, matched_refs) -> None:
         nonlocal pairs, ply_points, pair_counter
@@ -774,8 +781,16 @@ def run_dense_pipeline(
     xyz, rgb, err = np.concatenate(parts_xyz, axis=0), np.concatenate(parts_rgb, axis=0), np.concatenate(parts_err, axis=0)
     n_views = np.concatenate(parts_nv, axis=0) if getattr(config, "multiview", False) else None
     ref_uid = np.concatenate(parts_ref, axis=0)
-    consistent = None
-    if depth_kept is not None:
+    consistent = fused_views = None
+    if fusion:
+        # the fused maps replace the sampled cloud (its test includes depth_consistency's); the intermediate PLYs above stay
+        # those of the sampled path
+        if progress_callback:
+            progress_callback(93.0, "Fusing depth maps...")
+        xyz, rgb, err, ref_uid, fused_views, consistent = _fuse_depth_maps(depth_kept, tri_ctx)
+        depth_kept = None
+        n_views = None                         # the multiview counts belong to the sampled points
+    elif depth_kept is not None:
         # visibility test against the other reference views' maps, before the outlier filter, normals and Gaussians; the
         # intermediate PLYs above stay unfiltered
         if progress_callback:
@@ -806,6 +821,8 @@ def run_dense_pipeline(
             n_views = n_views[keep]
         if consistent is not None:
             consistent = consistent[keep]
+        if fused_views is not None:
+            fused_views = fused_views[keep]
     if k_nrm > 0:
         # every point faces the camera it was triangulated from (its reference view, a contributing view in every mode)
         if progress_callback:
@@ -826,7 +843,26 @@ def run_dense_pipeline(
                            opacity=float(config.gaussian_opacity), flatten=float(config.gaussian_flatten))
         gaussians = {name: getattr(g, name).cpu().numpy() for name in ("sh_dc", "opacity", "scales", "rotations")}
     return PipelineResult(xyz=xyz, rgb=rgb, err=err, elapsed_seconds=time.time() - t0, pairs_processed=pairs, n_views=n_views,
-                          normals=normals, gaussians=gaussians, depth_paths=depth_paths, consistent_views=consistent)
+                          normals=normals, gaussians=gaussians, depth_paths=depth_paths, consistent_views=consistent,
+                          fused_views=fused_views)
+
+
+def _fuse_depth_maps(depth_kept: list, tri_ctx: _TriangulationContext):
+    """``output.fuse_depth_maps`` of the kept maps (``collect_refs``), views in collection order.  Returns host arrays
+    (xyz, rgb, err, reference camera uid of each point's source view, n_views, n_consistent)."""
+    from ..engine import DepthViews
+    from ..output import fuse_depth_maps
+    cfg = tri_ctx.config
+    m0 = depth_kept[0][1]
+    views = DepthViews(int(m0.shape[0]), int(m0.shape[1]), tri_ctx.w_match, tri_ctx.h_match, m0.device)
+    for uid, depth, cam, xyz, rgb, err in depth_kept:
+        views.add(depth, cam, xyz=xyz, rgb=rgb, err=err)
+    f = fuse_depth_maps(views, rel_tol=float(cfg.consistency_rel_tol), min_views=int(cfg.consistency_min_views),
+                        max_violations=int(cfg.consistency_max_violations))
+    uids = np.array([e[0] for e in depth_kept], np.int64)
+    src_view = (f.source // (views.H * views.W)).cpu().numpy()
+    return (f.xyz.cpu().numpy(), f.rgb.cpu().numpy(), f.err.cpu().numpy(), uids[src_view], f.n_views.cpu().numpy(),
+            f.n_consistent.cpu().numpy())
 
 
 def _check_consistency(xyz: np.ndarray, ref_uid: np.ndarray, depth_kept: list, tri_ctx: _TriangulationContext):
@@ -838,7 +874,7 @@ def _check_consistency(xyz: np.ndarray, ref_uid: np.ndarray, depth_kept: list, t
     m0 = depth_kept[0][1]
     views = DepthViews(int(m0.shape[0]), int(m0.shape[1]), tri_ctx.w_match, tri_ctx.h_match, m0.device)
     index: Dict[int, int] = {}
-    for uid, depth, cam in depth_kept:
+    for uid, depth, cam, *_ in depth_kept:
         index[uid] = views.add(depth, cam)
     uids, inv = np.unique(ref_uid, return_inverse=True)
     owner = np.array([index.get(int(u), -1) for u in uids], dtype=np.int32)[inv.reshape(-1)]

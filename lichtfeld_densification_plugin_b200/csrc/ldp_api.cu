@@ -15,6 +15,7 @@
 #include "ldp_voxel.cu"
 #include "ldp_outlier.cu"
 #include "ldp_consistency.cu"
+#include "ldp_fusion.cu"
 
 namespace {
 
@@ -1394,6 +1395,105 @@ int ldp_depth_consistency(const float* xyz, int64_t n, const int32_t* owner, con
     const unsigned kgrid = (unsigned)((n + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
     return launch("ldp_outlier_kept_kernel", ldp::ldp_outlier_kept_kernel, dim3(kgrid), dim3(ldp::KV_THREADS), 0, st, (const int*)pl.flag,
                   (const int*)pl.rank, (long long)n, reinterpret_cast<long long*>(kept_idx_out));
+}
+
+// ---- depth-map fusion (ldp_fusion.cu; the compaction is the outlier filter's scan + ldp_outlier_kept_kernel).  Last in the
+// file for the reason given above the consistency check.
+int ldp_depth_colors(const ldp_params* params, const ldp_ref_desc* refs, const uint8_t* flags, float* rgb_out, void* stream) {
+    begin_call();
+    DepthPlan dp;
+    int rc = make_depth_plan(params, nullptr, &dp);
+    if (rc != LDP_OK) return rc;
+    if (params->n_refs == 0) return LDP_OK;
+    if (!refs || !flags || !rgb_out) return fail(LDP_ERR_INVALID, "null refs / flags / rgb_out");
+    const int R = params->n_refs, N = params->H * params->W;
+    const int tiles = (N + ldp::K2_THREADS - 1) / ldp::K2_THREADS;
+    const int per_view = std::max(1, std::min(tiles, (sm_count() * 16 + R - 1) / R));
+    KernelTimer kt(static_cast<cudaStream_t>(stream), "ldp_depth_color_kernel");
+    return launch("ldp_depth_color_kernel", ldp::ldp_depth_color_kernel, dim3((unsigned)per_view, (unsigned)R), dim3(ldp::K2_THREADS), 0,
+                  static_cast<cudaStream_t>(stream), *params, refs, flags, rgb_out, N);
+}
+
+struct FusionPlan {
+    uint8_t* kept;                         // [V*N] pass 1's keep flags
+    int* n_cons;                           // [V*N] pass 1's consistent counts
+    int* flag;                             // [V*N] emit flags
+    int* rank;                             // [V*N] their exclusive prefix
+    int* block_tot;                        // the scan's per-block totals
+};
+
+static int fusion_plan(int32_t n_views, int32_t H, int32_t W, void* base, FusionPlan* pl, size_t* bytes) {
+    if (n_views < 0 || H <= 0 || W <= 0 || (long long)H * W > 0x3fffffffLL) return fail(LDP_ERR_INVALID, "bad view count or map shape");
+    const long long total = (long long)n_views * H * W;
+    if (total >= (1ll << 31)) return fail(LDP_ERR_INVALID, "fusion: n_views * H * W must be below 2^31 (int32 ranks)");
+    const size_t T = (size_t)std::max<long long>(total, 1);
+    Carver c{static_cast<char*>(base)};
+    pl->kept = c.take<uint8_t>(T);
+    pl->n_cons = c.take<int>(T);
+    pl->flag = c.take<int>(T);
+    pl->rank = c.take<int>(T);
+    pl->block_tot = c.take<int>(T / ldp::SC_THREADS + 2);
+    *bytes = c.off;
+    return LDP_OK;
+}
+
+int ldp_fuse_workspace_bytes(int32_t n_views, int32_t H, int32_t W, size_t* bytes_out) {
+    if (!bytes_out) return fail(LDP_ERR_INVALID, "null bytes_out");
+    FusionPlan pl;
+    return fusion_plan(n_views, H, W, nullptr, &pl, bytes_out);
+}
+
+int ldp_fuse_depth_maps(const float* const* depth_ptrs, const float* const* xyz_ptrs, const float* const* rgb_ptrs,
+                        const float* const* err_ptrs, int32_t n_views, int32_t H, int32_t W, const float* P, const double* scales,
+                        const ldp_lens* lens, double rel_tol, int32_t min_views, int32_t max_violations, float* xyz_out,
+                        float* rgb_out, float* err_out, int32_t* n_views_out, int32_t* n_consistent_out, int64_t* source_out,
+                        int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream) {
+    begin_call();
+    if (!(rel_tol > 0.0 && rel_tol < 1.0)) return fail(LDP_ERR_INVALID, "rel_tol must lie in (0, 1)");
+    if (min_views < 0 || max_violations < 0) return fail(LDP_ERR_INVALID, "min_views and max_violations must be >= 0");
+    FusionPlan pl;
+    size_t need = 0;
+    int rc = fusion_plan(n_views, H, W, nullptr, &pl, &need);
+    if (rc != LDP_OK) return rc;
+    if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    rc = check(cudaMemsetAsync(status_out, 0, 2 * sizeof(int32_t), st), "cudaMemsetAsync(status)");
+    if (rc != LDP_OK || n_views == 0) return rc;
+    if (!depth_ptrs || !xyz_ptrs || !rgb_ptrs || !err_ptrs || !P || !scales) return fail(LDP_ERR_INVALID, "null view table");
+    if (!xyz_out || !rgb_out || !err_out || !n_views_out || !n_consistent_out || !source_out || !workspace)
+        return fail(LDP_ERR_INVALID, "null output or workspace");
+    if ((rc = fusion_plan(n_views, H, W, workspace, &pl, &need)) != LDP_OK) return rc;
+    if (workspace_bytes < need) return fail(LDP_ERR_WORKSPACE, "fusion workspace too small");
+    const long long total = (long long)n_views * H * W;
+    const ldp::FusionArgs a{depth_ptrs, xyz_ptrs, rgb_ptrs, err_ptrs, P, scales, lens, pl.kept, pl.n_cons, pl.flag,
+                            reinterpret_cast<const long long*>(source_out), xyz_out, rgb_out, err_out, (int*)n_views_out,
+                            (int*)n_consistent_out, (int*)status_out, total, rel_tol, (int)n_views, (int)H, (int)W, (int)(H * W),
+                            (int)min_views, (int)max_violations};
+    rc = launch("ldp_fusion_check_kernel", ldp::ldp_fusion_check_kernel, dim3((unsigned)((n_views + ldp::CS_THREADS - 1) / ldp::CS_THREADS)),
+                dim3(ldp::CS_THREADS), 0, st, a);
+    if (rc != LDP_OK) return rc;
+    // a few resident CTAs per SM; each strides over the maps, so a table of one chunk is staged once per CTA
+    const unsigned grid = (unsigned)std::min<long long>((total + ldp::CS_THREADS - 1) / ldp::CS_THREADS, (long long)sm_count() * 8);
+    {
+        KernelTimer kt(st, "ldp_fusion_verdict_kernel");
+        rc = launch("ldp_fusion_verdict_kernel", lens ? ldp::ldp_fusion_verdict_kernel<true> : ldp::ldp_fusion_verdict_kernel<false>,
+                    dim3(grid), dim3(ldp::CS_THREADS), 0, st, a);
+        if (rc != LDP_OK) return rc;
+    }
+    {
+        KernelTimer kt(st, "ldp_fusion_emit_kernel");
+        rc = launch("ldp_fusion_emit_kernel", lens ? ldp::ldp_fusion_emit_kernel<true> : ldp::ldp_fusion_emit_kernel<false>,
+                    dim3(grid), dim3(ldp::CS_THREADS), 0, st, a);
+        if (rc != LDP_OK) return rc;
+    }
+    if ((rc = scan_exclusive(pl.flag, pl.rank, total, pl.block_tot, (int*)status_out + 1, st)) != LDP_OK) return rc;
+    const unsigned kgrid = (unsigned)((total + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
+    rc = launch("ldp_outlier_kept_kernel", ldp::ldp_outlier_kept_kernel, dim3(kgrid), dim3(ldp::KV_THREADS), 0, st, (const int*)pl.flag,
+                (const int*)pl.rank, total, reinterpret_cast<long long*>(source_out));
+    if (rc != LDP_OK) return rc;
+    KernelTimer kt(st, "ldp_fusion_sum_kernel");
+    return launch("ldp_fusion_sum_kernel", lens ? ldp::ldp_fusion_sum_kernel<true> : ldp::ldp_fusion_sum_kernel<false>, dim3(grid),
+                  dim3(ldp::CS_THREADS), 0, st, a);
 }
 
 }  // extern "C"

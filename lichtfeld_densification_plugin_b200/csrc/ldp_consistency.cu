@@ -57,6 +57,34 @@ __device__ __forceinline__ double cons_row(const float* p, double X, double Y, d
                      (double)p[3]);
 }
 
+// Steps 1-3 of the rule for one point (X, Y, Z) and one view (its P rows p, map scales s, map D, lens L): ++nc where the view
+// supports the point, ++nv where it looks through it; returns true iff it supports it, and then pix is the map pixel.
+// Shared by ldp_consistency_kernel and the fusion kernels (ldp_fusion.cu), so both apply one test.
+template <bool LENS>
+__device__ __forceinline__ bool cons_test(const float* p, const double* s, const float* D, const ldp_lens& L, double X, double Y,
+                                          double Z, int W, int H, double rel_tol, int& nc, int& nv, size_t& pix) {
+    const double z = cons_row(p + 8, X, Y, Z);
+    if (!(z > 0.0)) return false;
+    double u = __ddiv_rn(cons_row(p, X, Y, Z), z), v = __ddiv_rn(cons_row(p + 4, X, Y, Z), z);
+    if constexpr (LENS) {
+        if (L.model != LDP_LENS_PINHOLE) {
+            const double fx = L.fx, fy = L.fy, cx = L.cx, cy = L.cy;
+            double xd, yd;
+            lens_distort(L, (u - cx) / fx, (v - cy) / fy, xd, yd);
+            u = fx * xd + cx; v = fy * yd + cy;
+        }
+    }
+    const double fxm = floor(__dmul_rn(u, s[0])), fym = floor(__dmul_rn(v, s[1]));
+    if (!(fxm >= 0.0 && fxm < (double)W && fym >= 0.0 && fym < (double)H)) return false;
+    pix = (size_t)fym * (size_t)W + (size_t)fxm;
+    const double Dp = (double)__ldg(D + pix);
+    if (!(Dp > 0.0)) return false;               // NaN (no depth) or not in front: no evidence
+    const double d = __dsub_rn(z, Dp), t = __dmul_rn(rel_tol, Dp);
+    if (fabs(d) <= t) { ++nc; return true; }
+    if (d < -t) ++nv;
+    return false;
+}
+
 template <bool LENS>
 __global__ void __launch_bounds__(CS_THREADS)
 ldp_consistency_kernel(const ConsistencyArgs a)
@@ -103,26 +131,8 @@ ldp_consistency_kernel(const ConsistencyArgs a)
             if (!live) continue;
             for (int j = 0; j < cn; ++j) {
                 if (c0 + j == own) continue;           // a point is never checked against the view it came from
-                const float* p = s_P[j];
-                const double z = cons_row(p + 8, X, Y, Z);
-                if (!(z > 0.0)) continue;
-                double u = __ddiv_rn(cons_row(p, X, Y, Z), z), v = __ddiv_rn(cons_row(p + 4, X, Y, Z), z);
-                if constexpr (LENS) {
-                    const ldp_lens& L = s_L[j];
-                    if (L.model != LDP_LENS_PINHOLE) {
-                        const double fx = L.fx, fy = L.fy, cx = L.cx, cy = L.cy;
-                        double xd, yd;
-                        lens_distort(L, (u - cx) / fx, (v - cy) / fy, xd, yd);
-                        u = fx * xd + cx; v = fy * yd + cy;
-                    }
-                }
-                const double fxm = floor(__dmul_rn(u, s_S[j][0])), fym = floor(__dmul_rn(v, s_S[j][1]));
-                if (!(fxm >= 0.0 && fxm < (double)W && fym >= 0.0 && fym < (double)H)) continue;
-                const double D = (double)__ldg(s_D[j] + ((size_t)fym * (size_t)W + (size_t)fxm));
-                if (!(D > 0.0)) continue;                // NaN (no depth) or not in front: no evidence
-                const double d = __dsub_rn(z, D), t = __dmul_rn(a.rel_tol, D);
-                if (fabs(d) <= t) ++nc;
-                else if (d < -t) ++nv;
+                size_t pix;
+                cons_test<LENS>(s_P[j], s_S[j], s_D[j], s_L[LENS ? j : 0], X, Y, Z, W, H, a.rel_tol, nc, nv, pix);
             }
         }
         if (live) {

@@ -560,6 +560,27 @@ __device__ __forceinline__ void gather_sample(const ldp_params& P, const RefCons
     rec.k_cert = (uint32_t)k;
 }
 
+// bilinear blend of the four texels at image position (fx, fy) with clipped corners (core/pipeline.py:661-679): f64 weights,
+// left-to-right sum like the reference; /255.0 as an FMA-corrected reciprocal multiply.  Shared by eval_sample and the colour
+// maps (ldp_depth_colors), so a kept map pixel gets the colour of a sampled pixel with the same winner.
+__device__ __forceinline__ void bilinear_rgb(float fx, float fy, int x0, int y0, int x1, int y1, const float t00[3], const float t01[3],
+                                             const float t10[3], const float t11[3], float col[3]) {
+    const double dfx = (double)fx, dfy = (double)fy;
+    const double ax = __dsub_rn((double)x1, dfx), bx = __dsub_rn(dfx, (double)x0);
+    const double ay = __dsub_rn((double)y1, dfy), by = __dsub_rn(dfy, (double)y0);
+    const double w00 = __dmul_rn(ax, ay), w01 = __dmul_rn(bx, ay), w10 = __dmul_rn(ax, by), w11 = __dmul_rn(bx, by);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        double acc = __dmul_rn((double)t00[c], w00);
+        acc = __dadd_rn(acc, __dmul_rn((double)t01[c], w01));
+        acc = __dadd_rn(acc, __dmul_rn((double)t10[c], w10));
+        acc = __dadd_rn(acc, __dmul_rn((double)t11[c], w11));
+        const double q0 = acc * (1.0 / 255.0);
+        const double rr = fma(-q0, 255.0, acc);
+        col[c] = (float)fma(rr, 1.0 / 255.0, q0);                                 // == acc / 255.0 rounded; .astype(f32) at :754
+    }
+}
+
 // ---- compute: everything else the reference computes for one sampled pixel (core/pipeline.py:653-769)
 // LENS: the launch has lens cameras (ldp_params.lens); lt = the view's staged lens table, [0] reference camera, [1 + k]
 // neighbour k.  A lens camera's observed pixels are undistorted before the Sampson gate and the DLT, and its reprojection
@@ -621,22 +642,9 @@ __device__ __forceinline__ void eval_sample(const ldp_params& P, const RefConst&
         if (!(n2 == n2) || !(den == den)) o.good = 0;                            // NaN: comparison is False in numpy
     }
 
-    {   // bilinear blend, f64, left-to-right sum like the reference; /255.0 as an FMA-corrected reciprocal multiply
-        const double dfx = (double)fx, dfy = (double)fy;
-        const double ax = __dsub_rn((double)x1, dfx), bx = __dsub_rn(dfx, (double)x0);
-        const double ay = __dsub_rn((double)y1, dfy), by = __dsub_rn(dfy, (double)y0);
-        const double w00 = __dmul_rn(ax, ay), w01 = __dmul_rn(bx, ay), w10 = __dmul_rn(ax, by), w11 = __dmul_rn(bx, by);
+    {
         float col[3];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            double acc = __dmul_rn((double)t00[c], w00);
-            acc = __dadd_rn(acc, __dmul_rn((double)t01[c], w01));
-            acc = __dadd_rn(acc, __dmul_rn((double)t10[c], w10));
-            acc = __dadd_rn(acc, __dmul_rn((double)t11[c], w11));
-            const double q0 = acc * (1.0 / 255.0);
-            const double rr = fma(-q0, 255.0, acc);
-            col[c] = (float)fma(rr, 1.0 / 255.0, q0);                             // == acc / 255.0 rounded; .astype(f32) at :754
-        }
+        bilinear_rgb(fx, fy, x0, y0, x1, y1, t00, t01, t10, t11, col);
         o.cr = col[0]; o.cg = col[1]; o.cb = col[2];
     }
 

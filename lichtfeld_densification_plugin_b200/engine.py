@@ -333,6 +333,7 @@ class DepthMaps:
     err: Optional[torch.Tensor] = None        # f32 [R, H, W]: reprojection error where triangulated, NaN elsewhere
     xyz: Optional[torch.Tensor] = None        # f32 [R, H, W, 3]: world point where kept, NaN elsewhere
     flags: Optional[torch.Tensor] = None      # u8 [R, H, W]: bit 0 candidate, 1 Sampson pass, 2 kept, bits 4-7 winning slot
+    rgb: Optional[torch.Tensor] = None        # f32 [R, H, W, 3]: colour of the kept pixel (ldp_depth_colors), NaN elsewhere
     ready: Optional[torch.cuda.Event] = None  # DensifyRing.submit_depth_maps: recorded on the ring stream after the launch
 
 
@@ -364,25 +365,38 @@ class DepthViews:
         depth_map_scales(1, 1, self.H, self.W, self.w_match, self.h_match)         # validates the matcher size
         self.maps: List[torch.Tensor] = []
         self.cameras: List[CameraRecord] = []
+        self.xyz: List[Optional[torch.Tensor]] = []      # per view, what fusion needs beside the depth (None where not given)
+        self.rgb: List[Optional[torch.Tensor]] = []
+        self.err: List[Optional[torch.Tensor]] = []
         self._tables = None
+        self._fusion_tables = None
 
     def __len__(self) -> int:
         return len(self.maps)
 
-    def add(self, depth, camera: CameraRecord) -> int:
+    def add(self, depth, camera: CameraRecord, *, xyz=None, rgb=None, err=None) -> int:
         """Append one view: its f32 [H, W] map (a device tensor or a host array; NaN = no depth) and the ``CameraRecord`` its
         map was made with (the P1 and lens of the launch, its full-resolution width and height).  Returns the view index,
-        the value ``owner`` takes for the points of this view."""
-        if isinstance(depth, np.ndarray):
-            depth = torch.from_numpy(np.ascontiguousarray(depth, dtype=np.float32)).to(self.device)
-        if not isinstance(depth, torch.Tensor) or depth.device != self.device or depth.dtype != torch.float32 \
-                or tuple(depth.shape) != (self.H, self.W):
-            raise ValueError(f"a depth map must be a float32 ({self.H}, {self.W}) tensor on {self.device} or a host array")
+        the value ``owner`` takes for the points of this view.  ``xyz`` / ``rgb`` ([H, W, 3]) and ``err`` ([H, W]), f32 like the
+        map (``DepthMaps.xyz`` / ``.rgb`` / ``.err`` of the view): what ``output.fuse_depth_maps`` needs beside the depth."""
+        depth = self._map(depth, (self.H, self.W), "a depth map")
+        xyz, rgb, err = (None if t is None else self._map(t, shape, what) for t, shape, what in
+                         ((xyz, (self.H, self.W, 3), "xyz"), (rgb, (self.H, self.W, 3), "rgb"), (err, (self.H, self.W), "err")))
         check_lens(camera)
-        self.maps.append(depth.contiguous())
+        self.maps.append(depth)
         self.cameras.append(camera)
-        self._tables = None
+        self.xyz.append(xyz)
+        self.rgb.append(rgb)
+        self.err.append(err)
+        self._tables = self._fusion_tables = None
         return len(self.maps) - 1
+
+    def _map(self, t, shape, what: str) -> torch.Tensor:
+        if isinstance(t, np.ndarray):
+            t = torch.from_numpy(np.ascontiguousarray(t, dtype=np.float32)).to(self.device)
+        if not isinstance(t, torch.Tensor) or t.device != self.device or t.dtype != torch.float32 or tuple(t.shape) != shape:
+            raise ValueError(f"{what} must be a float32 {shape} tensor on {self.device} or a host array")
+        return t.contiguous()
 
     @classmethod
     def from_depth_dir(cls, depth_dir: str, cameras: Sequence[CameraRecord], device=None) -> "DepthViews":
@@ -430,6 +444,23 @@ class DepthViews:
                 lens = torch.frombuffer(bytearray(bytes(arr)), dtype=torch.uint8).to(dev)
             self._tables = (ptrs, torch.from_numpy(P).to(dev), torch.from_numpy(S).to(dev), lens)
         return self._tables
+
+    def fusion_tables(self):
+        """Device tables of ``ldp_fuse_depth_maps`` beside ``tables()``: pointers to each view's xyz, rgb and err maps (int64
+        [V] each).  Raises if a view lacks one of them."""
+        if self._fusion_tables is None:
+            for v in range(len(self.maps)):
+                missing = [n for n, t in (("xyz", self.xyz[v]), ("rgb", self.rgb[v])) if t is None]
+                if missing:
+                    raise ValueError(f"view {v} has no {' / '.join(missing)} map: fusion needs the xyz and rgb maps of every view "
+                                     "(DepthViews.add(..., xyz=, rgb=, err=) with the device maps of DensifyEngine.depth_maps; "
+                                     "the .npy files of depth_dir hold depth only and cannot be fused)")
+            for v in range(len(self.maps)):                   # without err maps the fused err is NaN
+                if self.err[v] is None:
+                    self.err[v] = torch.full((self.H, self.W), float("nan"), dtype=torch.float32, device=self.device)
+            ptrs = lambda ts: torch.tensor([t.data_ptr() for t in ts] or [0], dtype=torch.int64).to(self.device)  # noqa: E731
+            self._fusion_tables = (ptrs(self.xyz), ptrs(self.rgb), ptrs(self.err))
+        return self._fusion_tables
 
 
 class DensifyEngine:
@@ -541,10 +572,11 @@ class DensifyEngine:
         return self.prepare(batch, cfg, uniforms, collect_debug, taps, descs_dev, outputs).launch()
 
     def depth_maps(self, batch: RefBatch, cfg: PathConfig, min_certainty: float, want_err: bool = False,
-                   want_xyz: bool = False, want_flags: bool = False) -> DepthMaps:
+                   want_xyz: bool = False, want_flags: bool = False, want_rgb: bool = False) -> DepthMaps:
         """``ldp_depth_maps``: every pixel of every view of ``batch`` whose best certainty is >= ``min_certainty`` (in (0, 1])
-        triangulated and filtered as a sampled pixel with the same winner is by ``densify(batch, cfg)``.  Enqueued on the
-        current torch stream."""
+        triangulated and filtered as a sampled pixel with the same winner is by ``densify(batch, cfg)``.  ``want_rgb``: also
+        the colour maps (``ldp_depth_colors``: a kept pixel's colour is that of a sampled pixel with the same winner); they
+        need the flags, which are then returned too.  Enqueued on the current torch stream."""
         if not 0.0 < float(min_certainty) <= 1.0:
             raise ValueError("min_certainty must lie in (0, 1]")
         R, H, W = len(batch), batch.H, batch.W
@@ -554,7 +586,8 @@ class DensifyEngine:
         out = DepthMaps(depth=torch.empty((R, H, W), **f32), kept=torch.zeros((R,), dtype=torch.int64, device=dev),
                         err=torch.empty((R, H, W), **f32) if want_err else None,
                         xyz=torch.empty((R, H, W, 3), **f32) if want_xyz else None,
-                        flags=torch.empty((R, H, W), dtype=torch.uint8, device=dev) if want_flags else None)
+                        flags=torch.empty((R, H, W), dtype=torch.uint8, device=dev) if (want_flags or want_rgb) else None,
+                        rgb=torch.empty((R, H, W, 3), **f32) if want_rgb else None)
         if R == 0:
             return out
         need = C.c_size_t(0)
@@ -569,6 +602,9 @@ class DensifyEngine:
         rc = self.lib.ldp_depth_maps(C.byref(params), ptr(descs), float(min_certainty), ptr(out.depth), ptr(out.err), ptr(out.xyz),
                                      ptr(out.flags), ptr(out.kept), ptr(ws), C.c_size_t(ws.numel()), C.c_void_p(stream))
         N.check(rc, "ldp_depth_maps")
+        if want_rgb:
+            N.check(self.lib.ldp_depth_colors(C.byref(params), ptr(descs), ptr(out.flags), ptr(out.rgb), C.c_void_p(stream)),
+                    "ldp_depth_colors")
         out._keep = (descs, batch)          # read by the kernels: alive until the stream is done with them
         return out
 

@@ -12,6 +12,8 @@ Mirrors, on tensors that stay on the GPU (SURVEY.md 8a row a15, 8f rows 2 and 4)
   the exact nearest neighbours, optionally flattened along the normals) and its ``save_ply`` layout
 * ``check_depth_consistency``          not in the reference: MVS fusion's visibility test of a cloud against the reference
   views' depth maps (``engine.DepthViews``)
+* ``fuse_depth_maps``                  not in the reference: MVS fusion of the reference views' depth maps into one dense
+  coloured cloud, each surface point emitted once and averaged over the views that agree with it
 * ``apply_point_cap``                  reference densify.py:110-120 (the indices are numpy's own
   ``default_rng(seed).choice`` on the host - PCG64 + a sequential shuffle, microseconds; only the gather is device work)
 * ``subsample_preview_matches``        reference core/pipeline.py:573-582 (debug preview subsample of the kept matches)
@@ -475,6 +477,62 @@ def check_depth_consistency(xyz: torch.Tensor, views, *, owner=None, rel_tol: fl
     if bad & 2:
         raise ValueError("an owner index is out of range")
     return DepthConsistency(kept_idx=kept[:m], n_consistent=nc, n_violations=nv)
+
+
+@dataclass
+class FusedCloud:
+    """What ``fuse_depth_maps`` returns (device tensors, one row per emitted point, ascending ``source``).  ``write_ply`` and
+    ``write_points3D_bin`` take ``xyz`` / ``rgb`` (/ ``err``) like any other cloud."""
+    xyz: torch.Tensor                   # [m, 3] f32: mean of the point and its members
+    rgb: torch.Tensor                   # [m, 3] f32: mean colour, in [0, 1]
+    err: torch.Tensor                   # [m] f32: reprojection error of the emitting pixel
+    n_views: torch.Tensor               # [m] int32: views averaged (members + 1)
+    n_consistent: torch.Tensor          # [m] int32: other views whose depth agrees with the emitting pixel
+    source: torch.Tensor                # [m] int64: emitting pixel, view * H * W + pixel index
+
+
+def fuse_depth_maps(views, *, rel_tol: float = 0.01, min_views: int = 1, max_violations: int = 0) -> FusedCloud:
+    """MVS fusion of the maps of ``views`` (``engine.DepthViews`` whose views carry xyz and rgb maps) into one cloud in which
+    each surface point appears once: a pixel is kept iff at least ``min_views`` other views agree with its depth (within
+    ``rel_tol``) and at most ``max_violations`` look through it (``check_depth_consistency``'s test); a kept pixel is
+    emitted iff no lower view holds a kept pixel that agrees with it, and its xyz and rgb are averaged over itself and the
+    kept pixels of the views that agree with it.  The rule is in include/ldp_b200.h (ldp_fuse_depth_maps).  Raises on a
+    view without xyz or rgb maps and on a non-finite xyz where the depth is finite.  Synchronises once, to read the
+    emitted count."""
+    if not 0.0 < float(rel_tol) < 1.0:
+        raise ValueError("rel_tol must lie in (0, 1)")
+    if int(min_views) < 0 or int(max_violations) < 0:
+        raise ValueError("min_views and max_violations must be >= 0")
+    dev = views.device
+    if dev.type != "cuda":
+        raise N.NativeLibraryError("fusion runs on a CUDA device (there is no CPU fallback)")
+    V, H, W = len(views), views.H, views.W
+    if V * H * W >= 2 ** 31:
+        raise ValueError("fusion needs n_views * H * W < 2^31")
+    xyz_p, rgb_p, err_p = views.fusion_tables()
+    lib, stream = N.load(), torch.cuda.current_stream(dev).cuda_stream
+    need = C.c_size_t(0)
+    N.check(lib.ldp_fuse_workspace_bytes(V, H, W, C.byref(need)), "ldp_fuse_workspace_bytes")
+    ws = torch.empty((max(1, need.value),), dtype=torch.uint8, device=dev)
+    cap = max(1, V * H * W)
+    f32 = dict(dtype=torch.float32, device=dev)
+    xyz, rgb, err = torch.empty((cap, 3), **f32), torch.empty((cap, 3), **f32), torch.empty((cap,), **f32)
+    nv, nc = torch.empty((cap,), dtype=torch.int32, device=dev), torch.empty((cap,), dtype=torch.int32, device=dev)
+    src = torch.empty((cap,), dtype=torch.int64, device=dev)
+    status = torch.zeros((2,), dtype=torch.int32, device=dev)
+    ptrs, P, S, lens = views.tables()
+    ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)          # noqa: E731
+    N.check(lib.ldp_fuse_depth_maps(ptr(ptrs), ptr(xyz_p), ptr(rgb_p), ptr(err_p), V, H, W, ptr(P), ptr(S), ptr(lens), float(rel_tol),
+                                    int(min_views), int(max_violations), ptr(xyz), ptr(rgb), ptr(err), ptr(nv), ptr(nc), ptr(src),
+                                    ptr(status), ptr(ws), C.c_size_t(need.value), C.c_void_p(stream)), "ldp_fuse_depth_maps")
+    bad, m = (int(v) for v in status.cpu().tolist())
+    if bad & 1:
+        raise ValueError("a view's xyz map is not finite where its depth is")
+    if bad & 2:
+        raise ValueError("a view's map pointer is NULL")
+    # copies of the first m rows: the capacity (one row per map pixel) is released
+    return FusedCloud(xyz=xyz[:m].clone(), rgb=rgb[:m].clone(), err=err[:m].clone(), n_views=nv[:m].clone(),
+                      n_consistent=nc[:m].clone(), source=src[:m].clone())
 
 
 def gaussian_record_bytes(sh_degree: int) -> int:
