@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define LDP_ABI_VERSION 21
+#define LDP_ABI_VERSION 22
 #define LDP_MAX_NN 16          /* neighbours per reference view (the panel clamps to 10) */
 #define LDP_MAX_BINS 4096      /* coverage tiles per map: ceil(W/tile)*ceil(H/tile), tile = max(1, W/24) */
 
@@ -508,6 +508,40 @@ int ldp_depth_consistency(const float* xyz, int64_t n, const int32_t* owner, con
 int ldp_depth_colors(const ldp_params* params, const ldp_ref_desc* refs, const uint8_t* flags, float* rgb_out, void* stream);
 int ldp_fuse_workspace_bytes(int32_t n_views, int32_t H, int32_t W, size_t* bytes_out);
 int ldp_fuse_depth_maps(const float* const* depth_ptrs, const float* const* xyz_ptrs, const float* const* rgb_ptrs, const float* const* err_ptrs, int32_t n_views, int32_t H, int32_t W, const float* P, const double* scales, const ldp_lens* lens, double rel_tol, int32_t min_views, int32_t max_violations, float* xyz_out, float* rgb_out, float* err_out, int32_t* n_views_out, int32_t* n_consistent_out, int64_t* source_out, int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- normal maps and oriented fusion (not in the reference) -------------------------------------------------------------
+ * ldp_depth_normals: one oriented normal per map pixel, from the pixel's depth-continuous map window.  V = n_views maps of
+ * one shape H x W; per view v, DEVICE: depth_ptrs[v] (f32 [H*W], NaN = no depth) and xyz_ptrs[v] (f32 [H*W*3]) as
+ * ldp_depth_maps writes them; centers f32 [V,3] DEVICE, each view's camera centre.  radius in [1, 3], rel_tol in (0, 1).
+ * For every pixel p = (y, x) of view v whose depth D_p is finite:
+ *   1. Neighbourhood: the pixels q = (y + dy, x + dx), dy and dx in [-radius, radius], in row-major order (dy ascending, then
+ *      dx ascending), that lie inside the map, have a finite D_q and satisfy |D_q - D_p| <= rel_tol * D_p, in f64 without
+ *      FMA (cons_test's depth test: d = D_q - D_p and t = rel_tol * D_p each rounded once).  p itself qualifies (D_p > 0).
+ *      k = their count.
+ *   2. Normal: steps 2-5 of ldp_estimate_normals' rule over their xyz in that order (two-pass f64 covariance without FMA,
+ *      cyclic Jacobi, undefined when k < 3, trace 0 or l1 <= 1e-12 * l2, canonical sign, then flipped to face centers[v]
+ *      from xyz_p) - the same device function.
+ *   3. Outputs: the normal rounded to f32, curvature l0 / ((l0 + l1) + l2) rounded to f32.  Where the depth is not finite
+ *      or the normal is undefined, normal and curvature are NaN.
+ * normals_out f32 [V*H*W*3] DEVICE; curvature_out f32 [V*H*W] DEVICE or NULL.  status_out int32 [2] DEVICE = {bit mask:
+ * 1 a non-finite xyz where the depth is finite, 2 a NULL map pointer (with either bit nothing else is written); pixels
+ * with a finite depth and an undefined normal}.  n_views * H * W < 2^31, n_views <= 65535.  n_views = 0 zeroes status_out
+ * and writes nothing else.  No host synchronisation.  Results do not depend on the launch configuration.
+ *
+ * ldp_fuse_depth_maps_oriented: ldp_fuse_depth_maps with COLMAP fusion's normal test.  Arguments as there, plus
+ * normal_ptrs[v] (f32 [H*W*3] DEVICE, e.g. ldp_depth_normals' output; NaN = no normal), cos_max in (0, 1) and normals_out
+ * f32 [capacity, 3] DEVICE.  The rule is ldp_fuse_depth_maps' with two changes:
+ *   a. Verdict.  For the pixel (r, i) with normal n and view v, the verdict at map pixel j is consistent iff the depth test
+ *      says consistent, m = the normal of (v, j) is finite and ((n0 m0 + n1 m1) + n2 m2) >= cos_max in f64 without FMA
+ *      (the products of f32 values are exact).  A view whose depth agrees and whose normal does not counts for nothing
+ *      (neither consistent nor a violation); violations are unchanged.  A pixel whose own normal is not finite is not kept.
+ *      This verdict is the one of step 1 (n_consistent, kept), of membership (step 2) and so of emission (step 3).
+ *   b. Fused normal: s = the f64 sum of the normals of (r, i) and its members, added one by one in ascending view order;
+ *      normals_out = f32(s / sqrt((sx^2 + sy^2) + sz^2)), the length in f64 without FMA and the division correctly rounded.
+ *      s is not 0: every member passed the angle test against (r, i) and cos_max > 0.
+ * Status bit 2 also marks a NULL normal map pointer.  Workspace: ldp_fuse_workspace_bytes. */
+int ldp_depth_normals(const float* const* depth_ptrs, const float* const* xyz_ptrs, int32_t n_views, int32_t H, int32_t W, const float* centers, int32_t radius, double rel_tol, float* normals_out, float* curvature_out, int32_t* status_out, void* stream);
+int ldp_fuse_depth_maps_oriented(const float* const* depth_ptrs, const float* const* xyz_ptrs, const float* const* rgb_ptrs, const float* const* err_ptrs, const float* const* normal_ptrs, int32_t n_views, int32_t H, int32_t W, const float* P, const double* scales, const ldp_lens* lens, double rel_tol, double cos_max, int32_t min_views, int32_t max_violations, float* xyz_out, float* rgb_out, float* err_out, float* normals_out, int32_t* n_views_out, int32_t* n_consistent_out, int64_t* source_out, int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream);
 
 /* SMs the one-CTA-per-SM first draw kernel leaves free when ldp_params.sm_reserve is -1 (process-wide default, initially 0).
  * With several launches in flight on different streams (engine.DensifyRing) or a collective running beside the path, the

@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-LDP_ABI_VERSION = 21
+LDP_ABI_VERSION = 22
 LDP_MAX_NN = 16
 LDP_MAX_BINS = 4096
 
@@ -148,6 +148,9 @@ SIGNATURES = {
     "ldp_depth_colors": (C.c_int, [_P, _P, _P, _P, _P]),
     "ldp_fuse_workspace_bytes": (C.c_int, [_I32, _I32, _I32, _SZ_OUT]),
     "ldp_fuse_depth_maps": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _I32, _P, _P, _P, C.c_double, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "ldp_depth_normals": (C.c_int, [_P, _P, _I32, _I32, _I32, _P, _I32, C.c_double, _P, _P, _P, _P]),
+    "ldp_fuse_depth_maps_oriented": (C.c_int, [_P, _P, _P, _P, _P, _I32, _I32, _I32, _P, _P, _P, C.c_double, C.c_double, _I32, _I32,
+                                               _P, _P, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "ldp_set_sm_reserve": (C.c_int, [C.c_int]),
     "ldp_last_launch_count": (C.c_int, []),
     "ldp_profile_enable": (C.c_int, [C.c_int]),

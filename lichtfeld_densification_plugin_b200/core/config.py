@@ -83,6 +83,17 @@ class DensePipelineConfig:
                                      # includes depth_consistency's test).  The depth, xyz, rgb and err maps of every view
                                      # stay on the device until the end: about 32 bytes per pixel (46 views at 512^2: 386 MB,
                                      # 250 views at 640^2: 3.3 GB)
+    depth_normal_radius: int = 0     # 1..3: oriented normal maps of the reference views, PCA over each pixel's
+                                     # (2r + 1)^2 map window (include/ldp_b200.h: ldp_depth_normals), written to
+                                     # <depth_dir>/normals/ and used by depth_fusion; needs depth_dir or depth_fusion.  With
+                                     # depth_fusion the maps stay on the device beside the others: 12 bytes more per pixel
+                                     # (46 views at 512^2: 145 MB, 250 views at 640^2: 1.2 GB).  0 = off
+    depth_normal_rel_tol: float = 0.05   # normal maps: relative depth difference of a window pixel that still counts as the
+                                     # same surface, in (0, 1); a slanted surface changes depth across the window by more
+                                     # than consistency_rel_tol does
+    depth_fusion_max_normal_angle: float = 0.0   # (0, 90) degrees: depth_fusion also requires agreeing normals (COLMAP
+                                     # fusion's test; its default is 10) and PipelineResult.normals become the fused normals
+                                     # unless normal_neighbors is set; needs depth_fusion and depth_normal_radius.  0 = off
 
     def validate(self) -> "DensePipelineConfig":
         if self.matches_per_ref < 0:
@@ -103,8 +114,8 @@ class DensePipelineConfig:
             raise ValueError("gaussian_opacity must lie in (0, 1)")
         if not 0.0 < float(self.gaussian_flatten) <= 1.0:
             raise ValueError("gaussian_flatten must lie in (0, 1]")
-        if float(self.gaussian_flatten) < 1.0 and int(self.normal_neighbors) == 0:
-            raise ValueError("gaussian_flatten < 1 needs normal_neighbors")
+        if float(self.gaussian_flatten) < 1.0 and int(self.normal_neighbors) == 0 and not self.fused_normals():
+            raise ValueError("gaussian_flatten < 1 needs normal_neighbors (or depth_fusion_max_normal_angle)")
         if not isinstance(self.depth_dir, str):
             raise ValueError("depth_dir must be a string (\"\" = off)")
         if not 0.0 < float(self.depth_min_certainty) <= 1.0:
@@ -115,9 +126,23 @@ class DensePipelineConfig:
             raise ValueError("consistency_min_views must be >= 0")
         if int(self.consistency_max_violations) < 0:
             raise ValueError("consistency_max_violations must be >= 0")
+        if not 0 <= int(self.depth_normal_radius) <= 3:
+            raise ValueError("depth_normal_radius must lie in [0, 3] (0 = off)")
+        if int(self.depth_normal_radius) > 0 and not (self.depth_dir or self.depth_fusion):
+            raise ValueError("depth_normal_radius needs depth_dir or depth_fusion")
+        if not 0.0 < float(self.depth_normal_rel_tol) < 1.0:
+            raise ValueError("depth_normal_rel_tol must lie in (0, 1)")
+        if not 0.0 <= float(self.depth_fusion_max_normal_angle) < 90.0:
+            raise ValueError("depth_fusion_max_normal_angle must lie in [0, 90) degrees (0 = off)")
+        if float(self.depth_fusion_max_normal_angle) > 0.0 and not (self.depth_fusion and int(self.depth_normal_radius) > 0):
+            raise ValueError("depth_fusion_max_normal_angle needs depth_fusion and depth_normal_radius")
         if self.rng_mode not in (RNG_PHILOX, RNG_NUMPY_GLOBAL, RNG_EXPLICIT):
             raise ValueError(f"unknown rng_mode {self.rng_mode!r}")
         return self
+
+    def fused_normals(self) -> bool:
+        """Whether depth fusion runs with the normal test and so yields a normal per fused point."""
+        return bool(self.depth_fusion) and int(self.depth_normal_radius) > 0 and float(self.depth_fusion_max_normal_angle) > 0.0
 
     @classmethod
     def from_reference(cls, cfg: Any, **overrides) -> "DensePipelineConfig":

@@ -41,7 +41,9 @@ class PipelineResult:
     pairs_processed: int
     n_views: Optional[np.ndarray] = None          # extra, config.multiview: uint8 cameras per point, the reference view included
     normals: Optional[np.ndarray] = None          # extra, config.normal_neighbors: f32 [n,3] unit normals facing each point's
-                                                  # reference camera; (0, 0, 0) where undefined
+                                                  # reference camera; (0, 0, 0) where undefined.  Without normal_neighbors,
+                                                  # config.depth_fusion_max_normal_angle: the fused normals (unit, each facing
+                                                  # its source camera)
     gaussians: Optional[Dict[str, np.ndarray]] = None   # extra, config.gaussian_neighbors: 3DGS's initial splats, f32
                                                   # sh_dc [n,3], opacity [n], scales [n,3] (log), rotations [n,4] (w, x, y, z)
     depth_paths: Optional[Dict[int, str]] = None  # extra, config.depth_dir: reference camera uid -> its depth map file
@@ -357,7 +359,7 @@ def submit_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triangulati
     depth = None
     fusion = bool(getattr(cfg, "depth_fusion", False))
     want_depth = bool(getattr(cfg, "depth_dir", "")) or bool(getattr(cfg, "depth_consistency", False)) or fusion
-    maps = dict(want_err=True, want_xyz=True, want_rgb=True) if fusion else {}
+    maps = dict(want_err=True, want_xyz=True, want_rgb=True) if fusion else (dict(want_xyz=True) if _normal_radius(cfg) else {})
     if ring is None:
         out = eng.densify(batch, pcfg, uniforms=u_dev, collect_debug=collect_debug_matches)
         if want_depth:
@@ -370,6 +372,34 @@ def submit_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triangulati
                           ref_cams=ref_cams)
 
 
+def _fused_normals(cfg) -> bool:
+    """Depth fusion with the normal test (config.depth_fusion_max_normal_angle): the fused cloud has normals."""
+    return (bool(getattr(cfg, "depth_fusion", False)) and int(getattr(cfg, "depth_normal_radius", 0)) > 0
+            and float(getattr(cfg, "depth_fusion_max_normal_angle", 0.0)) > 0.0)
+
+
+def _normal_radius(cfg) -> int:
+    """Window radius of the launches' normal maps; 0 when no consumer (depth_dir files, the fusion's normal test) wants them."""
+    r = int(getattr(cfg, "depth_normal_radius", 0))
+    return r if (r > 0 and (getattr(cfg, "depth_dir", "") or _fused_normals(cfg))) else 0
+
+
+def _launch_normal_maps(pending: "_PendingLaunch", tri_ctx: _TriangulationContext, ok: List[bool]) -> Dict[int, torch.Tensor]:
+    """``output.estimate_depth_normals`` of the launch's maps, on the current stream: {view index: f32 [H, W, 3]} for every view
+    whose sampling succeeded."""
+    from ..engine import DepthViews
+    from ..output import estimate_depth_normals
+    cfg, dm = tri_ctx.config, pending.depth
+    rs = [r for r in range(pending.n) if ok[r]]
+    if not rs:
+        return {}
+    views = DepthViews(int(dm.depth.shape[1]), int(dm.depth.shape[2]), tri_ctx.w_match, tri_ctx.h_match, dm.depth.device)
+    for r in rs:
+        views.add(dm.depth[r], pending.ref_cams[r], xyz=dm.xyz[r])
+    res = estimate_depth_normals(views, radius=int(cfg.depth_normal_radius), rel_tol=float(cfg.depth_normal_rel_tol))
+    return {r: res.normals[i] for i, r in enumerate(rs)}
+
+
 def depth_map_name(cameras, uid: int) -> str:
     """File name of reference view ``uid``'s depth map: the stem of its image path (its uid when it has none) + ``.npy``."""
     path = cameras.path_by.get(int(uid), "") if hasattr(cameras, "path_by") else ""
@@ -378,30 +408,37 @@ def depth_map_name(cameras, uid: int) -> str:
 
 
 def _write_depth_maps(pending: _PendingLaunch, tri_ctx: _TriangulationContext, ok: List[bool], ring,
-                      depth_paths: Optional[Dict[int, str]]) -> None:
-    """The launch's depth maps, one file per view whose sampling succeeded (the views the cloud has too)."""
+                      depth_paths: Optional[Dict[int, str]], normal_maps: Optional[Dict[int, torch.Tensor]] = None) -> None:
+    """The launch's depth maps, one file per view whose sampling succeeded (the views the cloud has too); with
+    ``normal_maps`` also each view's normal map, f32 [H, W, 3], under the same name in ``normals/``."""
     from ..output import write_depth_map
     if ring is not None:
         ring.wait(pending.depth)
     maps = pending.depth.depth.cpu().numpy()              # only these maps travel to the host, one launch at a time
     out_dir = tri_ctx.config.depth_dir
     os.makedirs(out_dir, exist_ok=True)
+    if normal_maps is not None:
+        os.makedirs(os.path.join(out_dir, "normals"), exist_ok=True)
     for r in range(pending.n):
         if not ok[r]:
             continue
         uid = int(pending.batch.ref_uids[r])
         path = os.path.join(out_dir, depth_map_name(tri_ctx.cameras, uid))
         write_depth_map(path, maps[r])
+        if normal_maps is not None:
+            np.save(os.path.join(out_dir, "normals", depth_map_name(tri_ctx.cameras, uid)),
+                    np.ascontiguousarray(normal_maps[r].cpu().numpy(), dtype=np.float32), allow_pickle=False)
         if depth_paths is not None:
             depth_paths[uid] = path
 
 
 def collect_refs(pending: _PendingLaunch, errors: Optional[list] = None, ring=None, tri_ctx: Optional[_TriangulationContext] = None,
-                 depth_paths: Optional[Dict[int, str]] = None, depth_kept: Optional[list] = None) -> List[Optional[_TriangulatedReference]]:
+                 depth_paths: Optional[Dict[int, str]] = None, depth_kept: Optional[list] = None,
+                 normals_kept: Optional[list] = None) -> List[Optional[_TriangulatedReference]]:
     """Second half: one synchronising read of the launch's results, split per view.  A launch with depth maps writes them
     under ``tri_ctx.config.depth_dir`` and records each file in ``depth_paths`` (reference camera uid -> path); with
     ``depth_kept`` it appends (uid, device map [H, W], reference camera, xyz, rgb, err maps or None) for every view whose
-    sampling succeeded."""
+    sampling succeeded, and with ``normals_kept`` each such view's normal map [H, W, 3] (config.depth_normal_radius)."""
     out, batch = pending.out, pending.batch
     if ring is not None:
         ring.wait(out)                                 # the current stream (which does the read-back) follows the ring stream
@@ -423,8 +460,13 @@ def collect_refs(pending: _PendingLaunch, errors: Optional[list] = None, ring=No
     if pending.depth is not None:
         if tri_ctx is None:
             raise ValueError("a launch with depth maps is collected with its tri_ctx")
+        normal_maps = None
+        if _normal_radius(tri_ctx.config):
+            if ring is not None:
+                ring.wait(pending.depth)           # computed on the current stream, which reads the maps
+            normal_maps = _launch_normal_maps(pending, tri_ctx, ok)
         if getattr(tri_ctx.config, "depth_dir", ""):
-            _write_depth_maps(pending, tri_ctx, ok, ring, depth_paths)
+            _write_depth_maps(pending, tri_ctx, ok, ring, depth_paths, normal_maps)
         if depth_kept is not None:
             if ring is not None:
                 ring.wait(pending.depth)           # the maps are read later on the current stream
@@ -433,6 +475,8 @@ def collect_refs(pending: _PendingLaunch, errors: Optional[list] = None, ring=No
                     dm = pending.depth
                     depth_kept.append((int(pending.batch.ref_uids[r]), dm.depth[r], pending.ref_cams[r],
                                        *(None if t is None else t[r] for t in (dm.xyz, dm.rgb, dm.err))))
+                    if normals_kept is not None:
+                        normals_kept.append(normal_maps[r])
     triangulate_refs.last_launches = out.launches
     return results
 
@@ -443,7 +487,7 @@ def triangulate_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triang
                      weight_sums: Optional[Sequence[float]] = None,
                      errors: Optional[list] = None, ply_records: bool = False,
                      depth_paths: Optional[Dict[int, str]] = None,
-                     depth_kept: Optional[list] = None) -> List[Optional[_TriangulatedReference]]:
+                     depth_kept: Optional[list] = None, normals_kept: Optional[list] = None) -> List[Optional[_TriangulatedReference]]:
     """Batched ``_triangulate_ref``: every view of ``matched_refs`` in one launch sequence.
 
     RNG: ``uniforms`` (f64 [n, U], explicit parity stream per view) or Philox keyed by
@@ -451,19 +495,19 @@ def triangulate_refs(matched_refs: Sequence[_MatchedReference], tri_ctx: _Triang
     None; the exception a per-view call would raise is appended to ``errors`` as (index, exc).
     ``ply_records``: also return every view's PLY vertex records (built on the device, 15 bytes per point).
     ``config.depth_dir``: also write every view's depth map there (``depth_paths``: see ``collect_refs``);
-    ``depth_kept``: keep the maps on the device (see ``collect_refs``).
+    ``depth_kept`` / ``normals_kept``: keep the maps on the device (see ``collect_refs``).
     """
     if len(matched_refs) == 0:
         return []
     pending = submit_refs(matched_refs, tri_ctx, collect_debug_matches, rng_streams=rng_streams, uniforms=uniforms,
                           weight_sums=weight_sums, ply_records=ply_records)
-    return collect_refs(pending, errors, tri_ctx=tri_ctx, depth_paths=depth_paths, depth_kept=depth_kept)
+    return collect_refs(pending, errors, tri_ctx=tri_ctx, depth_paths=depth_paths, depth_kept=depth_kept, normals_kept=normals_kept)
 
 
 def _triangulate_ref(matched_ref: _MatchedReference, tri_ctx: _TriangulationContext,
                      collect_debug_matches: bool = False, *,
                      depth_paths: Optional[Dict[int, str]] = None,
-                     depth_kept: Optional[list] = None) -> Optional[_TriangulatedReference]:
+                     depth_kept: Optional[list] = None, normals_kept: Optional[list] = None) -> Optional[_TriangulatedReference]:
     """Triangulate matches for a single reference view (reference core/pipeline.py:602-780).
 
     ``config.rng_mode``: "numpy" consumes the process-global MT19937 stream like the reference's ``np.random.choice``:
@@ -486,14 +530,17 @@ def _triangulate_ref(matched_ref: _MatchedReference, tri_ctx: _TriangulationCont
         while True:
             U = _mt_stream_from_global(n_uni)
             kept_here: Optional[list] = [] if depth_kept is not None else None
+            normals_here: Optional[list] = [] if normals_kept is not None else None
             res = triangulate_refs([matched_ref], tri_ctx, collect_debug_matches, uniforms=U[None, :], errors=errs,
-                                   depth_paths=depth_paths, depth_kept=kept_here)
+                                   depth_paths=depth_paths, depth_kept=kept_here, normals_kept=normals_here)
             if errs and "exhausted" in str(errs[0][1]):
                 errs.clear()
                 n_uni *= 2
                 continue
             if depth_kept is not None:
                 depth_kept += kept_here
+            if normals_kept is not None:
+                normals_kept += normals_here
             break
         used = int(triangulate_refs.last_uniforms_used[0])
         if used > 0:
@@ -501,7 +548,7 @@ def _triangulate_ref(matched_ref: _MatchedReference, tri_ctx: _TriangulationCont
     else:
         res = triangulate_refs([matched_ref], tri_ctx, collect_debug_matches,
                                rng_streams=[int(matched_ref.packed.ref_id)], errors=errs, depth_paths=depth_paths,
-                               depth_kept=depth_kept)
+                               depth_kept=depth_kept, normals_kept=normals_kept)
     if errs:
         raise errs[0][1]
     return res[0]
@@ -699,6 +746,7 @@ def run_dense_pipeline(
     depth_paths: Optional[Dict[int, str]] = {} if getattr(config, "depth_dir", "") else None
     fusion = bool(getattr(config, "depth_fusion", False))
     depth_kept: Optional[list] = [] if (getattr(config, "depth_consistency", False) or fusion) else None
+    normals_kept: Optional[list] = [] if _fused_normals(config) else None      # beside depth_kept, entry for entry
 
     def consume(outs, done: int, matched_refs) -> None:
         nonlocal pairs, ply_points, pair_counter
@@ -748,13 +796,15 @@ def run_dense_pipeline(
                 outs = []
                 for m in mrs:
                     try:
-                        outs.append(_triangulate_ref(m, tri_ctx, collect_debug, depth_paths=depth_paths, depth_kept=depth_kept))
+                        outs.append(_triangulate_ref(m, tri_ctx, collect_debug, depth_paths=depth_paths, depth_kept=depth_kept,
+                                                     normals_kept=normals_kept))
                     except Exception:
                         outs.append(None)
                 consume(outs, done, mrs)
             elif ring is None:
                 consume(triangulate_refs(mrs, tri_ctx, collect_debug, rng_streams=[int(r) for r, _ in matched],
-                                         ply_records=ply_base is not None, depth_paths=depth_paths, depth_kept=depth_kept),
+                                         ply_records=ply_base is not None, depth_paths=depth_paths, depth_kept=depth_kept,
+                                         normals_kept=normals_kept),
                         done, mrs)
             else:
                 # several launches in flight: the next chunk is uploaded and enqueued before the oldest one is read back
@@ -762,11 +812,13 @@ def run_dense_pipeline(
                                                     ply_records=ply_base is not None, ring=ring), mrs))
                 if len(in_flight) >= ring.depth:
                     d, pend, pm = in_flight.pop(0)
-                    consume(collect_refs(pend, ring=ring, tri_ctx=tri_ctx, depth_paths=depth_paths, depth_kept=depth_kept), d, pm)
+                    consume(collect_refs(pend, ring=ring, tri_ctx=tri_ctx, depth_paths=depth_paths, depth_kept=depth_kept,
+                                 normals_kept=normals_kept), d, pm)
         for d, pend, pm in in_flight:
             if _is_cancelled(cancel_requested):
                 raise PipelineCancelled("Cancelled")
-            consume(collect_refs(pend, ring=ring, tri_ctx=tri_ctx, depth_paths=depth_paths, depth_kept=depth_kept), d, pm)
+            consume(collect_refs(pend, ring=ring, tri_ctx=tri_ctx, depth_paths=depth_paths, depth_kept=depth_kept,
+                                 normals_kept=normals_kept), d, pm)
     finally:
         if debug_state is not None and hasattr(debug_state, "release_waiters"):
             debug_state.release_waiters()                              # core/pipeline.py:547-548
@@ -781,14 +833,17 @@ def run_dense_pipeline(
     xyz, rgb, err = np.concatenate(parts_xyz, axis=0), np.concatenate(parts_rgb, axis=0), np.concatenate(parts_err, axis=0)
     n_views = np.concatenate(parts_nv, axis=0) if getattr(config, "multiview", False) else None
     ref_uid = np.concatenate(parts_ref, axis=0)
-    consistent = fused_views = None
+    consistent = fused_views = fused_normals = None
     if fusion:
         # the fused maps replace the sampled cloud (its test includes depth_consistency's); the intermediate PLYs above stay
         # those of the sampled path
         if progress_callback:
             progress_callback(93.0, "Fusing depth maps...")
-        xyz, rgb, err, ref_uid, fused_views, consistent = _fuse_depth_maps(depth_kept, tri_ctx)
-        depth_kept = None
+        if normals_kept is None:
+            xyz, rgb, err, ref_uid, fused_views, consistent = _fuse_depth_maps(depth_kept, tri_ctx)
+        else:                                  # with the normal test: one normal per fused point
+            xyz, rgb, err, ref_uid, fused_views, consistent, fused_normals = _fuse_depth_maps(depth_kept, tri_ctx, normals=normals_kept)
+        depth_kept = normals_kept = None
         n_views = None                         # the multiview counts belong to the sampled points
     elif depth_kept is not None:
         # visibility test against the other reference views' maps, before the outlier filter, normals and Gaussians; the
@@ -803,7 +858,7 @@ def run_dense_pipeline(
     k_out = int(getattr(config, "outlier_neighbors", 0))
     k_nrm = int(getattr(config, "normal_neighbors", 0))
     k_gs = int(getattr(config, "gaussian_neighbors", 0))
-    normals = gaussians = None
+    normals = gaussians = nrm_dev = None
     if k_out > 0 or k_nrm > 0 or k_gs > 0:
         dev = torch.device("cuda", torch.cuda.current_device())
         xyz_dev = torch.from_numpy(np.ascontiguousarray(xyz, dtype=np.float32)).to(dev)
@@ -823,6 +878,8 @@ def run_dense_pipeline(
             consistent = consistent[keep]
         if fused_views is not None:
             fused_views = fused_views[keep]
+        if fused_normals is not None:
+            fused_normals = fused_normals[keep]
     if k_nrm > 0:
         # every point faces the camera it was triangulated from (its reference view, a contributing view in every mode)
         if progress_callback:
@@ -832,14 +889,19 @@ def run_dense_pipeline(
         centers = np.stack([np.asarray(cameras.C_by[int(u)], np.float64).reshape(3) for u in uids]).astype(np.float32)
         nres = estimate_normals(xyz_dev, nb_neighbors=k_nrm, centers=torch.from_numpy(centers).to(dev),
                                 center_idx=torch.from_numpy(center_idx.astype(np.int32)).to(dev))
-        normals = nres.normals.cpu().numpy()
+        normals, nrm_dev = nres.normals.cpu().numpy(), nres.normals
+    elif fused_normals is not None:
+        # the fused normals (averaged over each point's members, facing its source camera) in place of a k-NN search
+        normals = fused_normals
+        if k_gs > 0:
+            nrm_dev = torch.from_numpy(np.ascontiguousarray(normals)).to(dev)
     if k_gs > 0:
         # the final cloud, after the outlier filter; discs along the normals above when there are any
         if progress_callback:
             progress_callback(98.0, "Initialising Gaussians...")
         from ..output import init_gaussians
         rgb_dev = torch.from_numpy(np.ascontiguousarray(rgb, dtype=np.float32)).to(dev)
-        g = init_gaussians(xyz_dev, rgb_dev, normals=nres.normals if k_nrm > 0 else None, nb_neighbors=k_gs,
+        g = init_gaussians(xyz_dev, rgb_dev, normals=nrm_dev, nb_neighbors=k_gs,
                            opacity=float(config.gaussian_opacity), flatten=float(config.gaussian_flatten))
         gaussians = {name: getattr(g, name).cpu().numpy() for name in ("sh_dc", "opacity", "scales", "rotations")}
     return PipelineResult(xyz=xyz, rgb=rgb, err=err, elapsed_seconds=time.time() - t0, pairs_processed=pairs, n_views=n_views,
@@ -847,22 +909,25 @@ def run_dense_pipeline(
                           fused_views=fused_views)
 
 
-def _fuse_depth_maps(depth_kept: list, tri_ctx: _TriangulationContext):
+def _fuse_depth_maps(depth_kept: list, tri_ctx: _TriangulationContext, normals: Optional[list] = None):
     """``output.fuse_depth_maps`` of the kept maps (``collect_refs``), views in collection order.  Returns host arrays
-    (xyz, rgb, err, reference camera uid of each point's source view, n_views, n_consistent)."""
+    (xyz, rgb, err, reference camera uid of each point's source view, n_views, n_consistent); with ``normals`` (each kept
+    view's normal map, ``collect_refs``' ``normals_kept``) the fusion takes the normal test and the fused normals follow."""
     from ..engine import DepthViews
     from ..output import fuse_depth_maps
     cfg = tri_ctx.config
     m0 = depth_kept[0][1]
     views = DepthViews(int(m0.shape[0]), int(m0.shape[1]), tri_ctx.w_match, tri_ctx.h_match, m0.device)
-    for uid, depth, cam, xyz, rgb, err in depth_kept:
-        views.add(depth, cam, xyz=xyz, rgb=rgb, err=err)
+    for v, (uid, depth, cam, xyz, rgb, err) in enumerate(depth_kept):
+        views.add(depth, cam, xyz=xyz, rgb=rgb, err=err, normals=None if normals is None else normals[v])
     f = fuse_depth_maps(views, rel_tol=float(cfg.consistency_rel_tol), min_views=int(cfg.consistency_min_views),
-                        max_violations=int(cfg.consistency_max_violations))
+                        max_violations=int(cfg.consistency_max_violations),
+                        max_normal_angle=None if normals is None else float(cfg.depth_fusion_max_normal_angle))
     uids = np.array([e[0] for e in depth_kept], np.int64)
     src_view = (f.source // (views.H * views.W)).cpu().numpy()
-    return (f.xyz.cpu().numpy(), f.rgb.cpu().numpy(), f.err.cpu().numpy(), uids[src_view], f.n_views.cpu().numpy(),
-            f.n_consistent.cpu().numpy())
+    out = (f.xyz.cpu().numpy(), f.rgb.cpu().numpy(), f.err.cpu().numpy(), uids[src_view], f.n_views.cpu().numpy(),
+           f.n_consistent.cpu().numpy())
+    return out if normals is None else out + (f.normals.cpu().numpy(),)
 
 
 def _check_consistency(xyz: np.ndarray, ref_uid: np.ndarray, depth_kept: list, tri_ctx: _TriangulationContext):
@@ -892,8 +957,11 @@ def _write_depth_index(config: DensePipelineConfig, tri_ctx: _TriangulationConte
     for uid, path in depth_paths.items():
         H, W = np.load(path, mmap_mode="r").shape
         width, height = tri_ctx.cameras.size_by[uid]
-        maps.append(dict(file=os.path.basename(path), camera_uid=int(uid), H=int(H), W=int(W), w_match=int(tri_ctx.w_match),
-                         h_match=int(tri_ctx.h_match), width=int(width), height=int(height)))
+        entry = dict(file=os.path.basename(path), camera_uid=int(uid), H=int(H), W=int(W), w_match=int(tri_ctx.w_match),
+                     h_match=int(tri_ctx.h_match), width=int(width), height=int(height))
+        if _normal_radius(config):
+            entry["normals_file"] = "normals/" + os.path.basename(path)         # f32 [H, W, 3], NaN = no normal
+        maps.append(entry)
     index = dict(min_certainty=float(config.depth_min_certainty), nan="no depth", maps=maps)
     with open(os.path.join(config.depth_dir, "depth_maps.json"), "w") as f:
         json.dump(index, f, indent=1)

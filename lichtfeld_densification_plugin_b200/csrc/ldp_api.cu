@@ -1443,12 +1443,13 @@ int ldp_fuse_workspace_bytes(int32_t n_views, int32_t H, int32_t W, size_t* byte
     return fusion_plan(n_views, H, W, nullptr, &pl, bytes_out);
 }
 
-int ldp_fuse_depth_maps(const float* const* depth_ptrs, const float* const* xyz_ptrs, const float* const* rgb_ptrs,
-                        const float* const* err_ptrs, int32_t n_views, int32_t H, int32_t W, const float* P, const double* scales,
-                        const ldp_lens* lens, double rel_tol, int32_t min_views, int32_t max_violations, float* xyz_out,
-                        float* rgb_out, float* err_out, int32_t* n_views_out, int32_t* n_consistent_out, int64_t* source_out,
-                        int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream) {
-    begin_call();
+// both fusion entry points; normal_ptrs = NULL: ldp_fuse_depth_maps (the <LENS, false> kernels)
+static int fuse_maps(const float* const* depth_ptrs, const float* const* xyz_ptrs, const float* const* rgb_ptrs,
+                     const float* const* err_ptrs, const float* const* normal_ptrs, int32_t n_views, int32_t H, int32_t W,
+                     const float* P, const double* scales, const ldp_lens* lens, double rel_tol, double cos_max, int32_t min_views,
+                     int32_t max_violations, float* xyz_out, float* rgb_out, float* err_out, float* normals_out,
+                     int32_t* n_views_out, int32_t* n_consistent_out, int64_t* source_out, int32_t* status_out, void* workspace,
+                     size_t workspace_bytes, void* stream) {
     if (!(rel_tol > 0.0 && rel_tol < 1.0)) return fail(LDP_ERR_INVALID, "rel_tol must lie in (0, 1)");
     if (min_views < 0 || max_violations < 0) return fail(LDP_ERR_INVALID, "min_views and max_violations must be >= 0");
     FusionPlan pl;
@@ -1465,26 +1466,28 @@ int ldp_fuse_depth_maps(const float* const* depth_ptrs, const float* const* xyz_
     if ((rc = fusion_plan(n_views, H, W, workspace, &pl, &need)) != LDP_OK) return rc;
     if (workspace_bytes < need) return fail(LDP_ERR_WORKSPACE, "fusion workspace too small");
     const long long total = (long long)n_views * H * W;
+    const bool nrm = normal_ptrs != nullptr;
     const ldp::FusionArgs a{depth_ptrs, xyz_ptrs, rgb_ptrs, err_ptrs, P, scales, lens, pl.kept, pl.n_cons, pl.flag,
                             reinterpret_cast<const long long*>(source_out), xyz_out, rgb_out, err_out, (int*)n_views_out,
                             (int*)n_consistent_out, (int*)status_out, total, rel_tol, (int)n_views, (int)H, (int)W, (int)(H * W),
-                            (int)min_views, (int)max_violations};
-    rc = launch("ldp_fusion_check_kernel", ldp::ldp_fusion_check_kernel, dim3((unsigned)((n_views + ldp::CS_THREADS - 1) / ldp::CS_THREADS)),
-                dim3(ldp::CS_THREADS), 0, st, a);
+                            (int)min_views, (int)max_violations, normal_ptrs, normals_out, cos_max};
+    rc = launch("ldp_fusion_check_kernel", nrm ? ldp::ldp_fusion_check_kernel<true> : ldp::ldp_fusion_check_kernel<false>,
+                dim3((unsigned)((n_views + ldp::CS_THREADS - 1) / ldp::CS_THREADS)), dim3(ldp::CS_THREADS), 0, st, a);
     if (rc != LDP_OK) return rc;
     // a few resident CTAs per SM; each strides over the maps, so a table of one chunk is staged once per CTA
     const unsigned grid = (unsigned)std::min<long long>((total + ldp::CS_THREADS - 1) / ldp::CS_THREADS, (long long)sm_count() * 8);
+    const int which = (lens ? 2 : 0) + (nrm ? 1 : 0);
     {
         KernelTimer kt(st, "ldp_fusion_verdict_kernel");
-        rc = launch("ldp_fusion_verdict_kernel", lens ? ldp::ldp_fusion_verdict_kernel<true> : ldp::ldp_fusion_verdict_kernel<false>,
-                    dim3(grid), dim3(ldp::CS_THREADS), 0, st, a);
-        if (rc != LDP_OK) return rc;
+        auto* k = (which == 0) ? ldp::ldp_fusion_verdict_kernel<false, false> : (which == 1) ? ldp::ldp_fusion_verdict_kernel<false, true>
+                : (which == 2) ? ldp::ldp_fusion_verdict_kernel<true, false> : ldp::ldp_fusion_verdict_kernel<true, true>;
+        if ((rc = launch("ldp_fusion_verdict_kernel", k, dim3(grid), dim3(ldp::CS_THREADS), 0, st, a)) != LDP_OK) return rc;
     }
     {
         KernelTimer kt(st, "ldp_fusion_emit_kernel");
-        rc = launch("ldp_fusion_emit_kernel", lens ? ldp::ldp_fusion_emit_kernel<true> : ldp::ldp_fusion_emit_kernel<false>,
-                    dim3(grid), dim3(ldp::CS_THREADS), 0, st, a);
-        if (rc != LDP_OK) return rc;
+        auto* k = (which == 0) ? ldp::ldp_fusion_emit_kernel<false, false> : (which == 1) ? ldp::ldp_fusion_emit_kernel<false, true>
+                : (which == 2) ? ldp::ldp_fusion_emit_kernel<true, false> : ldp::ldp_fusion_emit_kernel<true, true>;
+        if ((rc = launch("ldp_fusion_emit_kernel", k, dim3(grid), dim3(ldp::CS_THREADS), 0, st, a)) != LDP_OK) return rc;
     }
     if ((rc = scan_exclusive(pl.flag, pl.rank, total, pl.block_tot, (int*)status_out + 1, st)) != LDP_OK) return rc;
     const unsigned kgrid = (unsigned)((total + ldp::KV_THREADS - 1) / ldp::KV_THREADS);
@@ -1492,8 +1495,64 @@ int ldp_fuse_depth_maps(const float* const* depth_ptrs, const float* const* xyz_
                 (const int*)pl.rank, total, reinterpret_cast<long long*>(source_out));
     if (rc != LDP_OK) return rc;
     KernelTimer kt(st, "ldp_fusion_sum_kernel");
-    return launch("ldp_fusion_sum_kernel", lens ? ldp::ldp_fusion_sum_kernel<true> : ldp::ldp_fusion_sum_kernel<false>, dim3(grid),
-                  dim3(ldp::CS_THREADS), 0, st, a);
+    auto* k = (which == 0) ? ldp::ldp_fusion_sum_kernel<false, false> : (which == 1) ? ldp::ldp_fusion_sum_kernel<false, true>
+            : (which == 2) ? ldp::ldp_fusion_sum_kernel<true, false> : ldp::ldp_fusion_sum_kernel<true, true>;
+    return launch("ldp_fusion_sum_kernel", k, dim3(grid), dim3(ldp::CS_THREADS), 0, st, a);
+}
+
+int ldp_fuse_depth_maps(const float* const* depth_ptrs, const float* const* xyz_ptrs, const float* const* rgb_ptrs,
+                        const float* const* err_ptrs, int32_t n_views, int32_t H, int32_t W, const float* P, const double* scales,
+                        const ldp_lens* lens, double rel_tol, int32_t min_views, int32_t max_violations, float* xyz_out,
+                        float* rgb_out, float* err_out, int32_t* n_views_out, int32_t* n_consistent_out, int64_t* source_out,
+                        int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream) {
+    begin_call();
+    return fuse_maps(depth_ptrs, xyz_ptrs, rgb_ptrs, err_ptrs, nullptr, n_views, H, W, P, scales, lens, rel_tol, 0.0, min_views,
+                     max_violations, xyz_out, rgb_out, err_out, nullptr, n_views_out, n_consistent_out, source_out, status_out,
+                     workspace, workspace_bytes, stream);
+}
+
+int ldp_fuse_depth_maps_oriented(const float* const* depth_ptrs, const float* const* xyz_ptrs, const float* const* rgb_ptrs,
+                                 const float* const* err_ptrs, const float* const* normal_ptrs, int32_t n_views, int32_t H, int32_t W,
+                                 const float* P, const double* scales, const ldp_lens* lens, double rel_tol, double cos_max,
+                                 int32_t min_views, int32_t max_violations, float* xyz_out, float* rgb_out, float* err_out,
+                                 float* normals_out, int32_t* n_views_out, int32_t* n_consistent_out, int64_t* source_out,
+                                 int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream) {
+    begin_call();
+    if (!(cos_max > 0.0 && cos_max < 1.0)) return fail(LDP_ERR_INVALID, "cos_max must lie in (0, 1)");
+    if (n_views > 0 && (!normal_ptrs || !normals_out)) return fail(LDP_ERR_INVALID, "null normal_ptrs / normals_out");
+    return fuse_maps(depth_ptrs, xyz_ptrs, rgb_ptrs, err_ptrs, normal_ptrs, n_views, H, W, P, scales, lens, rel_tol, cos_max,
+                     min_views, max_violations, xyz_out, rgb_out, err_out, normals_out, n_views_out, n_consistent_out, source_out,
+                     status_out, workspace, workspace_bytes, stream);
+}
+
+int ldp_depth_normals(const float* const* depth_ptrs, const float* const* xyz_ptrs, int32_t n_views, int32_t H, int32_t W,
+                      const float* centers, int32_t radius, double rel_tol, float* normals_out, float* curvature_out,
+                      int32_t* status_out, void* stream) {
+    begin_call();
+    if (radius < 1 || radius > 3) return fail(LDP_ERR_INVALID, "radius must lie in [1, 3]");
+    if (!(rel_tol > 0.0 && rel_tol < 1.0)) return fail(LDP_ERR_INVALID, "rel_tol must lie in (0, 1)");
+    if (n_views < 0 || n_views > 65535 || H <= 0 || W <= 0) return fail(LDP_ERR_INVALID, "bad view count or map shape");
+    if ((long long)n_views * H * W >= (1ll << 31)) return fail(LDP_ERR_INVALID, "normal maps: n_views * H * W must be below 2^31");
+    if (!status_out) return fail(LDP_ERR_INVALID, "null status_out");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    int rc = check(cudaMemsetAsync(status_out, 0, 2 * sizeof(int32_t), st), "cudaMemsetAsync(status)");
+    if (rc != LDP_OK || n_views == 0) return rc;
+    if (!depth_ptrs || !xyz_ptrs || !centers || !normals_out) return fail(LDP_ERR_INVALID, "null map table / centers / normals_out");
+    const int N = H * W;
+    const int tiles_x = (W + ldp::DN_TILE - 1) / ldp::DN_TILE, tiles = tiles_x * ((H + ldp::DN_TILE - 1) / ldp::DN_TILE);
+    const ldp::DepthNormalArgs a{depth_ptrs, xyz_ptrs, centers, normals_out, curvature_out, (int*)status_out, rel_tol, (int)n_views,
+                                 (int)H, (int)W, N, tiles_x};
+    const int per_view = std::max(1, std::min((N + ldp::CS_THREADS - 1) / ldp::CS_THREADS, (sm_count() * 8 + n_views - 1) / n_views));
+    {
+        KernelTimer kt(st, "ldp_depth_normals_check_kernel");
+        rc = launch("ldp_depth_normals_check_kernel", ldp::ldp_depth_normals_check_kernel, dim3((unsigned)per_view, (unsigned)n_views),
+                    dim3(ldp::CS_THREADS), 0, st, a);
+        if (rc != LDP_OK) return rc;
+    }
+    KernelTimer kt(st, "ldp_depth_normals_kernel");
+    auto* k = (radius == 1) ? ldp::ldp_depth_normals_kernel<1> : (radius == 2) ? ldp::ldp_depth_normals_kernel<2>
+                                                                                : ldp::ldp_depth_normals_kernel<3>;
+    return launch("ldp_depth_normals_kernel", k, dim3((unsigned)tiles, (unsigned)n_views), dim3(ldp::DN_THREADS), 0, st, a);
 }
 
 }  // extern "C"

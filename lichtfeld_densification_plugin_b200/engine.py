@@ -368,27 +368,32 @@ class DepthViews:
         self.xyz: List[Optional[torch.Tensor]] = []      # per view, what fusion needs beside the depth (None where not given)
         self.rgb: List[Optional[torch.Tensor]] = []
         self.err: List[Optional[torch.Tensor]] = []
+        self.normals: List[Optional[torch.Tensor]] = []   # per view, what the oriented fusion needs (None where not given)
         self._tables = None
         self._fusion_tables = None
+        self._normal_table = None
 
     def __len__(self) -> int:
         return len(self.maps)
 
-    def add(self, depth, camera: CameraRecord, *, xyz=None, rgb=None, err=None) -> int:
+    def add(self, depth, camera: CameraRecord, *, xyz=None, rgb=None, err=None, normals=None) -> int:
         """Append one view: its f32 [H, W] map (a device tensor or a host array; NaN = no depth) and the ``CameraRecord`` its
         map was made with (the P1 and lens of the launch, its full-resolution width and height).  Returns the view index,
         the value ``owner`` takes for the points of this view.  ``xyz`` / ``rgb`` ([H, W, 3]) and ``err`` ([H, W]), f32 like the
-        map (``DepthMaps.xyz`` / ``.rgb`` / ``.err`` of the view): what ``output.fuse_depth_maps`` needs beside the depth."""
+        map (``DepthMaps.xyz`` / ``.rgb`` / ``.err`` of the view): what ``output.fuse_depth_maps`` needs beside the depth.
+        ``normals`` ([H, W, 3], e.g. ``output.estimate_depth_normals(...).normals[v]``): what its normal test needs."""
         depth = self._map(depth, (self.H, self.W), "a depth map")
-        xyz, rgb, err = (None if t is None else self._map(t, shape, what) for t, shape, what in
-                         ((xyz, (self.H, self.W, 3), "xyz"), (rgb, (self.H, self.W, 3), "rgb"), (err, (self.H, self.W), "err")))
+        xyz, rgb, err, normals = (None if t is None else self._map(t, shape, what) for t, shape, what in
+                                  ((xyz, (self.H, self.W, 3), "xyz"), (rgb, (self.H, self.W, 3), "rgb"), (err, (self.H, self.W), "err"),
+                                   (normals, (self.H, self.W, 3), "normals")))
         check_lens(camera)
         self.maps.append(depth)
         self.cameras.append(camera)
         self.xyz.append(xyz)
         self.rgb.append(rgb)
         self.err.append(err)
-        self._tables = self._fusion_tables = None
+        self.normals.append(normals)
+        self._tables = self._fusion_tables = self._normal_table = None
         return len(self.maps) - 1
 
     def _map(self, t, shape, what: str) -> torch.Tensor:
@@ -461,6 +466,26 @@ class DepthViews:
             ptrs = lambda ts: torch.tensor([t.data_ptr() for t in ts] or [0], dtype=torch.int64).to(self.device)  # noqa: E731
             self._fusion_tables = (ptrs(self.xyz), ptrs(self.rgb), ptrs(self.err))
         return self._fusion_tables
+
+    def xyz_table(self):
+        """Device table of ``ldp_depth_normals`` beside the map pointers of ``tables()``: pointers to each view's xyz map (int64
+        [V]).  Raises if a view lacks one."""
+        missing = [v for v in range(len(self.maps)) if self.xyz[v] is None]
+        if missing:
+            raise ValueError(f"view {missing[0]} has no xyz map: normal maps need the xyz map of every view "
+                             "(DepthViews.add(..., xyz=) with DensifyEngine.depth_maps(want_xyz=True))")
+        return torch.tensor([t.data_ptr() for t in self.xyz] or [0], dtype=torch.int64).to(self.device)
+
+    def normal_table(self):
+        """Device table of ``ldp_fuse_depth_maps_oriented`` beside ``fusion_tables()``: pointers to each view's normal map
+        (int64 [V]).  Raises if a view lacks one."""
+        if self._normal_table is None:
+            missing = [v for v in range(len(self.maps)) if self.normals[v] is None]
+            if missing:
+                raise ValueError(f"view {missing[0]} has no normal map: the normal test needs the normal map of every view "
+                                 "(DepthViews.add(..., normals=) with output.estimate_depth_normals)")
+            self._normal_table = torch.tensor([t.data_ptr() for t in self.normals] or [0], dtype=torch.int64).to(self.device)
+        return self._normal_table
 
 
 class DensifyEngine:

@@ -13,7 +13,10 @@ Mirrors, on tensors that stay on the GPU (SURVEY.md 8a row a15, 8f rows 2 and 4)
 * ``check_depth_consistency``          not in the reference: MVS fusion's visibility test of a cloud against the reference
   views' depth maps (``engine.DepthViews``)
 * ``fuse_depth_maps``                  not in the reference: MVS fusion of the reference views' depth maps into one dense
-  coloured cloud, each surface point emitted once and averaged over the views that agree with it
+  coloured cloud, each surface point emitted once and averaged over the views that agree with it (optionally in depth and
+  normal, with the fused normals)
+* ``estimate_depth_normals``           not in the reference: oriented normal maps of the reference views, PCA over each
+  pixel's depth-continuous map window
 * ``apply_point_cap``                  reference densify.py:110-120 (the indices are numpy's own
   ``default_rng(seed).choice`` on the host - PCG64 + a sequential shuffle, microseconds; only the gather is device work)
 * ``subsample_preview_matches``        reference core/pipeline.py:573-582 (debug preview subsample of the kept matches)
@@ -26,6 +29,7 @@ No CPU fallback: every function needs the CUDA library (``NativeLibraryError`` o
 from __future__ import annotations
 
 import ctypes as C
+import math
 from dataclasses import dataclass
 from typing import Optional, Tuple
 
@@ -489,18 +493,28 @@ class FusedCloud:
     n_views: torch.Tensor               # [m] int32: views averaged (members + 1)
     n_consistent: torch.Tensor          # [m] int32: other views whose depth agrees with the emitting pixel
     source: torch.Tensor                # [m] int64: emitting pixel, view * H * W + pixel index
+    normals: Optional[torch.Tensor] = None   # [m, 3] f32 unit normals averaged over the point and its members (max_normal_angle)
 
 
-def fuse_depth_maps(views, *, rel_tol: float = 0.01, min_views: int = 1, max_violations: int = 0) -> FusedCloud:
+def fuse_depth_maps(views, *, rel_tol: float = 0.01, min_views: int = 1, max_violations: int = 0,
+                    max_normal_angle: Optional[float] = None) -> FusedCloud:
     """MVS fusion of the maps of ``views`` (``engine.DepthViews`` whose views carry xyz and rgb maps) into one cloud in which
     each surface point appears once: a pixel is kept iff at least ``min_views`` other views agree with its depth (within
     ``rel_tol``) and at most ``max_violations`` look through it (``check_depth_consistency``'s test); a kept pixel is
     emitted iff no lower view holds a kept pixel that agrees with it, and its xyz and rgb are averaged over itself and the
     kept pixels of the views that agree with it.  The rule is in include/ldp_b200.h (ldp_fuse_depth_maps).  Raises on a
     view without xyz or rgb maps and on a non-finite xyz where the depth is finite.  Synchronises once, to read the
-    emitted count."""
+    emitted count.
+
+    ``max_normal_angle`` (degrees in (0, 90); COLMAP: 10) adds COLMAP fusion's normal test: a view agrees only where its
+    normal map (``DepthViews.add(..., normals=)``, e.g. ``estimate_depth_normals``) is within that angle of the pixel's
+    normal too, a pixel without a normal is not kept, and ``FusedCloud.normals`` holds the normalised sum of the point's and
+    its members' normals (include/ldp_b200.h: ldp_fuse_depth_maps_oriented).  Raises if a view has no normal map.
+    None: no normal test and no normals."""
     if not 0.0 < float(rel_tol) < 1.0:
         raise ValueError("rel_tol must lie in (0, 1)")
+    if max_normal_angle is not None and not 0.0 < float(max_normal_angle) < 90.0:
+        raise ValueError("max_normal_angle must lie in (0, 90) degrees (None = off)")
     if int(min_views) < 0 or int(max_violations) < 0:
         raise ValueError("min_views and max_violations must be >= 0")
     dev = views.device
@@ -510,6 +524,7 @@ def fuse_depth_maps(views, *, rel_tol: float = 0.01, min_views: int = 1, max_vio
     if V * H * W >= 2 ** 31:
         raise ValueError("fusion needs n_views * H * W < 2^31")
     xyz_p, rgb_p, err_p = views.fusion_tables()
+    nrm_p = views.normal_table() if max_normal_angle is not None else None
     lib, stream = N.load(), torch.cuda.current_stream(dev).cuda_stream
     need = C.c_size_t(0)
     N.check(lib.ldp_fuse_workspace_bytes(V, H, W, C.byref(need)), "ldp_fuse_workspace_bytes")
@@ -522,9 +537,19 @@ def fuse_depth_maps(views, *, rel_tol: float = 0.01, min_views: int = 1, max_vio
     status = torch.zeros((2,), dtype=torch.int32, device=dev)
     ptrs, P, S, lens = views.tables()
     ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)          # noqa: E731
-    N.check(lib.ldp_fuse_depth_maps(ptr(ptrs), ptr(xyz_p), ptr(rgb_p), ptr(err_p), V, H, W, ptr(P), ptr(S), ptr(lens), float(rel_tol),
-                                    int(min_views), int(max_violations), ptr(xyz), ptr(rgb), ptr(err), ptr(nv), ptr(nc), ptr(src),
-                                    ptr(status), ptr(ws), C.c_size_t(need.value), C.c_void_p(stream)), "ldp_fuse_depth_maps")
+    nrm = None
+    if nrm_p is None:
+        N.check(lib.ldp_fuse_depth_maps(ptr(ptrs), ptr(xyz_p), ptr(rgb_p), ptr(err_p), V, H, W, ptr(P), ptr(S), ptr(lens),
+                                        float(rel_tol), int(min_views), int(max_violations), ptr(xyz), ptr(rgb), ptr(err), ptr(nv),
+                                        ptr(nc), ptr(src), ptr(status), ptr(ws), C.c_size_t(need.value), C.c_void_p(stream)),
+                "ldp_fuse_depth_maps")
+    else:
+        nrm = torch.empty((cap, 3), **f32)
+        cos_max = math.cos(math.radians(float(max_normal_angle)))
+        N.check(lib.ldp_fuse_depth_maps_oriented(ptr(ptrs), ptr(xyz_p), ptr(rgb_p), ptr(err_p), ptr(nrm_p), V, H, W, ptr(P), ptr(S),
+                                                 ptr(lens), float(rel_tol), cos_max, int(min_views), int(max_violations), ptr(xyz),
+                                                 ptr(rgb), ptr(err), ptr(nrm), ptr(nv), ptr(nc), ptr(src), ptr(status), ptr(ws),
+                                                 C.c_size_t(need.value), C.c_void_p(stream)), "ldp_fuse_depth_maps_oriented")
     bad, m = (int(v) for v in status.cpu().tolist())
     if bad & 1:
         raise ValueError("a view's xyz map is not finite where its depth is")
@@ -532,7 +557,53 @@ def fuse_depth_maps(views, *, rel_tol: float = 0.01, min_views: int = 1, max_vio
         raise ValueError("a view's map pointer is NULL")
     # copies of the first m rows: the capacity (one row per map pixel) is released
     return FusedCloud(xyz=xyz[:m].clone(), rgb=rgb[:m].clone(), err=err[:m].clone(), n_views=nv[:m].clone(),
-                      n_consistent=nc[:m].clone(), source=src[:m].clone())
+                      n_consistent=nc[:m].clone(), source=src[:m].clone(), normals=None if nrm is None else nrm[:m].clone())
+
+
+@dataclass
+class DepthNormals:
+    """What ``estimate_depth_normals`` returns (device tensors, one map per view of the ``DepthViews``)."""
+    normals: torch.Tensor               # [V, H, W, 3] f32 unit normals facing the view's camera; NaN where there is none
+    curvature: torch.Tensor             # [V, H, W] f32 surface variation l0 / (l0 + l1 + l2); NaN where there is no normal
+    undefined: int                      # pixels with a depth but no normal (fewer than 3 window pixels, a line)
+
+
+def estimate_depth_normals(views, *, radius: int = 2, rel_tol: float = 0.05) -> DepthNormals:
+    """Oriented normal maps of ``views`` (``engine.DepthViews`` whose views carry xyz maps): for every pixel with a depth,
+    PCA over the xyz of the pixels of its (2 radius + 1)^2 map window whose depth lies within ``rel_tol`` of its own (the
+    window stops at depth edges), the eigenvector of the smallest eigenvalue of their f64 covariance, facing the view's
+    camera centre (``CameraRecord.C``).  A slice ``normals[v]`` is what ``DepthViews.add(..., normals=)`` takes.  The rule
+    is in include/ldp_b200.h (ldp_depth_normals).  Raises on a view without an xyz map and on a non-finite xyz where the
+    depth is finite.  Synchronises once, to read the status."""
+    if not 1 <= int(radius) <= 3:
+        raise ValueError("radius must lie in [1, 3]")
+    if not 0.0 < float(rel_tol) < 1.0:
+        raise ValueError("rel_tol must lie in (0, 1)")
+    dev = views.device
+    if dev.type != "cuda":
+        raise N.NativeLibraryError("normal maps run on a CUDA device (there is no CPU fallback)")
+    V, H, W = len(views), views.H, views.W
+    if V * H * W >= 2 ** 31:
+        raise ValueError("normal maps need n_views * H * W < 2^31")
+    xyz_p = views.xyz_table()
+    ptrs = views.tables()[0]
+    centers = np.zeros((max(V, 1), 3), np.float32)
+    for v, cam in enumerate(views.cameras):
+        centers[v] = np.asarray(cam.C, np.float64).reshape(3).astype(np.float32)
+    centers_dev = torch.from_numpy(centers).to(dev)
+    normals = torch.empty((V, H, W, 3), dtype=torch.float32, device=dev)
+    curvature = torch.empty((V, H, W), dtype=torch.float32, device=dev)
+    status = torch.zeros((2,), dtype=torch.int32, device=dev)
+    lib, stream = N.load(), torch.cuda.current_stream(dev).cuda_stream
+    ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)          # noqa: E731
+    N.check(lib.ldp_depth_normals(ptr(ptrs), ptr(xyz_p), V, H, W, ptr(centers_dev), int(radius), float(rel_tol), ptr(normals),
+                                  ptr(curvature), ptr(status), C.c_void_p(stream)), "ldp_depth_normals")
+    bad, undefined = (int(v) for v in status.cpu().tolist())
+    if bad & 1:
+        raise ValueError("a view's xyz map is not finite where its depth is")
+    if bad & 2:
+        raise ValueError("a view's map pointer is NULL")
+    return DepthNormals(normals=normals, curvature=curvature, undefined=undefined)
 
 
 def gaussian_record_bytes(sh_degree: int) -> int:
